@@ -7,7 +7,7 @@ public call `graph2graph.train_step` from pinned HOST buffers (H2D of the five c
 and D2H of the loss inside the timed region).  `--impl reference` times the CPU restatement of
 the reference (oracle/) on the host cores instead.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload glide|cfg2|cfg3|cfg4] [--variant 2]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload glide|cfg2|cfg3|cfg4] [--variant 2] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
          --master-port P bench.py --gpus N --steps K --warmup W
 """
@@ -34,6 +34,22 @@ WORKLOADS = {   # BASELINE.json configs; B = commits per GPU per step
 }
 L2_BYTES = 126 * 2 ** 20
 METRIC = "train commits/sec (fwd+bwd+Adam)"
+DUMP_BYTES = 64 * 10 ** 6      # --dump-outputs writes at most this much, .npy headers included
+
+
+def write_outputs(out_dir, arrays):
+    """arrays: name -> NumPy array, written as out_dir/<name>.npy in float32 (float arrays) or float64 (integer arrays).
+    If they exceed DUMP_BYTES, `probs` keeps a fixed, seeded sample of its commits (rows), listed in probs_commits.npy."""
+    arrays = {k: a.astype(np.float32 if a.dtype == np.float32 else np.float64, copy=False) for k, a in arrays.items()}
+    p = arrays["probs"]
+    rest = sum(a.nbytes for k, a in arrays.items() if k != "probs") + 4096      # + room for the headers
+    if rest + p.nbytes > DUMP_BYTES:
+        keep = (DUMP_BYTES - rest) // (p[0].nbytes + 8)
+        rows = np.sort(np.random.default_rng(0).choice(p.shape[0], keep, replace=False))
+        arrays["probs"], arrays["probs_commits"] = p[rows], rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def flops_fwd_per_commit(Ne, Nc, variant):
@@ -172,7 +188,10 @@ def main():
     ap.add_argument("--variant", type=int, default=2)
     ap.add_argument("--batch", type=int, default=0, help="commits per GPU per step (default: workload's)")
     ap.add_argument("--ref-sample", type=int, default=0, help="commits per step of the CPU reference arm (default: the workload's B)")
-    ap.add_argument("--repeats", type=int, default=25, help="timed blocks of K steps each; the median block is reported")
+    ap.add_argument("--repeats", type=int, default=1,
+                    help="consecutive blocks the K timed steps are split into; the median block's time per step is reported")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (probabilities, losses, parameters, Adam state) as DIR/<name>.npy")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--loop-train", action="store_true", default=True, help="also time graph2graph.train() epochs (N=1)")
     ap.add_argument("--no-loop-train", dest="loop_train", action="store_false")
@@ -181,6 +200,8 @@ def main():
     ap.add_argument("--rows-e", type=int, default=0)
     ap.add_argument("--rows-c", type=int, default=0)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     wl = dict(WORKLOADS[args.workload])
     if args.batch:
         wl["B"] = args.batch
@@ -256,46 +277,59 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    def last_step_outputs():
+        """What a caller of the timed step holds after its last step: probabilities, losses (CE, map MSE, parameter
+        penalty; the CE is this rank's share on the multi-kernel path), the updated parameters and the Adam state."""
+        torch.cuda.synchronize()
+        losses = loss3 if world == 1 or model.peer else torch.cat([loss, model.reg])
+        out = {"probs": probs, "losses": losses, "params": model.params, "adam_m": model.m, "adam_v": model.v,
+               "adam_step": model.step_counter}
+        return {k: t.detach().cpu().numpy() for k, t in out.items()}
+
     def timed(fn, steps, warmup, repeats, sample_clocks=False):
-        """`repeats` timed blocks of exactly `steps` steps, each bracketed by a barrier + synchronize on both sides and
-        timed with CUDA events (max over ranks per block).  Returns the per-block milliseconds, launches of one block, clocks."""
+        """`warmup` untimed steps, then exactly `steps` timed steps in `repeats` consecutive blocks of (nearly) equal length,
+        each bracketed by a barrier + synchronize on both sides and timed with CUDA events (max over ranks per block).
+        Returns (milliseconds, steps) per block, launches of the timed steps, clocks."""
+        sampler = ClockSampler(local) if sample_clocks else None
+        if sampler:         # the sampler's start-up wait comes before the warm-up, so the GPU is busy going into the timed steps
+            sampler.start()
+            time.sleep(0.15)
         for k in range(warmup):
             fn(k)
         barrier()
-        sampler = ClockSampler(local) if sample_clocks else None
-        if sampler:
-            sampler.start()
-            time.sleep(0.15)
         blocks, launches, k0 = [], 0, warmup
-        for rep in range(repeats):
+        for n_steps in (len(a) for a in np.array_split(np.arange(steps), min(max(repeats, 1), steps))):
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             barrier()
             e0.record()
-            n = 0
-            for k in range(steps):
-                n += fn(k0 + k) or 0
+            for k in range(n_steps):
+                launches += fn(k0 + k) or 0
             e1.record()
             barrier()
-            k0 += steps
-            launches = n
+            k0 += n_steps
             t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
             if world > 1:
                 dist.all_reduce(t, op=dist.ReduceOp.MAX)
-            blocks.append(float(t.item()))
+            blocks.append((float(t.item()), n_steps))
         clocks = sampler.stop() if sampler else None
         return blocks, launches, clocks
 
+    def per_step(blocks):
+        return np.asarray([ms / n for ms, n in blocks])
+
     def spread(blocks):
-        a = np.asarray(blocks) / args.steps
+        a = per_step(blocks)
         return {"blocks": len(blocks), "ms_per_step_median": float(np.median(a)), "ms_per_step_min": float(a.min()),
                 "ms_per_step_max": float(a.max())}
 
     blocks_dev, launches, clocks = timed(device_step, args.steps, args.warmup, args.repeats, sample_clocks=True)
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, last_step_outputs())
     model.initialize(model.params.clone())      # reset Adam state, keep weights
     blocks_e2e, _, _ = timed(host_step, args.steps, args.warmup, args.repeats)
-    ms_dev, ms_e2e = float(np.median(blocks_dev)), float(np.median(blocks_e2e))
-    value = Bg * args.steps / (ms_dev * 1e-3)
-    e2e_value = Bg * args.steps / (ms_e2e * 1e-3)
+    ms_dev, ms_e2e = float(np.median(per_step(blocks_dev))), float(np.median(per_step(blocks_e2e)))     # per step
+    value = Bg / (ms_dev * 1e-3)
+    e2e_value = Bg / (ms_e2e * 1e-3)
 
     # the whole public loop: graph2graph.train() epochs (batch upload, step, accuracy counters, per-epoch log) on a
     # synthetic data set of 4 batches -- what `main.py --Type train` costs per step next to the bare step above
@@ -451,14 +485,14 @@ def main():
                                        else "one CTA per commit")}
         line = {
             "metric": METRIC, "value": value, "unit": "commits/s", "n_gpus": world, "steps": args.steps,
-            "warmup": args.warmup, "ms_per_step": ms_dev / args.steps, "higher_is_better": True, "scaling": "weak",
+            "warmup": args.warmup, "ms_per_step": ms_dev, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": config, "setup": setup,
             "timing": {"device": spread(blocks_dev), "e2e": spread(blocks_e2e),
-                       "note": f"{args.repeats} blocks of exactly {args.steps} steps, each bracketed by barrier + synchronize and timed with CUDA events "
-                               "(max over ranks); value / e2e are the MEDIAN block"},
+                       "note": f"{args.warmup} warm-up steps, then exactly {args.steps} timed steps in {len(blocks_dev)} block(s), each bracketed by "
+                               "barrier + synchronize and timed with CUDA events (max over ranks); value / e2e are the MEDIAN block's time per step"},
             "clocks": clocks,
-            "e2e": {"value": e2e_value, "unit": "commits/s", "ms_per_step": ms_e2e / args.steps,
+            "e2e": {"value": e2e_value, "unit": "commits/s", "ms_per_step": ms_e2e,
                     "h2d_bytes_per_step": host_pool[0].nbytes(), "d2h_bytes_per_step": 12,
                     "wire_format": "label grids as bitmaps (HDGNN_F_LABEL_BITS), x f32, hmap i32, L i32" if model.host_bits else "label grids as u8",
                     "api": "hdgnn_b200.model.graph2graph.train_step: pinned host buffers -> hdgnn_train_step_host (1 GPU) / "
