@@ -43,30 +43,32 @@ __host__ __device__ __forceinline__ int ent2_slots(int b, int N, int R) {
 }
 __host__ __device__ __forceinline__ int ent2_max_slots(int N, int R) { return (N + R - 1) / R + 1; }
 
-__host__ __device__ inline size_t ent2_smem_bytes(int CWT, int NRG, int N, int R, int WP, bool bwd) {
+__host__ __device__ inline size_t ent2_smem_bytes(int CWT, int N, int R, int WP, bool bwd) {
     const int RC = R < N ? R : N;
     size_t off = (size_t)round_up(RC * WP * 4, 128);                      // bitmap rows
     off += (size_t)RC * PROW * 4;                                           // P01
     off += (size_t)RC * HD * 4 * (bwd ? 3 : 2);                             // rowacc, diag (, GRt)
-    off += (size_t)(NRG / 2 > 0 ? NRG / 2 : 1) * CWT * 32 * HD * 4;         // column combine scratch
-    off += (size_t)(5 * HD + NRG * HD + 3 * 8 * HD + 4 * HD + 2 * HD) * 4;  // weights, lsw, red, acc80, dvw+pad
+    // unused column-combine scratch of the multi-row-group layouts: dropping it would change ent2_occupancy, hence the chunking
+    // and the summation order of the dense path
+    off += (size_t)CWT * 32 * HD * 4;
+    off += (size_t)(5 * HD + HD + 3 * 8 * HD + 4 * HD + 2 * HD) * 4;       // weights, lsw, red, acc80, dvw+pad
     return off + 16;
 }
 
-// launch bounds: 20 resident warps per SM (4 / 2 / 1 CTAs for NRG = 1 / 2 / 4)
-template <int CWT, int NRG>
-__global__ void __launch_bounds__(KG * NRG * 32, 4 / NRG) ent_fwd2_kernel(const Ent2Args a) {
+// one row group of KG warps (rg = 0); launch bounds: 20 resident warps per SM
+template <int CWT>
+__global__ void __launch_bounds__(KG * 32, 4) ent_fwd2_kernel(const Ent2Args a) {
     extern __shared__ __align__(128) unsigned char smem[];
     const int N = a.N, WP = a.WP, RC = a.R < N ? a.R : N;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, kg = warp % KG, rg = warp / KG;
-    constexpr int NT = KG * NRG * 32;
+    constexpr int NT = KG * 32;
     uint32_t* sbits = reinterpret_cast<uint32_t*>(smem);
     float* P01 = reinterpret_cast<float*>(smem + round_up(RC * WP * 4, 128));
     float* rowacc = P01 + (size_t)RC * PROW;
     float* diag = rowacc + (size_t)RC * HD;
-    float* scratch = diag + (size_t)RC * HD;
-    float* wts = scratch + (size_t)(NRG / 2 > 0 ? NRG / 2 : 1) * CWT * 32 * HD;   // U V bsum D
-    uint64_t* bar = reinterpret_cast<uint64_t*>(wts + 5 * HD + NRG * HD + 3 * 8 * HD + 4 * HD + 2 * HD);
+    float* scratch = diag + (size_t)RC * HD;      // unused (ent2_smem_bytes)
+    float* wts = scratch + (size_t)CWT * 32 * HD;   // U V bsum D
+    uint64_t* bar = reinterpret_cast<uint64_t*>(wts + 5 * HD + HD + 3 * 8 * HD + 4 * HD + 2 * HD);
 
     if (tid == 0) { mbar_init(bar, 1); fence_mbar_init(); }
     if (a.head) pdl_wait();
@@ -128,9 +130,8 @@ __global__ void __launch_bounds__(KG * NRG * 32, 4 / NRG) ent_fwd2_kernel(const 
                 Q[sg][1] = ok ? pk2(xj * V2, xj * V3) : pk2(NEG_BIG, NEG_BIG);
                 col[sg][0] = 0ull; col[sg][1] = 0ull;
             }
-            if (pass == 0) sweep2_fwd<CWT, false>(P01, sbits, WP, nr, rg, NRG, kg, Q, col, rowacc, lane);
-            else sweep2_fwd<CWT, true>(P01, sbits + pass * CWT, WP, nr, rg, NRG, kg, Q, col, rowacc, lane);
-            combine_cols<CWT>(col, scratch, rg, NRG, kg, lane);
+            if (pass == 0) sweep2_fwd<CWT, false>(P01, sbits, WP, nr, rg, 1, kg, Q, col, rowacc, lane);
+            else sweep2_fwd<CWT, true>(P01, sbits + pass * CWT, WP, nr, rg, 1, kg, Q, col, rowacc, lane);
             if (rg == 0) {
 #pragma unroll
                 for (int sg = 0; sg < CWT; ++sg) {
@@ -156,21 +157,21 @@ __global__ void __launch_bounds__(KG * NRG * 32, 4 / NRG) ent_fwd2_kernel(const 
     }
 }
 
-template <int CWT, int NRG>
-__global__ void __launch_bounds__(KG * NRG * 32, NRG == 1 ? 3 : 1) ent_bwd2_kernel(const Ent2Args a) {
+template <int CWT>
+__global__ void __launch_bounds__(KG * 32, 3) ent_bwd2_kernel(const Ent2Args a) {
     extern __shared__ __align__(128) unsigned char smem[];
     const int N = a.N, WP = a.WP, RC = a.R < N ? a.R : N;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, kg = warp % KG, rg = warp / KG;
-    constexpr int NT = KG * NRG * 32;
+    constexpr int NT = KG * 32;
     uint32_t* sbits = reinterpret_cast<uint32_t*>(smem);
     float* P01 = reinterpret_cast<float*>(smem + round_up(RC * WP * 4, 128));
     float* rowacc = P01 + (size_t)RC * PROW;
     float* dgv = rowacc + (size_t)RC * HD;
     float* GRt = dgv + (size_t)RC * HD;
-    float* scratch = GRt + (size_t)RC * HD;
-    float* wts = scratch + (size_t)(NRG / 2 > 0 ? NRG / 2 : 1) * CWT * 32 * HD;   // U V bsum D (W unused slot)
-    float* lsw = wts + 5 * HD;                  // [NRG][20]
-    float* red = lsw + NRG * HD;                // [3][8][20]
+    float* scratch = GRt + (size_t)RC * HD;       // unused (ent2_smem_bytes)
+    float* wts = scratch + (size_t)CWT * 32 * HD;   // U V bsum D (W unused slot)
+    float* lsw = wts + 5 * HD;                  // [20]
+    float* red = lsw + HD;                      // [3][8][20]
     float* acc80 = red + 3 * 8 * HD;            // [4][20] db dU dV LS over the CTA's sub-tiles
     float* dvw = acc80 + 4 * HD;                // [20] dV of the current sub-tile
     uint64_t* bar = reinterpret_cast<uint64_t*>(dvw + 2 * HD);
@@ -248,9 +249,8 @@ __global__ void __launch_bounds__(KG * NRG * 32, NRG == 1 ? 3 : 1) ent_bwd2_kern
                 GC[sg][0] = g.x; GC[sg][1] = g.y;
                 col[sg][0] = 0ull; col[sg][1] = 0ull;
             }
-            if (pass == 0) sweep2_bwd<CWT, false>(P01, GRt, sbits, WP, nr, rg, NRG, kg, Q, GC, col, lacc, rowacc, lane);
-            else sweep2_bwd<CWT, true>(P01, GRt, sbits + pass * CWT, WP, nr, rg, NRG, kg, Q, GC, col, lacc, rowacc, lane);
-            combine_cols<CWT>(col, scratch, rg, NRG, kg, lane);
+            if (pass == 0) sweep2_bwd<CWT, false>(P01, GRt, sbits, WP, nr, rg, 1, kg, Q, GC, col, lacc, rowacc, lane);
+            else sweep2_bwd<CWT, true>(P01, GRt, sbits + pass * CWT, WP, nr, rg, 1, kg, Q, GC, col, lacc, rowacc, lane);
             if (rg == 0) {       // dV partial of this pass: sum_j x_j (col_j - diag_j)
                 u64 dv0 = 0ull, dv1 = 0ull;
 #pragma unroll
@@ -273,7 +273,7 @@ __global__ void __launch_bounds__(KG * NRG * 32, NRG == 1 ? 3 : 1) ent_bwd2_kern
                 if ((lane & 7) == 0) dvw[k0 + ch] += t;
             }
         }
-        {   // label-1 sums: warp totals, then row groups in order
+        {   // label-1 sums: warp totals
             const float t = reduce4(lacc[0], lacc[1], lane);
             if ((lane & 7) == 0) lsw[rg * HD + k0 + ch] = t;
         }
@@ -294,7 +294,7 @@ __global__ void __launch_bounds__(KG * NRG * 32, NRG == 1 ? 3 : 1) ent_bwd2_kern
             const int k = tid;
             float sb = 0.f, su = 0.f, ls = 0.f;
             for (int p = 0; p < 8; ++p) { sb += red[(0 * 8 + p) * HD + k]; su += red[(1 * 8 + p) * HD + k]; }
-            for (int w = 0; w < NRG; ++w) ls += lsw[w * HD + k];
+            ls += lsw[k];
             acc80[k] += sb; acc80[HD + k] += su; acc80[2 * HD + k] += dvw[k]; acc80[3 * HD + k] += ls;
         }
         __syncthreads();

@@ -69,8 +69,6 @@ struct FinalArgs {
     float* reg_losses;       // {loss_map, loss_para} at the pre-update parameters, or null
     float* l2part;           // (gridDim.x) scratch
     unsigned int* counter;   // zero-initialised; reset by the last CTA
-    int* done_flag; int done_seq;    // host-fed steps: *done_flag = done_seq once the per-commit kernel has completed (its staging
-                                     // slot may be refilled: the copy stream waits on this value, cuStreamWaitValue32), or null
 };
 
 // lr_t = lr sqrt(1 - b2^t) / (1 - b1^t) (tf.train.AdamOptimizer), with 1 - b^t = -expm1(t log b) so that the
@@ -134,10 +132,6 @@ __global__ void __launch_bounds__(FIN_P * FIN_SL) reduce_adam_kernel(const Final
         th[0] = a.params[o]; th[1] = a.params[o + 1];
     }
     pdl_wait();                     // gradient partials come from mid2 / ent_bwd2
-    if (a.done_flag && blockIdx.x == 0 && tid == 0) {      // every kernel that reads the staged inputs has completed
-        *reinterpret_cast<volatile int*>(a.done_flag) = a.done_seq;
-        __threadfence_system();
-    }
     float acc = 0.f;
     if (p < a.total) {
         for (int bb = sl; bb < a.B; bb += 16 * FIN_SL) {      // sixteen guarded loads in flight, fixed summation order

@@ -8,14 +8,14 @@
 namespace hdgnn {
 
 // kernel handle for cudaFuncSetAttribute / occupancy queries (nullptr if not instantiated)
-const void* ent2_fn_rt(int cwt, int nrg, bool bwd);
+const void* ent2_fn_rt(int cwt, bool bwd);
 const void* mid2_fn_rt(int cwt, bool train, bool gt, bool cl = false);
 int mid2_max_clusters(int cwt, bool train, size_t smem);
 // which table placements are compiled for a hunk-grid width: shared memory for cwt <= 5, global memory for cwt >= 5
 bool mid2_gt_supported(int cwt, bool gt);
 // pdl: launch with programmatic stream serialization (the kernel calls pdl_wait() before it reads its
 // predecessor's outputs, so its prologue overlaps the predecessor's tail)
-void launch_ent2(int cwt, int nrg, bool bwd, int grid, size_t smem, cudaStream_t st, const Ent2Args& a, bool pdl);
+void launch_ent2(int cwt, bool bwd, int grid, size_t smem, cudaStream_t st, const Ent2Args& a, bool pdl);
 void launch_mid2(int cwt, bool train, bool gt, bool cl, int grid, size_t smem, cudaStream_t st, const Mid2Args& a, bool pdl);
 
 // cluster: CTAs per thread-block cluster (1 = none; the grid must be a multiple)
@@ -45,12 +45,6 @@ inline cudaError_t launch_ex(Kern kern, int grid, int block, size_t smem, cudaSt
         case 3: { constexpr int CWT = 3; __VA_ARGS__; } break; case 4: { constexpr int CWT = 4; __VA_ARGS__; } break; \
         case 5: { constexpr int CWT = 5; __VA_ARGS__; } break; case 6: { constexpr int CWT = 6; __VA_ARGS__; } break; \
         case 7: { constexpr int CWT = 7; __VA_ARGS__; } break; case 8: { constexpr int CWT = 8; __VA_ARGS__; } break; \
-        default: break;                                                                             \
-    }
-#define HDGNN_NRG_SWITCH(nrg, ...)                                                                  \
-    switch (nrg) {                                                                                  \
-        case 1: { constexpr int NRG = 1; __VA_ARGS__; } break; case 2: { constexpr int NRG = 2; __VA_ARGS__; } break; \
-        case 4: { constexpr int NRG = 4; __VA_ARGS__; } break;                                     \
         default: break;                                                                             \
     }
 

@@ -16,7 +16,12 @@
 //             -> [E: score(edge, train: recompute + delta sums) -> head_bwd(edge) -> pairsum_bwd(edge)
 //                 -> rank1_grad(edge, tied)] -> grad_reduce
 //       opt : adam (regularisers fused)
-#include <cuda.h>
+//
+// Entry points: each checks its arguments and makes one call -- device_step for the device-resident entries, host_step for the
+// *_host entries.  host_step stages the host inputs into one of two slots on the handle's copy stream (stage_inputs), runs the
+// step on the slot, releases it by an event on the caller's stream (release_slot) and copies the outputs out.  The step
+// waits for its staged inputs through an event, or, when mid2 is its first kernel, by polling a tag the copy stream's last DMA
+// writes (an event wait would break the programmatic launch chain reduce_adam -> mid2).
 #include <cuda_runtime.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -93,7 +98,7 @@ struct Buf { void* p = nullptr; size_t bytes = 0; };
 
 }  // namespace
 
-constexpr int NSLOT = 3;         // staging slots of the *_host entry points
+constexpr int NSLOT = 2;         // staging slots of the *_host entry points
 
 struct hdgnn_handle_s {
     hdgnn_config_t cfg;
@@ -108,7 +113,7 @@ struct hdgnn_handle_s {
     // fused path: label bitmaps + balanced row chunks of the entity grid (ent2.cuh)
     int WPe = 0, WPc = 0;      // bitmap words per row
     int nsm = 148;
-    int fwd_nrg = 2, bwd_nrg = 1, fwd_cwt = 0, bwd_cwt = 0;   // warp layout / column segments per pass
+    int cwt = 0;                                               // column segments per pass of the entity sweeps
     int fwd_occ = 1, bwd_occ = 1;                              // resident CTAs per SM
     bool pdl = true;                                           // programmatic dependent launch between the fused kernels
     int bslot = 0;                                             // bitmap buffer of the current step (two alternate)
@@ -131,18 +136,10 @@ struct hdgnn_handle_s {
     cudaEvent_t prof_start = nullptr;
     std::vector<std::pair<std::string, std::pair<cudaEvent_t, cudaEvent_t>>> prof_ev;
     // host-entry staging: two slots filled on a private copy stream so the H2D copies of call k+1 overlap
-    // the kernels of call k (both calls only enqueue work; ordering is by events)
+    // the kernels of call k (both calls only enqueue work; the copies are ordered by events or by a tag, stage_inputs)
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t ev_copy[NSLOT] = {}, ev_done[NSLOT] = {};
     bool done_valid[NSLOT] = {};
-    // OPT-IN (HDGNN_WAIT_VALUE=1): host-fed training steps on the tag path release their slot by a VALUE the optimizer kernel
-    // writes (final.cuh: done_flag) and the copy stream waits on (cuStreamWaitValue32) instead of an event record / wait pair.
-    // Measured slower than the event (the stream memory operation reacts late): off by default
-    void* wait32 = nullptr;                // cuStreamWaitValue32 (driver entry point), null: events
-    bool flag_release = false;             // the step being enqueued releases its slot by value
-    bool want_flag_release = false;        // the entry point being served ends in reduce_adam (training)
-    unsigned int done_seq[NSLOT] = {};     // last value promised for a slot
-    bool done_by_flag[NSLOT] = {};
     int slot = 0, cur = 0, cur_B = 0;      // next slot, the slot (and its batch size) filled by the last stage_inputs call
     // peer exchange (commit sharding over NVLink, final.cuh): own mailbox + the peers' mailboxes mapped through CUDA IPC
     PeerArgs peer{};
@@ -545,13 +542,13 @@ void ent2_grid(hdgnn_handle_t h, int B, int occ, int* G, int* R) {
 }
 
 // largest number of co-resident CTAs per SM (<= 4) whose row chunk fits next to each other
-int ent2_occupancy(hdgnn_handle_t h, int cwt, int nrg, bool bwd) {
-    const void* fn = ent2_fn_rt(cwt, nrg, bwd);
+int ent2_occupancy(hdgnn_handle_t h, bool bwd) {
+    const void* fn = ent2_fn_rt(h->cwt, bwd);
     for (int occ = 4; occ > 1; --occ) {
         int G, R, got = 0;
         ent2_grid(h, h->cfg.max_batch, occ, &G, &R);
-        const size_t smem = ent2_smem_bytes(cwt, nrg, h->Ne, R, h->WPe, bwd);
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&got, fn, KG * nrg * 32, smem) == cudaSuccess && got >= occ) return occ;
+        const size_t smem = ent2_smem_bytes(h->cwt, h->Ne, R, h->WPe, bwd);
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&got, fn, KG * 32, smem) == cudaSuccess && got >= occ) return occ;
     }
     return 1;
 }
@@ -602,9 +599,9 @@ int fused_forward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float
         ent2_grid(h, B, h->fwd_occ, &h->Gf, &h->Rf);
         h->SLf = ent2_max_slots(h->Ne, h->Rf);
         a.R = h->Rf; a.SL = h->SLf; a.RS = F(h, "RS1"); a.CSp = F(h, "CS1P"); a.head = head ? 1 : 0;
-        const size_t smem = ent2_smem_bytes(h->fwd_cwt, h->fwd_nrg, h->Ne, h->Rf, h->WPe, false);
+        const size_t smem = ent2_smem_bytes(h->cwt, h->Ne, h->Rf, h->WPe, false);
         PROF_BEGIN(h, st);
-        launch_ent2(h->fwd_cwt, h->fwd_nrg, false, h->Gf, smem, st, a, h->pdl);
+        launch_ent2(h->cwt, false, h->Gf, smem, st, a, h->pdl);
         LAUNCH_CHECK(h, "ent_fwd", st);
     }
     Mid2Args m{};
@@ -656,9 +653,9 @@ int fused_backward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, floa
         Ent2Args a = ent2_args(h, B, in);
         ent2_grid(h, B, h->bwd_occ, &h->Gb, &h->Rb);
         a.R = h->Rb; a.SL = 0; a.GR = F(h, "GE"); a.GC = F(h, "GE"); a.gpart = F(h, "GPE");
-        const size_t smem = ent2_smem_bytes(h->bwd_cwt, h->bwd_nrg, h->Ne, h->Rb, h->WPe, true);
+        const size_t smem = ent2_smem_bytes(h->cwt, h->Ne, h->Rb, h->WPe, true);
         PROF_BEGIN(h, st);
-        launch_ent2(h->bwd_cwt, h->bwd_nrg, true, h->Gb, smem, st, a, h->pdl);
+        launch_ent2(h->cwt, true, h->Gb, smem, st, a, h->pdl);
         LAUNCH_CHECK(h, "ent_bwd", st);
     }
     FinalArgs f{};
@@ -672,11 +669,6 @@ int fused_backward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, floa
         f.o_t1 = h->po.theta1; f.o_t2 = h->po.theta2; f.lr = adam->lr; f.b1 = adam->b1; f.b2 = adam->b2; f.eps = adam->eps;
         f.reg_losses = adam->reg;
         if (adam->peer) f.peer = h->peer;
-    }
-    if (h->flag_release) {
-        const int s = h->cur;
-        f.done_flag = (int*)h->ws["H_DONE"].p + s; f.done_seq = (int)++h->done_seq[s];
-        h->done_by_flag[s] = true; h->done_valid[s] = true;
     }
     PROF_BEGIN(h, st);
     launch_ex(reduce_adam_kernel, (h->po.total + FIN_P - 1) / FIN_P, FIN_P * FIN_SL, 0, st, h->pdl, f);
@@ -722,11 +714,11 @@ cudaError_t setup_fused(hdgnn_handle_t h, int optin) {
         }
     }
     if (h->ent) {
-        acc(cudaFuncSetAttribute(ent2_fn_rt(h->fwd_cwt, h->fwd_nrg, false), A, optin));
-        acc(cudaFuncSetAttribute(ent2_fn_rt(h->bwd_cwt, h->bwd_nrg, true), A, optin));
+        acc(cudaFuncSetAttribute(ent2_fn_rt(h->cwt, false), A, optin));
+        acc(cudaFuncSetAttribute(ent2_fn_rt(h->cwt, true), A, optin));
         if (e != cudaSuccess) return e;
-        h->fwd_occ = ent2_occupancy(h, h->fwd_cwt, h->fwd_nrg, false);
-        h->bwd_occ = ent2_occupancy(h, h->bwd_cwt, h->bwd_nrg, true);
+        h->fwd_occ = ent2_occupancy(h, false);
+        h->bwd_occ = ent2_occupancy(h, true);
     }
     return e;
 }
@@ -817,17 +809,8 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
     h->debug = (cfg->flags & HDGNN_F_DEBUG) != 0;
     h->nsm = prop.multiProcessorCount;
     h->WPe = bit_words(h->Ne); h->WPc = bit_words(h->Nc);
-    h->fwd_cwt = h->bwd_cwt = ent2_cwt(h->Ne);
-    {   // tuning overrides: a pass width below the row width must be a multiple of 4 (16-byte bitmap loads)
-        const int f = env_int("HDGNN_FWD_CWT", 0), bw = env_int("HDGNN_BWD_CWT", 0);
-        if ((f == 4 || f == 8) && f < h->fwd_cwt) h->fwd_cwt = f;
-        if ((bw == 4 || bw == 8) && bw < h->bwd_cwt) h->bwd_cwt = bw;
-    }
-    h->pdl = env_int("HDGNN_PDL", 1) != 0 && !h->debug;
-    h->fwd_nrg = env_int("HDGNN_FWD_NRG", 1);
-    h->bwd_nrg = env_int("HDGNN_BWD_NRG", 1);
-    if (h->fwd_nrg != 1 && h->fwd_nrg != 2 && h->fwd_nrg != 4) h->fwd_nrg = 1;
-    if (h->bwd_nrg != 1 && h->bwd_nrg != 2 && h->bwd_nrg != 4) h->bwd_nrg = 1;
+    h->cwt = ent2_cwt(h->Ne);
+    h->pdl = !h->debug;
     // the fused path needs the per-commit state of mid2 in one SM's shared memory and a hunk grid of <= 8 segments.  The twelve
     // hunk-stage tables (12 Nc 20 floats) either sit in shared memory (compiled for Nc <= 160) or in a per-commit slice of global
     // memory (compiled for Nc > 128: mid2_kernel<.., GT>); the placement that admits the inline entity stage wins, shared memory
@@ -835,7 +818,7 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
     {
         const size_t lim = (size_t)prop.sharedMemPerBlockOptin;
         const int cwc = (h->Nc + 31) / 32;
-        const bool want_inl = h->ent && !(cfg->flags & HDGNN_F_DENSE_SWEEP) && env_int("HDGNN_DENSE_SWEEP", 0) == 0;
+        const bool want_inl = h->ent && !(cfg->flags & HDGNN_F_DENSE_SWEEP);
         struct Plan { bool fused = false, dlt_global = false, scache = false, inl = false, scg = false; };
         // above 256 hunks only the forward kernel exists (BASELINE config 5: the inference sweep to Nc = 512); variants 1-3
         const bool fwd_only = h->Nc > 256;
@@ -866,7 +849,7 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
     if (h->edge) {
         // variant 4 on the fused path: needs the inline entity stage, the soft-edge head tables (Ne x 60 floats + a 128-row
         // staging tile) and the edge branch's pair sums (2 Ne x 20) side by side in mid2's union region
-        bool ok = h->fused && h->inl && env_int("HDGNN_V4_FUSED", 1) != 0;
+        bool ok = h->fused && h->inl;
         if (ok) {
             const size_t lim = (size_t)prop.sharedMemPerBlockOptin;
             h->dlt_global = mid2_smem_bytes(h->Ne, h->Nc, true, true, true, true, true, h->gt, h->scg) > lim;
@@ -874,7 +857,7 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
             ok = (size_t)L.total * 4 + 16 <= lim && h->Ne * 60 + (M2_T / KG) * HD <= (L.sc - L.uni) - 2 * h->Ne * HD;
         }
         h->edge_fused = ok;
-        bool okt = ok && env_int("HDGNN_V4_FUSED_TRAIN", 1) != 0;
+        bool okt = ok;
         if (okt) {      // backward: head tables + column delta sums + a 32-row de tile; later five Ne x 20 arrays + GCe at the end;
                         // the general-attribute form of ent_bwd needs two sets of suffix tables beside GCe
             const Mid2Smem L = mid2_layout(h->Ne, h->Nc, true, !h->dlt_global, true, true, true, h->gt, h->scg);
@@ -947,8 +930,7 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
         {"H_HMAP1", B * Ne * sizeof(int32_t), !h->host_bits}, {"H_L1", B * sizeof(int32_t), !h->host_bits},
         // label-bitmap wire block of a staging slot: [entity bitmaps][hunk bitmaps][x][hmap][L], 16-byte aligned sections
         {"H_WIRE0", wire_layout(h, cfg->max_batch).total, h->host_bits}, {"H_WIRE1", wire_layout(h, cfg->max_batch).total, h->host_bits},
-        {"H_WIRE2", wire_layout(h, cfg->max_batch).total, h->host_bits},
-        {"H_FLAG", 16, true}, {"H_DONE", 16, true}, {"H_PROBS", B * 2 * Nc * (Nc - 1) * f, true}, {"H_LOSS", 4 * f, true}, {"H_GRADS", (size_t)h->po.total * f, true},
+        {"H_FLAG", 16, true}, {"H_PROBS", B * 2 * Nc * (Nc - 1) * f, true}, {"H_LOSS", 4 * f, true}, {"H_GRADS", (size_t)h->po.total * f, true},
     };
     for (auto& p : plan) {
         if (!p.need) continue;
@@ -960,15 +942,9 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
         }
     }
     bool ok = cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking) == cudaSuccess;
-    if (ok && env_int("HDGNN_TAG_WAIT", 1) != 0 && cudaHostAlloc((void**)&h->tag_table, 256 * sizeof(uint32_t), cudaHostAllocDefault) == cudaSuccess) {
+    if (ok && cudaHostAlloc((void**)&h->tag_table, 256 * sizeof(uint32_t), cudaHostAllocDefault) == cudaSuccess) {
         for (int i = 0; i < 256; ++i) h->tag_table[i] = (uint32_t)i;
     } else { cudaGetLastError(); h->tag_table = nullptr; }
-    if (ok && env_int("HDGNN_WAIT_VALUE", 0) != 0) {      // opt-in (measured slower than the event: 113 vs 101 us per step); driver entry point, no link-time dependency on libcuda
-        void* fn = nullptr;
-        cudaDriverEntryPointQueryResult qr;
-        if (cudaGetDriverEntryPoint("cuStreamWaitValue32", &fn, cudaEnableDefault, &qr) == cudaSuccess && qr == cudaDriverEntryPointSuccess) h->wait32 = fn;
-        else cudaGetLastError();
-    }
     for (int i = 0; i < NSLOT && ok; ++i)
         ok = cudaEventCreateWithFlags(&h->ev_copy[i], cudaEventDisableTiming) == cudaSuccess &&
              cudaEventCreateWithFlags(&h->ev_done[i], cudaEventDisableTiming) == cudaSuccess;
@@ -1088,8 +1064,6 @@ int hdgnn_peer_status(hdgnn_handle_t h) {
 
 // forward [+ backward [+ adam]] on device-resident inputs; dispatches to the fused or the
 // multi-kernel path.
-static int release_slot(hdgnn_handle_t h, cudaStream_t st);
-
 static int run_step(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float* logits, float* probs, float* loss,
                     float* grads, const AdamArgs* adam, cudaStream_t st) {
     const bool train = grads != nullptr;
@@ -1116,15 +1090,29 @@ static int run_step(hdgnn_handle_t h, int B, int B_global, const Inputs& in, flo
                      adam->reg, st);
 }
 
+// the step of a device entry point whose arguments have been checked
+static int device_step(hdgnn_handle_t h, int B, int B_global, const uint8_t* adj, const float* x, const int32_t* hmap,
+                       const int32_t* L, const uint8_t* Y, const float* params, float* logits, float* probs, float* loss,
+                       float* grads, const AdamArgs* adam, void* stream) {
+    h->launches = 0;
+    Inputs in{adj, x, hmap, L, Y, params};
+    alias_bits(h, in);
+    return run_step(h, B, B_global, in, logits, probs, loss, grads, adam, (cudaStream_t)stream);
+}
+
+// the peer-exchange steps: peers attached, equal shards
+static int check_peer(hdgnn_handle_t h, int B, int B_global) {
+    if (!h->peer_ready) return fail(h, HDGNN_E_INVALID, "hdgnn_peer_attach has not been called");
+    if (B_global != B * h->peer.world) return fail(h, HDGNN_E_INVALID, "B_global must be B * world (equal shards)");
+    return HDGNN_OK;
+}
+
 int hdgnn_forward(hdgnn_handle_t h, int B, const uint8_t* adj, int adj_pitch, const float* x, const int32_t* hmap,
                   const int32_t* L, const uint8_t* Y, int y_pitch, const float* params, float* logits, float* probs,
                   float* loss, void* stream) {
     int rc = check_inputs(h, B, adj, adj_pitch, x, hmap, L, Y, y_pitch, params);
     if (rc) return rc;
-    h->launches = 0;
-    Inputs in{adj, x, hmap, L, Y, params};
-    alias_bits(h, in);
-    return run_step(h, B, B, in, logits, probs, loss, nullptr, nullptr, (cudaStream_t)stream);
+    return device_step(h, B, B, adj, x, hmap, L, Y, params, logits, probs, loss, nullptr, nullptr, stream);
 }
 
 int hdgnn_forward_backward(hdgnn_handle_t h, int B, int B_global, const uint8_t* adj, int adj_pitch, const float* x,
@@ -1134,10 +1122,7 @@ int hdgnn_forward_backward(hdgnn_handle_t h, int B, int B_global, const uint8_t*
     if (rc) return rc;
     if (!grads) return fail(h, HDGNN_E_INVALID, "grads is null");
     if (B_global < B) return fail(h, HDGNN_E_INVALID, "B_global < B");
-    h->launches = 0;
-    Inputs in{adj, x, hmap, L, Y, params};
-    alias_bits(h, in);
-    return run_step(h, B, B_global, in, logits, probs, loss, grads, nullptr, (cudaStream_t)stream);
+    return device_step(h, B, B_global, adj, x, hmap, L, Y, params, logits, probs, loss, grads, nullptr, stream);
 }
 
 int hdgnn_adam_step(hdgnn_handle_t h, float* params, const float* grads, float* m, float* v, int32_t* step_counter,
@@ -1155,16 +1140,14 @@ int hdgnn_train_step(hdgnn_handle_t h, int B, const uint8_t* adj, int adj_pitch,
     int rc = check_inputs(h, B, adj, adj_pitch, x, hmap, L, Y, y_pitch, params);
     if (rc) return rc;
     if (!m || !v || !step_counter || !loss3) return fail(h, HDGNN_E_INVALID, "null pointer");
-    h->launches = 0;
-    Inputs in{adj, x, hmap, L, Y, params};
-    alias_bits(h, in);
-    AdamArgs ad{params, m, v, step_counter, lr, beta1, beta2, eps, loss3 + 1};
-    return run_step(h, B, B, in, logits, probs, loss3, F(h, "H_GRADS"), &ad, (cudaStream_t)stream);
+    const AdamArgs ad{params, m, v, step_counter, lr, beta1, beta2, eps, loss3 + 1};
+    return device_step(h, B, B, adj, x, hmap, L, Y, params, logits, probs, loss3, F(h, "H_GRADS"), &ad, stream);
 }
 
 // Host buffers -> staging slot `h->cur` (un-pitched rows are re-pitched on the device).  Outside stream capture the
 // copies run on the handle's copy stream: slot s is reused only after the kernels that read it (two calls ago)
-// have finished, and the caller's stream waits for the copies, so consecutive calls overlap copy and compute.
+// have finished, and the step waits for the copies (an event, or the tag mid2 polls), so consecutive calls overlap copy
+// and compute.
 static std::string slot_name(const char* base, int slot) { return std::string(base) + (char)('0' + slot); }
 
 static int stage_inputs(hdgnn_handle_t h, int B, const uint8_t* adj_host, const float* x_host, const int32_t* hmap_host,
@@ -1175,18 +1158,9 @@ static int stage_inputs(hdgnn_handle_t h, int B, const uint8_t* adj_host, const 
     const bool side = cap == cudaStreamCaptureStatusNone;
     const int slot = h->slot;
     h->cur = slot;
-    h->slot = (slot + 1) % (h->host_bits && env_int("HDGNN_SLOTS", 2) == 3 ? 3 : 2);     // a third slot (label bitmaps) is there to try: no gain measured
+    h->slot = slot ^ 1;
     cudaStream_t cs = side ? h->copy_stream : st;
-    if (side && h->done_valid[slot]) {
-        if (h->done_by_flag[slot]) {
-            typedef CUresult (*wait32_t)(CUstream, CUdeviceptr, cuuint32_t, unsigned int);
-            const CUresult r = ((wait32_t)h->wait32)((CUstream)cs, (CUdeviceptr)((int*)h->ws["H_DONE"].p + slot), (cuuint32_t)h->done_seq[slot],
-                                                     CU_STREAM_WAIT_VALUE_GEQ);
-            if (r != CUDA_SUCCESS) return fail(h, HDGNN_E_CUDA, "cuStreamWaitValue32 failed");
-        } else {
-            CK(h, cudaStreamWaitEvent(cs, h->ev_done[slot], 0));
-        }
-    }
+    if (side && h->done_valid[slot]) CK(h, cudaStreamWaitEvent(cs, h->ev_done[slot], 0));
     h->cur_B = B;
     if (h->host_bits) {
         // one staging block per slot; host arrays that already sit back to back in that layout (one pinned block, what
@@ -1239,7 +1213,6 @@ static int stage_inputs(hdgnn_handle_t h, int B, const uint8_t* adj_host, const 
             const int tag = (int)(++h->slot_uses[slot] & 0xffu);
             CK(h, cudaMemcpyAsync((int*)h->ws["H_FLAG"].p + slot, h->tag_table + tag, sizeof(int), cudaMemcpyHostToDevice, cs));
             h->cur_tag = tag;
-            h->flag_release = h->wait32 != nullptr && h->want_flag_release;      // set by the training entry points (reduce_adam follows)
         } else {
             CK(h, cudaEventRecord(h->ev_copy[slot], cs));
             CK(h, cudaStreamWaitEvent(st, h->ev_copy[slot], 0));
@@ -1266,12 +1239,11 @@ static Inputs staged_inputs(hdgnn_handle_t h, const float* params) {
 
 // the kernels reading slot h->cur have been enqueued on `st`: the slot may be refilled once they are done
 static int release_slot(hdgnn_handle_t h, cudaStream_t st) {
-    if (h->flag_release) { h->flag_release = false; return HDGNN_OK; }      // released by value (fused_backward)
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     cudaStreamIsCapturing(st, &cap);
     if (cap != cudaStreamCaptureStatusNone) return HDGNN_OK;
     CK(h, cudaEventRecord(h->ev_done[h->cur], st));
-    h->done_valid[h->cur] = true; h->done_by_flag[h->cur] = false;
+    h->done_valid[h->cur] = true;
     return HDGNN_OK;
 }
 
@@ -1285,32 +1257,54 @@ static float* host_alias(float* host_ptr) {
     return (float*)at.devicePointer;
 }
 
+// argument checks every *_host entry point makes
+static int check_host_inputs(hdgnn_handle_t h, int B, const void* adj_host, const void* x_host, const void* hmap_host,
+                             const void* L_host, const void* Y_host, const void* params) {
+    if (!h) return HDGNN_E_INVALID;
+    if (B < 1 || B > h->cfg.max_batch) return fail(h, HDGNN_E_INVALID, "B out of range [1, max_batch]");
+    if (!adj_host || !x_host || !hmap_host || !L_host || !Y_host || !params) return fail(h, HDGNN_E_INVALID, "null pointer");
+    return HDGNN_OK;
+}
+
+// The step of a *_host entry point whose arguments have been checked: stage the host inputs, run the step on the staging
+// slot, release the slot, copy the outputs out.
+//   to_host = false: probs / loss are device buffers the kernels write;
+//   to_host = true:  probs (may be null) and loss are host buffers, filled from H_PROBS / H_LOSS after the step -- except that
+//                    the fused optimizer step (reduce_adam; the peer steps always take it) stores the loss floats straight
+//                    into a pinned `loss` (host_alias).
+// After an optimizer step `loss` holds three floats (the loss, then the two regularisers, adam->reg), else one.
+static int host_step(hdgnn_handle_t h, int B, int B_global, const uint8_t* adj_host, const float* x_host,
+                     const int32_t* hmap_host, const int32_t* L_host, const uint8_t* Y_host, const float* params,
+                     float* probs, float* loss, float* grads, const AdamArgs* adam, bool to_host, void* stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    h->launches = 0;
+    int rc = stage_inputs(h, B, adj_host, x_host, hmap_host, L_host, Y_host, st);
+    if (rc) return rc;
+    const Inputs in = staged_inputs(h, params);
+    float* probs_d = to_host && probs ? F(h, "H_PROBS") : probs;
+    float* alias = to_host && adam && fused_for(h, true) ? host_alias(loss) : nullptr;
+    float* loss_d = to_host ? (alias ? alias : F(h, "H_LOSS")) : loss;
+    AdamArgs ad{};
+    if (adam) { ad = *adam; ad.reg = loss_d + 1; }
+    rc = run_step(h, B, B_global, in, nullptr, probs_d, loss_d, grads, adam ? &ad : nullptr, st);
+    if (rc) return rc;
+    if ((rc = release_slot(h, st)) || !to_host) return rc;
+    if (probs)
+        CK(h, cudaMemcpyAsync(probs, probs_d, (size_t)B * 2 * h->Nc * (h->Nc - 1) * sizeof(float), cudaMemcpyDefault, st));
+    if (loss && !alias) CK(h, cudaMemcpyAsync(loss, loss_d, (adam ? 3 : 1) * sizeof(float), cudaMemcpyDeviceToHost, st));
+    return HDGNN_OK;
+}
+
 int hdgnn_train_step_host(hdgnn_handle_t h, int B, const uint8_t* adj_host, const float* x_host,
                           const int32_t* hmap_host, const int32_t* L_host, const uint8_t* Y_host, float* params,
                           float* m, float* v, int32_t* step_counter, float lr, float beta1, float beta2, float eps,
                           float* probs_host, float* loss3_host, void* stream) {
-    if (!h) return HDGNN_E_INVALID;
-    if (B < 1 || B > h->cfg.max_batch) return fail(h, HDGNN_E_INVALID, "B out of range [1, max_batch]");
-    if (!adj_host || !x_host || !hmap_host || !L_host || !Y_host || !params || !m || !v || !step_counter || !loss3_host)
-        return fail(h, HDGNN_E_INVALID, "null pointer");
-    cudaStream_t st = (cudaStream_t)stream;
-    h->launches = 0;
-    h->want_flag_release = fused_for(h, true);
-    int rc = stage_inputs(h, B, adj_host, x_host, hmap_host, L_host, Y_host, st);
-    h->want_flag_release = false;
+    int rc = check_host_inputs(h, B, adj_host, x_host, hmap_host, L_host, Y_host, params);
     if (rc) return rc;
-    Inputs in = staged_inputs(h, params);
-    float* probs_d = probs_host ? F(h, "H_PROBS") : nullptr;
-    float* alias = fused_for(h, true) ? host_alias(loss3_host) : nullptr;
-    float* loss_d = alias ? alias : F(h, "H_LOSS");
-    AdamArgs ad{params, m, v, step_counter, lr, beta1, beta2, eps, loss_d + 1};
-    rc = run_step(h, B, B, in, nullptr, probs_d, loss_d, F(h, "H_GRADS"), &ad, st);
-    if (rc) return rc;
-    if ((rc = release_slot(h, st))) return rc;
-    if (probs_host)
-        CK(h, cudaMemcpyAsync(probs_host, probs_d, (size_t)B * 2 * h->Nc * (h->Nc - 1) * sizeof(float), cudaMemcpyDefault, st));
-    if (!alias) CK(h, cudaMemcpyAsync(loss3_host, loss_d, 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
-    return HDGNN_OK;
+    if (!m || !v || !step_counter || !loss3_host) return fail(h, HDGNN_E_INVALID, "null pointer");
+    const AdamArgs ad{params, m, v, step_counter, lr, beta1, beta2, eps, nullptr};
+    return host_step(h, B, B, adj_host, x_host, hmap_host, L_host, Y_host, params, probs_host, loss3_host, F(h, "H_GRADS"), &ad,
+                     true, stream);
 }
 
 int hdgnn_train_step_peer(hdgnn_handle_t h, int B, int B_global, const uint8_t* adj, int adj_pitch, const float* x,
@@ -1320,81 +1314,42 @@ int hdgnn_train_step_peer(hdgnn_handle_t h, int B, int B_global, const uint8_t* 
     int rc = check_inputs(h, B, adj, adj_pitch, x, hmap, L, Y, y_pitch, params);
     if (rc) return rc;
     if (!m || !v || !step_counter || !loss3) return fail(h, HDGNN_E_INVALID, "null pointer");
-    if (!h->peer_ready) return fail(h, HDGNN_E_INVALID, "hdgnn_peer_attach has not been called");
-    if (B_global != B * h->peer.world) return fail(h, HDGNN_E_INVALID, "B_global must be B * world (equal shards)");
-    h->launches = 0;
-    Inputs in{adj, x, hmap, L, Y, params};
-    alias_bits(h, in);
-    AdamArgs ad{params, m, v, step_counter, lr, beta1, beta2, eps, loss3 + 1, true};
-    return run_step(h, B, B_global, in, logits, probs, loss3, F(h, "H_GRADS"), &ad, (cudaStream_t)stream);
+    if ((rc = check_peer(h, B, B_global))) return rc;
+    const AdamArgs ad{params, m, v, step_counter, lr, beta1, beta2, eps, loss3 + 1, true};
+    return device_step(h, B, B_global, adj, x, hmap, L, Y, params, logits, probs, loss3, F(h, "H_GRADS"), &ad, stream);
 }
 
 int hdgnn_train_step_peer_host(hdgnn_handle_t h, int B, int B_global, const uint8_t* adj_host, const float* x_host,
                                const int32_t* hmap_host, const int32_t* L_host, const uint8_t* Y_host, float* params,
                                float* m, float* v, int32_t* step_counter, float lr, float beta1, float beta2, float eps,
                                float* probs_out, float* loss3_host, void* stream) {
-    if (!h) return HDGNN_E_INVALID;
-    if (B < 1 || B > h->cfg.max_batch) return fail(h, HDGNN_E_INVALID, "B out of range [1, max_batch]");
-    if (!adj_host || !x_host || !hmap_host || !L_host || !Y_host || !params || !m || !v || !step_counter || !loss3_host)
-        return fail(h, HDGNN_E_INVALID, "null pointer");
-    if (!h->peer_ready) return fail(h, HDGNN_E_INVALID, "hdgnn_peer_attach has not been called");
-    if (B_global != B * h->peer.world) return fail(h, HDGNN_E_INVALID, "B_global must be B * world (equal shards)");
-    cudaStream_t st = (cudaStream_t)stream;
-    h->launches = 0;
-    h->want_flag_release = true;            // the peer step always ends in reduce_adam (fused path only)
-    int rc = stage_inputs(h, B, adj_host, x_host, hmap_host, L_host, Y_host, st);
-    h->want_flag_release = false;
+    int rc = check_host_inputs(h, B, adj_host, x_host, hmap_host, L_host, Y_host, params);
     if (rc) return rc;
-    Inputs in = staged_inputs(h, params);
-    float* probs_d = probs_out ? F(h, "H_PROBS") : nullptr;
-    float* alias = host_alias(loss3_host);
-    float* loss_d = alias ? alias : F(h, "H_LOSS");
-    AdamArgs ad{params, m, v, step_counter, lr, beta1, beta2, eps, loss_d + 1, true};
-    rc = run_step(h, B, B_global, in, nullptr, probs_d, loss_d, F(h, "H_GRADS"), &ad, st);
-    if (rc) return rc;
-    if ((rc = release_slot(h, st))) return rc;
-    if (probs_out)
-        CK(h, cudaMemcpyAsync(probs_out, probs_d, (size_t)B * 2 * h->Nc * (h->Nc - 1) * sizeof(float), cudaMemcpyDefault, st));
-    if (!alias) CK(h, cudaMemcpyAsync(loss3_host, loss_d, 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
-    return HDGNN_OK;
+    if (!m || !v || !step_counter || !loss3_host) return fail(h, HDGNN_E_INVALID, "null pointer");
+    if ((rc = check_peer(h, B, B_global))) return rc;
+    const AdamArgs ad{params, m, v, step_counter, lr, beta1, beta2, eps, nullptr, true};
+    return host_step(h, B, B_global, adj_host, x_host, hmap_host, L_host, Y_host, params, probs_out, loss3_host, F(h, "H_GRADS"),
+                     &ad, true, stream);
 }
 
 int hdgnn_forward_backward_host(hdgnn_handle_t h, int B, int B_global, const uint8_t* adj_host, const float* x_host,
                                 const int32_t* hmap_host, const int32_t* L_host, const uint8_t* Y_host, const float* params,
                                 float* probs, float* loss, float* grads, void* stream) {
-    if (!h) return HDGNN_E_INVALID;
-    if (B < 1 || B > h->cfg.max_batch) return fail(h, HDGNN_E_INVALID, "B out of range [1, max_batch]");
-    if (!adj_host || !x_host || !hmap_host || !L_host || !Y_host || !params || !grads)
-        return fail(h, HDGNN_E_INVALID, "null pointer");
+    int rc = check_host_inputs(h, B, adj_host, x_host, hmap_host, L_host, Y_host, params);
+    if (rc) return rc;
+    if (!grads) return fail(h, HDGNN_E_INVALID, "null pointer");
     if (B_global < B) return fail(h, HDGNN_E_INVALID, "B_global < B");
-    cudaStream_t st = (cudaStream_t)stream;
-    h->launches = 0;
-    int rc = stage_inputs(h, B, adj_host, x_host, hmap_host, L_host, Y_host, st);
-    if (rc) return rc;
-    Inputs in = staged_inputs(h, params);
-    rc = run_step(h, B, B_global, in, nullptr, probs, loss, grads, nullptr, st);
-    if (rc) return rc;
-    return release_slot(h, st);
+    return host_step(h, B, B_global, adj_host, x_host, hmap_host, L_host, Y_host, params, probs, loss, grads, nullptr, false, stream);
 }
 
 int hdgnn_infer_host(hdgnn_handle_t h, int B, const uint8_t* adj_host, const float* x_host, const int32_t* hmap_host,
                      const int32_t* L_host, const uint8_t* Y_host, const float* params, float* probs_host,
                      float* loss_host, void* stream) {
-    if (!h) return HDGNN_E_INVALID;
-    if (B < 1 || B > h->cfg.max_batch) return fail(h, HDGNN_E_INVALID, "B out of range [1, max_batch]");
-    if (!adj_host || !x_host || !hmap_host || !L_host || !Y_host || !params || !probs_host)
-        return fail(h, HDGNN_E_INVALID, "null pointer");
-    cudaStream_t st = (cudaStream_t)stream;
-    h->launches = 0;
-    int rc = stage_inputs(h, B, adj_host, x_host, hmap_host, L_host, Y_host, st);
+    int rc = check_host_inputs(h, B, adj_host, x_host, hmap_host, L_host, Y_host, params);
     if (rc) return rc;
-    Inputs in = staged_inputs(h, params);
-    rc = run_step(h, B, B, in, nullptr, F(h, "H_PROBS"), F(h, "H_LOSS"), nullptr, nullptr, st);
-    if (rc) return rc;
-    if ((rc = release_slot(h, st))) return rc;
-    CK(h, cudaMemcpyAsync(probs_host, F(h, "H_PROBS"), (size_t)B * 2 * h->Nc * (h->Nc - 1) * sizeof(float), cudaMemcpyDefault, st));
-    if (loss_host) CK(h, cudaMemcpyAsync(loss_host, F(h, "H_LOSS"), sizeof(float), cudaMemcpyDeviceToHost, st));
-    return HDGNN_OK;
+    if (!probs_host) return fail(h, HDGNN_E_INVALID, "null pointer");
+    return host_step(h, B, B, adj_host, x_host, hmap_host, L_host, Y_host, params, probs_host, loss_host, nullptr, nullptr, true,
+                     stream);
 }
 
 int hdgnn_workspace(hdgnn_handle_t h, const char* name, void** ptr, size_t* bytes) {

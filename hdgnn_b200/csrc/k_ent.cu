@@ -3,20 +3,15 @@
 
 namespace hdgnn {
 
-template <int CWT, int NRG>
-static const void* ent2_fn(bool bwd) {
-    return bwd ? (const void*)ent_bwd2_kernel<CWT, NRG> : (const void*)ent_fwd2_kernel<CWT, NRG>;
-}
-
-const void* ent2_fn_rt(int cwt, int nrg, bool bwd) {
+const void* ent2_fn_rt(int cwt, bool bwd) {
     const void* fn = nullptr;
-    HDGNN_CWT_SWITCH(cwt, HDGNN_NRG_SWITCH(nrg, fn = ent2_fn<CWT, NRG>(bwd)));
+    HDGNN_CWT_SWITCH(cwt, fn = bwd ? (const void*)ent_bwd2_kernel<CWT> : (const void*)ent_fwd2_kernel<CWT>);
     return fn;
 }
 
-void launch_ent2(int cwt, int nrg, bool bwd, int grid, size_t smem, cudaStream_t st, const Ent2Args& a, bool pdl) {
-    if (bwd) { HDGNN_CWT_SWITCH(cwt, HDGNN_NRG_SWITCH(nrg, launch_ex(ent_bwd2_kernel<CWT, NRG>, grid, KG * NRG * 32, smem, st, pdl, a))); }
-    else { HDGNN_CWT_SWITCH(cwt, HDGNN_NRG_SWITCH(nrg, launch_ex(ent_fwd2_kernel<CWT, NRG>, grid, KG * NRG * 32, smem, st, pdl, a))); }
+void launch_ent2(int cwt, bool bwd, int grid, size_t smem, cudaStream_t st, const Ent2Args& a, bool pdl) {
+    if (bwd) { HDGNN_CWT_SWITCH(cwt, launch_ex(ent_bwd2_kernel<CWT>, grid, KG * 32, smem, st, pdl, a)); }
+    else { HDGNN_CWT_SWITCH(cwt, launch_ex(ent_fwd2_kernel<CWT>, grid, KG * 32, smem, st, pdl, a)); }
 }
 
 }  // namespace hdgnn

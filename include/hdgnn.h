@@ -144,10 +144,13 @@ int hdgnn_train_step(hdgnn_handle_t h, int B,
                      float* logits, float* probs, float* loss3, void* stream);
 
 /* One whole training step from HOST buffers (pinned recommended): H2D copies of the five
- * compact inputs, forward, backward, Adam, and a D2H copy of {CE, loss_map, loss_para} into
- * loss3_host.  The kernels and the D2H copy are enqueued on `stream`; the H2D copies go through two staging
- * slots on a copy stream owned by the handle (ordered against `stream` by events), so the copies of one call
- * overlap the kernels of the previous one.  Host buffers must stay unchanged until `stream` has passed the call.  Un-pitched host layouts: adj (B,Ne,Ne), Y (B,Nc,Nc).
+ * compact inputs, forward, backward, Adam, and {CE, loss_map, loss_para} into loss3_host (stored by the last kernel
+ * when loss3_host is pinned and the step runs on the fused path, else copied D2H).  The kernels and the D2H copies are
+ * enqueued on `stream`; the H2D copies go through two staging slots on a copy stream owned by the handle, so the copies
+ * of one call overlap the kernels of the previous one.  A slot is refilled after an event `stream` records behind the
+ * call's kernels; the kernels wait for the copies through an event, or, when the per-commit kernel is the first kernel
+ * of the step (label bitmaps, HDGNN_F_LABEL_BITS, and no dense entity sweep), by polling a tag the copy stream's last
+ * DMA writes, which keeps `stream` free of cross-stream waits.  Host buffers must stay unchanged until `stream` has passed the call.  Un-pitched host layouts: adj (B,Ne,Ne), Y (B,Nc,Nc).
  * probs_host may be NULL (otherwise B*2*Ncr floats are copied out; the pointer may also be a DEVICE buffer, e.g. to feed
  * hdgnn_eval_counts without a round trip through the host). */
 int hdgnn_train_step_host(hdgnn_handle_t h, int B,
@@ -168,9 +171,9 @@ int hdgnn_forward_backward_host(hdgnn_handle_t h, int B, int B_global,
 /* ---- commit sharding with the gradient all-reduce fused into the reduce + Adam kernel (one process per GPU) --------
  * The reference is single-device; this replaces what a data-parallel port would do with an NCCL all-reduce between
  * hdgnn_forward_backward and hdgnn_adam_step.  Every rank owns a mailbox in its HBM; the last kernel of the step pushes
- * its 128-parameter gradient slices into every peer's mailbox over NVLink (P2P stores of {sequence number : value}
+ * its 16-parameter gradient slices into every peer's mailbox over NVLink (P2P stores of {sequence number : value}
  * words, no flag and no fence), polls its own mailbox for the peers' slices, sums them in rank order (bitwise identical
- * on all ranks) and applies the regularisers + TF1 Adam -- the step has the same 5 launches as on one GPU and no NCCL call.
+ * on all ranks) and applies the regularisers + TF1 Adam -- the step has the same launches as on one GPU (two with label bitmaps) and no NCCL call.
  * Set-up: (1) every rank calls hdgnn_peer_export and receives a 64-byte CUDA IPC handle; (2) the handles are gathered by
  * the caller (torch.distributed / MPI / files) into world*64 bytes ordered by rank; (3) every rank calls
  * hdgnn_peer_attach, then the ranks synchronise once (barrier) before the first step.  Fused path only (Nc <= 256),

@@ -35,7 +35,7 @@ CASES = [
 ]
 
 
-F_DEBUG, F_LEGACY, F_DENSE = 2, 4, 16
+F_DEBUG, F_LEGACY, F_LABEL_BITS, F_DENSE = 2, 4, 8, 16
 PATH_FLAGS = {"default": 0, "dense": F_DENSE, "legacy": F_LEGACY}
 
 
@@ -182,20 +182,43 @@ def test_adam_step_matches_tf_formula():
     eng.close()
 
 
+# host inputs of the *_host entry points: byte grids (staged by events, re-pitched on the device); label bitmaps in one pinned
+# HostBatch block (one DMA, ordered by a tag the per-commit kernel polls) or in five separate pinned tensors (one DMA per
+# section); label bitmaps into a dense-sweep handle, whose first kernel is ent_fwd2 (ordered by an event instead of the tag)
+HOST_INPUTS = {"bytes": 0, "bits_block": F_LABEL_BITS, "bits_sections": F_LABEL_BITS, "dense_bits": F_LABEL_BITS | F_DENSE}
+
+
 def test_host_entry_points_match_device_entry_points():
-    from hdgnn_b200.engine import Engine, DeviceBatch
+    _host_entry_points_match_device_entry_points("bytes")
+
+
+@pytest.mark.parametrize("inputs", ["bits_block", "bits_sections", "dense_bits"])
+def test_host_entry_points_match_device_entry_points_label_bits(inputs):
+    _host_entry_points_match_device_entry_points(inputs)
+
+
+def _host_entry_points_match_device_entry_points(inputs):
+    from hdgnn_b200.engine import Engine, DeviceBatch, pack_label_bits
+    from hdgnn_b200.model import HostBatch
     B, Ne, Nc, variant = 4, 50, 20, 2      # Ne, Nc not multiples of 16: exercises the pitched staging copy
     cb = make_commits(B, Ne, Nc, seed=21)
     flat = _params(variant).float()
-    eng = Engine(Ne, Nc, variant=variant, max_batch=B)
-    db = DeviceBatch.from_numpy(cb.adj, cb.x, cb.hmap, cb.L, cb.Y, eng.tdev)
+    flags = HOST_INPUTS[inputs]
+    bits = bool(flags & F_LABEL_BITS)
+    eng = Engine(Ne, Nc, variant=variant, max_batch=B, flags=flags)
+    db = DeviceBatch.from_numpy(cb.adj, cb.x, cb.hmap, cb.L, cb.Y, eng.tdev, bits=bits)
     params = flat.cuda()
     probs, _, loss, grads = eng.forward_backward(db, params)
     p_ref = params.clone(); m = torch.zeros_like(params); v = torch.zeros_like(params)
     step = torch.zeros(1, dtype=torch.int32, device="cuda"); reg = torch.zeros(2, device="cuda")
     eng.adam_step(p_ref, grads, m, v, step, reg_losses=reg)
     pin = lambda a: torch.as_tensor(np.ascontiguousarray(a)).pin_memory()
-    h = [pin(cb.adj), pin(cb.x), pin(cb.hmap), pin(cb.L), pin(cb.Y)]
+    if inputs == "bits_sections":
+        h = [pin(pack_label_bits(cb.adj).view(np.int32)), pin(cb.x), pin(cb.hmap), pin(cb.L), pin(pack_label_bits(cb.Y).view(np.int32))]
+    elif bits:
+        h = list(HostBatch(cb, bits=True).tensors())
+    else:
+        h = [pin(cb.adj), pin(cb.x), pin(cb.hmap), pin(cb.L), pin(cb.Y)]
     p2 = flat.cuda(); m2 = torch.zeros_like(p2); v2 = torch.zeros_like(p2)
     step2 = torch.zeros(1, dtype=torch.int32, device="cuda")
     loss3 = torch.zeros(3).pin_memory(); probs_h = torch.zeros(B, 2, eng.Ncr).pin_memory()
