@@ -16,6 +16,8 @@
 //             -> [E: score(edge, train: recompute + delta sums) -> head_bwd(edge) -> pairsum_bwd(edge)
 //                 -> rank1_grad(edge, tied)] -> grad_reduce
 //       opt : adam (regularisers fused)
+// Which path each mode (forward only / training) takes, and the form of the fused path -- table placement, inline or dense
+// entity stage, mid2's shared-memory layout, the cluster form -- is decided once at hdgnn_create by plan_fused (FusedPlan).
 //
 // Entry points: each checks its arguments and makes one call -- device_step for the device-resident entries, host_step for the
 // *_host entries.  host_step stages the host inputs into one of two slots on the handle's copy stream (stage_inputs), runs the
@@ -96,6 +98,26 @@ ParamOff make_off(int variant) {
 
 struct Buf { void* p = nullptr; size_t bytes = 0; };
 
+// mid2 in one mode of a handle (FusedPlan::mode[0]: forward only, mode[1]: training)
+struct Mid2Mode {
+    bool fused = false;        // this mode runs on the fused path, else on the multi-kernel path
+    Mid2Opts opt;              // mid2's options, normalised; opt.dlt_smem = false: the dL/dlogit table is the DLT workspace
+    Mid2Smem lay{}; size_t smem = 0;     // the layout they give and its dynamic shared memory
+    int clusters = 0;          // co-resident clusters of two CTAs of the cluster form (mid2.cuh); 0: one CTA per commit
+};
+
+// the fused path of a handle, fixed at create by plan_fused; the fields below `mode` apply when mode[0].fused
+struct FusedPlan {
+    Mid2Mode mode[2];
+    bool gt = false;           // mid2's hunk-stage tables in global memory (Nc > 128), workspace TABS; see also Mid2Opts::scg
+    bool inl = false;          // entity pair layer inside mid2 (entsp.cuh)
+    bool dense = false;        // the entity branch runs as the dense sweeps ent_fwd2 / ent_bwd2 around mid2 (ent2.cuh)
+    bool mid2_first = false;   // no dense sweeps: mid2 is the step's first kernel (after pack_bits for byte grids)
+    bool edge = false;         // variant 4: the entity-edge branch inside mid2 (its backward too when mode[1].fused)
+    int fwd_occ = 1, bwd_occ = 1;  // resident CTAs per SM of the dense sweeps
+    bool pdl = true;           // programmatic dependent launch between the fused kernels (off with HDGNN_F_DEBUG)
+};
+
 }  // namespace
 
 constexpr int NSLOT = 2;         // staging slots of the *_host entry points
@@ -108,26 +130,13 @@ struct hdgnn_handle_s {
     int RTe, Se, CWe;          // entity grid tiling
     int RTc, Sc, CWc;          // hunk grid tiling
     bool ent, edge;            // branches that feed the loss
-    bool fused = false;        // ent_fwd -> mid -> ent_bwd -> reduce(+adam) path (variants 1-3)
     bool debug = false;
+    FusedPlan plan;
     // fused path: label bitmaps + balanced row chunks of the entity grid (ent2.cuh)
     int WPe = 0, WPc = 0;      // bitmap words per row
     int nsm = 148;
     int cwt = 0;                                               // column segments per pass of the entity sweeps
-    int fwd_occ = 1, bwd_occ = 1;                              // resident CTAs per SM
-    bool pdl = true;                                           // programmatic dependent launch between the fused kernels
     int bslot = 0;                                             // bitmap buffer of the current step (two alternate)
-    bool dlt_global = false;                                   // mid2's dL/dlogit table in HBM instead of shared memory
-    bool gt = false;                                           // mid2's hunk-stage tables in global memory (Nc > 128), workspace TABS
-    bool scg = false;                                          // ... and its S / GE rows in the GE workspace instead of shared memory
-    bool cl_ok = false;                                        // the cluster form of mid2 (two CTAs share a commit) exists for this handle
-    int cl_max[2] = {0, 0};                                    // co-resident clusters of two: [inference, training] shared-memory size
-    bool infer_only = false;                                   // 256 < Nc <= 512: the fused kernel exists forward-only; training takes the multi-kernel path
-    bool mid_scache = false;                                   // mid2 keeps the entity effect sums in shared memory for its backward
-    bool inl = false;                                          // entity pair layer inside mid2 (entsp.cuh): no ent_fwd2 / ent_bwd2 launch
-    bool edge_fused = false;                                   // variant 4: the entity-edge branch inside mid2 as well
-    bool edge_fused_train = false;                             // ... including its backward
-    int Gf = 0, Gb = 0, Rf = 0, Rb = 0, SLf = 0;               // grids / rows per CTA / slots of the last launch
     std::map<std::string, Buf> ws;
     std::string err;
     int launches = 0;
@@ -194,12 +203,6 @@ namespace {
             (h)->prof_ev.push_back({what, {(h)->prof_start, stop_}});                             \
         }                                                                                         \
     } while (0)
-
-// which path a call takes: variant 4 runs its forward on the fused path as soon as the edge branch fits (edge_fused), its
-// training step only with edge_fused_train; everything else follows h->fused
-bool fused_for(hdgnn_handle_t h, bool train) {
-    return h->fused && !(train && h->infer_only) && (!h->edge || (train ? h->edge_fused_train : h->edge_fused));
-}
 
 int fail(hdgnn_handle_t h, int code, const std::string& msg) {
     if (h) h->err = msg; else g_create_error = msg;
@@ -531,23 +534,23 @@ struct AdamArgs { float* params; float* m; float* v; int32_t* step; float lr, b1
 // column segments per pass of an entity sweep: the whole row when it fits 8 segments, else passes of 8
 int ent2_cwt(int N) { const int cw = (N + 31) / 32; return cw <= 8 ? cw : 8; }
 
-// Grid of an entity sweep for a batch of B commits: `occ` resident CTAs on each SM, one wave, the
+// Grid of an entity sweep over B commits of N entities: `occ` resident CTAs on each of `nsm` SMs, one wave, the
 // B*N rows cut into equal chunks (at least 8 rows each).
-void ent2_grid(hdgnn_handle_t h, int B, int occ, int* G, int* R) {
-    const long long rows = (long long)B * h->Ne;
-    long long g = (long long)occ * h->nsm;
+void ent2_grid(int B, int N, int occ, int nsm, int* G, int* R) {
+    const long long rows = (long long)B * N;
+    long long g = (long long)occ * nsm;
     if (g > rows / 8) g = rows / 8 > 0 ? rows / 8 : 1;
     *R = (int)((rows + g - 1) / g);
     *G = (int)((rows + *R - 1) / *R);
 }
 
-// largest number of co-resident CTAs per SM (<= 4) whose row chunk fits next to each other
-int ent2_occupancy(hdgnn_handle_t h, bool bwd) {
-    const void* fn = ent2_fn_rt(h->cwt, bwd);
+// largest number of co-resident CTAs per SM (<= 4) whose row chunk of a full batch fits next to each other
+int ent2_occupancy(const hdgnn_config_t& cfg, int nsm, bool bwd) {
+    const int cwt = ent2_cwt(cfg.Ne); const void* fn = ent2_fn_rt(cwt, bwd);
     for (int occ = 4; occ > 1; --occ) {
         int G, R, got = 0;
-        ent2_grid(h, h->cfg.max_batch, occ, &G, &R);
-        const size_t smem = ent2_smem_bytes(h->cwt, h->Ne, R, h->WPe, bwd);
+        ent2_grid(cfg.max_batch, cfg.Ne, occ, nsm, &G, &R);
+        const size_t smem = ent2_smem_bytes(cwt, cfg.Ne, R, bit_words(cfg.Ne), bwd);
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&got, fn, KG * 32, smem) == cudaSuccess && got >= occ) return occ;
     }
     return 1;
@@ -575,6 +578,7 @@ int debug_scatter(hdgnn_handle_t h, int B, cudaStream_t st) {
 
 int fused_forward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float* logits, float* probs, bool train,
                   cudaStream_t st) {
+    const FusedPlan& P = h->plan; const Mid2Mode& md = P.mode[train];
     // bitmaps given: nothing to pack.  The first kernel then follows the previous step's optimizer kernel directly and reads
     // the weights it updates: ent_fwd2 defers those loads behind its pdl_wait (Ent2Args::head), mid2 is launched normally
     const bool head = in.ebits != nullptr;
@@ -590,22 +594,23 @@ int fused_forward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float
         p.B = B;
         const long long rows = (long long)B * (h->Ne + h->Nc);
         PROF_BEGIN(h, st);
-        if (h->pe <= 256 && h->pc <= 256) launch_ex(pack_bits_kernel<16>, (int)((rows + 15) / 16), 256, 0, st, h->pdl, p);
-        else launch_ex(pack_bits_kernel<32>, (int)((rows + 7) / 8), 256, 0, st, h->pdl, p);
+        if (h->pe <= 256 && h->pc <= 256) launch_ex(pack_bits_kernel<16>, (int)((rows + 15) / 16), 256, 0, st, P.pdl, p);
+        else launch_ex(pack_bits_kernel<32>, (int)((rows + 7) / 8), 256, 0, st, P.pdl, p);
         LAUNCH_CHECK(h, "pack_bits", st);
     }
-    if (h->ent && !h->inl) {
+    int G, R = 0, SL = 0;       // grid and row chunks of ent_fwd2, which mid2 reads back
+    if (P.dense) {
         Ent2Args a = ent2_args(h, B, in);
-        ent2_grid(h, B, h->fwd_occ, &h->Gf, &h->Rf);
-        h->SLf = ent2_max_slots(h->Ne, h->Rf);
-        a.R = h->Rf; a.SL = h->SLf; a.RS = F(h, "RS1"); a.CSp = F(h, "CS1P"); a.head = head ? 1 : 0;
-        const size_t smem = ent2_smem_bytes(h->cwt, h->Ne, h->Rf, h->WPe, false);
+        ent2_grid(B, h->Ne, P.fwd_occ, h->nsm, &G, &R);
+        SL = ent2_max_slots(h->Ne, R);
+        a.R = R; a.SL = SL; a.RS = F(h, "RS1"); a.CSp = F(h, "CS1P"); a.head = head ? 1 : 0;
+        const size_t smem = ent2_smem_bytes(h->cwt, h->Ne, R, h->WPe, false);
         PROF_BEGIN(h, st);
-        launch_ent2(h->cwt, false, h->Gf, smem, st, a, h->pdl);
+        launch_ent2(h->cwt, false, G, smem, st, a, P.pdl);
         LAUNCH_CHECK(h, "ent_fwd", st);
     }
     Mid2Args m{};
-    m.Ne = h->Ne; m.Nc = h->Nc; m.ent = h->ent ? 1 : 0; m.R = h->Rf; m.SL = h->SLf;
+    m.Ne = h->Ne; m.Nc = h->Nc; m.ent = h->ent ? 1 : 0; m.R = R; m.SL = SL;
     m.ebits = h->eb; m.WPe = h->WPe;
     m.ybits = h->yb; m.WPc = h->WPc;
     m.x = in.x; m.hmap = in.hmap; m.L = in.L;
@@ -615,33 +620,29 @@ int fused_forward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float
     m.GE = F(h, "GE"); m.gpart = F(h, "GPART"); m.total = h->po.total;
     m.dbg = h->debug ? F(h, "DBG") : nullptr;
     m.clk = h->debug ? (long long*)h->ws["CLK"].p : nullptr;
-    const bool dlt_g = train && h->dlt_global;
-    m.dlt_g = dlt_g ? F(h, "DLT") : nullptr;
-    m.scache = ((train && h->ent && h->mid_scache) || h->inl) ? 1 : 0;
-    m.inl = h->inl ? 1 : 0;
+    m.dlt_g = md.opt.dlt_smem ? nullptr : F(h, "DLT");
+    m.scache = md.opt.scache ? 1 : 0;
+    m.inl = P.inl ? 1 : 0;
     m.wait_flag = in.wait_flag; m.wait_tag = in.wait_tag;
     m.hits_acc = h->hits_acc;
     m.evc = h->evc;
-    m.edge = h->edge_fused ? 1 : 0;
+    m.edge = P.edge ? 1 : 0;
     if (m.edge) { m.RSEg = F(h, "RSEG"); m.CSEg = F(h, "CSEG"); m.REg = F(h, "REG"); m.CEg = F(h, "CEG"); m.A1F = F(h, "A1F"); m.PREg = F(h, "PREG"); }
-    m.lay = mid2_layout(h->Ne, h->Nc, train, !dlt_g, m.scache != 0, h->inl, h->edge_fused, h->gt, h->scg);
-    m.tabs_g = h->gt ? F(h, "TABS") : nullptr;
-    const size_t smem = mid2_smem_bytes(h->Ne, h->Nc, train, !dlt_g, m.scache != 0, h->inl, h->edge_fused, h->gt, h->scg);
-    const int cwc = (h->Nc + 31) / 32;
+    m.lay = md.lay;
+    m.tabs_g = P.gt ? F(h, "TABS") : nullptr;
     // Batches below one wave of SMs: clusters of two CTAs, the `S` costliest commits shared by both CTAs of a cluster (mid2.cuh),
     // as many as there are spare SMs and co-resident clusters
     bool cl = false;
     int grid = B;
-    if (h->cl_ok && B < h->nsm) {
-        const int maxc = h->cl_max[train ? 1 : 0];
+    if (md.clusters > 0 && B < h->nsm) {
         int S = B < h->nsm - B ? B : h->nsm - B;
-        if (S > 2 * maxc - B) S = 2 * maxc - B;
+        if (S > 2 * md.clusters - B) S = 2 * md.clusters - B;
         if (S > 0) { cl = true; m.B = B; m.nsplit = S; grid = 2 * (S + (B - S + 1) / 2); }
     }
     PROF_BEGIN(h, st);
     // inline entity stage: this kernel reads the weights after its pdl_wait, so it may follow the previous step's optimizer
     // kernel (or pack_bits) under programmatic dependent launch; otherwise PDL only behind ent_fwd2
-    launch_mid2(cwc, train, h->gt, cl, grid, smem, st, m, h->pdl && (h->ent || h->inl));
+    launch_mid2(h->CWc, train, P.gt, cl, grid, md.smem, st, m, P.pdl && (h->ent || P.inl));
     LAUNCH_CHECK(h, train ? "mid(train)" : "mid(infer)", st);
     if (h->debug) return debug_scatter(h, B, st);
     return HDGNN_OK;
@@ -649,18 +650,20 @@ int fused_forward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float
 
 int fused_backward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float* loss, float* grads,
                    const AdamArgs* adam, cudaStream_t st) {
-    if (h->ent && !h->inl) {
+    const FusedPlan& P = h->plan;
+    int G = 0, R;               // grid (reduce_adam adds its gradient partials) and row chunks of ent_bwd2
+    if (P.dense) {
         Ent2Args a = ent2_args(h, B, in);
-        ent2_grid(h, B, h->bwd_occ, &h->Gb, &h->Rb);
-        a.R = h->Rb; a.SL = 0; a.GR = F(h, "GE"); a.GC = F(h, "GE"); a.gpart = F(h, "GPE");
-        const size_t smem = ent2_smem_bytes(h->cwt, h->Ne, h->Rb, h->WPe, true);
+        ent2_grid(B, h->Ne, P.bwd_occ, h->nsm, &G, &R);
+        a.R = R; a.SL = 0; a.GR = F(h, "GE"); a.GC = F(h, "GE"); a.gpart = F(h, "GPE");
+        const size_t smem = ent2_smem_bytes(h->cwt, h->Ne, R, h->WPe, true);
         PROF_BEGIN(h, st);
-        launch_ent2(h->cwt, true, h->Gb, smem, st, a, h->pdl);
+        launch_ent2(h->cwt, true, G, smem, st, a, P.pdl);
         LAUNCH_CHECK(h, "ent_bwd", st);
     }
     FinalArgs f{};
     f.B = B; f.total = h->po.total; f.gpart = F(h, "GPART");
-    if (h->ent && !h->inl) f.ent = {F(h, "GPE"), h->Gb, h->po.ent_w1, h->po.ent_w1 + HD, h->po.ent_b1, h->po.ent_w1 + 2 * HD};
+    if (P.dense) f.ent = {F(h, "GPE"), G, h->po.ent_w1, h->po.ent_w1 + HD, h->po.ent_b1, h->po.ent_w1 + 2 * HD};
     f.cep = F(h, "CEP"); f.ncep = B; f.loss_denom = (float)B_global * (float)(h->Nc * (h->Nc - 1)); f.loss = loss;
     f.grads = grads;
     f.l2part = F(h, "FIN_L2"); f.counter = (unsigned int*)h->ws["FIN_CNT"].p;
@@ -671,12 +674,10 @@ int fused_backward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, floa
         if (adam->peer) f.peer = h->peer;
     }
     PROF_BEGIN(h, st);
-    launch_ex(reduce_adam_kernel, (h->po.total + FIN_P - 1) / FIN_P, FIN_P * FIN_SL, 0, st, h->pdl, f);
+    launch_ex(reduce_adam_kernel, (h->po.total + FIN_P - 1) / FIN_P, FIN_P * FIN_SL, 0, st, P.pdl, f);
     LAUNCH_CHECK(h, adam ? (adam->peer ? "reduce_allreduce_adam(peer)" : "reduce_adam") : "grad_reduce", st);
     return HDGNN_OK;
 }
-
-int env_int(const char* name, int dflt);
 
 // HDGNN_F_LABEL_BITS: byte offsets of the five inputs of a batch of B commits inside one staging block (every section starts at
 // the next multiple of 16 bytes).  Host buffers laid out the same way travel in ONE DMA (stage_inputs).
@@ -691,41 +692,97 @@ WireOff wire_layout(hdgnn_handle_t h, int B) {
     return w;
 }
 
-// opt-in shared memory + occupancy of the fused kernels for this handle's shapes
-cudaError_t setup_fused(hdgnn_handle_t h, int optin) {
-    const cudaFuncAttribute A = cudaFuncAttributeMaxDynamicSharedMemorySize;
-    cudaError_t e = cudaSuccess;
-    auto acc = [&](cudaError_t x) { if (e == cudaSuccess) e = x; };
-    const int cwc = (h->Nc + 31) / 32;
-    if (!h->infer_only) acc(cudaFuncSetAttribute(mid2_fn_rt(cwc, true, h->gt), A, optin));
-    acc(cudaFuncSetAttribute(mid2_fn_rt(cwc, false, h->gt), A, optin));
-    // cluster form: shared-memory tables, at most 128 hunks, no global side outputs of the entity stage (inline stage or no entity
-    // branch), not variant 4, not the debug dumps
-    h->cl_ok = !h->gt && cwc <= 4 && (h->inl || !h->ent) && !h->edge && !h->debug && env_int("HDGNN_CLUSTER", 1) != 0;
-    if (h->cl_ok) {
-        acc(cudaFuncSetAttribute(mid2_fn_rt(cwc, true, false, true), A, optin));
-        acc(cudaFuncSetAttribute(mid2_fn_rt(cwc, false, false, true), A, optin));
-        if (e == cudaSuccess) {
-            const bool dlt_g = h->dlt_global;
-            const bool sc_t = (h->ent && h->mid_scache) || h->inl, sc_i = h->inl;
-            h->cl_max[1] = mid2_max_clusters(cwc, true, mid2_smem_bytes(h->Ne, h->Nc, true, !dlt_g, sc_t, h->inl, false, false, false));
-            h->cl_max[0] = mid2_max_clusters(cwc, false, mid2_smem_bytes(h->Ne, h->Nc, false, true, sc_i, h->inl, false, false, false));
-            if (h->cl_max[0] <= 0 || h->cl_max[1] <= 0) h->cl_ok = false;
-        }
-    }
-    if (h->ent) {
-        acc(cudaFuncSetAttribute(ent2_fn_rt(h->cwt, false), A, optin));
-        acc(cudaFuncSetAttribute(ent2_fn_rt(h->cwt, true), A, optin));
-        if (e != cudaSuccess) return e;
-        h->fwd_occ = ent2_occupancy(h, false);
-        h->bwd_occ = ent2_occupancy(h, true);
-    }
-    return e;
-}
-
 int env_int(const char* name, int dflt) {
     const char* v = getenv(name);
     return v && *v ? atoi(v) : dflt;
+}
+
+// The form of the fused path for a handle: first, from the shapes and the flags alone, which modes fit one SM's `optin` bytes
+// of shared memory, and how; then the kernels' shared-memory opt-in and their co-residency on `nsm` SMs.  The fused path needs
+// the per-commit state of mid2 in one SM's shared memory and a hunk grid of <= 8 segments (forward only: <= 16).  The twelve
+// hunk-stage tables (12 Nc 20 floats) either sit in shared memory (compiled for Nc <= 160) or in a per-commit slice of global
+// memory (compiled for Nc > 128: mid2_kernel<.., GT>); the placement that admits the inline entity stage wins, shared memory on
+// a tie.
+FusedPlan plan_fused(const hdgnn_config_t& cfg, int optin, int nsm, cudaError_t* err) {
+    const int Ne = cfg.Ne, Nc = cfg.Nc, cwc = (Nc + 31) / 32;
+    const bool ent = cfg.variant == 2 || cfg.variant == 4, edge = cfg.variant == 4;
+    const size_t lim = (size_t)optin;
+    const bool tr = Nc <= 256;      // above 256 hunks only the forward kernel exists (BASELINE config 5: the inference sweep)
+    auto fits = [&](const Mid2Opts& o) { return mid2_smem_bytes(Ne, Nc, o) <= lim; };
+    // mid2 with its hunk-stage tables placed as `gt` says, in the layout it must fit: training, or forward only above 256 hunks.
+    // opt.scache: S also fits beside the rest for the training kernel's backward
+    struct Place { bool fused = false; Mid2Opts opt; };
+    auto place = [&](bool gt) {
+        Place p;
+        if ((cfg.flags & HDGNN_F_LEGACY) || (!tr && edge) || !mid2_gt_supported(cwc, gt)) return p;
+        Mid2Opts& o = p.opt; o.train = tr; o.gt = gt;
+        // per-commit state of mid2 in one SM; the per-pair dL/dlogit table may spill to HBM (L2-resident)
+        o.dlt_smem = !tr || fits(o);
+        p.fused = fits(o);
+        Mid2Opts s = o; s.scache = true;
+        o.scache = ent && p.fused && fits(s);
+        if (p.fused && ent && !(cfg.flags & HDGNN_F_DENSE_SWEEP)) {
+            // entity pair layer inside mid2 (sorted prefix sums + edge walk) when its extra state fits beside mid2's: with the
+            // dL/dlogit table in shared memory, else in HBM, else (global tables only) with the S / GE rows in global memory as
+            // well (Ne = 512 beside Nc = 256)
+            Mid2Opts i = o; i.inl = i.scache = true;
+            Mid2Opts d = i; d.dlt_smem = false;
+            Mid2Opts g = i; g.dlt_smem = !tr; g.scg = true;
+            if (fits(i)) o = i;
+            else if (tr && fits(d)) o = d;
+            else if (gt && fits(g)) o = g;
+        }
+        return p;
+    };
+    const Place ps = place(false), pg = place(true);
+    Place pp = pg.fused && (!ps.fused || (pg.opt.inl && !ps.opt.inl)) ? pg : ps;
+    bool edge_train = false;
+    if (edge && pp.fused) {
+        // variant 4 on the fused path: needs the inline entity stage and room for the edge branch in mid2's union region, with
+        // the dL/dlogit table in HBM if need be
+        Mid2Opts& o = pp.opt; o.edge = o.dlt_smem = true;
+        o.dlt_smem = fits(o);
+        const Mid2Smem L = mid2_layout(Ne, Nc, o);
+        pp.fused = o.inl && mid2_smem_bytes(L) <= lim && mid2_edge_fwd_fits(Ne, L);
+        edge_train = pp.fused && mid2_edge_bwd_fits(Ne, L);
+    }
+    FusedPlan P;
+    P.pdl = !(cfg.flags & HDGNN_F_DEBUG);
+    cudaError_t& e = *err = cudaSuccess;
+    if (!pp.fused) return P;
+    P.gt = pp.opt.gt; P.inl = pp.opt.inl; P.edge = edge;
+    P.dense = ent && !P.inl; P.mid2_first = !P.dense;
+    auto resolve = [&](Mid2Mode& md, bool fused, const Mid2Opts& o) {
+        md.fused = fused; md.opt = mid2_normalize(o); md.lay = mid2_layout(Ne, Nc, md.opt); md.smem = mid2_smem_bytes(md.lay);
+    };
+    Mid2Opts f = pp.opt; f.train = false; f.dlt_smem = true; f.scache = false;
+    Mid2Opts t = pp.opt; t.train = true;
+    resolve(P.mode[0], true, f);
+    resolve(P.mode[1], tr && (!edge || edge_train), t);     // also when not fused (variant 4): its dlt_smem sizes DLT
+
+    const cudaFuncAttribute A = cudaFuncAttributeMaxDynamicSharedMemorySize;
+    auto acc = [&](cudaError_t x) { if (e == cudaSuccess) e = x; };
+    if (P.mode[1].fused) acc(cudaFuncSetAttribute(mid2_fn_rt(cwc, true, P.gt), A, optin));
+    acc(cudaFuncSetAttribute(mid2_fn_rt(cwc, false, P.gt), A, optin));
+    // cluster form: shared-memory tables, at most 128 hunks, no global side outputs of the entity stage, not variant 4, not the
+    // debug dumps
+    if (!P.gt && cwc <= 4 && P.mid2_first && !P.edge && !(cfg.flags & HDGNN_F_DEBUG) && env_int("HDGNN_CLUSTER", 1) != 0) {
+        acc(cudaFuncSetAttribute(mid2_fn_rt(cwc, true, false, true), A, optin));
+        acc(cudaFuncSetAttribute(mid2_fn_rt(cwc, false, false, true), A, optin));
+        if (e == cudaSuccess) {
+            const int ct = mid2_max_clusters(cwc, true, P.mode[1].smem), cf = mid2_max_clusters(cwc, false, P.mode[0].smem);
+            if (ct > 0 && cf > 0) { P.mode[1].clusters = ct; P.mode[0].clusters = cf; }
+        }
+    }
+    // the occupancy of the sweeps also sizes CS1P and GPE, so it is taken for the inline entity stage as well
+    if (ent) {
+        const int cwt = ent2_cwt(Ne);
+        acc(cudaFuncSetAttribute(ent2_fn_rt(cwt, false), A, optin));
+        acc(cudaFuncSetAttribute(ent2_fn_rt(cwt, true), A, optin));
+        if (e != cudaSuccess) return P;
+        P.fwd_occ = ent2_occupancy(cfg, nsm, false); P.bwd_occ = ent2_occupancy(cfg, nsm, true);
+    }
+    return P;
 }
 
 int pick_rt(int N, int B, int requested) {
@@ -810,88 +867,29 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
     h->nsm = prop.multiProcessorCount;
     h->WPe = bit_words(h->Ne); h->WPc = bit_words(h->Nc);
     h->cwt = ent2_cwt(h->Ne);
-    h->pdl = !h->debug;
-    // the fused path needs the per-commit state of mid2 in one SM's shared memory and a hunk grid of <= 8 segments.  The twelve
-    // hunk-stage tables (12 Nc 20 floats) either sit in shared memory (compiled for Nc <= 160) or in a per-commit slice of global
-    // memory (compiled for Nc > 128: mid2_kernel<.., GT>); the placement that admits the inline entity stage wins, shared memory
-    // on a tie
-    {
-        const size_t lim = (size_t)prop.sharedMemPerBlockOptin;
-        const int cwc = (h->Nc + 31) / 32;
-        const bool want_inl = h->ent && !(cfg->flags & HDGNN_F_DENSE_SWEEP);
-        struct Plan { bool fused = false, dlt_global = false, scache = false, inl = false, scg = false; };
-        // above 256 hunks only the forward kernel exists (BASELINE config 5: the inference sweep to Nc = 512); variants 1-3
-        const bool fwd_only = h->Nc > 256;
-        const bool tr = !fwd_only;                  // the layout the plan must fit: training, or forward only
-        auto plan = [&](bool gt) {
-            Plan p;
-            if ((cfg->flags & HDGNN_F_LEGACY) || (fwd_only && cfg->variant == 4) || !mid2_gt_supported(cwc, gt)) return p;
-            // per-commit state of mid2 in one SM; the per-pair dL/dlogit table may spill to HBM (L2-resident)
-            p.dlt_global = tr && mid2_smem_bytes(h->Ne, h->Nc, tr, true, false, false, false, gt) > lim;
-            p.fused = mid2_smem_bytes(h->Ne, h->Nc, tr, !p.dlt_global, false, false, false, gt) <= lim;
-            p.scache = p.fused && mid2_smem_bytes(h->Ne, h->Nc, tr, !p.dlt_global, true, false, false, gt) <= lim;
-            if (p.fused && want_inl) {
-                // entity pair layer inside mid2 (sorted prefix sums + edge walk) when its extra state fits beside mid2's
-                if (mid2_smem_bytes(h->Ne, h->Nc, tr, true, true, true, false, gt) <= lim) { p.inl = true; p.dlt_global = false; }
-                else if (tr && mid2_smem_bytes(h->Ne, h->Nc, tr, false, true, true, false, gt) <= lim) { p.inl = true; p.dlt_global = true; }
-                // ... or (global tables only) with the S / GE rows in global memory as well: Ne = 512 beside Nc = 256
-                else if (gt && mid2_smem_bytes(h->Ne, h->Nc, tr, false, true, true, false, gt, true) <= lim) { p.inl = true; p.dlt_global = tr; p.scg = true; }
-                if (p.inl) p.scache = true;
-            }
-            return p;
-        };
-        h->infer_only = fwd_only;
-        const Plan ps = plan(false), pg = plan(env_int("HDGNN_GT", 1) != 0);
-        const bool use_gt = env_int("HDGNN_GT", 1) == 2 ? pg.fused : (pg.fused && (!ps.fused || (pg.inl && !ps.inl)));
-        const Plan& pp = use_gt ? pg : ps;
-        h->gt = use_gt; h->fused = pp.fused; h->dlt_global = pp.dlt_global; h->mid_scache = pp.scache; h->inl = pp.inl; h->scg = pp.scg;
-    }
-    if (h->edge) {
-        // variant 4 on the fused path: needs the inline entity stage, the soft-edge head tables (Ne x 60 floats + a 128-row
-        // staging tile) and the edge branch's pair sums (2 Ne x 20) side by side in mid2's union region
-        bool ok = h->fused && h->inl;
-        if (ok) {
-            const size_t lim = (size_t)prop.sharedMemPerBlockOptin;
-            h->dlt_global = mid2_smem_bytes(h->Ne, h->Nc, true, true, true, true, true, h->gt, h->scg) > lim;
-            const Mid2Smem L = mid2_layout(h->Ne, h->Nc, true, !h->dlt_global, true, true, true, h->gt, h->scg);
-            ok = (size_t)L.total * 4 + 16 <= lim && h->Ne * 60 + (M2_T / KG) * HD <= (L.sc - L.uni) - 2 * h->Ne * HD;
-        }
-        h->edge_fused = ok;
-        bool okt = ok;
-        if (okt) {      // backward: head tables + column delta sums + a 32-row de tile; later five Ne x 20 arrays + GCe at the end;
-                        // the general-attribute form of ent_bwd needs two sets of suffix tables beside GCe
-            const Mid2Smem L = mid2_layout(h->Ne, h->Nc, true, !h->dlt_global, true, true, true, h->gt, h->scg);
-            const int uf = L.sc - L.uni, wue = (h->Ne + 31) / 32;
-            okt = h->Ne * 80 + 32 * wue * 32 <= uf && h->Ne * 120 <= uf && 40 * (h->Ne + 1) + 8 * M2_T + h->Ne * HD <= uf;
-        }
-        h->edge_fused_train = okt;
-        if (!ok) { h->fused = false; h->inl = false; }
-    }
+    cudaError_t e;
+    h->plan = plan_fused(*cfg, (int)prop.sharedMemPerBlockOptin, h->nsm, &e);
+    const FusedPlan& P = h->plan;
     h->host_bits = (cfg->flags & HDGNN_F_LABEL_BITS) != 0;
-    if (h->host_bits && !fused_for(h, true)) {
+    if (h->host_bits && !P.mode[1].fused) {
         delete h;
         return fail(nullptr, HDGNN_E_UNSUPPORTED, "HDGNN_F_LABEL_BITS needs the fused training path (Nc <= 256, per-commit state within one SM)");
     }
-    cudaError_t e = set_attrs(h, (int)prop.sharedMemPerBlockOptin);
-    if (e == cudaSuccess && h->fused) e = setup_fused(h, (int)prop.sharedMemPerBlockOptin);
+    if (e == cudaSuccess) e = set_attrs(h, (int)prop.sharedMemPerBlockOptin);
     if (e != cudaSuccess) {
         std::string m = std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(e);
         delete h;
         return fail(nullptr, HDGNN_E_CUDA, m);
     }
-    int Gf_max = 0, Gb_max = 0, Rtmp = 0;
-    if (h->fused && h->ent) {
-        ent2_grid(h, cfg->max_batch, h->fwd_occ, &Gf_max, &Rtmp);
-        ent2_grid(h, cfg->max_batch, h->bwd_occ, &Gb_max, &Rtmp);
-        Gf_max = h->fwd_occ * h->nsm; Gb_max = h->bwd_occ * h->nsm;
-    }
+    const bool fused = P.mode[0].fused;       // the forward is fused whenever the training step is
+    const int Gf_max = fused && h->ent ? P.fwd_occ * h->nsm : 0, Gb_max = fused && h->ent ? P.bwd_occ * h->nsm : 0;
 
     const size_t B = cfg->max_batch, Ne = h->Ne, Nc = h->Nc, Se = h->Se, Sc = h->Sc, f = sizeof(float);
     // (B, SL, Ne, 20) column partials of ent_fwd2: B * SL <= grid + 2 B for every batch size <= max_batch
     const size_t cs1p_f = ((size_t)Gf_max + 2 * B + 2) * Ne * HD * f, cs1p_l = B * Se * Ne * HD * f;
-    const bool mixed = h->fused && !fused_for(h, true);        // variant 4: fused forward, multi-kernel training
-    const size_t cs1p = !h->fused ? cs1p_l : (mixed && cs1p_l > cs1p_f ? cs1p_l : cs1p_f);
-    const bool lg = !fused_for(h, true) || !fused_for(h, false);     // buffers only the multi-kernel path needs (kept when debugging: dump targets)
+    const bool mixed = fused && !P.mode[1].fused;        // variant 4: fused forward, multi-kernel training
+    const size_t cs1p = !fused ? cs1p_l : (mixed && cs1p_l > cs1p_f ? cs1p_l : cs1p_f);
+    const bool lg = !P.mode[1].fused;     // buffers only the multi-kernel path needs (kept when debugging: dump targets)
     const bool dbgbuf = lg || h->debug;
     struct { const char* n; size_t bytes; bool need; } plan[] = {
         {"RS1", B * Ne * HD * f, h->ent}, {"CS1P", cs1p, h->ent}, {"S1", B * Ne * HD * f, dbgbuf},
@@ -905,15 +903,15 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
         {"DNB", B * Nc * 4 * f, dbgbuf}, {"GE", B * Ne * HD * f, true}, {"DX2", B * Ne * f, dbgbuf},
         {"RS1D", B * Ne * HD * f, h->ent && lg}, {"CS1DP", B * Se * Ne * HD * f, h->ent && lg}, {"LS1P", B * Se * HD * f, h->ent && lg},
         {"GPART", 2 * B * (size_t)h->po.total * f, true},       // second half: spare rows of the cluster form (mid2.cuh)
-        {"GPE", ((size_t)Gb_max + 1) * 4 * HD * f, h->fused && h->ent}, {"FIN_L2", 256 * f, h->fused}, {"FIN_CNT", 16, h->fused},
-        {"EBITS0", B * Ne * (size_t)h->WPe * 4, h->fused}, {"YBITS0", B * Nc * (size_t)h->WPc * 4, h->fused},
-        {"EBITS1", B * Ne * (size_t)h->WPe * 4, h->fused}, {"YBITS1", B * Nc * (size_t)h->WPc * 4, h->fused},
-        {"DBG", B * mid2_dbg_floats(h->Ne, h->Nc) * f, h->fused && h->debug},
-        {"CLK", B * 24 * sizeof(long long), h->fused && h->debug},
-        {"DLT", B * Nc * (size_t)((h->Nc + 31) / 32 * 32) * f, h->fused && h->dlt_global},
-        {"TABS", B * (size_t)mid2_tab_floats(h->Nc) * f, h->fused && h->gt},
-        {"RSEG", B * Ne * HD * f, h->edge_fused}, {"CSEG", B * Ne * HD * f, h->edge_fused}, {"REG", B * Ne * HD * f, h->edge_fused},
-        {"CEG", B * Ne * HD * f, h->edge_fused}, {"A1F", B * Ne * (Ne - 1) * f, h->edge_fused}, {"PREG", B * Ne * 60 * f, h->edge_fused},
+        {"GPE", ((size_t)Gb_max + 1) * 4 * HD * f, fused && h->ent}, {"FIN_L2", 256 * f, fused}, {"FIN_CNT", 16, fused},
+        {"EBITS0", B * Ne * (size_t)h->WPe * 4, fused}, {"YBITS0", B * Nc * (size_t)h->WPc * 4, fused},
+        {"EBITS1", B * Ne * (size_t)h->WPe * 4, fused}, {"YBITS1", B * Nc * (size_t)h->WPc * 4, fused},
+        {"DBG", B * mid2_dbg_floats(h->Ne, h->Nc) * f, fused && h->debug},
+        {"CLK", B * 24 * sizeof(long long), fused && h->debug},
+        {"DLT", B * Nc * (size_t)((h->Nc + 31) / 32 * 32) * f, fused && !P.mode[1].opt.dlt_smem},
+        {"TABS", B * (size_t)mid2_tab_floats(h->Nc) * f, fused && P.gt},
+        {"RSEG", B * Ne * HD * f, P.edge}, {"CSEG", B * Ne * HD * f, P.edge}, {"REG", B * Ne * HD * f, P.edge},
+        {"CEG", B * Ne * HD * f, P.edge}, {"A1F", B * Ne * (Ne - 1) * f, P.edge}, {"PREG", B * Ne * 60 * f, P.edge},
         {"RSE", B * Ne * HD * f, h->edge}, {"CSEP", B * Se * Ne * HD * f, h->edge}, {"CSEF", B * Ne * HD * f, h->edge},
         {"PRE", B * Ne * HD * f, h->edge}, {"PCE", B * Ne * HD * f, h->edge},
         {"SOFT", B * Ne * Ne * 2 * f, h->edge}, {"DSOFT", B * Ne * Ne * 2 * f, h->edge},
@@ -982,7 +980,7 @@ static void peer_layout(int world, int total, int* stride, int* ncta, size_t* of
 int hdgnn_peer_export(hdgnn_handle_t h, int world, unsigned char* ipc_handle_out) {
     if (!h) return HDGNN_E_INVALID;
     if (world < 2 || world > PEER_MAX || !ipc_handle_out) return fail(h, HDGNN_E_INVALID, "world must be 2..8");
-    if (!fused_for(h, true)) return fail(h, HDGNN_E_UNSUPPORTED, "the peer exchange is fused into the reduce+Adam kernel of the fused path (Nc <= 256, per-commit state within one SM)");
+    if (!h->plan.mode[1].fused) return fail(h, HDGNN_E_UNSUPPORTED, "the peer exchange is fused into the reduce+Adam kernel of the fused path (Nc <= 256, per-commit state within one SM)");
     static_assert(sizeof(cudaIpcMemHandle_t) == HDGNN_IPC_HANDLE_BYTES, "IPC handle size");
     CK(h, cudaSetDevice(h->cfg.device));
     if (h->peer_box) return fail(h, HDGNN_E_INVALID, "hdgnn_peer_export was already called on this handle");
@@ -1040,14 +1038,14 @@ int hdgnn_peer_attach(hdgnn_handle_t h, int rank, int world, const unsigned char
 
 int hdgnn_set_hits_accumulator(hdgnn_handle_t h, uint64_t* acc) {
     if (!h) return HDGNN_E_INVALID;
-    if (acc && !fused_for(h, true)) return fail(h, HDGNN_E_UNSUPPORTED, "the hit counter lives in the fused per-commit kernel (Nc <= 256, per-commit state within one SM); use hdgnn_eval_counts");
+    if (acc && !h->plan.mode[1].fused) return fail(h, HDGNN_E_UNSUPPORTED, "the hit counter lives in the fused per-commit kernel (Nc <= 256, per-commit state within one SM); use hdgnn_eval_counts");
     h->hits_acc = (unsigned long long*)acc;
     return HDGNN_OK;
 }
 
 int hdgnn_set_eval_counters(hdgnn_handle_t h, int64_t* counts) {
     if (!h) return HDGNN_E_INVALID;
-    if (counts && !fused_for(h, false)) return fail(h, HDGNN_E_UNSUPPORTED, "the evaluation counters live in the fused per-commit kernel; use hdgnn_eval_counts");
+    if (counts && !h->plan.mode[0].fused) return fail(h, HDGNN_E_UNSUPPORTED, "the evaluation counters live in the fused per-commit kernel; use hdgnn_eval_counts");
     if ((uintptr_t)counts & 7) return fail(h, HDGNN_E_INVALID, "counts must be 8-byte aligned");
     h->evc = (unsigned long long*)counts;
     return HDGNN_OK;
@@ -1068,7 +1066,7 @@ static int run_step(hdgnn_handle_t h, int B, int B_global, const Inputs& in, flo
                     float* grads, const AdamArgs* adam, cudaStream_t st) {
     const bool train = grads != nullptr;
     int rc;
-    if (fused_for(h, train)) {
+    if (h->plan.mode[train].fused) {
         rc = fused_forward(h, B, B_global, in, logits, probs, train, st);
         if (rc) return rc;
 
@@ -1208,7 +1206,7 @@ static int stage_inputs(hdgnn_handle_t h, int B, const uint8_t* adj_host, const 
     }
     h->cur_tag = -1;
     if (side) {
-        if (h->tag_table && h->host_bits && h->fused && (h->inl || !h->ent)) {
+        if (h->tag_table && h->host_bits && h->plan.mid2_first) {
             // mid2 is the first kernel of the step and reads every staged input: order it by a tag instead of an event
             const int tag = (int)(++h->slot_uses[slot] & 0xffu);
             CK(h, cudaMemcpyAsync((int*)h->ws["H_FLAG"].p + slot, h->tag_table + tag, sizeof(int), cudaMemcpyHostToDevice, cs));
@@ -1282,7 +1280,7 @@ static int host_step(hdgnn_handle_t h, int B, int B_global, const uint8_t* adj_h
     if (rc) return rc;
     const Inputs in = staged_inputs(h, params);
     float* probs_d = to_host && probs ? F(h, "H_PROBS") : probs;
-    float* alias = to_host && adam && fused_for(h, true) ? host_alias(loss) : nullptr;
+    float* alias = to_host && adam && h->plan.mode[1].fused ? host_alias(loss) : nullptr;
     float* loss_d = to_host ? (alias ? alias : F(h, "H_LOSS")) : loss;
     AdamArgs ad{};
     if (adam) { ad = *adam; ad.reg = loss_d + 1; }

@@ -58,14 +58,30 @@ struct Mid2Smem {
     int stg;                                 // (GT kernels) staging region of the hunk sweeps' row tables (3 Nc 20 floats), behind the dlt table
 };
 
-// dlt_smem: keep the per-pair dL/dlogit table of the training path in shared memory (else it lives in HBM / L2)
-// gt: the twelve hunk-stage tables live in global memory (per-commit scratch, L1/L2-resident) -- the form for hunk grids whose
-//     tables do not fit one SM beside the rest of the commit's state (Nc > 128)
-__host__ __device__ inline Mid2Smem mid2_layout(int Ne, int Nc, bool train, bool dlt_smem = true, bool scache = false, bool inl = false, bool edge = false,
-                                                bool gt = false, bool scg = false) {
+// what a mid2 launch keeps where; mid2_layout turns it into offsets
+struct Mid2Opts {
+    bool train = false;      // the training kernel (forward + backward)
+    bool dlt_smem = true;    // the per-pair dL/dlogit table of the training path in shared memory (else it lives in HBM / L2)
+    bool scache = false;     // the entity effect sums S (Ne x 20) in shared memory from the forward to the backward
+    bool inl = false;        // entity pair layer inside mid2 (entsp.cuh); implies scache
+    bool edge = false;       // variant 4: the entity-edge branch inside mid2 as well
+    bool gt = false;         // the twelve hunk-stage tables in global memory (per-commit scratch, L1/L2-resident) -- the form
+                             // for hunk grids whose tables do not fit one SM beside the rest of the commit's state (Nc > 128)
+    bool scg = false;        // ... and the S / GE rows in global memory as well; only with gt
+};
+
+// the options as mid2 runs with them: every layout and every kernel flag derives from these
+__host__ __device__ inline Mid2Opts mid2_normalize(Mid2Opts o) {
+    if (o.inl) o.scache = true;
+    if (!o.gt) o.scg = false;
+    return o;
+}
+
+__host__ __device__ inline Mid2Smem mid2_layout(int Ne, int Nc, Mid2Opts opt) {
+    const Mid2Opts no = mid2_normalize(opt);
+    const bool train = no.train, dlt_smem = no.dlt_smem, scache = no.scache, inl = no.inl, edge = no.edge, gt = no.gt;
     Mid2Smem m;
-    m.gt = gt ? 1 : 0; m.scg = (gt && scg) ? 1 : 0;
-    if (inl) scache = true;
+    m.gt = gt ? 1 : 0; m.scg = no.scg ? 1 : 0;
     int o = 0;
     auto take = [&](int n) { int r = o; o += (n + 7) & ~7; return r; };      // 32-byte granules
     m.blk1 = take(M2_BLK1); m.blk2 = take(M2_BLK2); m.gam = take(20); m.Dh = take(20); m.Dg = take(20); m.G1g = take(400);
@@ -114,9 +130,19 @@ __host__ __device__ inline Mid2Smem mid2_layout(int Ne, int Nc, bool train, bool
     m.total = o;
     return m;
 }
-__host__ __device__ inline size_t mid2_smem_bytes(int Ne, int Nc, bool train, bool dlt_smem = true, bool scache = false, bool inl = false, bool edge = false,
-                                                  bool gt = false, bool scg = false) {
-    return (size_t)mid2_layout(Ne, Nc, train, dlt_smem, scache, inl, edge, gt, scg).total * 4 + 16;
+__host__ __device__ inline size_t mid2_smem_bytes(const Mid2Smem& m) { return (size_t)m.total * 4 + 16; }
+__host__ __device__ inline size_t mid2_smem_bytes(int Ne, int Nc, const Mid2Opts& o) { return mid2_smem_bytes(mid2_layout(Ne, Nc, o)); }
+
+// Variant 4 (layout m with Mid2Opts::edge): the forward of the entity-edge branch keeps the soft-edge head tables (Ne x 60 floats
+// + a 128-row staging tile) and the edge branch's pair sums (2 Ne x 20) side by side in the union region
+__host__ __device__ inline bool mid2_edge_fwd_fits(int Ne, const Mid2Smem& m) {
+    return Ne * 60 + (M2_T / KG) * HD <= (m.sc - m.uni) - 2 * Ne * HD;
+}
+// ... its backward needs the head tables + column delta sums + a 32-row de tile; later five Ne x 20 arrays + GCe at the end; the
+// general-attribute form of ent_bwd needs two sets of suffix tables beside GCe
+__host__ __device__ inline bool mid2_edge_bwd_fits(int Ne, const Mid2Smem& m) {
+    const int uf = m.sc - m.uni, wue = (Ne + 31) / 32;
+    return Ne * 80 + 32 * wue * 32 <= uf && Ne * 120 <= uf && 40 * (Ne + 1) + 8 * M2_T + Ne * HD <= uf;
 }
 
 struct Mid2Args {
