@@ -13,12 +13,17 @@
 // 1-D TMA bulk copy; the degree scan runs while the tile is resident and packs the rows into bitmaps, the
 // bitmap is transposed with ballots when the reference's A^T form is asked for, and the propagation walks the
 // set bits (lanes = output channels).  HBM traffic = the adjacency bytes once + H in + out.
+//
+// Every kernel takes the adjacency in either format (template parameter BITS): byte grids, or with
+// HDGNN_P_LABEL_BITS the label bitmaps of HDGNN_F_LABEL_BITS (bits.cuh; pitch = 4 * bit_words(N) bytes).  Only the
+// stage that turns the staged tile into edge bits and degrees differs; diagonal and padding bits are masked there,
+// as the byte stage ignores the diagonal byte and the padding columns.
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
 #include <stdint.h>
 
 #include "../../include/hdgnn.h"
-#include "common.cuh"
+#include "bits.cuh"
 
 namespace hdgnn {
 
@@ -36,7 +41,7 @@ struct ConvArgs {
 __host__ __device__ inline int conv_words(int N) { return (N + 31) / 32; }
 __host__ __device__ inline size_t conv_smem_bytes(int N, int pitch, int d_out) {
     const int WP = conv_words(N), NP = WP * 32;
-    size_t off = 16 + (size_t)round_up(N * pitch, 128);     // mbarrier, byte tile
+    size_t off = 16 + (size_t)round_up(N * pitch, 128);     // mbarrier, staged tile
     off += (size_t)2 * NP * WP * 4;                          // row bitmap, column bitmap (padded to 32 rows)
     off += (size_t)N * 4;                                    // dinv
     off += (size_t)N * (d_out > 0 ? d_out : 1) * 4;          // Hs (or x scaled)
@@ -67,24 +72,43 @@ __device__ __forceinline__ ConvSmem conv_carve(unsigned char* smem, int N, int p
     return s;
 }
 
+// Word sg of row j of the edge bitmap (bit l = column 32 sg + l) from a label-bitmap tile (row stride bit_words(N)
+// words): the diagonal and the columns >= N cleared, 0 for the padding rows j >= N.
+__device__ __forceinline__ uint32_t bits_row_word(const uint8_t* tile, int j, int N, int pitch, int sg) {
+    if (j >= N) return 0u;
+    uint32_t w = reinterpret_cast<const uint32_t*>(tile + (size_t)j * pitch)[sg];
+    const int c0 = sg * 32;
+    if (c0 + 32 > N) w &= (c0 >= N) ? 0u : (0xffffffffu >> (c0 + 32 - N));
+    if ((j >> 5) == sg) w &= ~(1u << (j & 31));
+    return w;
+}
+
+template <bool BITS>
 __device__ __forceinline__ void conv_degree_scan(const ConvSmem& s, int N, int pitch, bool self_loop, float eps, bool transpose) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, WP = conv_words(N), NP = WP * 32;
-    // rows: 32 lanes x 16 bytes cover 512 columns; one row per warp iteration
+    // rows: 32 lanes x 16 bytes cover 512 columns (a bitmap row: lane = word); one row per warp iteration
     for (int j = warp; j < NP; j += CONV_T / 32) {
-        uint32_t m = 0u;
-        if (j < N && lane * 16 < pitch) {
-            const uint4 v = *reinterpret_cast<const uint4*>(s.tile + (size_t)j * pitch + lane * 16);
-            m = nz4(v.x) | (nz4(v.y) << 4) | (nz4(v.z) << 8) | (nz4(v.w) << 12);
-        }
-        const uint32_t hi = __shfl_down_sync(0xffffffffu, m, 1);
         uint32_t w = 0u;
-        const int sg = lane >> 1;
-        if ((lane & 1) == 0 && sg < WP) {
-            w = m | (hi << 16);
-            const int c0 = sg * 32;
-            if (c0 + 32 > N) w &= (c0 >= N) ? 0u : (0xffffffffu >> (c0 + 32 - N));
-            if ((j >> 5) == sg) w &= ~(1u << (j & 31));
-            s.rbits[(size_t)j * WP + sg] = w;
+        if constexpr (BITS) {
+            if (lane < WP) {
+                w = bits_row_word(s.tile, j, N, pitch, lane);
+                s.rbits[(size_t)j * WP + lane] = w;
+            }
+        } else {
+            uint32_t m = 0u;
+            if (j < N && lane * 16 < pitch) {
+                const uint4 v = *reinterpret_cast<const uint4*>(s.tile + (size_t)j * pitch + lane * 16);
+                m = nz4(v.x) | (nz4(v.y) << 4) | (nz4(v.z) << 8) | (nz4(v.w) << 12);
+            }
+            const uint32_t hi = __shfl_down_sync(0xffffffffu, m, 1);
+            const int sg = lane >> 1;
+            if ((lane & 1) == 0 && sg < WP) {
+                w = m | (hi << 16);
+                const int c0 = sg * 32;
+                if (c0 + 32 > N) w &= (c0 >= N) ? 0u : (0xffffffffu >> (c0 + 32 - N));
+                if ((j >> 5) == sg) w &= ~(1u << (j & 31));
+                s.rbits[(size_t)j * WP + sg] = w;
+            }
         }
         const int deg = __reduce_add_sync(0xffffffffu, __popc(w));
         if (lane == 0 && j < N) s.dinv[j] = 1.f / sqrtf((float)deg + (self_loop ? 1.f : 0.f) + eps);
@@ -107,6 +131,7 @@ __device__ __forceinline__ void conv_degree_scan(const ConvSmem& s, int N, int p
     }
 }
 
+template <bool BITS>
 __global__ void __launch_bounds__(CONV_T) propagate_kernel(const ConvArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     const int N = a.N, pitch = a.pitch, b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -132,7 +157,7 @@ __global__ void __launch_bounds__(CONV_T) propagate_kernel(const ConvArgs a) {
     mbar_wait(s.bar, 0);
     __syncthreads();
     const bool self_loop = a.flags & HDGNN_P_SELF_LOOP, transpose = !(a.flags & HDGNN_P_NO_TRANSPOSE);
-    conv_degree_scan(s, N, pitch, self_loop, a.eps, transpose);
+    conv_degree_scan<BITS>(s, N, pitch, self_loop, a.eps, transpose);
     for (int idx = tid; idx < N * d_out; idx += CONV_T) s.Hs[idx] *= s.dinv[idx / d_out];
     if (a.dinv_out) for (int j = tid; j < N; j += CONV_T) a.dinv_out[(size_t)b * N + j] = s.dinv[j];
     __syncthreads();
@@ -171,7 +196,7 @@ __host__ __device__ inline int tc_mp(int N) { return N <= 128 ? 128 : 256; }
 __host__ __device__ inline size_t tc_smem_bytes(int N, int pitch, int d_in, int d_out) {
     const int WP = conv_words(N), NP32 = WP * 32, KP = round_up(N, 16);
     const size_t tile = (size_t)round_up(N * pitch, 128), sa = (size_t)tc_mp(N) * KP * 2;
-    size_t off = 32 + (tile > sa ? tile : sa);                 // mbarrier + tmem slot | byte tile, later the A operand
+    size_t off = 32 + (tile > sa ? tile : sa);                 // mbarrier + tmem slot | staged tile, later the A operand
     off += (size_t)tc_np(d_out) * KP * 2;                      // B operand
     off += (size_t)NP32 * WP * 4;                              // row bitmap
     off += (size_t)round_up(N, 4) * 4 + (size_t)round_up(N * d_out, 4) * 4;     // dinv, Hs
@@ -190,6 +215,7 @@ __device__ __forceinline__ uint32_t umma_idesc(int M, int N) {
     return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
+template <bool BITS>
 __global__ void __launch_bounds__(TC_T, 1) propagate_tc_kernel(const ConvArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     const int N = a.N, pitch = a.pitch, b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -199,7 +225,7 @@ __global__ void __launch_bounds__(TC_T, 1) propagate_tc_kernel(const ConvArgs a)
     uint64_t* bar_mma = bar_tma + 1;
     uint32_t* tslot = reinterpret_cast<uint32_t*>(bar_tma + 2);
     uint8_t* tile = smem + 32;
-    __nv_bfloat16* sA = reinterpret_cast<__nv_bfloat16*>(smem + 32);                    // aliases the byte tile
+    __nv_bfloat16* sA = reinterpret_cast<__nv_bfloat16*>(smem + 32);                    // aliases the staged tile
     const size_t tile_b = (size_t)round_up(N * pitch, 128), sa_b = (size_t)MP * KP * 2;
     __nv_bfloat16* sB = reinterpret_cast<__nv_bfloat16*>(smem + 32 + (tile_b > sa_b ? tile_b : sa_b));
     uint32_t* rbits = reinterpret_cast<uint32_t*>(sB + (size_t)NPc * KP);
@@ -241,27 +267,34 @@ __global__ void __launch_bounds__(TC_T, 1) propagate_tc_kernel(const ConvArgs a)
         Hs[idx] = acc;
     }
     const bool self_loop = a.flags & HDGNN_P_SELF_LOOP, transpose = !(a.flags & HDGNN_P_NO_TRANSPOSE);
-    // degree scan + row bitmap while the byte tile is resident (same as conv_degree_scan, no transpose needed)
+    // degree scan + row bitmap while the tile is resident (same as conv_degree_scan, no transpose needed)
     for (int j = warp; j < NP32; j += TC_T / 32) {
-        uint32_t m = 0u;
-        if (j < N && lane * 16 < pitch) {
-            const uint4 v = *reinterpret_cast<const uint4*>(tile + (size_t)j * pitch + lane * 16);
-            m = nz4(v.x) | (nz4(v.y) << 4) | (nz4(v.z) << 8) | (nz4(v.w) << 12);
-        }
-        const uint32_t hi = __shfl_down_sync(0xffffffffu, m, 1);
         uint32_t w = 0u;
-        const int sg = lane >> 1;
-        if ((lane & 1) == 0 && sg < WP) {
-            w = m | (hi << 16);
-            const int c0 = sg * 32;
-            if (c0 + 32 > N) w &= (c0 >= N) ? 0u : (0xffffffffu >> (c0 + 32 - N));
-            if ((j >> 5) == sg) w &= ~(1u << (j & 31));
-            rbits[(size_t)j * WP + sg] = w;
+        if constexpr (BITS) {
+            if (lane < WP) {
+                w = bits_row_word(tile, j, N, pitch, lane);
+                rbits[(size_t)j * WP + lane] = w;
+            }
+        } else {
+            uint32_t m = 0u;
+            if (j < N && lane * 16 < pitch) {
+                const uint4 v = *reinterpret_cast<const uint4*>(tile + (size_t)j * pitch + lane * 16);
+                m = nz4(v.x) | (nz4(v.y) << 4) | (nz4(v.z) << 8) | (nz4(v.w) << 12);
+            }
+            const uint32_t hi = __shfl_down_sync(0xffffffffu, m, 1);
+            const int sg = lane >> 1;
+            if ((lane & 1) == 0 && sg < WP) {
+                w = m | (hi << 16);
+                const int c0 = sg * 32;
+                if (c0 + 32 > N) w &= (c0 >= N) ? 0u : (0xffffffffu >> (c0 + 32 - N));
+                if ((j >> 5) == sg) w &= ~(1u << (j & 31));
+                rbits[(size_t)j * WP + sg] = w;
+            }
         }
         const int deg = __reduce_add_sync(0xffffffffu, __popc(w));
         if (lane == 0 && j < N) dinv[j] = 1.f / sqrtf((float)deg + (self_loop ? 1.f : 0.f) + a.eps);
     }
-    __syncthreads();                    // the byte tile is dead from here on: sA overwrites it
+    __syncthreads();                    // the staged tile is dead from here on: sA overwrites it
     if (a.dinv_out) for (int j = tid; j < N; j += TC_T) a.dinv_out[(size_t)b * N + j] = dinv[j];
     // A operand: A_mma[m = i][k = j] = adj[j][i] (reference form) or adj[i][j]; + I with the self loop; zero padding
     const uint32_t one = 0x3F80u;       // bf16 1.0
@@ -362,9 +395,10 @@ __global__ void __launch_bounds__(TC_T, 1) propagate_tc_kernel(const ConvArgs a)
 // canonical no-swizzle layouts only differ in which of LBO / SBO strides over which index:
 //   reference form  out_i = sum_j adj[j][i] z_j : k = r, n = 8 c8 + u  -> MN-major B (SBO = KP * 16 B, LBO = 128 B)
 //   un-transposed   out_i = sum_j adj[i][j] z_j : n = r, k = 8 c8 + u  -> K-major  B (LBO = KP * 16 B, SBO = 128 B)
-// so there is no bit transpose at all; the row degrees fall out of the same pass over the bytes.  A CTA is persistent
-// over commits: as soon as a byte tile has been converted the TMA for the CTA's next commit is issued into the same
-// buffer and lands while the operands are finished, the MMA chain runs and the epilogue drains TMEM.
+// so there is no bit transpose at all; the row degrees fall out of the same pass over the bytes.  From a label bitmap the
+// 8-column edge mask of a chunk is simply byte c8 of the row's bitmap.  A CTA is persistent over commits: as soon as a
+// tile has been converted the TMA for the CTA's next commit is issued into the same buffer and lands while the operands
+// are finished, the MMA chain runs and the epilogue drains TMEM.
 constexpr int TC2_T = 512;
 // four bytes -> four bits (bit i = byte i != 0): bytes to 0/1, then one multiply gathers them into the top nibble
 __device__ __forceinline__ uint32_t nzn(uint32_t v) {
@@ -378,7 +412,7 @@ __host__ __device__ inline size_t tc2_adj_bytes(int KP) {
 __host__ __device__ inline size_t tc2_smem_bytes(int N, int pitch, int d_in) {
     const int KP = round_up(N, 16), K8 = KP / 8, KS = KP + 1;   // KS: chunk stride per c8 (odd: conflict-free 16-byte stores)
     size_t off = 256;                                           // two mbarriers + TMEM slot, nibble table
-    off += (size_t)round_up(N * pitch, 128);                    // byte tile (TMA destination)
+    off += (size_t)round_up(N * pitch, 128);                    // staged tile (TMA destination)
     off += tc2_adj_bytes(KP);                                   // adjacency chunks [c8][r] | epilogue staging [3][KP][32] f32
     off += (size_t)K8 * 128 * 16;                               // feature chunks   [k8][m], m = 4 c + term
     off += (size_t)round_up(N * d_in, 4) * 4;                   // H tile (TMA destination)
@@ -388,6 +422,7 @@ __host__ __device__ inline size_t tc2_smem_bytes(int N, int pitch, int d_in) {
     return off + 128;
 }
 
+template <bool BITS>
 __global__ void __launch_bounds__(TC2_T, 1) propagate_tc2_kernel(const ConvArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     const int N = a.N, pitch = a.pitch, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -438,22 +473,27 @@ __global__ void __launch_bounds__(TC2_T, 1) propagate_tc2_kernel(const ConvArgs 
     uint32_t ph = 0;
     for (; b < a.B; b += gridDim.x, ph ^= 1u) {
         mbar_wait(bar_tma, ph);
-        // bytes -> bf16 chunks + row degrees: a warp takes four rows at a time (all loads first), a lane per 8 columns
+        // tile -> bf16 chunks + row degrees: a warp takes four rows at a time (all loads first), a lane per 8 columns
+        // (8 bytes of a byte row, or byte `lane` of a bitmap row)
         for (int r0 = warp; r0 < KP; r0 += 4 * (TC2_T / 32)) {
             uint32_t lo[4], hi[4];
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
                 const int r = r0 + q * (TC2_T / 32);
                 lo[q] = 0u; hi[q] = 0u;
-                if (lane < K8 && r < N && lane * 8 < pitch) {
-                    const uint2 v = *reinterpret_cast<const uint2*>(tile + (size_t)r * pitch + lane * 8);
-                    lo[q] = v.x; hi[q] = v.y;
+                if constexpr (BITS) {
+                    if (lane < K8 && r < N) lo[q] = tile[(size_t)r * pitch + lane];
+                } else {
+                    if (lane < K8 && r < N && lane * 8 < pitch) {
+                        const uint2 v = *reinterpret_cast<const uint2*>(tile + (size_t)r * pitch + lane * 8);
+                        lo[q] = v.x; hi[q] = v.y;
+                    }
                 }
             }
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
                 const int r = r0 + q * (TC2_T / 32);
-                uint32_t m = (nzn(lo[q]) | (nzn(hi[q]) << 4)) & colmask;                 // bit u = column 8 lane + u is an edge
+                uint32_t m = (BITS ? lo[q] : (nzn(lo[q]) | (nzn(hi[q]) << 4))) & colmask;    // bit u = column 8 lane + u is an edge
                 const bool dg = (r >> 3) == lane;
                 if (dg) m &= ~(1u << (r & 7));                                            // the diagonal is not an edge
                 if (r < KP) mask8[r * 32 + lane] = (uint8_t)m;                            // edge masks of the row, for the degree
@@ -470,7 +510,7 @@ __global__ void __launch_bounds__(TC2_T, 1) propagate_tc2_kernel(const ConvArgs 
             const int deg = __popc(m0.x) + __popc(m0.y) + __popc(m0.z) + __popc(m0.w) + __popc(m1.x) + __popc(m1.y) + __popc(m1.z) + __popc(m1.w);
             dinv[j] = 1.f / sqrtf((float)deg + (self_loop ? 1.f : 0.f) + a.eps);
         }
-        fence_proxy_async();            // the generic reads of the byte tile are ordered before the next bulk copy into it
+        fence_proxy_async();            // the generic reads of the tile are ordered before the next bulk copy into it
         __syncthreads();
         const int nb = b + gridDim.x;
         if (tid == 0 && nb < a.B) {     // prefetch: the tile buffer is free, the H buffer after the operand build below
@@ -575,6 +615,7 @@ __global__ void __launch_bounds__(TC2_T, 1) propagate_tc2_kernel(const ConvArgs 
 }
 
 // per commit: q_b = x^T (t0 x + t1 ((2/lam)(x - A_hat x) - x)),  t = softmax(theta)
+template <bool BITS>
 __global__ void __launch_bounds__(CONV_T) map_conv_kernel(const ConvArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     const int N = a.N, pitch = a.pitch, b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -589,7 +630,7 @@ __global__ void __launch_bounds__(CONV_T) map_conv_kernel(const ConvArgs a) {
     __syncthreads();
     mbar_wait(s.bar, 0);
     const bool self_loop = a.flags & HDGNN_P_SELF_LOOP, transpose = !(a.flags & HDGNN_P_NO_TRANSPOSE);
-    conv_degree_scan(s, N, pitch, self_loop, a.eps, false);
+    conv_degree_scan<BITS>(s, N, pitch, self_loop, a.eps, false);
     const float* xb = a.x + (size_t)b * N;
     for (int j = tid; j < N; j += CONV_T) s.Hs[j] = xb[j] * s.dinv[j];
     __syncthreads();
@@ -622,25 +663,29 @@ __global__ void __launch_bounds__(CONV_T) map_conv_kernel(const ConvArgs a) {
     (void)lane; (void)warp;
 }
 
-// ---- map_conv for the reference's (transposed) form, straight on the byte tile ---------------------------------------
-// (A_hat x)_i = dinv_i sum_j A[j][i] dinv_j x_j is a weighted COLUMN sum of the byte tile: no bitmap, no transpose.
+// ---- map_conv for the reference's (transposed) form, straight on the staged tile ---------------------------------------
+// (A_hat x)_i = dinv_i sum_j A[j][i] dinv_j x_j is a weighted COLUMN sum of the tile: no bitmap, no transpose.
 // Pass 1: row degrees, one thread per row (16-byte loads; at pitch 208 the rows of 8 lanes fall on distinct banks).
-// Pass 2: one 4-byte word (4 columns) per thread and row, the rows split over the thread groups.  The quadratic form
-// is reduced in a fixed order.  The tile (one buffer, 1-D TMA bulk copy) is 42 KB at N = 200, so five CTAs share an SM
-// and cover each other's copy latency; a CTA walks commits b, b + grid, ...
+// Pass 2: 4 columns per thread and row (one 4-byte word of a byte row, one nibble of a bitmap word), the rows split
+// over the thread groups.  A bitmap tile keeps the byte tile's partition (WR = label_pitch(N) / 4 column groups), so
+// both formats add the same terms in the same order.  The quadratic form is reduced in a fixed order.  The tile (one
+// buffer, 1-D TMA bulk copy) is 42 KB at N = 200 as bytes, so five CTAs share an SM and cover each other's copy
+// latency; a CTA walks commits b, b + grid, ...
 constexpr int MC2_T = 256;
-__host__ __device__ inline size_t mc2_smem_bytes(int N, int pitch) {
-    const int WR = pitch / 4, G = MC2_T / WR > 0 ? MC2_T / WR : 1;
+// WR: 4-column groups of pass 2 per row, pitch / 4 for a byte tile, label_pitch(N) / 4 for a bitmap tile
+__host__ __device__ inline size_t mc2_smem_bytes(int N, int pitch, int WR) {
+    const int G = MC2_T / WR > 0 ? MC2_T / WR : 1;
     return 64 + (size_t)round_up(N * pitch, 128) + (size_t)(2 * round_up(N, 4) + G * WR * 4 + 64) * 4 + 64;
 }
 __device__ __forceinline__ int nzcount4(uint32_t v) {      // number of non-zero bytes
     return __popc((((v & 0x7f7f7f7fu) + 0x7f7f7f7fu) | v) & 0x80808080u);
 }
 
+template <bool BITS>
 __global__ void __launch_bounds__(MC2_T) map_conv2_kernel(const ConvArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     const int N = a.N, pitch = a.pitch, tid = threadIdx.x;
-    const int WR = pitch >> 2;                              // words per tile row
+    const int WR = BITS ? round_up(N, 16) >> 2 : pitch >> 2;   // 4-column groups per row (words per byte tile row)
     const int G = MC2_T / WR > 0 ? MC2_T / WR : 1;          // row groups of pass 2 (4 at N = 200)
     uint64_t* bar = reinterpret_cast<uint64_t*>(smem);
     const uint32_t tbytes = (uint32_t)N * pitch;
@@ -665,42 +710,52 @@ __global__ void __launch_bounds__(MC2_T) map_conv2_kernel(const ConvArgs a) {
         mbar_wait(bar, ph);
         // pass 1: row degrees, thread per row
         for (int j = tid; j < N; j += MC2_T) {
-            const uint4* row = reinterpret_cast<const uint4*>(tile + (size_t)j * pitch);
             int c = 0;
-            for (int q = 0; q * 16 < N; ++q) {
-                const uint4 v = row[q];
-                uint32_t w[4] = {v.x, v.y, v.z, v.w};
+            if constexpr (BITS) {
+                for (int w = 0; w < conv_words(N); ++w) c += __popc(bits_row_word(tile, j, N, pitch, w));
+                // the diagonal is not an edge: cleared in the tile, so pass 2 needs no correction
+                reinterpret_cast<uint32_t*>(tile + (size_t)j * pitch)[j >> 5] &= ~(1u << (j & 31));
+            } else {
+                const uint4* row = reinterpret_cast<const uint4*>(tile + (size_t)j * pitch);
+                for (int q = 0; q * 16 < N; ++q) {
+                    const uint4 v = row[q];
+                    uint32_t w[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    const int c0 = q * 16 + k * 4;
-                    if (c0 + 4 > N) w[k] = c0 >= N ? 0u : (w[k] & (0xffffffffu >> (8 * (c0 + 4 - N))));     // columns >= N
-                    c += nzcount4(w[k]);
+                    for (int k = 0; k < 4; ++k) {
+                        const int c0 = q * 16 + k * 4;
+                        if (c0 + 4 > N) w[k] = c0 >= N ? 0u : (w[k] & (0xffffffffu >> (8 * (c0 + 4 - N))));     // columns >= N
+                        c += nzcount4(w[k]);
+                    }
                 }
+                c -= tile[(size_t)j * pitch + j] != 0;      // the diagonal is not an edge
             }
-            c -= tile[(size_t)j * pitch + j] != 0;          // the diagonal is not an edge
             const float d = 1.f / sqrtf((float)c + (self_loop ? 1.f : 0.f) + a.eps);
             dinv[j] = d; xs[j] = (j == tid ? xmine : xb[j]) * d;
         }
         __syncthreads();
-        // pass 2: weighted column sums; thread = (row group g, word w), 4 columns per thread
+        // pass 2: weighted column sums; thread = (row group g, column group w), 4 columns per thread
         {
             const int g = tid / WR, w = tid - g * WR;
             if (g < G) {
                 const int r0 = (g * N) / G, r1 = ((g + 1) * N) / G;
                 float c0 = 0.f, c1 = 0.f, c2 = 0.f, c3 = 0.f;
-                const uint32_t* col = reinterpret_cast<const uint32_t*>(tile) + w;
+                // byte tile: word w of the row, a byte per column; bitmap tile: nibble w & 7 of word w >> 3, a bit per column
+                const uint32_t* col = reinterpret_cast<const uint32_t*>(tile) + (BITS ? w >> 3 : w);
+                const int rs = BITS ? pitch >> 2 : WR;
+                const uint32_t m0 = BITS ? 1u << (4 * (w & 7)) : 0x000000ffu;
+                const uint32_t m1 = BITS ? m0 << 1 : 0x0000ff00u, m2 = BITS ? m0 << 2 : 0x00ff0000u, m3 = BITS ? m0 << 3 : 0xff000000u;
 #pragma unroll 8
                 for (int j = r0; j < r1; ++j) {
-                    const uint32_t v = col[(size_t)j * WR];
+                    const uint32_t v = col[(size_t)j * rs];
                     const float xj = xs[j];
-                    c0 += (v & 0x000000ffu) ? xj : 0.f; c1 += (v & 0x0000ff00u) ? xj : 0.f;
-                    c2 += (v & 0x00ff0000u) ? xj : 0.f; c3 += (v & 0xff000000u) ? xj : 0.f;
+                    c0 += (v & m0) ? xj : 0.f; c1 += (v & m1) ? xj : 0.f;
+                    c2 += (v & m2) ? xj : 0.f; c3 += (v & m3) ? xj : 0.f;
                 }
                 // the diagonal entry is not an edge: take it out again (row i of column i lies in exactly one group)
 #pragma unroll
                 for (int u = 0; u < 4; ++u) {
                     const int i = 4 * w + u;
-                    if (i < N && i >= r0 && i < r1 && tile[(size_t)i * pitch + i]) {
+                    if (!BITS && i < N && i >= r0 && i < r1 && tile[(size_t)i * pitch + i]) {
                         const float xi = xs[i];
                         if (u == 0) c0 -= xi; else if (u == 1) c1 -= xi; else if (u == 2) c2 -= xi; else c3 -= xi;
                     }
@@ -734,63 +789,70 @@ __global__ void mean_kernel(const float* v, int n, float* out) {
 
 using namespace hdgnn;
 
-static int conv_check(int B, int N, int pitch, const void* adj) {
-    if (B < 1 || N < 2 || N > HDGNN_MAX_N || !adj) return HDGNN_E_INVALID;
-    if (pitch < N || (pitch & 15) || ((uintptr_t)adj & 15)) return HDGNN_E_INVALID;
+static int conv_check(int B, int N, int pitch, const void* adj, int flags) {
+    if (B < 1 || N < 2 || N > HDGNN_MAX_N || !adj || !legacy_adj_ok(N, pitch, adj, flags)) return HDGNN_E_INVALID;
     return HDGNN_OK;
 }
 
 extern "C" int hdgnn_normalize_propagate(int B, int N, const uint8_t* adj, int pitch, const float* H, int d_in, const float* W,
                                          const float* bias, int d_out, float eps, int flags, float* out, float* dinv_out,
                                          void* stream) {
-    int rc = conv_check(B, N, pitch, adj);
+    int rc = conv_check(B, N, pitch, adj, flags);
     if (rc) return rc;
     if (!H || !out || d_in < 1 || d_in > CONV_MAXD || d_out < 1 || d_out > CONV_MAXD) return HDGNN_E_INVALID;
     if (!W && d_in != d_out) return HDGNN_E_INVALID;
     int dev = 0, optin = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
         return HDGNN_E_CUDA;
+    const bool bits = flags & HDGNN_P_LABEL_BITS;
     ConvArgs a{};
     a.B = B; a.N = N; a.pitch = pitch; a.d_in = d_in; a.d_out = d_out; a.flags = flags; a.eps = eps;
     a.adj = adj; a.H = H; a.W = W; a.bias = bias; a.out = out; a.dinv_out = dinv_out;
     // tensor-core paths (tcgen05), N <= 256: the persistent kernel with the adjacency as the wide operand when its
-    // buffers fit one SM, else the one-CTA-per-commit kernel; else the set-bit walk on the CUDA cores
+    // buffers fit one SM, else the one-CTA-per-commit kernel; else the set-bit walk on the CUDA cores.  Every size is
+    // that of the tile as staged (N * pitch bytes): a bitmap tile is 1/8 of a byte tile, so the persistent kernel takes
+    // bitmaps up to N = 240 at d_in = 20 where byte grids fall back to the one-CTA-per-commit kernel above N = 208.
     const size_t smem_tc2 = tc2_smem_bytes(N, pitch, d_in);
     if (!(flags & (HDGNN_P_NO_TENSOR | HDGNN_P_TENSOR_V1)) && N <= 256 && smem_tc2 <= (size_t)optin) {
         int sms = 148;
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (cudaFuncSetAttribute(propagate_tc2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) != cudaSuccess) return HDGNN_E_CUDA;
-        propagate_tc2_kernel<<<B < sms ? B : sms, TC2_T, smem_tc2, (cudaStream_t)stream>>>(a);
+        const auto k = bits ? propagate_tc2_kernel<true> : propagate_tc2_kernel<false>;
+        if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) != cudaSuccess) return HDGNN_E_CUDA;
+        k<<<B < sms ? B : sms, TC2_T, smem_tc2, (cudaStream_t)stream>>>(a);
         return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
     }
     const size_t smem_tc = tc_smem_bytes(N, pitch, d_in, d_out);
     if (!(flags & HDGNN_P_NO_TENSOR) && N <= 256 && smem_tc <= (size_t)optin) {
-        if (cudaFuncSetAttribute(propagate_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) != cudaSuccess) return HDGNN_E_CUDA;
-        propagate_tc_kernel<<<B, TC_T, smem_tc, (cudaStream_t)stream>>>(a);
+        const auto k = bits ? propagate_tc_kernel<true> : propagate_tc_kernel<false>;
+        if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) != cudaSuccess) return HDGNN_E_CUDA;
+        k<<<B, TC_T, smem_tc, (cudaStream_t)stream>>>(a);
         return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
     }
     const size_t smem = conv_smem_bytes(N, pitch, d_out);
     if (smem > (size_t)optin) return HDGNN_E_UNSUPPORTED;       // the per-commit tile must fit one SM
-    if (cudaFuncSetAttribute(propagate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) != cudaSuccess) return HDGNN_E_CUDA;
-    propagate_kernel<<<B, CONV_T, smem, (cudaStream_t)stream>>>(a);
+    const auto k = bits ? propagate_kernel<true> : propagate_kernel<false>;
+    if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) != cudaSuccess) return HDGNN_E_CUDA;
+    k<<<B, CONV_T, smem, (cudaStream_t)stream>>>(a);
     return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
 }
 
 extern "C" int hdgnn_map_conv(int B, int N, const uint8_t* adj, int pitch, const float* x, const float* theta, float lam_max,
                               float eps, int flags, float* per_commit, float* loss, void* stream) {
-    int rc = conv_check(B, N, pitch, adj);
+    int rc = conv_check(B, N, pitch, adj, flags);
     if (rc) return rc;
     if (!x || !theta || !per_commit || lam_max <= 0.f) return HDGNN_E_INVALID;
+    const bool bits = flags & HDGNN_P_LABEL_BITS;
     const size_t smem = conv_smem_bytes(N, pitch, 1);
     int dev = 0, optin = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
         return HDGNN_E_CUDA;
-    // the reference's (transposed) form: persistent kernel on the byte tile, two tiles in flight, two CTAs per SM
-    const size_t smem2 = mc2_smem_bytes(N, pitch);
+    // the reference's (transposed) form: persistent kernel on the staged tile, several tiles in flight per SM
+    const size_t smem2 = mc2_smem_bytes(N, pitch, bits ? round_up(N, 16) / 4 : pitch / 4);
     if (!(flags & (HDGNN_P_NO_TRANSPOSE | HDGNN_P_TENSOR_V1)) && smem2 <= (size_t)optin) {
         int sms = 148;
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (cudaFuncSetAttribute(map_conv2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2) != cudaSuccess) return HDGNN_E_CUDA;
+        const auto k2 = bits ? map_conv2_kernel<true> : map_conv2_kernel<false>;
+        if (cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2) != cudaSuccess) return HDGNN_E_CUDA;
         ConvArgs a2{};
         a2.B = B; a2.N = N; a2.pitch = pitch; a2.flags = flags; a2.eps = eps; a2.lam_max = lam_max;
         a2.adj = adj; a2.x = x; a2.theta = theta; a2.per_commit = per_commit;
@@ -798,16 +860,17 @@ extern "C" int hdgnn_map_conv(int B, int N, const uint8_t* adj, int pitch, const
         per_sm = per_sm < 1 ? 1 : (per_sm > 8 ? 8 : per_sm);
         const int grid = B < sms * per_sm ? B : sms * per_sm;
         if (!x || !theta || !per_commit || lam_max <= 0.f) return HDGNN_E_INVALID;
-        map_conv2_kernel<<<grid, MC2_T, smem2, (cudaStream_t)stream>>>(a2);
+        k2<<<grid, MC2_T, smem2, (cudaStream_t)stream>>>(a2);
         if (loss) mean_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(per_commit, B, loss);
         return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
     }
     if (smem > (size_t)optin) return HDGNN_E_UNSUPPORTED;
-    if (cudaFuncSetAttribute(map_conv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) != cudaSuccess) return HDGNN_E_CUDA;
+    const auto k = bits ? map_conv_kernel<true> : map_conv_kernel<false>;
+    if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) != cudaSuccess) return HDGNN_E_CUDA;
     ConvArgs a{};
     a.B = B; a.N = N; a.pitch = pitch; a.flags = flags; a.eps = eps; a.lam_max = lam_max;
     a.adj = adj; a.x = x; a.theta = theta; a.per_commit = per_commit;
-    map_conv_kernel<<<B, CONV_T, smem, (cudaStream_t)stream>>>(a);
+    k<<<B, CONV_T, smem, (cudaStream_t)stream>>>(a);
     if (loss) mean_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(per_commit, B, loss);
     return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
 }

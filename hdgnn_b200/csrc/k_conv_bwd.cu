@@ -12,10 +12,11 @@
 //  * hdgnn_map_conv_backward: loss = mean_b s_b^2, s_b = x^T (t0 I + t1 L~) x, t = softmax(theta), L~ = (2/lam)(I - A_hat) - I:
 //        ds/dx = 2 t0 x + t1 ((4/lam - 2) x - (2/lam)(A_hat + A_hat^T) x),
 //        dloss/dx_b = (2 s_b / B) ds/dx,   dloss/dt0 = sum_b (2 s_b / B) x^T x,   dloss/dt1 = sum_b (2 s_b / B) x^T L~ x,
-//    then through the softmax.  One CTA per commit on the byte tile: degrees, then the row and column mat-vecs in two passes.
+//    then through the softmax.  One CTA per commit on the staged tile (byte grid, or label bitmap with HDGNN_P_LABEL_BITS):
+//    degrees, then the row and column mat-vecs in two passes.
 // All sums run in a fixed order (no float atomics).
 #include "../../include/hdgnn.h"
-#include "common.cuh"
+#include "bits.cuh"
 
 namespace hdgnn {
 
@@ -107,6 +108,7 @@ struct McbArgs {
     float* dx; float* part;      // part (B,2): (2 s_b g / B) x^T x, (2 s_b g / B) x^T L~ x
 };
 
+template <bool BITS>
 __global__ void __launch_bounds__(CB_T) map_conv_bwd_kernel(const McbArgs a) {
     extern __shared__ __align__(16) unsigned char smraw[];
     const int N = a.N, pitch = a.pitch, b = blockIdx.x, tid = threadIdx.x;
@@ -130,13 +132,24 @@ __global__ void __launch_bounds__(CB_T) map_conv_bwd_kernel(const McbArgs a) {
     mbar_wait(bar, 0);
     const bool self = (a.flags & HDGNN_P_SELF_LOOP) != 0, notr = (a.flags & HDGNN_P_NO_TRANSPOSE) != 0;
     const int NW = pitch >> 2;
+    // a bitmap row: bit (j & 31) of word j >> 5; only columns < N are read below, and the diagonal is skipped
+    const uint32_t* tbits = reinterpret_cast<const uint32_t*>(tile);
     for (int i = tid; i < N; i += CB_T) {                     // degrees (diagonal ignored)
         const uint32_t* row = reinterpret_cast<const uint32_t*>(tile + (size_t)i * pitch);
         int deg = 0;
-        for (int w = 0; w < NW; ++w) {
-            uint32_t v = row[w];
-            if ((i >> 2) == w) v &= ~(0xffu << (8 * (i & 3)));
-            deg += ((v & 0xffu) != 0) + ((v & 0xff00u) != 0) + ((v & 0xff0000u) != 0) + ((v & 0xff000000u) != 0);
+        if constexpr (BITS) {
+            for (int w = 0; w < (N + 31) / 32; ++w) {
+                uint32_t v = row[w];
+                if (32 * w + 32 > N) v &= 0xffffffffu >> (32 * w + 32 - N);
+                if ((i >> 5) == w) v &= ~(1u << (i & 31));
+                deg += __popc(v);
+            }
+        } else {
+            for (int w = 0; w < NW; ++w) {
+                uint32_t v = row[w];
+                if ((i >> 2) == w) v &= ~(0xffu << (8 * (i & 3)));
+                deg += ((v & 0xffu) != 0) + ((v & 0xff00u) != 0) + ((v & 0xff0000u) != 0) + ((v & 0xff000000u) != 0);
+            }
         }
         const float di = rsqrtf((float)deg + (self ? 1.f : 0.f) + a.eps);
         dinv[i] = di; u[i] = di * xs[i];
@@ -145,12 +158,24 @@ __global__ void __launch_bounds__(CB_T) map_conv_bwd_kernel(const McbArgs a) {
     for (int i = tid; i < N; i += CB_T) {                     // rr_i = sum_j A_ij u_j
         const uint8_t* row = tile + (size_t)i * pitch;
         float acc = self ? u[i] : 0.f;
-        for (int j = 0; j < N; ++j) acc += (row[j] != 0 && j != i) ? u[j] : 0.f;
+        if constexpr (BITS) {
+            for (int j0 = 0; j0 < N; j0 += 32) {              // one word load per 32 columns, the same additions as below
+                const uint32_t v = tbits[(size_t)i * NW + (j0 >> 5)];
+                const int j1 = j0 + 32 < N ? j0 + 32 : N;
+                for (int j = j0; j < j1; ++j) acc += (((v >> (j & 31)) & 1u) && j != i) ? u[j] : 0.f;
+            }
+        } else {
+            for (int j = 0; j < N; ++j) acc += (row[j] != 0 && j != i) ? u[j] : 0.f;
+        }
         rr[i] = acc;
     }
     for (int j = tid; j < N; j += CB_T) {                     // pp_j = sum_i A_ij u_i
         float acc = self ? u[j] : 0.f;
-        for (int i = 0; i < N; ++i) acc += (tile[(size_t)i * pitch + j] != 0 && i != j) ? u[i] : 0.f;
+        if constexpr (BITS) {
+            for (int i = 0; i < N; ++i) acc += (((tbits[(size_t)i * NW + (j >> 5)] >> (j & 31)) & 1u) && i != j) ? u[i] : 0.f;
+        } else {
+            for (int i = 0; i < N; ++i) acc += (tile[(size_t)i * pitch + j] != 0 && i != j) ? u[i] : 0.f;
+        }
         pp[j] = acc;
     }
     __syncthreads();
@@ -202,6 +227,7 @@ extern "C" int hdgnn_normalize_propagate_backward(int B, int N, const uint8_t* a
                                                   const float* W, int d_out, float eps, int flags, const float* out, const float* dOut,
                                                   float* dH, float* dW, float* dbias, float* work, void* stream) {
     if (B < 1 || N < 2 || N > HDGNN_MAX_N || !adj || !H || !dOut || !work) return HDGNN_E_INVALID;
+    if (!legacy_adj_ok(N, adj_pitch, adj, flags)) return HDGNN_E_INVALID;
     if (d_in < 1 || d_in > CB_MAXD || d_out < 1 || d_out > CB_MAXD || (!W && d_in != d_out)) return HDGNN_E_INVALID;
     if ((flags & HDGNN_P_RELU) && !out) return HDGNN_E_INVALID;
     cudaStream_t st = (cudaStream_t)stream;
@@ -213,7 +239,7 @@ extern "C" int hdgnn_normalize_propagate_backward(int B, int N, const uint8_t* a
         dpre_src = dPre;
     }
     // dZ = A_hat^T dPre: the forward operator with the transposition flipped, no weights, no bias, no activation
-    const int keep = flags & (HDGNN_P_SELF_LOOP | HDGNN_P_NO_TENSOR | HDGNN_P_TENSOR_V1);
+    const int keep = flags & (HDGNN_P_SELF_LOOP | HDGNN_P_NO_TENSOR | HDGNN_P_TENSOR_V1 | HDGNN_P_LABEL_BITS);
     const int flipped = keep | ((flags & HDGNN_P_NO_TRANSPOSE) ? 0 : HDGNN_P_NO_TRANSPOSE);
     int rc = hdgnn_normalize_propagate(B, N, adj, adj_pitch, dpre_src, d_out, nullptr, nullptr, d_out, eps, flipped, dZ, nullptr, stream);
     if (rc) return rc;
@@ -236,7 +262,7 @@ extern "C" int hdgnn_normalize_propagate_backward(int B, int N, const uint8_t* a
 extern "C" int hdgnn_map_conv_backward(int B, int N, const uint8_t* adj, int adj_pitch, const float* x, const float* theta, float lam_max,
                                        float eps, int flags, float gscale, float* dx, float* dtheta, float* work, void* stream) {
     if (B < 1 || N < 2 || N > HDGNN_MAX_N || !adj || !x || !theta || lam_max <= 0.f) return HDGNN_E_INVALID;
-    if (adj_pitch < N || (adj_pitch & 15) || ((uintptr_t)adj & 15)) return HDGNN_E_INVALID;
+    if (!legacy_adj_ok(N, adj_pitch, adj, flags)) return HDGNN_E_INVALID;
     if (dtheta && !work) return HDGNN_E_INVALID;
     cudaStream_t st = (cudaStream_t)stream;
     const size_t smem = 16 + (size_t)round_up(N * adj_pitch, 16) + (size_t)(5 * N + 32) * sizeof(float);
@@ -244,11 +270,12 @@ extern "C" int hdgnn_map_conv_backward(int B, int N, const uint8_t* adj, int adj
     if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
         return HDGNN_E_CUDA;
     if (smem > (size_t)optin) return HDGNN_E_UNSUPPORTED;
-    if (cudaFuncSetAttribute(map_conv_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return HDGNN_E_CUDA;
+    const auto k = (flags & HDGNN_P_LABEL_BITS) ? map_conv_bwd_kernel<true> : map_conv_bwd_kernel<false>;
+    if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return HDGNN_E_CUDA;
     McbArgs a{};
     a.B = B; a.N = N; a.pitch = adj_pitch; a.flags = flags; a.eps = eps; a.lam_max = lam_max; a.gscale = gscale;
     a.adj = adj; a.x = x; a.theta = theta; a.dx = dx; a.part = dtheta ? work : nullptr;
-    map_conv_bwd_kernel<<<B, CB_T, smem, st>>>(a);
+    k<<<B, CB_T, smem, st>>>(a);
     if (dtheta) theta_grad_kernel<<<1, 256, 0, st>>>(work, B, theta, dtheta);
     return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
 }

@@ -308,7 +308,7 @@ class Engine:
 
 
 # -- legacy operator of model.py (normalize_adj + propagation, Chebyshev map_conv) -------------------------------
-P_SELF_LOOP, P_RELU, P_NO_TRANSPOSE, P_NO_TENSOR = 1, 2, 4, 8
+P_SELF_LOOP, P_RELU, P_NO_TRANSPOSE, P_NO_TENSOR, P_TENSOR_V1, P_LABEL_BITS = 1, 2, 4, 8, 16, 32
 
 
 def _pitched(adj: torch.Tensor) -> torch.Tensor:
@@ -322,14 +322,29 @@ def _pitched(adj: torch.Tensor) -> torch.Tensor:
     return out
 
 
+def _adjacency(adj: torch.Tensor, flags: int):
+    """The legacy operator's adjacency argument -> (tensor, row pitch in bytes, flags).  An int32 / uint32 tensor is a label
+    bitmap (B,N,bit_words(N)) as pack_label_bits_device returns it and sets P_LABEL_BITS; a uint8 tensor is a byte grid."""
+    if adj.dtype in (torch.int32, torch.uint32):
+        B, N, wp = adj.shape
+        if wp != bit_words(N):
+            raise ValueError(f"a label bitmap of N = {N} has bit_words(N) = {bit_words(N)} words per row, got {wp}")
+        return adj.contiguous(), 4 * wp, flags | P_LABEL_BITS
+    if flags & P_LABEL_BITS:
+        raise ValueError("P_LABEL_BITS needs an int32 / uint32 label bitmap, got a byte grid")
+    a = _pitched(adj)
+    return a, a.shape[2], flags
+
+
 def normalize_propagate(adj: torch.Tensor, H: torch.Tensor, W: Optional[torch.Tensor] = None,
                         bias: Optional[torch.Tensor] = None, eps: float = 1e-3, flags: int = 0):
-    """act(A_hat (H W) + b) with the reference's normalize_adj (model.py:360-367).  adj (B,N,N|pitch) uint8 cuda,
-    H (B,N,d_in) float32 cuda.  Returns (out (B,N,d_out), dinv (B,N))."""
+    """act(A_hat (H W) + b) with the reference's normalize_adj (model.py:360-367).  adj (B,N,N|pitch) uint8 cuda, or a
+    (B,N,bit_words(N)) int32 / uint32 label bitmap (the same operator, P_LABEL_BITS is set here), H (B,N,d_in) float32
+    cuda.  Returns (out (B,N,d_out), dinv (B,N))."""
+    a, pitch, flags = _adjacency(adj, flags)
     if not (adj.is_cuda and H.is_cuda):
         raise RuntimeError("normalize_propagate needs CUDA tensors; there is no CPU fallback")
-    a = _pitched(adj)
-    B, N, pitch = a.shape
+    B, N = a.shape[:2]
     H = H.contiguous().float()
     d_in = H.shape[2]
     d_out = d_in if W is None else W.shape[1]
@@ -344,11 +359,12 @@ def normalize_propagate(adj: torch.Tensor, H: torch.Tensor, W: Optional[torch.Te
 
 def map_conv(adj: torch.Tensor, x: torch.Tensor, theta: torch.Tensor, lam_max: float = 1.5, eps: float = 1e-3,
              flags: int = 0):
-    """map_conv of model.py:394-403 (k = 2, Ds = 1).  Returns (loss scalar tensor, per-commit (B,))."""
+    """map_conv of model.py:394-403 (k = 2, Ds = 1); adj as for normalize_propagate.  Returns (loss scalar tensor,
+    per-commit (B,))."""
+    a, pitch, flags = _adjacency(adj, flags)
     if not (adj.is_cuda and x.is_cuda):
         raise RuntimeError("map_conv needs CUDA tensors; there is no CPU fallback")
-    a = _pitched(adj)
-    B, N, pitch = a.shape
+    B, N = a.shape[:2]
     per = torch.empty(B, dtype=torch.float32, device=a.device)
     loss = torch.empty(1, dtype=torch.float32, device=a.device)
     st = C.c_void_p(torch.cuda.current_stream(a.device).cuda_stream)
@@ -360,11 +376,12 @@ def map_conv(adj: torch.Tensor, x: torch.Tensor, theta: torch.Tensor, lam_max: f
 def normalize_propagate_backward(adj: torch.Tensor, H: torch.Tensor, dOut: torch.Tensor, W: Optional[torch.Tensor] = None,
                                  out: Optional[torch.Tensor] = None, eps: float = 1e-3, flags: int = 0):
     """Backward of normalize_propagate w.r.t. H, W and the bias (the adjacency carries no gradient: model.py:337 takes its
-    argmax).  `out` = the forward's output, needed with P_RELU.  Returns (dH (B,N,d_in), dW (d_in,d_out) or None, dbias (d_out))."""
+    argmax); adj as for normalize_propagate.  `out` = the forward's output, needed with P_RELU.  Returns (dH (B,N,d_in),
+    dW (d_in,d_out) or None, dbias (d_out))."""
+    a, pitch, flags = _adjacency(adj, flags)
     if not (adj.is_cuda and H.is_cuda and dOut.is_cuda):
         raise RuntimeError("normalize_propagate_backward needs CUDA tensors; there is no CPU fallback")
-    a = _pitched(adj)
-    B, N, pitch = a.shape
+    B, N = a.shape[:2]
     H = H.contiguous().float(); dOut = dOut.contiguous().float()
     d_in, d_out = H.shape[2], dOut.shape[2]
     dH = torch.empty(B, N, d_in, dtype=torch.float32, device=a.device)
@@ -380,11 +397,12 @@ def normalize_propagate_backward(adj: torch.Tensor, H: torch.Tensor, dOut: torch
 
 def map_conv_backward(adj: torch.Tensor, x: torch.Tensor, theta: torch.Tensor, lam_max: float = 1.5, eps: float = 1e-3,
                       flags: int = 0, gscale: float = 1.0):
-    """Gradient of map_conv's loss w.r.t. x (B,N) and theta (2) (model.py:394-403; no gradient to the adjacency)."""
+    """Gradient of map_conv's loss w.r.t. x (B,N) and theta (2) (model.py:394-403; no gradient to the adjacency); adj as
+    for normalize_propagate."""
+    a, pitch, flags = _adjacency(adj, flags)
     if not (adj.is_cuda and x.is_cuda):
         raise RuntimeError("map_conv_backward needs CUDA tensors; there is no CPU fallback")
-    a = _pitched(adj)
-    B, N, pitch = a.shape
+    B, N = a.shape[:2]
     dx = torch.empty(B, N, dtype=torch.float32, device=a.device)
     dth = torch.empty(2, dtype=torch.float32, device=a.device)
     work = torch.empty(2 * B, dtype=torch.float32, device=a.device)

@@ -210,14 +210,21 @@ int hdgnn_infer_host(hdgnn_handle_t h, int B,
  * out (B,N,d_out) = act( A_hat (H W) + bias ),  A_hat = D^-1/2 A^T D^-1/2,  D = rowsum(A) + eps: the
  * normalize_adj of model.py:360-367 (eps = 1e-3, no self loop, transposed) fused with one propagation.
  * H (B,N,d_in); W (d_in,d_out) row-major or NULL (then d_in == d_out); bias (d_out) or NULL; d_in, d_out <= 32;
- * dinv_out (B,N) optionally receives D^-1/2.  flags select the variants.  Stateless (no handle); the
- * per-commit state (N * pitch bytes of adjacency + two bitmaps + N * d_out floats) must fit one SM's shared
- * memory (N ~ 380 at d_out = 20), else HDGNN_E_UNSUPPORTED. */
+ * dinv_out (B,N) optionally receives D^-1/2.  flags select the variants.  Stateless (no handle).
+ * The adjacency of the four legacy entry points is either
+ *   - a byte grid: uint8 (B, N, adj_pitch), A_ij != 0 is an edge, adj_pitch >= N and a multiple of 16; or
+ *   - with HDGNN_P_LABEL_BITS, a label bitmap in the layout of HDGNN_F_LABEL_BITS: (B, N, hdgnn_bit_words(N)) uint32,
+ *     bit k of word w of row i = A_i,32w+k, adj_pitch = 4 * hdgnn_bit_words(N) exactly (what hdgnn_pack_label_bits writes).
+ * Either way adj is 16-byte aligned, and the diagonal (and for bitmaps the padding bits, columns >= N) is ignored.
+ * The per-commit state (N * adj_pitch bytes of adjacency + two bitmaps + N * d_out floats) must fit one SM's shared
+ * memory, else HDGNN_E_UNSUPPORTED: byte grids up to N ~ 380 at d_out = 20, label bitmaps up to N = HDGNN_MAX_N = 512
+ * (a 32 KB tile).  With bitmaps the persistent tcgen05 kernel is the default up to N = 240 at d_in = 20 (byte grids: N = 208). */
 #define HDGNN_P_SELF_LOOP     1   /* normalise and propagate A + I (the textbook GCN form) */
 #define HDGNN_P_RELU          2
 #define HDGNN_P_NO_TRANSPOSE  4   /* A_hat = D^-1/2 A D^-1/2 */
 #define HDGNN_P_NO_TENSOR     8   /* force the CUDA-core set-bit walk (default for N <= 256: tcgen05, bf16 x 3 split, fp32 in TMEM) */
 #define HDGNN_P_TENSOR_V1    16   /* force the one-CTA-per-commit tcgen05 kernel (default: the persistent kernel when its buffers fit) */
+#define HDGNN_P_LABEL_BITS   32   /* adj is a label bitmap, not a byte grid (see above); same kernels, same results */
 int hdgnn_normalize_propagate(int B, int N, const uint8_t* adj, int adj_pitch, const float* H, int d_in,
                               const float* W, const float* bias, int d_out, float eps, int flags,
                               float* out, float* dinv_out, void* stream);
