@@ -2,12 +2,13 @@
 // ownership, the launch sequence of one forward / forward+backward / optimizer step, staging of host buffers, the
 // peer-memory set-up.  No torch types.
 //
-// Launch sequences of a training step:
+// Launch sequences of a training step.  Byte-grid inputs are first turned into label bitmaps (bits.cuh) by pack_bits
+// (pack_step); no kernel after it reads a byte grid.  With HDGNN_F_LABEL_BITS the inputs are bitmaps and there is no pack_bits.
 //   fused path (all four variants, Nc <= 256, forward only up to Nc = 512; mid2.cuh, entsp.cuh, final.cuh):
-//       [pack_bits, byte-grid inputs only] -> mid2 (the whole per-commit forward + backward; above 128 hunks with its hunk-stage
-//       tables in the per-commit global slice TABS) -> reduce_adam (gradient reduction [+ peer all-reduce] + regularisers +
-//       TF-Adam).  With HDGNN_F_DENSE_SWEEP, or when the inline entity state does not fit (Ne = 512 beside Nc <= 128):
-//       [pack_bits] -> ent_fwd2 -> mid2 -> ent_bwd2 -> reduce_adam (ent2.cuh).
+//       mid2 (the whole per-commit forward + backward; above 128 hunks with its hunk-stage tables in the per-commit global
+//       slice TABS) -> reduce_adam (gradient reduction [+ peer all-reduce] + regularisers + TF-Adam).  With
+//       HDGNN_F_DENSE_SWEEP, or when the inline entity state does not fit (Ne = 512 beside Nc <= 128):
+//       ent_fwd2 -> mid2 -> ent_bwd2 -> reduce_adam (ent2.cuh).
 //   multi-kernel path (HDGNN_F_LEGACY, training with Nc > 256; pairsum.cuh, score.cuh, node.cuh;
 //   [E] = entity-edge branch of model_4.py:92-98):
 //       fwd : pairsum(ent) -> [E: pairsum(edge) -> head_fwd(edge) -> score(edge, soft out)] -> pool_fwd
@@ -126,17 +127,16 @@ struct hdgnn_handle_s {
     hdgnn_config_t cfg;
     ParamOff po;
     HeadOff ho_hunk, ho_edge;
-    int Ne, Nc, pe, pc;        // sizes and label pitches
+    int Ne, Nc, pe, pc;        // sizes and byte-grid label pitches
+    int WPe = 0, WPc = 0;      // label-bitmap words per row
     int RTe, Se, CWe;          // entity grid tiling
     int RTc, Sc, CWc;          // hunk grid tiling
     bool ent, edge;            // branches that feed the loss
     bool debug = false;
     FusedPlan plan;
-    // fused path: label bitmaps + balanced row chunks of the entity grid (ent2.cuh)
-    int WPe = 0, WPc = 0;      // bitmap words per row
     int nsm = 148;
-    int cwt = 0;                                               // column segments per pass of the entity sweeps
-    int bslot = 0;                                             // bitmap buffer of the current step (two alternate)
+    int cwt = 0;                                               // column segments per pass of the entity sweeps (ent2.cuh)
+    int bslot = 0;                                             // bitmap buffer of the current device-fed step (two alternate)
     std::map<std::string, Buf> ws;
     std::string err;
     int launches = 0;
@@ -164,9 +164,8 @@ struct hdgnn_handle_s {
     uint32_t* tag_table = nullptr;         // pinned, tag_table[i] = i: immutable DMA source
     unsigned int slot_uses[NSLOT] = {};
     int cur_tag = -1;                      // tag of the staging slot filled by the last stage_inputs call, -1 = ordered by event
-    // HDGNN_F_LABEL_BITS: the *_host entry points receive label bitmaps (bits.cuh layout) instead of byte grids
+    // HDGNN_F_LABEL_BITS: the entry points receive label bitmaps (bits.cuh layout) instead of byte grids
     bool host_bits = false;
-    const uint32_t* eb = nullptr; const uint32_t* yb = nullptr;   // bitmaps of the current step
 };
 
 namespace {
@@ -272,16 +271,16 @@ cudaError_t set_attrs(hdgnn_handle_t h, int optin) {
 }
 
 // grid: which N x N grid a launch runs on
-struct GridCfg { int N, RT, S, CW, pitch; };
-GridCfg ent_grid(hdgnn_handle_t h) { return {h->Ne, h->RTe, h->Se, h->CWe, h->pe}; }
-GridCfg hunk_grid(hdgnn_handle_t h) { return {h->Nc, h->RTc, h->Sc, h->CWc, h->pc}; }
+struct GridCfg { int N, RT, S, CW, WP; };
+GridCfg ent_grid(hdgnn_handle_t h) { return {h->Ne, h->RTe, h->Se, h->CWe, h->WPe}; }
+GridCfg hunk_grid(hdgnn_handle_t h) { return {h->Nc, h->RTc, h->Sc, h->CWc, h->WPc}; }
 
 int launch_pairsum(hdgnn_handle_t h, const char* what, const GridCfg& g, int B, bool bwd, bool rank1, PairSumArgs a, cudaStream_t st) {
-    a.N = g.N; a.RT = g.RT; a.S = g.S; a.pitch = g.pitch;
+    a.N = g.N; a.RT = g.RT; a.S = g.S; a.WP = g.WP;
     const dim3 grid(g.S, B), block(32 * HD);
     PROF_BEGIN(h, st);
     CW_SWITCH(g.CW, {
-        const size_t smem = pairsum_smem_bytes(CW, g.RT, g.pitch, bwd);
+        const size_t smem = pairsum_smem_bytes(CW, g.RT, 4 * g.WP, bwd);
         if (bwd) {
             if (rank1) pairsum_kernel<CW, true, true><<<grid, block, smem, st>>>(a);
             else pairsum_kernel<CW, true, false><<<grid, block, smem, st>>>(a);
@@ -295,11 +294,11 @@ int launch_pairsum(hdgnn_handle_t h, const char* what, const GridCfg& g, int B, 
 }
 
 int launch_score(hdgnn_handle_t h, const char* what, const GridCfg& g, int B, bool train, ScoreArgs a, cudaStream_t st) {
-    a.N = g.N; a.RT = g.RT; a.S = g.S; a.pitch = g.pitch;
+    a.N = g.N; a.RT = g.RT; a.S = g.S; a.WP = g.WP;
     const dim3 grid(g.S, B), block(32 * HD);
     PROF_BEGIN(h, st);
     CW_SWITCH(g.CW, {
-        const size_t smem = score_smem_bytes(CW, g.RT, g.pitch, train);
+        const size_t smem = score_smem_bytes(CW, g.RT, 4 * g.WP, train);
         if (train) score_kernel<CW, true><<<grid, block, smem, st>>>(a);
         else score_kernel<CW, false><<<grid, block, smem, st>>>(a);
     });
@@ -323,20 +322,13 @@ int check_inputs(hdgnn_handle_t h, int B, const void* adj, int adj_pitch, const 
     return HDGNN_OK;
 }
 
-struct Inputs;
-static void alias_bits(hdgnn_handle_t h, Inputs& in);
-
+// the device inputs of a step, its label grids as bitmaps (bits.cuh): given, or made by pack_step
 struct Inputs {
-    const uint8_t* adj; const float* x; const int32_t* hmap; const int32_t* L; const uint8_t* Y;
+    const uint32_t* ebits; const uint32_t* ybits;
+    const float* x; const int32_t* hmap; const int32_t* L;
     const float* params;
-    const uint32_t* ebits = nullptr; const uint32_t* ybits = nullptr;   // set: bitmaps are given, adj / Y are not read (fused path)
     const int* wait_flag = nullptr; int wait_tag = 0;                    // staged inputs ordered by a DMA-written tag (mid2 polls it)
 };
-
-// HDGNN_F_LABEL_BITS: the adj / Y arguments of the device entry points ARE the bitmaps
-static void alias_bits(hdgnn_handle_t h, Inputs& in) {
-    if (h->host_bits && !in.ebits) { in.ebits = (const uint32_t*)in.adj; in.ybits = (const uint32_t*)in.Y; }
-}
 
 int forward_impl(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float* logits, float* probs,
                  float* loss, bool train, cudaStream_t st) {
@@ -345,14 +337,14 @@ int forward_impl(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float*
     int rc;
     if (h->ent) {
         PairSumArgs a{};
-        a.lab = in.adj; a.params = in.params; a.x = in.x;
+        a.bits = in.ebits; a.params = in.params; a.x = in.x;
         a.o_u = po.ent_w1; a.o_v = po.ent_w1 + HD; a.o_b = po.ent_b1; a.o_l = po.ent_w1 + 2 * HD;
         a.RS = F(h, "RS1"); a.CSp = F(h, "CS1P");
         if ((rc = launch_pairsum(h, "pairsum_fwd(ent)", ge, B, false, true, a, st))) return rc;
     }
     if (h->edge) {
         PairSumArgs a{};
-        a.lab = in.adj; a.params = in.params; a.x = in.x;
+        a.bits = in.ebits; a.params = in.params; a.x = in.x;
         a.o_u = po.edg_w11; a.o_v = po.edg_w11; a.o_b = po.edg_b1; a.o_l = po.edg_w12;
         a.RS = F(h, "RSE"); a.CSp = F(h, "CSEP");
         if ((rc = launch_pairsum(h, "pairsum_fwd(edge)", ge, B, false, true, a, st))) return rc;
@@ -363,7 +355,7 @@ int forward_impl(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float*
         head_fwd_kernel<<<B, NODE_THREADS, head_fwd_smem_bytes(), st>>>(hf);
         LAUNCH_CHECK(h, "head_fwd_kernel(edge)", st);
         ScoreArgs s{};
-        s.lab = in.adj; s.PR = F(h, "PRE"); s.PC = F(h, "PCE"); s.params = in.params;
+        s.bits = in.ebits; s.PR = F(h, "PRE"); s.PC = F(h, "PCE"); s.params = in.params;
         s.o_l = po.eup_w1; s.o_w2 = po.eup_w2; s.o_b2 = po.eup_b2;
         s.soft = F(h, "SOFT");
         if ((rc = launch_score(h, "score_fwd(edge)", ge, B, false, s, st))) return rc;
@@ -372,7 +364,7 @@ int forward_impl(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float*
         PoolFwdArgs a{};
         a.Ne = h->Ne; a.Nc = h->Nc; a.Se = h->Se; a.ent = h->ent ? 1 : 0;
         a.x = in.x; a.RS1 = F(h, "RS1"); a.CS1p = F(h, "CS1P"); a.params = in.params; a.po = po;
-        a.adj = in.adj; a.pitch = h->pe; a.soft = h->edge ? F(h, "SOFT") : nullptr;
+        a.bits = in.ebits; a.WP = h->WPe; a.soft = h->edge ? F(h, "SOFT") : nullptr;
         a.hmap = in.hmap; a.L = in.L;
         a.S1 = F(h, "S1"); a.X2 = F(h, "X2"); a.NB = F(h, "NB"); a.PH = F(h, "PH"); a.QH = F(h, "QH");
         PROF_BEGIN(h, st);
@@ -381,7 +373,7 @@ int forward_impl(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float*
     }
     {
         PairSumArgs a{};
-        a.lab = in.Y; a.params = in.params; a.o_l = po.hnk_w1 + 8 * HD;
+        a.bits = in.ybits; a.params = in.params; a.o_l = po.hnk_w1 + 8 * HD;
         a.Ptab = F(h, "PH"); a.Qtab = F(h, "QH");
         a.RS = F(h, "RS3"); a.CSp = F(h, "CS3P");
         if ((rc = launch_pairsum(h, "pairsum_fwd(hunk)", gc, B, false, false, a, st))) return rc;
@@ -396,7 +388,7 @@ int forward_impl(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float*
     }
     {
         ScoreArgs s{};
-        s.lab = in.Y; s.PR = F(h, "PR"); s.PC = F(h, "PC"); s.params = in.params;
+        s.bits = in.ybits; s.PR = F(h, "PR"); s.PC = F(h, "PC"); s.params = in.params;
         s.o_l = po.scr_w1; s.o_w2 = po.scr_w2; s.o_b2 = po.scr_b2;
         s.logits = logits; s.probs = probs; s.cep = F(h, "CEP");
         s.scale = 10.f / ((float)B_global * (float)(h->Nc * (h->Nc - 1)));
@@ -427,7 +419,7 @@ int backward_impl(hdgnn_handle_t h, int B, const Inputs& in, float* grads, cudaS
     }
     {
         PairSumArgs a{};
-        a.lab = in.Y; a.params = in.params; a.o_l = po.hnk_w1 + 8 * HD;
+        a.bits = in.ybits; a.params = in.params; a.o_l = po.hnk_w1 + 8 * HD;
         a.Ptab = F(h, "PH"); a.Qtab = F(h, "QH"); a.GR = F(h, "GRH"); a.GC = F(h, "GCH");
         a.RS = F(h, "RS3D"); a.CSp = F(h, "CS3DP"); a.LSp = F(h, "LS3P");
         if ((rc = launch_pairsum(h, "pairsum_bwd(hunk)", gc, B, true, false, a, st))) return rc;
@@ -446,7 +438,7 @@ int backward_impl(hdgnn_handle_t h, int B, const Inputs& in, float* grads, cudaS
     }
     if (h->ent) {
         PairSumArgs a{};
-        a.lab = in.adj; a.params = in.params; a.x = in.x;
+        a.bits = in.ebits; a.params = in.params; a.x = in.x;
         a.o_u = po.ent_w1; a.o_v = po.ent_w1 + HD; a.o_b = po.ent_b1; a.o_l = po.ent_w1 + 2 * HD;
         a.GR = F(h, "GE"); a.GC = F(h, "GE");
         a.RS = F(h, "RS1D"); a.CSp = F(h, "CS1DP"); a.LSp = F(h, "LS1P");
@@ -461,7 +453,7 @@ int backward_impl(hdgnn_handle_t h, int B, const Inputs& in, float* grads, cudaS
     }
     if (h->edge) {
         ScoreArgs s{};
-        s.lab = in.adj; s.PR = F(h, "PRE"); s.PC = F(h, "PCE"); s.params = in.params;
+        s.bits = in.ebits; s.PR = F(h, "PRE"); s.PC = F(h, "PCE"); s.params = in.params;
         s.o_l = po.eup_w1; s.o_w2 = po.eup_w2; s.o_b2 = po.eup_b2;
         s.dsoft = F(h, "DSOFT");
         s.RSm = F(h, "RSME"); s.CSmp = F(h, "CSMEP"); s.LSmp = F(h, "LSMEP"); s.HSp = F(h, "HSEP"); s.dsump = F(h, "DSUMEP");
@@ -475,7 +467,7 @@ int backward_impl(hdgnn_handle_t h, int B, const Inputs& in, float* grads, cudaS
         head_bwd_kernel<<<B, NODE_THREADS, head_bwd_smem_bytes(), st>>>(a);
         LAUNCH_CHECK(h, "head_bwd_kernel(edge)", st);
         PairSumArgs p{};
-        p.lab = in.adj; p.params = in.params; p.x = in.x;
+        p.bits = in.ebits; p.params = in.params; p.x = in.x;
         p.o_u = po.edg_w11; p.o_v = po.edg_w11; p.o_b = po.edg_b1; p.o_l = po.edg_w12;
         p.GR = F(h, "GRE"); p.GC = F(h, "GCE");
         p.RS = F(h, "RSED"); p.CSp = F(h, "CSEDP"); p.LSp = F(h, "LSEP");
@@ -526,7 +518,7 @@ __global__ void repitch_kernel(const uint8_t* __restrict__ src, uint8_t* __restr
 }
 
 // ================================================================================================
-// fused path: pack_bits -> ent_fwd2 -> mid2 -> ent_bwd2 -> reduce (+ adam)
+// pack step (both paths); fused path: ent_fwd2 -> mid2 -> ent_bwd2 -> reduce (+ adam)
 // ================================================================================================
 
 struct AdamArgs { float* params; float* m; float* v; int32_t* step; float lr, b1, b2, eps; float* reg; bool peer = false; };
@@ -558,7 +550,7 @@ int ent2_occupancy(const hdgnn_config_t& cfg, int nsm, bool bwd) {
 
 Ent2Args ent2_args(hdgnn_handle_t h, int B, const Inputs& in) {
     Ent2Args a{};
-    a.bits = h->eb; a.WP = h->WPe; a.N = h->Ne; a.B = B;
+    a.bits = in.ebits; a.WP = h->WPe; a.N = h->Ne; a.B = B;
     a.params = in.params; a.x = in.x;
     a.o_u = h->po.ent_w1; a.o_v = h->po.ent_w1 + HD; a.o_b = h->po.ent_b1; a.o_l = h->po.ent_w1 + 2 * HD;
     return a;
@@ -576,28 +568,32 @@ int debug_scatter(hdgnn_handle_t h, int B, cudaStream_t st) {
     return HDGNN_OK;
 }
 
-int fused_forward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float* logits, float* probs, bool train,
+// Byte grids adj / Y -> the label bitmaps of the step, in.ebits / in.ybits: a staging slot's bitmap sections when the host
+// entry points stage them, else the next of the two alternating EBITS / YBITS buffers (pack_bits may overlap the previous
+// step's last kernel, pack.cuh).
+int pack_step(hdgnn_handle_t h, int B, const uint8_t* adj, const uint8_t* Y, Inputs& in, cudaStream_t st) {
+    if (!in.ebits) {
+        h->bslot ^= 1;
+        in.ebits = (const uint32_t*)h->ws[h->bslot ? "EBITS1" : "EBITS0"].p;
+        in.ybits = (const uint32_t*)h->ws[h->bslot ? "YBITS1" : "YBITS0"].p;
+    }
+    PackArgs p{};
+    p.adj = adj; p.Ne = h->Ne; p.pe = h->pe; p.WPe = h->WPe; p.ebits = const_cast<uint32_t*>(in.ebits);
+    p.Y = Y; p.Nc = h->Nc; p.pc = h->pc; p.WPc = h->WPc; p.ybits = const_cast<uint32_t*>(in.ybits);
+    p.B = B;
+    const long long rows = (long long)B * (h->Ne + h->Nc);
+    PROF_BEGIN(h, st);
+    if (h->pe <= 256 && h->pc <= 256) launch_ex(pack_bits_kernel<16>, (int)((rows + 15) / 16), 256, 0, st, h->plan.pdl, p);
+    else launch_ex(pack_bits_kernel<32>, (int)((rows + 7) / 8), 256, 0, st, h->plan.pdl, p);
+    LAUNCH_CHECK(h, "pack_bits", st);
+    return HDGNN_OK;
+}
+
+// head: no pack_bits in front of the step.  Its first kernel then follows the previous step's optimizer kernel directly and
+// reads the weights it updates: ent_fwd2 defers those loads behind its pdl_wait (Ent2Args::head), mid2 is launched normally
+int fused_forward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float* logits, float* probs, bool train, bool head,
                   cudaStream_t st) {
     const FusedPlan& P = h->plan; const Mid2Mode& md = P.mode[train];
-    // bitmaps given: nothing to pack.  The first kernel then follows the previous step's optimizer kernel directly and reads
-    // the weights it updates: ent_fwd2 defers those loads behind its pdl_wait (Ent2Args::head), mid2 is launched normally
-    const bool head = in.ebits != nullptr;
-    if (head) {
-        h->eb = in.ebits; h->yb = in.ybits;
-    } else {
-        h->bslot ^= 1;
-        h->eb = (const uint32_t*)h->ws[h->bslot ? "EBITS1" : "EBITS0"].p;
-        h->yb = (const uint32_t*)h->ws[h->bslot ? "YBITS1" : "YBITS0"].p;
-        PackArgs p{};
-        p.adj = in.adj; p.Ne = h->Ne; p.pe = h->pe; p.WPe = h->WPe; p.ebits = (uint32_t*)h->ws[h->bslot ? "EBITS1" : "EBITS0"].p;
-        p.Y = in.Y; p.Nc = h->Nc; p.pc = h->pc; p.WPc = h->WPc; p.ybits = (uint32_t*)h->ws[h->bslot ? "YBITS1" : "YBITS0"].p;
-        p.B = B;
-        const long long rows = (long long)B * (h->Ne + h->Nc);
-        PROF_BEGIN(h, st);
-        if (h->pe <= 256 && h->pc <= 256) launch_ex(pack_bits_kernel<16>, (int)((rows + 15) / 16), 256, 0, st, P.pdl, p);
-        else launch_ex(pack_bits_kernel<32>, (int)((rows + 7) / 8), 256, 0, st, P.pdl, p);
-        LAUNCH_CHECK(h, "pack_bits", st);
-    }
     int G, R = 0, SL = 0;       // grid and row chunks of ent_fwd2, which mid2 reads back
     if (P.dense) {
         Ent2Args a = ent2_args(h, B, in);
@@ -611,8 +607,8 @@ int fused_forward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float
     }
     Mid2Args m{};
     m.Ne = h->Ne; m.Nc = h->Nc; m.ent = h->ent ? 1 : 0; m.R = R; m.SL = SL;
-    m.ebits = h->eb; m.WPe = h->WPe;
-    m.ybits = h->yb; m.WPc = h->WPc;
+    m.ebits = in.ebits; m.WPe = h->WPe;
+    m.ybits = in.ybits; m.WPc = h->WPc;
     m.x = in.x; m.hmap = in.hmap; m.L = in.L;
     m.params = in.params; m.po = h->po; m.RS1 = F(h, "RS1"); m.CS1p = F(h, "CS1P");
     m.logits = logits; m.probs = probs; m.cep = F(h, "CEP");
@@ -679,8 +675,8 @@ int fused_backward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, floa
     return HDGNN_OK;
 }
 
-// HDGNN_F_LABEL_BITS: byte offsets of the five inputs of a batch of B commits inside one staging block (every section starts at
-// the next multiple of 16 bytes).  Host buffers laid out the same way travel in ONE DMA (stage_inputs).
+// Byte offsets of the five inputs of a batch of B commits, labels as bitmaps, inside one staging block (every section starts
+// at the next multiple of 16 bytes).  Host buffers laid out the same way travel in ONE DMA (stage_inputs).
 struct WireOff { size_t eb, yb, x, hm, L, total; };
 WireOff wire_layout(hdgnn_handle_t h, int B) {
     WireOff w{};
@@ -855,9 +851,10 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
     h->RTe = pick_rt(h->Ne, cfg->max_batch, cfg->rows_per_cta_e);
     h->RTc = pick_rt(h->Nc, cfg->max_batch, cfg->rows_per_cta_c);
     h->Se = (h->Ne + h->RTe - 1) / h->RTe; h->Sc = (h->Nc + h->RTc - 1) / h->RTc;
+    h->WPe = bit_words(h->Ne); h->WPc = bit_words(h->Nc);
 
-    const size_t smem_need[] = {pairsum_smem_bytes(h->CWe, h->RTe, h->pe, true), score_smem_bytes(h->CWe, h->RTe, h->pe, true),
-                                pairsum_smem_bytes(h->CWc, h->RTc, h->pc, true), score_smem_bytes(h->CWc, h->RTc, h->pc, true)};
+    const size_t smem_need[] = {pairsum_smem_bytes(h->CWe, h->RTe, 4 * h->WPe, true), score_smem_bytes(h->CWe, h->RTe, 4 * h->WPe, true),
+                                pairsum_smem_bytes(h->CWc, h->RTc, 4 * h->WPc, true), score_smem_bytes(h->CWc, h->RTc, 4 * h->WPc, true)};
     for (size_t s : smem_need)
         if (s > (size_t)prop.sharedMemPerBlockOptin) {
             delete h;
@@ -865,16 +862,11 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
         }
     h->debug = (cfg->flags & HDGNN_F_DEBUG) != 0;
     h->nsm = prop.multiProcessorCount;
-    h->WPe = bit_words(h->Ne); h->WPc = bit_words(h->Nc);
     h->cwt = ent2_cwt(h->Ne);
     cudaError_t e;
     h->plan = plan_fused(*cfg, (int)prop.sharedMemPerBlockOptin, h->nsm, &e);
     const FusedPlan& P = h->plan;
     h->host_bits = (cfg->flags & HDGNN_F_LABEL_BITS) != 0;
-    if (h->host_bits && !P.mode[1].fused) {
-        delete h;
-        return fail(nullptr, HDGNN_E_UNSUPPORTED, "HDGNN_F_LABEL_BITS needs the fused training path (Nc <= 256, per-commit state within one SM)");
-    }
     if (e == cudaSuccess) e = set_attrs(h, (int)prop.sharedMemPerBlockOptin);
     if (e != cudaSuccess) {
         std::string m = std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(e);
@@ -904,8 +896,9 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
         {"RS1D", B * Ne * HD * f, h->ent && lg}, {"CS1DP", B * Se * Ne * HD * f, h->ent && lg}, {"LS1P", B * Se * HD * f, h->ent && lg},
         {"GPART", 2 * B * (size_t)h->po.total * f, true},       // second half: spare rows of the cluster form (mid2.cuh)
         {"GPE", ((size_t)Gb_max + 1) * 4 * HD * f, fused && h->ent}, {"FIN_L2", 256 * f, fused}, {"FIN_CNT", 16, fused},
-        {"EBITS0", B * Ne * (size_t)h->WPe * 4, fused}, {"YBITS0", B * Nc * (size_t)h->WPc * 4, fused},
-        {"EBITS1", B * Ne * (size_t)h->WPe * 4, fused}, {"YBITS1", B * Nc * (size_t)h->WPc * 4, fused},
+        // pack_bits' output for the device entry points taking byte grids
+        {"EBITS0", B * Ne * (size_t)h->WPe * 4, !h->host_bits}, {"YBITS0", B * Nc * (size_t)h->WPc * 4, !h->host_bits},
+        {"EBITS1", B * Ne * (size_t)h->WPe * 4, !h->host_bits}, {"YBITS1", B * Nc * (size_t)h->WPc * 4, !h->host_bits},
         {"DBG", B * mid2_dbg_floats(h->Ne, h->Nc) * f, fused && h->debug},
         {"CLK", B * 24 * sizeof(long long), fused && h->debug},
         {"DLT", B * Nc * (size_t)((h->Nc + 31) / 32 * 32) * f, fused && !P.mode[1].opt.dlt_smem},
@@ -919,15 +912,13 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
         {"HSEP", B * Se * HD * f, h->edge}, {"DSUMEP", B * Se * f, h->edge},
         {"GRE", B * Ne * HD * f, h->edge}, {"GCE", B * Ne * HD * f, h->edge},
         {"RSED", B * Ne * HD * f, h->edge}, {"CSEDP", B * Se * Ne * HD * f, h->edge}, {"LSEP", B * Se * HD * f, h->edge},
-        // staging for the *_host entry points
-        {"H_ADJ0", B * Ne * (size_t)h->pe, !h->host_bits}, {"H_Y0", B * Nc * (size_t)h->pc, !h->host_bits}, {"H_X0", B * Ne * f, !h->host_bits},
+        // staging slots of the *_host entry points: the wire block [entity bitmaps][hunk bitmaps][x][hmap][L] (16-byte aligned
+        // sections), and for byte grids the pitched grids pack_bits reads (+ the un-pitched rows, re-pitched on the device)
+        {"H_WIRE0", wire_layout(h, cfg->max_batch).total, true}, {"H_WIRE1", wire_layout(h, cfg->max_batch).total, true},
+        {"H_ADJ0", B * Ne * (size_t)h->pe, !h->host_bits}, {"H_Y0", B * Nc * (size_t)h->pc, !h->host_bits},
+        {"H_ADJ1", B * Ne * (size_t)h->pe, !h->host_bits}, {"H_Y1", B * Nc * (size_t)h->pc, !h->host_bits},
         {"H_ADJ_RAW0", B * Ne * Ne, !h->host_bits && h->pe != h->Ne}, {"H_Y_RAW0", B * Nc * Nc, !h->host_bits && h->pc != h->Nc},
-        {"H_HMAP0", B * Ne * sizeof(int32_t), !h->host_bits}, {"H_L0", B * sizeof(int32_t), !h->host_bits},
-        {"H_ADJ1", B * Ne * (size_t)h->pe, !h->host_bits}, {"H_Y1", B * Nc * (size_t)h->pc, !h->host_bits}, {"H_X1", B * Ne * f, !h->host_bits},
         {"H_ADJ_RAW1", B * Ne * Ne, !h->host_bits && h->pe != h->Ne}, {"H_Y_RAW1", B * Nc * Nc, !h->host_bits && h->pc != h->Nc},
-        {"H_HMAP1", B * Ne * sizeof(int32_t), !h->host_bits}, {"H_L1", B * sizeof(int32_t), !h->host_bits},
-        // label-bitmap wire block of a staging slot: [entity bitmaps][hunk bitmaps][x][hmap][L], 16-byte aligned sections
-        {"H_WIRE0", wire_layout(h, cfg->max_batch).total, h->host_bits}, {"H_WIRE1", wire_layout(h, cfg->max_batch).total, h->host_bits},
         {"H_FLAG", 16, true}, {"H_PROBS", B * 2 * Nc * (Nc - 1) * f, true}, {"H_LOSS", 4 * f, true}, {"H_GRADS", (size_t)h->po.total * f, true},
     };
     for (auto& p : plan) {
@@ -1060,14 +1051,15 @@ int hdgnn_peer_status(hdgnn_handle_t h) {
     return HDGNN_OK;
 }
 
-// forward [+ backward [+ adam]] on device-resident inputs; dispatches to the fused or the
-// multi-kernel path.
-static int run_step(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float* logits, float* probs, float* loss,
-                    float* grads, const AdamArgs* adam, cudaStream_t st) {
-    const bool train = grads != nullptr;
+// forward [+ backward [+ adam]] on device-resident inputs: the pack step when adj / Y are byte grids (else null, and `in`
+// holds the bitmaps), then the fused or the multi-kernel path.
+static int run_step(hdgnn_handle_t h, int B, int B_global, const uint8_t* adj, const uint8_t* Y, Inputs in, float* logits,
+                    float* probs, float* loss, float* grads, const AdamArgs* adam, cudaStream_t st) {
+    const bool train = grads != nullptr, packed = adj != nullptr;
     int rc;
+    if (packed && (rc = pack_step(h, B, adj, Y, in, st))) return rc;
     if (h->plan.mode[train].fused) {
-        rc = fused_forward(h, B, B_global, in, logits, probs, train, st);
+        rc = fused_forward(h, B, B_global, in, logits, probs, train, !packed, st);
         if (rc) return rc;
 
         if (!train) {
@@ -1093,9 +1085,12 @@ static int device_step(hdgnn_handle_t h, int B, int B_global, const uint8_t* adj
                        const int32_t* L, const uint8_t* Y, const float* params, float* logits, float* probs, float* loss,
                        float* grads, const AdamArgs* adam, void* stream) {
     h->launches = 0;
-    Inputs in{adj, x, hmap, L, Y, params};
-    alias_bits(h, in);
-    return run_step(h, B, B_global, in, logits, probs, loss, grads, adam, (cudaStream_t)stream);
+    if (h->host_bits) {         // HDGNN_F_LABEL_BITS: adj / Y are the bitmaps
+        const Inputs in{(const uint32_t*)adj, (const uint32_t*)Y, x, hmap, L, params};
+        return run_step(h, B, B_global, nullptr, nullptr, in, logits, probs, loss, grads, adam, (cudaStream_t)stream);
+    }
+    const Inputs in{nullptr, nullptr, x, hmap, L, params};
+    return run_step(h, B, B_global, adj, Y, in, logits, probs, loss, grads, adam, (cudaStream_t)stream);
 }
 
 // the peer-exchange steps: peers attached, equal shards
@@ -1149,7 +1144,7 @@ int hdgnn_train_step(hdgnn_handle_t h, int B, const uint8_t* adj, int adj_pitch,
 static std::string slot_name(const char* base, int slot) { return std::string(base) + (char)('0' + slot); }
 
 static int stage_inputs(hdgnn_handle_t h, int B, const uint8_t* adj_host, const float* x_host, const int32_t* hmap_host,
-                        const int32_t* L_host, const uint8_t* Y_host, cudaStream_t st) {
+                        const int32_t* L_host, const uint8_t* Y_host, bool train, cudaStream_t st) {
     const size_t Ne = h->Ne, Nc = h->Nc;
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     cudaStreamIsCapturing(st, &cap);
@@ -1160,53 +1155,50 @@ static int stage_inputs(hdgnn_handle_t h, int B, const uint8_t* adj_host, const 
     cudaStream_t cs = side ? h->copy_stream : st;
     if (side && h->done_valid[slot]) CK(h, cudaStreamWaitEvent(cs, h->ev_done[slot], 0));
     h->cur_B = B;
-    if (h->host_bits) {
-        // one staging block per slot; host arrays that already sit back to back in that layout (one pinned block, what
-        // HostBatch builds) are copied with a single DMA, anything else section by section
-        const WireOff W = wire_layout(h, B);
-        char* base = (char*)h->ws[slot_name("H_WIRE", slot)].p;
-        const char* hb = (const char*)adj_host;
-        const bool packed = (const char*)Y_host == hb + W.yb && (const char*)x_host == hb + W.x &&
-                            (const char*)hmap_host == hb + W.hm && (const char*)L_host == hb + W.L;
-        if (packed) {
-            CK(h, cudaMemcpyAsync(base, hb, W.L + (size_t)B * 4, cudaMemcpyHostToDevice, cs));
-        } else {
-            CK(h, cudaMemcpyAsync(base + W.eb, adj_host, (size_t)B * Ne * h->WPe * 4, cudaMemcpyHostToDevice, cs));
-            CK(h, cudaMemcpyAsync(base + W.yb, Y_host, (size_t)B * Nc * h->WPc * 4, cudaMemcpyHostToDevice, cs));
-            CK(h, cudaMemcpyAsync(base + W.x, x_host, (size_t)B * Ne * sizeof(float), cudaMemcpyHostToDevice, cs));
-            CK(h, cudaMemcpyAsync(base + W.hm, hmap_host, (size_t)B * Ne * sizeof(int32_t), cudaMemcpyHostToDevice, cs));
-            CK(h, cudaMemcpyAsync(base + W.L, L_host, (size_t)B * sizeof(int32_t), cudaMemcpyHostToDevice, cs));
+    // one wire block per slot (wire_layout).  Host bitmaps that already sit back to back with x, hmap and L in that layout
+    // (one pinned block, what HostBatch builds) are copied with a single DMA, anything else section by section.  Byte grids
+    // go to the slot's pitched buffers instead, and pack_bits fills the block's bitmap sections from them (pack_step).
+    const WireOff W = wire_layout(h, B);
+    char* base = (char*)h->ws[slot_name("H_WIRE", slot)].p;
+    const char* hb = (const char*)adj_host;
+    const bool whole = h->host_bits && (const char*)Y_host == hb + W.yb && (const char*)x_host == hb + W.x &&
+                       (const char*)hmap_host == hb + W.hm && (const char*)L_host == hb + W.L;
+    if (whole) {
+        CK(h, cudaMemcpyAsync(base, hb, W.L + (size_t)B * 4, cudaMemcpyHostToDevice, cs));
+    } else if (h->host_bits) {
+        CK(h, cudaMemcpyAsync(base + W.eb, adj_host, (size_t)B * Ne * h->WPe * 4, cudaMemcpyHostToDevice, cs));
+        CK(h, cudaMemcpyAsync(base + W.yb, Y_host, (size_t)B * Nc * h->WPc * 4, cudaMemcpyHostToDevice, cs));
+    } else {
+        const uint8_t* srcs[2] = {adj_host, Y_host};
+        const char* raw[2] = {"H_ADJ_RAW", "H_Y_RAW"};
+        const char* dstn[2] = {"H_ADJ", "H_Y"};
+        const size_t n[2] = {Ne, Nc};
+        const int pitch[2] = {h->pe, h->pc};
+        for (int t = 0; t < 2; ++t) {
+            const size_t rows = (size_t)B * n[t];
+            void* dst = h->ws[slot_name(dstn[t], slot)].p;
+            if (pitch[t] == (int)n[t]) {
+                CK(h, cudaMemcpyAsync(dst, srcs[t], rows * n[t], cudaMemcpyHostToDevice, cs));
+            } else {
+                void* rawp = h->ws[slot_name(raw[t], slot)].p;
+                CK(h, cudaMemcpyAsync(rawp, srcs[t], rows * n[t], cudaMemcpyHostToDevice, cs));
+                const size_t work = rows * (size_t)pitch[t] / 4;
+                int blocks = (int)((work + 255) / 256);
+                if (blocks > 148 * 8) blocks = 148 * 8;
+                PROF_BEGIN(h, cs);
+                repitch_kernel<<<blocks, 256, 0, cs>>>((const uint8_t*)rawp, (uint8_t*)dst, rows, (int)n[t], pitch[t]);
+                LAUNCH_CHECK(h, "repitch_kernel", cs);
+            }
         }
     }
-    const uint8_t* srcs[2] = {adj_host, Y_host};
-    const char* raw[2] = {"H_ADJ_RAW", "H_Y_RAW"};
-    const char* dstn[2] = {"H_ADJ", "H_Y"};
-    const size_t n[2] = {Ne, Nc};
-    const int pitch[2] = {h->pe, h->pc};
-    for (int t = 0; t < 2 && !h->host_bits; ++t) {
-        const size_t rows = (size_t)B * n[t];
-        void* dst = h->ws[slot_name(dstn[t], slot)].p;
-        if (pitch[t] == (int)n[t]) {
-            CK(h, cudaMemcpyAsync(dst, srcs[t], rows * n[t], cudaMemcpyHostToDevice, cs));
-        } else {
-            void* rawp = h->ws[slot_name(raw[t], slot)].p;
-            CK(h, cudaMemcpyAsync(rawp, srcs[t], rows * n[t], cudaMemcpyHostToDevice, cs));
-            const size_t work = rows * (size_t)pitch[t] / 4;
-            int blocks = (int)((work + 255) / 256);
-            if (blocks > 148 * 8) blocks = 148 * 8;
-            PROF_BEGIN(h, cs);
-            repitch_kernel<<<blocks, 256, 0, cs>>>((const uint8_t*)rawp, (uint8_t*)dst, rows, (int)n[t], pitch[t]);
-            LAUNCH_CHECK(h, "repitch_kernel", cs);
-        }
-    }
-    if (!h->host_bits) {
-        CK(h, cudaMemcpyAsync(h->ws[slot_name("H_X", slot)].p, x_host, (size_t)B * Ne * sizeof(float), cudaMemcpyHostToDevice, cs));
-        CK(h, cudaMemcpyAsync(h->ws[slot_name("H_HMAP", slot)].p, hmap_host, (size_t)B * Ne * sizeof(int32_t), cudaMemcpyHostToDevice, cs));
-        CK(h, cudaMemcpyAsync(h->ws[slot_name("H_L", slot)].p, L_host, (size_t)B * sizeof(int32_t), cudaMemcpyHostToDevice, cs));
+    if (!whole) {
+        CK(h, cudaMemcpyAsync(base + W.x, x_host, (size_t)B * Ne * sizeof(float), cudaMemcpyHostToDevice, cs));
+        CK(h, cudaMemcpyAsync(base + W.hm, hmap_host, (size_t)B * Ne * sizeof(int32_t), cudaMemcpyHostToDevice, cs));
+        CK(h, cudaMemcpyAsync(base + W.L, L_host, (size_t)B * sizeof(int32_t), cudaMemcpyHostToDevice, cs));
     }
     h->cur_tag = -1;
     if (side) {
-        if (h->tag_table && h->host_bits && h->plan.mid2_first) {
+        if (h->tag_table && h->host_bits && h->plan.mode[train].fused && h->plan.mid2_first) {
             // mid2 is the first kernel of the step and reads every staged input: order it by a tag instead of an event
             const int tag = (int)(++h->slot_uses[slot] & 0xffu);
             CK(h, cudaMemcpyAsync((int*)h->ws["H_FLAG"].p + slot, h->tag_table + tag, sizeof(int), cudaMemcpyHostToDevice, cs));
@@ -1219,19 +1211,17 @@ static int stage_inputs(hdgnn_handle_t h, int B, const uint8_t* adj_host, const 
     return HDGNN_OK;
 }
 
-// device-side views of the staging slot filled by the last stage_inputs call
-static Inputs staged_inputs(hdgnn_handle_t h, const float* params) {
+// Device-side views of the staging slot filled by the last stage_inputs call: the sections of its wire block, and, for byte
+// grids, the pitched grids (*adj, *Y; null with HDGNN_F_LABEL_BITS) that the pack step turns into the block's bitmaps.
+static Inputs staged_inputs(hdgnn_handle_t h, const float* params, const uint8_t** adj, const uint8_t** Y) {
     const int s = h->cur;
-    Inputs in{(const uint8_t*)h->ws[slot_name("H_ADJ", s)].p, (const float*)h->ws[slot_name("H_X", s)].p,
-              (const int32_t*)h->ws[slot_name("H_HMAP", s)].p, (const int32_t*)h->ws[slot_name("H_L", s)].p,
-              (const uint8_t*)h->ws[slot_name("H_Y", s)].p, params};
-    if (h->host_bits) {
-        const WireOff W = wire_layout(h, h->cur_B);
-        const char* base = (const char*)h->ws[slot_name("H_WIRE", s)].p;
-        in.ebits = (const uint32_t*)(base + W.eb); in.ybits = (const uint32_t*)(base + W.yb);
-        in.x = (const float*)(base + W.x); in.hmap = (const int32_t*)(base + W.hm); in.L = (const int32_t*)(base + W.L);
-    }
+    const WireOff W = wire_layout(h, h->cur_B);
+    const char* base = (const char*)h->ws[slot_name("H_WIRE", s)].p;
+    Inputs in{(const uint32_t*)(base + W.eb), (const uint32_t*)(base + W.yb), (const float*)(base + W.x),
+              (const int32_t*)(base + W.hm), (const int32_t*)(base + W.L), params};
     if (h->cur_tag >= 0) { in.wait_flag = (const int*)h->ws["H_FLAG"].p + s; in.wait_tag = h->cur_tag; }
+    *adj = h->host_bits ? nullptr : (const uint8_t*)h->ws[slot_name("H_ADJ", s)].p;
+    *Y = h->host_bits ? nullptr : (const uint8_t*)h->ws[slot_name("H_Y", s)].p;
     return in;
 }
 
@@ -1276,15 +1266,16 @@ static int host_step(hdgnn_handle_t h, int B, int B_global, const uint8_t* adj_h
                      float* probs, float* loss, float* grads, const AdamArgs* adam, bool to_host, void* stream) {
     cudaStream_t st = (cudaStream_t)stream;
     h->launches = 0;
-    int rc = stage_inputs(h, B, adj_host, x_host, hmap_host, L_host, Y_host, st);
+    int rc = stage_inputs(h, B, adj_host, x_host, hmap_host, L_host, Y_host, grads != nullptr, st);
     if (rc) return rc;
-    const Inputs in = staged_inputs(h, params);
+    const uint8_t *adj, *Y;
+    const Inputs in = staged_inputs(h, params, &adj, &Y);
     float* probs_d = to_host && probs ? F(h, "H_PROBS") : probs;
     float* alias = to_host && adam && h->plan.mode[1].fused ? host_alias(loss) : nullptr;
     float* loss_d = to_host ? (alias ? alias : F(h, "H_LOSS")) : loss;
     AdamArgs ad{};
     if (adam) { ad = *adam; ad.reg = loss_d + 1; }
-    rc = run_step(h, B, B_global, in, nullptr, probs_d, loss_d, grads, adam ? &ad : nullptr, st);
+    rc = run_step(h, B, B_global, adj, Y, in, nullptr, probs_d, loss_d, grads, adam ? &ad : nullptr, st);
     if (rc) return rc;
     if ((rc = release_slot(h, st)) || !to_host) return rc;
     if (probs)

@@ -23,7 +23,7 @@ struct PoolFwdArgs {
     const float* CS1p;      // (B,Se,Ne,20)
     const float* params;
     ParamOff po;
-    const uint8_t* adj; int pitch;
+    const uint32_t* bits; int WP;   // (B,Ne,WP) entity label bitmap (bits.cuh)
     const float* soft;      // (B,Ne,Ne,2) soft edges (variant 4) or nullptr
     const int* hmap;        // (B,Ne)
     const int* L;           // (B)
@@ -126,7 +126,7 @@ __global__ void __launch_bounds__(NODE_THREADS) pool_fwd_kernel(const PoolFwdArg
                 const float2 s2 = reinterpret_cast<const float2*>(a.soft)[((size_t)b * Ne + gi) * Ne + gj];
                 v2 = s2.x; v3 = s2.y;
             } else {
-                v3 = a.adj[((size_t)b * Ne + gi) * a.pitch + gj] != 0 ? 1.f : 0.f;
+                v3 = (a.bits[((size_t)b * Ne + gi) * a.WP + (gj >> 5)] >> (gj & 31)) & 1u ? 1.f : 0.f;
                 v2 = 1.f - v3;
             }
             acc0 += x2s[gi]; acc1 += x2s[gj]; acc2 += v2; acc3 += v3;

@@ -2,7 +2,7 @@
 //
 // For one commit and an N x N grid of ordered pairs (i != j) it evaluates the first layer of a
 // per-pair MLP in the separable form
-//        pre_ij[k] = P_i[k] + Q_j[k] + l_ij * D[k]          l_ij in {0,1} from the byte grid
+//        pre_ij[k] = P_i[k] + Q_j[k] + l_ij * D[k]          l_ij in {0,1} from the label bitmap
 // and reduces over the grid.  Because the second layer of every pair MLP in the reference is
 // linear and immediately row/column-summed by a one-hot matmul (model_2.py:172-188 entity
 // effects, model_2.py:263-275 hunk "edge translation", model_4.py:226-240 entity-edge effects)
@@ -15,7 +15,7 @@
 // Mapping: grid (S row tiles, B commits); one warp per hidden channel k (20 warps); lane owns
 // columns j = seg*32 + lane, seg < CW (column sums live in registers for the whole tile); rows
 // are swept four at a time, their sums reduced across lanes by a fixed-order shuffle butterfly.
-// The label tile (RT rows x pitch bytes, contiguous) is staged by one 1-D TMA bulk copy and
+// The label tile (RT bitmap rows of WP words, contiguous) is staged by one 1-D TMA bulk copy and
 // re-packed once per CTA into float4 {l(i..i+3, j)} so the inner loop issues one LDS.128 per four
 // pairs.  The diagonal pair (i,i) is carried through with l = 0 and subtracted once at the
 // end.  No atomics: every sum has a fixed order.
@@ -25,8 +25,8 @@
 namespace hdgnn {
 
 struct PairSumArgs {
-    const uint8_t* lab;   // (B, N, pitch) bytes
-    int pitch;
+    const uint32_t* bits; // (B, N, WP) label bitmap (bits.cuh)
+    int WP;
     int N, RT, S;         // grid size, rows per CTA (multiple of 4, >= 20), row tiles
     const float* params;
     // RANK1: P_i = x_i*par[o_u+k] + par[o_b+k] + par[o_l+k];  Q_j = x_j*par[o_v+k]
@@ -43,8 +43,8 @@ struct PairSumArgs {
     float* LSp;           // BWD: (B,S,20)
 };
 
-__host__ __device__ inline size_t pairsum_smem_bytes(int CW, int RT, int pitch, bool bwd) {
-    size_t off = round_up(RT * pitch, 128);
+__host__ __device__ inline size_t pairsum_smem_bytes(int CW, int RT, int row_bytes, bool bwd) {
+    size_t off = round_up(RT * row_bytes, 128);
     size_t labf = (size_t)(RT / 4) * (CW * 32) * 16;
     size_t cst = (size_t)(CW * 32) * HD * 4;
     off += labf > cst ? labf : cst;
@@ -56,14 +56,14 @@ template <int CW, bool BWD, bool RANK1>
 __global__ void __launch_bounds__(32 * HD) pairsum_kernel(const PairSumArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     constexpr int NP = CW * 32;
-    const int N = a.N, RT = a.RT, pitch = a.pitch;
+    const int N = a.N, RT = a.RT, WP = a.WP;
     const int b = blockIdx.y, s = blockIdx.x;
     const int r0 = s * RT;
     const int nrows = min(RT, N - r0);
     const int tid = threadIdx.x, lane = tid & 31, k = tid >> 5;
 
-    uint8_t* stage = smem;
-    size_t off = round_up(RT * pitch, 128);
+    uint32_t* stage = reinterpret_cast<uint32_t*>(smem);
+    size_t off = round_up(RT * WP * 4, 128);
     float4* labf = reinterpret_cast<float4*>(smem + off);
     float* CSt = reinterpret_cast<float*>(smem + off);          // reused after the sweep
     {
@@ -79,9 +79,9 @@ __global__ void __launch_bounds__(32 * HD) pairsum_kernel(const PairSumArgs a) {
     if (tid == 0) { mbar_init(bar, 1); fence_mbar_init(); }
     __syncthreads();
     if (tid == 0) {
-        const uint32_t bytes = (uint32_t)nrows * pitch;
+        const uint32_t bytes = (uint32_t)nrows * WP * 4;
         mbar_arrive_expect_tx(bar, bytes);
-        bulk_g2s(stage, a.lab + ((size_t)b * N + r0) * pitch, bytes, bar);
+        bulk_g2s(stage, a.bits + ((size_t)b * N + r0) * WP, bytes, bar);
     }
 
     const float* par = a.params;
@@ -110,7 +110,7 @@ __global__ void __launch_bounds__(32 * HD) pairsum_kernel(const PairSumArgs a) {
             if (BWD) GCr[seg] = a.GC[((size_t)b * N + j) * HD + k];
         }
     }
-    // labels: bytes -> float4 {rows 4rq..4rq+3} per column; diagonal and padding -> 0
+    // labels: bits -> float4 {rows 4rq..4rq+3} per column; diagonal and padding -> 0
     mbar_wait(bar, 0);
     for (int idx = tid; idx < (RT / 4) * NP; idx += blockDim.x) {
         const int rq = idx / NP, c = idx - rq * NP;
@@ -118,7 +118,7 @@ __global__ void __launch_bounds__(32 * HD) pairsum_kernel(const PairSumArgs a) {
 #pragma unroll
         for (int r = 0; r < 4; ++r) {
             const int row = 4 * rq + r;
-            v[r] = (row < nrows && c < N && c != r0 + row && stage[row * pitch + c] != 0) ? 1.f : 0.f;
+            v[r] = (row < nrows && c < N && c != r0 + row && ((stage[row * WP + (c >> 5)] >> (c & 31)) & 1u)) ? 1.f : 0.f;
         }
         labf[idx] = make_float4(v[0], v[1], v[2], v[3]);
     }

@@ -18,8 +18,8 @@
 namespace hdgnn {
 
 struct ScoreArgs {
-    const uint8_t* lab;
-    int pitch;
+    const uint32_t* bits; // (B, N, WP) label bitmap (bits.cuh)
+    int WP;
     int N, RT, S;
     const float* PR;      // (B,N,20), bias + label-0 row folded in
     const float* PC;      // (B,N,20)
@@ -38,9 +38,9 @@ struct ScoreArgs {
     float* dsump;         // (B,S)
 };
 
-__host__ __device__ inline size_t score_smem_bytes(int CW, int RT, int pitch, bool train) {
+__host__ __device__ inline size_t score_smem_bytes(int CW, int RT, int row_bytes, bool train) {
     const size_t NP = (size_t)CW * 32;
-    size_t off = round_up(RT * pitch, 128);
+    size_t off = round_up(RT * row_bytes, 128);
     size_t labf = (size_t)(RT / 4) * NP * 16;
     size_t cst = NP * HD * 4;
     off += labf > cst ? labf : cst;
@@ -55,14 +55,14 @@ template <int CW, bool TRAIN>
 __global__ void __launch_bounds__(32 * HD, 1) score_kernel(const ScoreArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     constexpr int NP = CW * 32;
-    const int N = a.N, RT = a.RT, pitch = a.pitch;
+    const int N = a.N, RT = a.RT, WP = a.WP;
     const int b = blockIdx.y, s = blockIdx.x;
     const int r0 = s * RT;
     const int nrows = min(RT, N - r0);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 
-    uint8_t* stage = smem;
-    size_t off = round_up(RT * pitch, 128);
+    uint32_t* stage = reinterpret_cast<uint32_t*>(smem);
+    size_t off = round_up(RT * WP * 4, 128);
     float4* labf = reinterpret_cast<float4*>(smem + off);
     float* CSt = reinterpret_cast<float*>(smem + off);
     const size_t labf_bytes = (size_t)(RT / 4) * NP * 16;
@@ -81,9 +81,9 @@ __global__ void __launch_bounds__(32 * HD, 1) score_kernel(const ScoreArgs a) {
     if (tid == 0) { mbar_init(bar, 1); fence_mbar_init(); }
     __syncthreads();
     if (tid == 0) {
-        const uint32_t bytes = (uint32_t)nrows * pitch;
+        const uint32_t bytes = (uint32_t)nrows * WP * 4;
         mbar_arrive_expect_tx(bar, bytes);
-        bulk_g2s(stage, a.lab + ((size_t)b * N + r0) * pitch, bytes, bar);
+        bulk_g2s(stage, a.bits + ((size_t)b * N + r0) * WP, bytes, bar);
     }
     const float* par = a.params;
     if (tid < HD) {
@@ -107,7 +107,7 @@ __global__ void __launch_bounds__(32 * HD, 1) score_kernel(const ScoreArgs a) {
 #pragma unroll
         for (int r = 0; r < 4; ++r) {
             const int row = 4 * rq + r;
-            v[r] = (row < nrows && c < N && c != r0 + row && stage[row * pitch + c] != 0) ? 1.f : 0.f;
+            v[r] = (row < nrows && c < N && c != r0 + row && ((stage[row * WP + (c >> 5)] >> (c & 31)) & 1u)) ? 1.f : 0.f;
         }
         labf[idx] = make_float4(v[0], v[1], v[2], v[3]);
         if (TRAIN) delt[idx] = make_float4(0.f, 0.f, 0.f, 0.f);

@@ -15,7 +15,6 @@ from typing import Optional
 import numpy as np
 import torch
 
-from . import _lib
 from .engine import Engine, DeviceBatch, param_count, param_offsets, PARAM_NAMES, F_LABEL_BITS, F_DENSE_SWEEP, pack_label_bits
 from .synthetic import CommitBatch
 
@@ -172,14 +171,9 @@ class graph2graph(object):
     # ------------------------------------------------------------------------------------------
     def build_model(self):
         torch.cuda.set_device(self.device)
-        extra = F_DENSE_SWEEP if self._dense else 0
-        try:        # label grids as bitmaps on the wire (1/8 of the H2D bytes, no packing kernel): fused path only
-            self.engine = Engine(self.Ne, self.Nc, variant=self.variant, max_batch=self.max_batch, device=self.device,
-                                 flags=F_LABEL_BITS | extra)
-        except _lib.HdgnnError as e:
-            if e.code != _lib.E_UNSUPPORTED:
-                raise
-            self.engine = Engine(self.Ne, self.Nc, variant=self.variant, max_batch=self.max_batch, device=self.device, flags=extra)
+        # label grids as bitmaps on the wire (1/8 of the H2D bytes, no packing kernel)
+        self.engine = Engine(self.Ne, self.Nc, variant=self.variant, max_batch=self.max_batch, device=self.device,
+                             flags=F_LABEL_BITS | (F_DENSE_SWEEP if self._dense else 0))
         self.host_bits = self.engine.host_bits
         self.n_params = param_count(self.variant)
         self.offsets = param_offsets(self.variant)

@@ -74,8 +74,7 @@ typedef struct {
                                (B, Ne, hdgnn_bit_words(Ne)) uint32 and Y / Y_host (B, Nc, hdgnn_bit_words(Nc)) uint32, word w of a
                                row holding column 32 w + k at bit k (little-endian np.packbits order), diagonal and padding
                                bits ZERO; adj_pitch / y_pitch = 4 * hdgnn_bit_words(n).  1/8 of the bytes on the wire and
-                               in HBM and no packing kernel; fused path only (Nc <= 256; hdgnn_create fails with
-                               HDGNN_E_UNSUPPORTED otherwise).  The *_host entry points copy the five arrays with ONE DMA when
+                               in HBM and no packing kernel; the same results as byte grids.  The *_host entry points copy the five arrays with ONE DMA when
                                they sit back to back in one pinned block in the order adj, Y, x, hmap, L, every array starting
                                at the next multiple of 16 bytes (what hdgnn_b200.model.HostBatch builds); any other placement
                                is copied array by array.  hdgnn_pack_label_bits builds the format on the device. */

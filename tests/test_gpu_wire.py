@@ -1,10 +1,18 @@
 """The bit-packed wire format of the *_host entry points (HDGNN_F_LABEL_BITS): same kernels, same bitmaps, so a training
-run fed with host bitmaps is BITWISE identical to one fed with byte grids (which the device packs itself)."""
+run fed with host bitmaps is BITWISE identical to one fed with byte grids (which the device packs itself) -- on the fused
+path and on the multi-kernel path alike."""
 import numpy as np
 import pytest
 import torch
 
 from hdgnn_b200.synthetic import make_commits
+
+F_LEGACY = 4
+
+# (variant, Ne, Nc, B, extra flags): the fused path; HDGNN_F_LEGACY (the multi-kernel path) at variants 2 and 4; training
+# above 256 hunks, which runs on the multi-kernel path while its forward-only step stays fused
+WIRE_CASES = [(2, 48, 20, 5, 0), (2, 200, 74, 12, 0), (1, 33, 9, 4, 0), (3, 64, 40, 3, 0), (2, 250, 150, 3, 0),
+              (2, 200, 74, 12, F_LEGACY), (4, 200, 74, 6, F_LEGACY), (2, 48, 300, 3, 0)]
 
 
 def test_pack_label_bits_layout():
@@ -22,13 +30,14 @@ def test_pack_label_bits_layout():
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("variant,Ne,Nc,B", [(2, 48, 20, 5), (2, 200, 74, 12), (1, 33, 9, 4), (3, 64, 40, 3), (2, 250, 150, 3)])
-def test_host_bits_training_is_bitwise_identical_to_byte_grids(variant, Ne, Nc, B):
+@pytest.mark.parametrize("variant,Ne,Nc,B,extra", WIRE_CASES,
+                         ids=["-".join(map(str, c[:4])) + ("-legacy" if c[4] else "") for c in WIRE_CASES])
+def test_host_bits_training_is_bitwise_identical_to_byte_grids(variant, Ne, Nc, B, extra):
     from hdgnn_b200.engine import Engine, F_LABEL_BITS
     from hdgnn_b200.model import HostBatch, truncated_normal_init
     res = []
     for flags in (0, F_LABEL_BITS):
-        eng = Engine(Ne, Nc, variant=variant, max_batch=B, flags=flags)
+        eng = Engine(Ne, Nc, variant=variant, max_batch=B, flags=flags | extra)
         params = truncated_normal_init(variant, 3).cuda()
         m = torch.zeros_like(params); v = torch.zeros_like(params)
         step = torch.zeros(1, dtype=torch.int32, device="cuda")
@@ -67,40 +76,29 @@ def test_device_packer_equals_host_packer(n):
 
 @pytest.mark.gpu
 def test_label_bits_device_entry_points_bitwise():
-    """Device-resident bitmaps through hdgnn_train_step / hdgnn_forward == byte grids."""
+    """Device-resident bitmaps through hdgnn_train_step / hdgnn_forward == byte grids, on the fused path and (HDGNN_F_LEGACY)
+    on the multi-kernel path."""
     from hdgnn_b200.engine import Engine, DeviceBatch, F_LABEL_BITS
     from hdgnn_b200.model import truncated_normal_init
     Ne, Nc, B, variant = 200, 74, 8, 2
     cb = make_commits(B, Ne, Nc, seed=9)
-    out = []
-    for flags in (0, F_LABEL_BITS):
-        eng = Engine(Ne, Nc, variant=variant, max_batch=B, flags=flags)
-        db = DeviceBatch.from_numpy(cb.adj, cb.x, cb.hmap, cb.L, cb.Y, eng.tdev, bits=bool(flags))
-        params = truncated_normal_init(variant, 3).cuda()
-        m = torch.zeros_like(params); v = torch.zeros_like(params)
-        step = torch.zeros(1, dtype=torch.int32, device="cuda"); loss3 = torch.zeros(3, device="cuda")
-        probs = torch.zeros(B, 2, Nc * (Nc - 1), device="cuda")
-        for _ in range(2):
-            eng.train_step(db, params, m, v, step, loss3, probs=probs)
-        p2, _, l2 = eng.forward(db, params, want_logits=False)
-        torch.cuda.synchronize()
-        out.append((params.cpu().numpy(), probs.cpu().numpy(), loss3.cpu().numpy(), p2.cpu().numpy(), l2.cpu().numpy(), eng.last_launch_count()))
-        eng.close()
-    for k in range(5):
-        assert np.array_equal(out[0][k], out[1][k]), k
-
-
-@pytest.mark.gpu
-def test_host_bits_refused_on_the_multi_kernel_path():
-    from hdgnn_b200 import _lib
-    from hdgnn_b200.engine import Engine, F_LABEL_BITS
-    with pytest.raises(_lib.HdgnnError) as e:
-        Engine(48, 300, variant=2, max_batch=4, flags=F_LABEL_BITS)         # Nc > 256: per-commit state beyond one SM
-    assert e.value.code == _lib.E_UNSUPPORTED
-    with pytest.raises(_lib.HdgnnError) as e:
-        Engine(48, 20, variant=4, max_batch=4, flags=F_LABEL_BITS | 4)      # HDGNN_F_LEGACY forces the multi-kernel path
-    assert e.value.code == _lib.E_UNSUPPORTED
-    Engine(48, 20, variant=4, max_batch=4, flags=F_LABEL_BITS).close()      # variant 4 runs on the fused path now
+    for extra in (0, F_LEGACY):
+        out = []
+        for flags in (0, F_LABEL_BITS):
+            eng = Engine(Ne, Nc, variant=variant, max_batch=B, flags=flags | extra)
+            db = DeviceBatch.from_numpy(cb.adj, cb.x, cb.hmap, cb.L, cb.Y, eng.tdev, bits=bool(flags))
+            params = truncated_normal_init(variant, 3).cuda()
+            m = torch.zeros_like(params); v = torch.zeros_like(params)
+            step = torch.zeros(1, dtype=torch.int32, device="cuda"); loss3 = torch.zeros(3, device="cuda")
+            probs = torch.zeros(B, 2, Nc * (Nc - 1), device="cuda")
+            for _ in range(2):
+                eng.train_step(db, params, m, v, step, loss3, probs=probs)
+            p2, _, l2 = eng.forward(db, params, want_logits=False)
+            torch.cuda.synchronize()
+            out.append((params.cpu().numpy(), probs.cpu().numpy(), loss3.cpu().numpy(), p2.cpu().numpy(), l2.cpu().numpy(), eng.last_launch_count()))
+            eng.close()
+        for k in range(5):
+            assert np.array_equal(out[0][k], out[1][k]), (extra, k)
 
 
 @pytest.mark.gpu

@@ -3,17 +3,13 @@ Prints commits/s and hunk pairs/s for the device-resident forward (hdgnn_forward
 import json, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
-from hdgnn_b200 import _lib
 from hdgnn_b200.engine import Engine, DeviceBatch, F_LABEL_BITS, eval_counts
 from hdgnn_b200.synthetic import make_commits
 
 B, Ne = 100, 200
 out = []
 for Nc in (74, 114, 150, 256, 384, 512):
-    try:        # label bitmaps resident in HBM on the fused path, byte grids on the multi-kernel path
-        eng = Engine(Ne, Nc, variant=2, max_batch=B, flags=F_LABEL_BITS)
-    except _lib.HdgnnError:
-        eng = Engine(Ne, Nc, variant=2, max_batch=B)
+    eng = Engine(Ne, Nc, variant=2, max_batch=B, flags=F_LABEL_BITS)      # label bitmaps resident in HBM
     pool, ybytes = [], []
     for i in range(8):
         cb = make_commits(B, Ne, Nc, seed=20260 + i)
