@@ -30,7 +30,7 @@
 #include <stdlib.h>
 #include <string.h>
 
-#include <map>
+#include <array>
 #include <string>
 #include <tuple>
 #include <vector>
@@ -99,6 +99,26 @@ ParamOff make_off(int variant) {
 
 struct Buf { void* p = nullptr; size_t bytes = 0; };
 
+// The handle's scratch buffers, in the order hdgnn_create allocates them (workspace_bytes sizes them).  The buffers of the
+// two staging slots of the *_host entry points are adjacent ids, base + slot.  hdgnn_peer_attach allocates PEER_SEQ and
+// PEER_STAMPS.
+#define HDGNN_WORKSPACE(X)                                                                                                  \
+    X(RS1) X(CS1P) X(S1) X(X2) X(NB) X(PH) X(QH) X(RS3) X(CS3P) X(CS3F) X(PR) X(PC) X(CEP)                                 \
+    X(RSM) X(CSMP) X(LSMP) X(HSP) X(DSUMP) X(GRH) X(GCH) X(RS3D) X(CS3DP) X(LS3P) X(DNB) X(GE) X(DX2)                      \
+    X(RS1D) X(CS1DP) X(LS1P) X(GPART) X(GPE) X(FIN_L2) X(FIN_CNT) X(EBITS0) X(EBITS1) X(YBITS0) X(YBITS1)                  \
+    X(DBG) X(CLK) X(DLT) X(TABS) X(RSEG) X(CSEG) X(REG) X(CEG) X(A1F) X(PREG)                                               \
+    X(RSE) X(CSEP) X(CSEF) X(PRE) X(PCE) X(SOFT) X(DSOFT) X(RSME) X(CSMEP) X(LSMEP) X(HSEP) X(DSUMEP)                      \
+    X(GRE) X(GCE) X(RSED) X(CSEDP) X(LSEP)                                                                                  \
+    X(H_WIRE0) X(H_WIRE1) X(H_ADJ0) X(H_ADJ1) X(H_Y0) X(H_Y1) X(H_ADJ_RAW0) X(H_ADJ_RAW1) X(H_Y_RAW0) X(H_Y_RAW1)          \
+    X(H_FLAG) X(H_PROBS) X(H_LOSS) X(H_GRADS) X(PEER_SEQ) X(PEER_STAMPS)
+
+#define WS_ID(n) WS_##n,
+enum WsId { HDGNN_WORKSPACE(WS_ID) WS_COUNT };
+#undef WS_ID
+#define WS_NAME(n) #n,
+const char* const kWsName[WS_COUNT] = {HDGNN_WORKSPACE(WS_NAME)};
+#undef WS_NAME
+
 // mid2 in one mode of a handle (FusedPlan::mode[0]: forward only, mode[1]: training)
 struct Mid2Mode {
     bool fused = false;        // this mode runs on the fused path, else on the multi-kernel path
@@ -137,7 +157,7 @@ struct hdgnn_handle_s {
     int nsm = 148;
     int cwt = 0;                                               // column segments per pass of the entity sweeps (ent2.cuh)
     int bslot = 0;                                             // bitmap buffer of the current device-fed step (two alternate)
-    std::map<std::string, Buf> ws;
+    Buf ws[WS_COUNT];                                          // p = nullptr: not allocated for this handle
     std::string err;
     int launches = 0;
     // opt-in per-launch timing (hdgnn_profile): events bracket every kernel launch
@@ -208,17 +228,28 @@ int fail(hdgnn_handle_t h, int code, const std::string& msg) {
     return code;
 }
 
-float* F(hdgnn_handle_t h, const char* name) { return static_cast<float*>(h->ws[name].p); }
+float* F(hdgnn_handle_t h, WsId id) { return static_cast<float*>(h->ws[id].p); }
 
-int alloc(hdgnn_handle_t h, const char* name, size_t bytes) {
-    Buf b;
+// a zeroed buffer (FIN_CNT, FIN_L2, H_FLAG and PEER_SEQ rely on starting at zero)
+int alloc(hdgnn_handle_t h, WsId id, size_t bytes) {
+    Buf& b = h->ws[id];
+    cudaError_t e = cudaMalloc(&b.p, bytes);
+    if (e != cudaSuccess) { b.p = nullptr; h->err = std::string("cudaMalloc(") + kWsName[id] + "): " + cudaGetErrorString(e); return HDGNN_E_NOMEM; }
     b.bytes = bytes;
-    cudaError_t e = cudaMalloc(&b.p, bytes ? bytes : 16);
-    if (e != cudaSuccess) { h->err = std::string("cudaMalloc(") + name + "): " + cudaGetErrorString(e); return HDGNN_E_NOMEM; }
-    e = cudaMemset(b.p, 0, bytes ? bytes : 16);
-    if (e != cudaSuccess) { h->err = std::string("cudaMemset(") + name + "): " + cudaGetErrorString(e); return HDGNN_E_CUDA; }
-    h->ws[name] = b;
+    e = cudaMemset(b.p, 0, bytes);
+    if (e != cudaSuccess) { h->err = std::string("cudaMemset(") + kWsName[id] + "): " + cudaGetErrorString(e); return HDGNN_E_CUDA; }
     return HDGNN_OK;
+}
+
+// hdgnn_workspace*: the buffer called `name`, if this handle has it
+int find_ws(hdgnn_handle_t h, const char* name, const Buf** out) {
+    for (int i = 0; i < WS_COUNT; ++i) {
+        if (strcmp(name, kWsName[i])) continue;
+        if (!h->ws[i].p) return fail(h, HDGNN_E_INVALID, std::string("workspace buffer ") + name + " is not allocated for this handle");
+        *out = &h->ws[i];
+        return HDGNN_OK;
+    }
+    return fail(h, HDGNN_E_INVALID, std::string("no workspace buffer named ") + name);
 }
 
 
@@ -339,34 +370,34 @@ int forward_impl(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float*
         PairSumArgs a{};
         a.bits = in.ebits; a.params = in.params; a.x = in.x;
         a.o_u = po.ent_w1; a.o_v = po.ent_w1 + HD; a.o_b = po.ent_b1; a.o_l = po.ent_w1 + 2 * HD;
-        a.RS = F(h, "RS1"); a.CSp = F(h, "CS1P");
+        a.RS = F(h, WS_RS1); a.CSp = F(h, WS_CS1P);
         if ((rc = launch_pairsum(h, "pairsum_fwd(ent)", ge, B, false, true, a, st))) return rc;
     }
     if (h->edge) {
         PairSumArgs a{};
         a.bits = in.ebits; a.params = in.params; a.x = in.x;
         a.o_u = po.edg_w11; a.o_v = po.edg_w11; a.o_b = po.edg_b1; a.o_l = po.edg_w12;
-        a.RS = F(h, "RSE"); a.CSp = F(h, "CSEP");
+        a.RS = F(h, WS_RSE); a.CSp = F(h, WS_CSEP);
         if ((rc = launch_pairsum(h, "pairsum_fwd(edge)", ge, B, false, true, a, st))) return rc;
         HeadFwdArgs hf{};
-        hf.N = h->Ne; hf.S = h->Se; hf.RS = F(h, "RSE"); hf.CSp = F(h, "CSEP"); hf.params = in.params;
-        hf.ho = h->ho_edge; hf.CSf = F(h, "CSEF"); hf.PR = F(h, "PRE"); hf.PC = F(h, "PCE");
+        hf.N = h->Ne; hf.S = h->Se; hf.RS = F(h, WS_RSE); hf.CSp = F(h, WS_CSEP); hf.params = in.params;
+        hf.ho = h->ho_edge; hf.CSf = F(h, WS_CSEF); hf.PR = F(h, WS_PRE); hf.PC = F(h, WS_PCE);
         PROF_BEGIN(h, st);
         head_fwd_kernel<<<B, NODE_THREADS, head_fwd_smem_bytes(), st>>>(hf);
         LAUNCH_CHECK(h, "head_fwd_kernel(edge)", st);
         ScoreArgs s{};
-        s.bits = in.ebits; s.PR = F(h, "PRE"); s.PC = F(h, "PCE"); s.params = in.params;
+        s.bits = in.ebits; s.PR = F(h, WS_PRE); s.PC = F(h, WS_PCE); s.params = in.params;
         s.o_l = po.eup_w1; s.o_w2 = po.eup_w2; s.o_b2 = po.eup_b2;
-        s.soft = F(h, "SOFT");
+        s.soft = F(h, WS_SOFT);
         if ((rc = launch_score(h, "score_fwd(edge)", ge, B, false, s, st))) return rc;
     }
     {
         PoolFwdArgs a{};
         a.Ne = h->Ne; a.Nc = h->Nc; a.Se = h->Se; a.ent = h->ent ? 1 : 0;
-        a.x = in.x; a.RS1 = F(h, "RS1"); a.CS1p = F(h, "CS1P"); a.params = in.params; a.po = po;
-        a.bits = in.ebits; a.WP = h->WPe; a.soft = h->edge ? F(h, "SOFT") : nullptr;
+        a.x = in.x; a.RS1 = F(h, WS_RS1); a.CS1p = F(h, WS_CS1P); a.params = in.params; a.po = po;
+        a.bits = in.ebits; a.WP = h->WPe; a.soft = h->edge ? F(h, WS_SOFT) : nullptr;
         a.hmap = in.hmap; a.L = in.L;
-        a.S1 = F(h, "S1"); a.X2 = F(h, "X2"); a.NB = F(h, "NB"); a.PH = F(h, "PH"); a.QH = F(h, "QH");
+        a.S1 = F(h, WS_S1); a.X2 = F(h, WS_X2); a.NB = F(h, WS_NB); a.PH = F(h, WS_PH); a.QH = F(h, WS_QH);
         PROF_BEGIN(h, st);
         pool_fwd_kernel<<<B, NODE_THREADS, pool_fwd_smem_bytes(h->Ne, h->Nc), st>>>(a);
         LAUNCH_CHECK(h, "pool_fwd_kernel", st);
@@ -374,30 +405,30 @@ int forward_impl(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float*
     {
         PairSumArgs a{};
         a.bits = in.ybits; a.params = in.params; a.o_l = po.hnk_w1 + 8 * HD;
-        a.Ptab = F(h, "PH"); a.Qtab = F(h, "QH");
-        a.RS = F(h, "RS3"); a.CSp = F(h, "CS3P");
+        a.Ptab = F(h, WS_PH); a.Qtab = F(h, WS_QH);
+        a.RS = F(h, WS_RS3); a.CSp = F(h, WS_CS3P);
         if ((rc = launch_pairsum(h, "pairsum_fwd(hunk)", gc, B, false, false, a, st))) return rc;
     }
     {
         HeadFwdArgs hf{};
-        hf.N = h->Nc; hf.S = h->Sc; hf.RS = F(h, "RS3"); hf.CSp = F(h, "CS3P"); hf.params = in.params;
-        hf.ho = h->ho_hunk; hf.CSf = F(h, "CS3F"); hf.PR = F(h, "PR"); hf.PC = F(h, "PC");
+        hf.N = h->Nc; hf.S = h->Sc; hf.RS = F(h, WS_RS3); hf.CSp = F(h, WS_CS3P); hf.params = in.params;
+        hf.ho = h->ho_hunk; hf.CSf = F(h, WS_CS3F); hf.PR = F(h, WS_PR); hf.PC = F(h, WS_PC);
         PROF_BEGIN(h, st);
         head_fwd_kernel<<<B, NODE_THREADS, head_fwd_smem_bytes(), st>>>(hf);
         LAUNCH_CHECK(h, "head_fwd_kernel(hunk)", st);
     }
     {
         ScoreArgs s{};
-        s.bits = in.ybits; s.PR = F(h, "PR"); s.PC = F(h, "PC"); s.params = in.params;
+        s.bits = in.ybits; s.PR = F(h, WS_PR); s.PC = F(h, WS_PC); s.params = in.params;
         s.o_l = po.scr_w1; s.o_w2 = po.scr_w2; s.o_b2 = po.scr_b2;
-        s.logits = logits; s.probs = probs; s.cep = F(h, "CEP");
+        s.logits = logits; s.probs = probs; s.cep = F(h, WS_CEP);
         s.scale = 10.f / ((float)B_global * (float)(h->Nc * (h->Nc - 1)));
-        s.RSm = F(h, "RSM"); s.CSmp = F(h, "CSMP"); s.LSmp = F(h, "LSMP"); s.HSp = F(h, "HSP"); s.dsump = F(h, "DSUMP");
+        s.RSm = F(h, WS_RSM); s.CSmp = F(h, WS_CSMP); s.LSmp = F(h, WS_LSMP); s.HSp = F(h, WS_HSP); s.dsump = F(h, WS_DSUMP);
         if ((rc = launch_score(h, "score(hunk)", gc, B, train, s, st))) return rc;
     }
     if (loss) {
         PROF_BEGIN(h, st);
-        loss_reduce_kernel<<<1, 256, 0, st>>>(F(h, "CEP"), B * h->Sc, (float)B_global * (float)(h->Nc * (h->Nc - 1)), loss);
+        loss_reduce_kernel<<<1, 256, 0, st>>>(F(h, WS_CEP), B * h->Sc, (float)B_global * (float)(h->Nc * (h->Nc - 1)), loss);
         LAUNCH_CHECK(h, "loss_reduce_kernel", st);
     }
     return HDGNN_OK;
@@ -410,9 +441,9 @@ int backward_impl(hdgnn_handle_t h, int B, const Inputs& in, float* grads, cudaS
     {
         HeadBwdArgs a{};
         a.N = h->Nc; a.S = h->Sc;
-        a.RSm = F(h, "RSM"); a.CSmp = F(h, "CSMP"); a.LSmp = F(h, "LSMP"); a.HSp = F(h, "HSP"); a.dsump = F(h, "DSUMP");
-        a.RS = F(h, "RS3"); a.CSf = F(h, "CS3F"); a.params = in.params; a.ho = h->ho_hunk;
-        a.gpart = F(h, "GPART"); a.total = po.total; a.GR = F(h, "GRH"); a.GC = F(h, "GCH");
+        a.RSm = F(h, WS_RSM); a.CSmp = F(h, WS_CSMP); a.LSmp = F(h, WS_LSMP); a.HSp = F(h, WS_HSP); a.dsump = F(h, WS_DSUMP);
+        a.RS = F(h, WS_RS3); a.CSf = F(h, WS_CS3F); a.params = in.params; a.ho = h->ho_hunk;
+        a.gpart = F(h, WS_GPART); a.total = po.total; a.GR = F(h, WS_GRH); a.GC = F(h, WS_GCH);
         PROF_BEGIN(h, st);
         head_bwd_kernel<<<B, NODE_THREADS, head_bwd_smem_bytes(), st>>>(a);
         LAUNCH_CHECK(h, "head_bwd_kernel(hunk)", st);
@@ -420,18 +451,18 @@ int backward_impl(hdgnn_handle_t h, int B, const Inputs& in, float* grads, cudaS
     {
         PairSumArgs a{};
         a.bits = in.ybits; a.params = in.params; a.o_l = po.hnk_w1 + 8 * HD;
-        a.Ptab = F(h, "PH"); a.Qtab = F(h, "QH"); a.GR = F(h, "GRH"); a.GC = F(h, "GCH");
-        a.RS = F(h, "RS3D"); a.CSp = F(h, "CS3DP"); a.LSp = F(h, "LS3P");
+        a.Ptab = F(h, WS_PH); a.Qtab = F(h, WS_QH); a.GR = F(h, WS_GRH); a.GC = F(h, WS_GCH);
+        a.RS = F(h, WS_RS3D); a.CSp = F(h, WS_CS3DP); a.LSp = F(h, WS_LS3P);
         if ((rc = launch_pairsum(h, "pairsum_bwd(hunk)", gc, B, true, false, a, st))) return rc;
     }
     {
         PoolBwdArgs a{};
         a.Ne = h->Ne; a.Nc = h->Nc; a.Sc = h->Sc; a.ent = h->ent ? 1 : 0;
-        a.RS3D = F(h, "RS3D"); a.CS3Dp = F(h, "CS3DP"); a.LS3p = F(h, "LS3P"); a.NB = F(h, "NB");
-        a.x = in.x; a.S1 = F(h, "S1"); a.X2 = F(h, "X2"); a.params = in.params; a.po = po;
-        a.hmap = in.hmap; a.L = in.L; a.gpart = F(h, "GPART"); a.total = po.total;
-        a.DNB = F(h, "DNB"); a.GE = F(h, "GE"); a.DX2 = F(h, "DX2");
-        a.dsoft = h->edge ? F(h, "DSOFT") : nullptr;
+        a.RS3D = F(h, WS_RS3D); a.CS3Dp = F(h, WS_CS3DP); a.LS3p = F(h, WS_LS3P); a.NB = F(h, WS_NB);
+        a.x = in.x; a.S1 = F(h, WS_S1); a.X2 = F(h, WS_X2); a.params = in.params; a.po = po;
+        a.hmap = in.hmap; a.L = in.L; a.gpart = F(h, WS_GPART); a.total = po.total;
+        a.DNB = F(h, WS_DNB); a.GE = F(h, WS_GE); a.DX2 = F(h, WS_DX2);
+        a.dsoft = h->edge ? F(h, WS_DSOFT) : nullptr;
         PROF_BEGIN(h, st);
         pool_bwd_kernel<<<B, NODE_THREADS, pool_bwd_smem_bytes(h->Ne, h->Nc), st>>>(a);
         LAUNCH_CHECK(h, "pool_bwd_kernel", st);
@@ -440,48 +471,48 @@ int backward_impl(hdgnn_handle_t h, int B, const Inputs& in, float* grads, cudaS
         PairSumArgs a{};
         a.bits = in.ebits; a.params = in.params; a.x = in.x;
         a.o_u = po.ent_w1; a.o_v = po.ent_w1 + HD; a.o_b = po.ent_b1; a.o_l = po.ent_w1 + 2 * HD;
-        a.GR = F(h, "GE"); a.GC = F(h, "GE");
-        a.RS = F(h, "RS1D"); a.CSp = F(h, "CS1DP"); a.LSp = F(h, "LS1P");
+        a.GR = F(h, WS_GE); a.GC = F(h, WS_GE);
+        a.RS = F(h, WS_RS1D); a.CSp = F(h, WS_CS1DP); a.LSp = F(h, WS_LS1P);
         if ((rc = launch_pairsum(h, "pairsum_bwd(ent)", ge, B, true, true, a, st))) return rc;
         Rank1GradArgs r{};
-        r.N = h->Ne; r.S = h->Se; r.x = in.x; r.RSd = F(h, "RS1D"); r.CSdp = F(h, "CS1DP"); r.LSp = F(h, "LS1P");
+        r.N = h->Ne; r.S = h->Se; r.x = in.x; r.RSd = F(h, WS_RS1D); r.CSdp = F(h, WS_CS1DP); r.LSp = F(h, WS_LS1P);
         r.o_u = po.ent_w1; r.o_v = po.ent_w1 + HD; r.o_b = po.ent_b1; r.o_l = po.ent_w1 + 2 * HD;
-        r.gpart = F(h, "GPART"); r.total = po.total;
+        r.gpart = F(h, WS_GPART); r.total = po.total;
         PROF_BEGIN(h, st);
         rank1_grad_kernel<<<B, 256, 0, st>>>(r);
         LAUNCH_CHECK(h, "rank1_grad_kernel(ent)", st);
     }
     if (h->edge) {
         ScoreArgs s{};
-        s.bits = in.ebits; s.PR = F(h, "PRE"); s.PC = F(h, "PCE"); s.params = in.params;
+        s.bits = in.ebits; s.PR = F(h, WS_PRE); s.PC = F(h, WS_PCE); s.params = in.params;
         s.o_l = po.eup_w1; s.o_w2 = po.eup_w2; s.o_b2 = po.eup_b2;
-        s.dsoft = F(h, "DSOFT");
-        s.RSm = F(h, "RSME"); s.CSmp = F(h, "CSMEP"); s.LSmp = F(h, "LSMEP"); s.HSp = F(h, "HSEP"); s.dsump = F(h, "DSUMEP");
+        s.dsoft = F(h, WS_DSOFT);
+        s.RSm = F(h, WS_RSME); s.CSmp = F(h, WS_CSMEP); s.LSmp = F(h, WS_LSMEP); s.HSp = F(h, WS_HSEP); s.dsump = F(h, WS_DSUMEP);
         if ((rc = launch_score(h, "score_bwd(edge)", ge, B, true, s, st))) return rc;
         HeadBwdArgs a{};
         a.N = h->Ne; a.S = h->Se;
-        a.RSm = F(h, "RSME"); a.CSmp = F(h, "CSMEP"); a.LSmp = F(h, "LSMEP"); a.HSp = F(h, "HSEP"); a.dsump = F(h, "DSUMEP");
-        a.RS = F(h, "RSE"); a.CSf = F(h, "CSEF"); a.params = in.params; a.ho = h->ho_edge;
-        a.gpart = F(h, "GPART"); a.total = po.total; a.GR = F(h, "GRE"); a.GC = F(h, "GCE");
+        a.RSm = F(h, WS_RSME); a.CSmp = F(h, WS_CSMEP); a.LSmp = F(h, WS_LSMEP); a.HSp = F(h, WS_HSEP); a.dsump = F(h, WS_DSUMEP);
+        a.RS = F(h, WS_RSE); a.CSf = F(h, WS_CSEF); a.params = in.params; a.ho = h->ho_edge;
+        a.gpart = F(h, WS_GPART); a.total = po.total; a.GR = F(h, WS_GRE); a.GC = F(h, WS_GCE);
         PROF_BEGIN(h, st);
         head_bwd_kernel<<<B, NODE_THREADS, head_bwd_smem_bytes(), st>>>(a);
         LAUNCH_CHECK(h, "head_bwd_kernel(edge)", st);
         PairSumArgs p{};
         p.bits = in.ebits; p.params = in.params; p.x = in.x;
         p.o_u = po.edg_w11; p.o_v = po.edg_w11; p.o_b = po.edg_b1; p.o_l = po.edg_w12;
-        p.GR = F(h, "GRE"); p.GC = F(h, "GCE");
-        p.RS = F(h, "RSED"); p.CSp = F(h, "CSEDP"); p.LSp = F(h, "LSEP");
+        p.GR = F(h, WS_GRE); p.GC = F(h, WS_GCE);
+        p.RS = F(h, WS_RSED); p.CSp = F(h, WS_CSEDP); p.LSp = F(h, WS_LSEP);
         if ((rc = launch_pairsum(h, "pairsum_bwd(edge)", ge, B, true, true, p, st))) return rc;
         Rank1GradArgs r{};
-        r.N = h->Ne; r.S = h->Se; r.x = in.x; r.RSd = F(h, "RSED"); r.CSdp = F(h, "CSEDP"); r.LSp = F(h, "LSEP");
+        r.N = h->Ne; r.S = h->Se; r.x = in.x; r.RSd = F(h, WS_RSED); r.CSdp = F(h, WS_CSEDP); r.LSp = F(h, WS_LSEP);
         r.o_u = po.edg_w11; r.o_v = po.edg_w11; r.o_b = po.edg_b1; r.o_l = po.edg_w12;
-        r.gpart = F(h, "GPART"); r.total = po.total;
+        r.gpart = F(h, WS_GPART); r.total = po.total;
         PROF_BEGIN(h, st);
         rank1_grad_kernel<<<B, 256, 0, st>>>(r);
         LAUNCH_CHECK(h, "rank1_grad_kernel(edge)", st);
     }
     PROF_BEGIN(h, st);
-    grad_reduce_kernel<<<(po.total + 127) / 128, 128, 0, st>>>(F(h, "GPART"), B, po.total, grads);
+    grad_reduce_kernel<<<(po.total + 127) / 128, 128, 0, st>>>(F(h, WS_GPART), B, po.total, grads);
     LAUNCH_CHECK(h, "grad_reduce_kernel", st);
     return HDGNN_OK;
 }
@@ -558,13 +589,13 @@ Ent2Args ent2_args(hdgnn_handle_t h, int B, const Inputs& in) {
 
 int debug_scatter(hdgnn_handle_t h, int B, cudaStream_t st) {
     const size_t Ne = h->Ne, Nc = h->Nc, T = Nc * HD, stride = mid2_dbg_floats(h->Ne, h->Nc) * 4;
-    const char* src = (const char*)h->ws["DBG"].p;
-    struct { const char* name; size_t off, n; } parts[] = {
-        {"S1", 0, Ne * HD}, {"X2", Ne * HD, Ne}, {"NB", Ne * 21, Nc * 4}, {"RS3", Ne * 21 + Nc * 4, T},
-        {"CS3F", Ne * 21 + Nc * 4 + T, T}, {"PR", Ne * 21 + Nc * 4 + 2 * T, T}, {"PC", Ne * 21 + Nc * 4 + 3 * T, T},
-        {"DNB", Ne * 21 + Nc * 4 + 4 * T, Nc * 4}, {"DX2", Ne * 21 + Nc * 8 + 4 * T, Ne}};
+    const char* src = (const char*)h->ws[WS_DBG].p;
+    struct { WsId id; size_t off, n; } parts[] = {
+        {WS_S1, 0, Ne * HD}, {WS_X2, Ne * HD, Ne}, {WS_NB, Ne * 21, Nc * 4}, {WS_RS3, Ne * 21 + Nc * 4, T},
+        {WS_CS3F, Ne * 21 + Nc * 4 + T, T}, {WS_PR, Ne * 21 + Nc * 4 + 2 * T, T}, {WS_PC, Ne * 21 + Nc * 4 + 3 * T, T},
+        {WS_DNB, Ne * 21 + Nc * 4 + 4 * T, Nc * 4}, {WS_DX2, Ne * 21 + Nc * 8 + 4 * T, Ne}};
     for (auto& p : parts)
-        CK(h, cudaMemcpy2DAsync(h->ws[p.name].p, p.n * 4, src + p.off * 4, stride, p.n * 4, B, cudaMemcpyDeviceToDevice, st));
+        CK(h, cudaMemcpy2DAsync(h->ws[p.id].p, p.n * 4, src + p.off * 4, stride, p.n * 4, B, cudaMemcpyDeviceToDevice, st));
     return HDGNN_OK;
 }
 
@@ -574,8 +605,8 @@ int debug_scatter(hdgnn_handle_t h, int B, cudaStream_t st) {
 int pack_step(hdgnn_handle_t h, int B, const uint8_t* adj, const uint8_t* Y, Inputs& in, cudaStream_t st) {
     if (!in.ebits) {
         h->bslot ^= 1;
-        in.ebits = (const uint32_t*)h->ws[h->bslot ? "EBITS1" : "EBITS0"].p;
-        in.ybits = (const uint32_t*)h->ws[h->bslot ? "YBITS1" : "YBITS0"].p;
+        in.ebits = (const uint32_t*)h->ws[WS_EBITS0 + h->bslot].p;
+        in.ybits = (const uint32_t*)h->ws[WS_YBITS0 + h->bslot].p;
     }
     PackArgs p{};
     p.adj = adj; p.Ne = h->Ne; p.pe = h->pe; p.WPe = h->WPe; p.ebits = const_cast<uint32_t*>(in.ebits);
@@ -599,7 +630,7 @@ int fused_forward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float
         Ent2Args a = ent2_args(h, B, in);
         ent2_grid(B, h->Ne, P.fwd_occ, h->nsm, &G, &R);
         SL = ent2_max_slots(h->Ne, R);
-        a.R = R; a.SL = SL; a.RS = F(h, "RS1"); a.CSp = F(h, "CS1P"); a.head = head ? 1 : 0;
+        a.R = R; a.SL = SL; a.RS = F(h, WS_RS1); a.CSp = F(h, WS_CS1P); a.head = head ? 1 : 0;
         const size_t smem = ent2_smem_bytes(h->cwt, h->Ne, R, h->WPe, false);
         PROF_BEGIN(h, st);
         launch_ent2(h->cwt, false, G, smem, st, a, P.pdl);
@@ -610,22 +641,22 @@ int fused_forward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float
     m.ebits = in.ebits; m.WPe = h->WPe;
     m.ybits = in.ybits; m.WPc = h->WPc;
     m.x = in.x; m.hmap = in.hmap; m.L = in.L;
-    m.params = in.params; m.po = h->po; m.RS1 = F(h, "RS1"); m.CS1p = F(h, "CS1P");
-    m.logits = logits; m.probs = probs; m.cep = F(h, "CEP");
+    m.params = in.params; m.po = h->po; m.RS1 = F(h, WS_RS1); m.CS1p = F(h, WS_CS1P);
+    m.logits = logits; m.probs = probs; m.cep = F(h, WS_CEP);
     m.scale = 10.f / ((float)B_global * (float)(h->Nc * (h->Nc - 1)));
-    m.GE = F(h, "GE"); m.gpart = F(h, "GPART"); m.total = h->po.total;
-    m.dbg = h->debug ? F(h, "DBG") : nullptr;
-    m.clk = h->debug ? (long long*)h->ws["CLK"].p : nullptr;
-    m.dlt_g = md.opt.dlt_smem ? nullptr : F(h, "DLT");
+    m.GE = F(h, WS_GE); m.gpart = F(h, WS_GPART); m.total = h->po.total;
+    m.dbg = h->debug ? F(h, WS_DBG) : nullptr;
+    m.clk = h->debug ? (long long*)h->ws[WS_CLK].p : nullptr;
+    m.dlt_g = md.opt.dlt_smem ? nullptr : F(h, WS_DLT);
     m.scache = md.opt.scache ? 1 : 0;
     m.inl = P.inl ? 1 : 0;
     m.wait_flag = in.wait_flag; m.wait_tag = in.wait_tag;
     m.hits_acc = h->hits_acc;
     m.evc = h->evc;
     m.edge = P.edge ? 1 : 0;
-    if (m.edge) { m.RSEg = F(h, "RSEG"); m.CSEg = F(h, "CSEG"); m.REg = F(h, "REG"); m.CEg = F(h, "CEG"); m.A1F = F(h, "A1F"); m.PREg = F(h, "PREG"); }
+    if (m.edge) { m.RSEg = F(h, WS_RSEG); m.CSEg = F(h, WS_CSEG); m.REg = F(h, WS_REG); m.CEg = F(h, WS_CEG); m.A1F = F(h, WS_A1F); m.PREg = F(h, WS_PREG); }
     m.lay = md.lay;
-    m.tabs_g = P.gt ? F(h, "TABS") : nullptr;
+    m.tabs_g = P.gt ? F(h, WS_TABS) : nullptr;
     // Batches below one wave of SMs: clusters of two CTAs, the `S` costliest commits shared by both CTAs of a cluster (mid2.cuh),
     // as many as there are spare SMs and co-resident clusters
     bool cl = false;
@@ -651,18 +682,18 @@ int fused_backward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, floa
     if (P.dense) {
         Ent2Args a = ent2_args(h, B, in);
         ent2_grid(B, h->Ne, P.bwd_occ, h->nsm, &G, &R);
-        a.R = R; a.SL = 0; a.GR = F(h, "GE"); a.GC = F(h, "GE"); a.gpart = F(h, "GPE");
+        a.R = R; a.SL = 0; a.GR = F(h, WS_GE); a.GC = F(h, WS_GE); a.gpart = F(h, WS_GPE);
         const size_t smem = ent2_smem_bytes(h->cwt, h->Ne, R, h->WPe, true);
         PROF_BEGIN(h, st);
         launch_ent2(h->cwt, true, G, smem, st, a, P.pdl);
         LAUNCH_CHECK(h, "ent_bwd", st);
     }
     FinalArgs f{};
-    f.B = B; f.total = h->po.total; f.gpart = F(h, "GPART");
-    if (P.dense) f.ent = {F(h, "GPE"), G, h->po.ent_w1, h->po.ent_w1 + HD, h->po.ent_b1, h->po.ent_w1 + 2 * HD};
-    f.cep = F(h, "CEP"); f.ncep = B; f.loss_denom = (float)B_global * (float)(h->Nc * (h->Nc - 1)); f.loss = loss;
+    f.B = B; f.total = h->po.total; f.gpart = F(h, WS_GPART);
+    if (P.dense) f.ent = {F(h, WS_GPE), G, h->po.ent_w1, h->po.ent_w1 + HD, h->po.ent_b1, h->po.ent_w1 + 2 * HD};
+    f.cep = F(h, WS_CEP); f.ncep = B; f.loss_denom = (float)B_global * (float)(h->Nc * (h->Nc - 1)); f.loss = loss;
     f.grads = grads;
-    f.l2part = F(h, "FIN_L2"); f.counter = (unsigned int*)h->ws["FIN_CNT"].p;
+    f.l2part = F(h, WS_FIN_L2); f.counter = (unsigned int*)h->ws[WS_FIN_CNT].p;
     if (adam) {
         f.apply_adam = 1; f.params = adam->params; f.m = adam->m; f.v = adam->v; f.step = adam->step;
         f.o_t1 = h->po.theta1; f.o_t2 = h->po.theta2; f.lr = adam->lr; f.b1 = adam->b1; f.b2 = adam->b2; f.eps = adam->eps;
@@ -678,7 +709,7 @@ int fused_backward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, floa
 // Byte offsets of the five inputs of a batch of B commits, labels as bitmaps, inside one staging block (every section starts
 // at the next multiple of 16 bytes).  Host buffers laid out the same way travel in ONE DMA (stage_inputs).
 struct WireOff { size_t eb, yb, x, hm, L, total; };
-WireOff wire_layout(hdgnn_handle_t h, int B) {
+WireOff wire_layout(const hdgnn_handle_s* h, int B) {
     WireOff w{};
     size_t o = 0;
     auto take = [&](size_t n) { const size_t r = o; o += (n + 15) & ~(size_t)15; return r; };
@@ -754,7 +785,7 @@ FusedPlan plan_fused(const hdgnn_config_t& cfg, int optin, int nsm, cudaError_t*
     Mid2Opts f = pp.opt; f.train = false; f.dlt_smem = true; f.scache = false;
     Mid2Opts t = pp.opt; t.train = true;
     resolve(P.mode[0], true, f);
-    resolve(P.mode[1], tr && (!edge || edge_train), t);     // also when not fused (variant 4): its dlt_smem sizes DLT
+    resolve(P.mode[1], tr && (!edge || edge_train), t);
 
     const cudaFuncAttribute A = cudaFuncAttributeMaxDynamicSharedMemorySize;
     auto acc = [&](cudaError_t x) { if (e == cudaSuccess) e = x; };
@@ -770,7 +801,8 @@ FusedPlan plan_fused(const hdgnn_config_t& cfg, int optin, int nsm, cudaError_t*
             if (ct > 0 && cf > 0) { P.mode[1].clusters = ct; P.mode[0].clusters = cf; }
         }
     }
-    // the occupancy of the sweeps also sizes CS1P and GPE, so it is taken for the inline entity stage as well
+    // the occupancy of the sweeps also sizes CS1P, so it is taken for the inline entity stage as well (variant 4 with a fused
+    // forward and multi-kernel training)
     if (ent) {
         const int cwt = ent2_cwt(Ne);
         acc(cudaFuncSetAttribute(ent2_fn_rt(cwt, false), A, optin));
@@ -789,6 +821,67 @@ int pick_rt(int N, int B, int requested) {
     while (rt > 16 && (long)B * ((N + rt - 1) / rt) < 2 * 148 * 3) rt -= 4;
     if (rt > round_up(N, 4)) rt = round_up(N, 4);
     return rt;
+}
+
+// Bytes of each workspace buffer of a handle, 0 for a buffer it does not have: a function of its configuration, its plan and the
+// sizes derived from them, without CUDA calls.  PEER_SEQ and PEER_STAMPS are 0 here (hdgnn_peer_attach).
+std::array<size_t, WS_COUNT> workspace_bytes(const hdgnn_handle_s& h) {
+    const FusedPlan& P = h.plan;
+    const bool fused = P.mode[0].fused;       // the forward is fused whenever the training step is
+    const int Gf_max = fused && h.ent ? P.fwd_occ * h.nsm : 0, Gb_max = fused && h.ent ? P.bwd_occ * h.nsm : 0;
+    const size_t B = h.cfg.max_batch, Ne = h.Ne, Nc = h.Nc, Se = h.Se, Sc = h.Sc, f = sizeof(float);
+    // (B, SL, Ne, 20) column partials of ent_fwd2: B * SL <= grid + 2 B for every batch size <= max_batch
+    const size_t cs1p_f = ((size_t)Gf_max + 2 * B + 2) * Ne * HD * f, cs1p_l = B * Se * Ne * HD * f;
+    const bool mixed = fused && !P.mode[1].fused;        // variant 4: fused forward, multi-kernel training
+    const size_t cs1p = !fused ? cs1p_l : (mixed && cs1p_l > cs1p_f ? cs1p_l : cs1p_f);
+    const bool lg = !P.mode[1].fused;     // buffers only the multi-kernel path needs (kept when debugging: dump targets)
+    const bool dbgbuf = lg || h.debug;
+    // the entity state in HBM: RS1 / CS1P and GE on the multi-kernel path and beside the dense sweeps.  The inline entity stage
+    // keeps S and GE in shared memory; GE holds its S / GE rows when they do not fit there (scg), and the debug dump of GE.
+    const bool ent_g = h.ent && (P.dense || lg);
+    const bool ge = dbgbuf || (h.ent && (P.dense || P.mode[0].lay.scg || P.mode[1].lay.scg));
+    const struct { WsId id; size_t bytes; bool need; } rows[] = {
+        {WS_RS1, B * Ne * HD * f, ent_g}, {WS_CS1P, cs1p, ent_g}, {WS_S1, B * Ne * HD * f, dbgbuf},
+        {WS_X2, B * Ne * f, dbgbuf}, {WS_NB, B * Nc * 4 * f, dbgbuf}, {WS_PH, B * Nc * HD * f, lg}, {WS_QH, B * Nc * HD * f, lg},
+        {WS_RS3, B * Nc * HD * f, dbgbuf}, {WS_CS3P, B * Sc * Nc * HD * f, lg}, {WS_CS3F, B * Nc * HD * f, dbgbuf},
+        {WS_PR, B * Nc * HD * f, dbgbuf}, {WS_PC, B * Nc * HD * f, dbgbuf}, {WS_CEP, B * Sc * f, true},
+        {WS_RSM, B * Nc * HD * f, lg}, {WS_CSMP, B * Sc * Nc * HD * f, lg}, {WS_LSMP, B * Sc * HD * f, lg},
+        {WS_HSP, B * Sc * HD * f, lg}, {WS_DSUMP, B * Sc * f, lg},
+        {WS_GRH, B * Nc * HD * f, lg}, {WS_GCH, B * Nc * HD * f, lg},
+        {WS_RS3D, B * Nc * HD * f, lg}, {WS_CS3DP, B * Sc * Nc * HD * f, lg}, {WS_LS3P, B * Sc * HD * f, lg},
+        {WS_DNB, B * Nc * 4 * f, dbgbuf}, {WS_GE, B * Ne * HD * f, ge}, {WS_DX2, B * Ne * f, dbgbuf},
+        {WS_RS1D, B * Ne * HD * f, h.ent && lg}, {WS_CS1DP, B * Se * Ne * HD * f, h.ent && lg}, {WS_LS1P, B * Se * HD * f, h.ent && lg},
+        {WS_GPART, 2 * B * (size_t)h.po.total * f, true},       // second half: spare rows of the cluster form (mid2.cuh)
+        {WS_GPE, ((size_t)Gb_max + 1) * 4 * HD * f, P.dense}, {WS_FIN_L2, 256 * f, fused}, {WS_FIN_CNT, 16, fused},
+        // pack_bits' output for the device entry points taking byte grids
+        {WS_EBITS0, B * Ne * (size_t)h.WPe * 4, !h.host_bits}, {WS_EBITS1, B * Ne * (size_t)h.WPe * 4, !h.host_bits},
+        {WS_YBITS0, B * Nc * (size_t)h.WPc * 4, !h.host_bits}, {WS_YBITS1, B * Nc * (size_t)h.WPc * 4, !h.host_bits},
+        {WS_DBG, B * mid2_dbg_floats(h.Ne, h.Nc) * f, fused && h.debug},
+        {WS_CLK, B * 24 * sizeof(long long), fused && h.debug},
+        {WS_DLT, B * Nc * (size_t)((h.Nc + 31) / 32 * 32) * f, P.mode[1].fused && !P.mode[1].opt.dlt_smem},
+        {WS_TABS, B * (size_t)mid2_tab_floats(h.Nc) * f, fused && P.gt},
+        {WS_RSEG, B * Ne * HD * f, P.edge}, {WS_CSEG, B * Ne * HD * f, P.edge}, {WS_REG, B * Ne * HD * f, P.edge},
+        {WS_CEG, B * Ne * HD * f, P.edge}, {WS_A1F, B * Ne * (Ne - 1) * f, P.edge}, {WS_PREG, B * Ne * 60 * f, P.edge},
+        {WS_RSE, B * Ne * HD * f, h.edge}, {WS_CSEP, B * Se * Ne * HD * f, h.edge}, {WS_CSEF, B * Ne * HD * f, h.edge},
+        {WS_PRE, B * Ne * HD * f, h.edge}, {WS_PCE, B * Ne * HD * f, h.edge},
+        {WS_SOFT, B * Ne * Ne * 2 * f, h.edge}, {WS_DSOFT, B * Ne * Ne * 2 * f, h.edge},
+        {WS_RSME, B * Ne * HD * f, h.edge}, {WS_CSMEP, B * Se * Ne * HD * f, h.edge}, {WS_LSMEP, B * Se * HD * f, h.edge},
+        {WS_HSEP, B * Se * HD * f, h.edge}, {WS_DSUMEP, B * Se * f, h.edge},
+        {WS_GRE, B * Ne * HD * f, h.edge}, {WS_GCE, B * Ne * HD * f, h.edge},
+        {WS_RSED, B * Ne * HD * f, h.edge}, {WS_CSEDP, B * Se * Ne * HD * f, h.edge}, {WS_LSEP, B * Se * HD * f, h.edge},
+        // staging slots of the *_host entry points: the wire block [entity bitmaps][hunk bitmaps][x][hmap][L] (16-byte aligned
+        // sections), and for byte grids the pitched grids pack_bits reads (+ the un-pitched rows, re-pitched on the device)
+        {WS_H_WIRE0, wire_layout(&h, h.cfg.max_batch).total, true}, {WS_H_WIRE1, wire_layout(&h, h.cfg.max_batch).total, true},
+        {WS_H_ADJ0, B * Ne * (size_t)h.pe, !h.host_bits}, {WS_H_ADJ1, B * Ne * (size_t)h.pe, !h.host_bits},
+        {WS_H_Y0, B * Nc * (size_t)h.pc, !h.host_bits}, {WS_H_Y1, B * Nc * (size_t)h.pc, !h.host_bits},
+        {WS_H_ADJ_RAW0, B * Ne * Ne, !h.host_bits && h.pe != h.Ne}, {WS_H_ADJ_RAW1, B * Ne * Ne, !h.host_bits && h.pe != h.Ne},
+        {WS_H_Y_RAW0, B * Nc * Nc, !h.host_bits && h.pc != h.Nc}, {WS_H_Y_RAW1, B * Nc * Nc, !h.host_bits && h.pc != h.Nc},
+        {WS_H_FLAG, 16, true}, {WS_H_PROBS, B * 2 * Nc * (Nc - 1) * f, true}, {WS_H_LOSS, 4 * f, true}, {WS_H_GRADS, (size_t)h.po.total * f, true},
+    };
+    std::array<size_t, WS_COUNT> bytes{};
+    for (auto& r : rows)
+        if (r.need) bytes[r.id] = r.bytes;
+    return bytes;
 }
 
 }  // namespace
@@ -865,7 +958,6 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
     h->cwt = ent2_cwt(h->Ne);
     cudaError_t e;
     h->plan = plan_fused(*cfg, (int)prop.sharedMemPerBlockOptin, h->nsm, &e);
-    const FusedPlan& P = h->plan;
     h->host_bits = (cfg->flags & HDGNN_F_LABEL_BITS) != 0;
     if (e == cudaSuccess) e = set_attrs(h, (int)prop.sharedMemPerBlockOptin);
     if (e != cudaSuccess) {
@@ -873,57 +965,10 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
         delete h;
         return fail(nullptr, HDGNN_E_CUDA, m);
     }
-    const bool fused = P.mode[0].fused;       // the forward is fused whenever the training step is
-    const int Gf_max = fused && h->ent ? P.fwd_occ * h->nsm : 0, Gb_max = fused && h->ent ? P.bwd_occ * h->nsm : 0;
-
-    const size_t B = cfg->max_batch, Ne = h->Ne, Nc = h->Nc, Se = h->Se, Sc = h->Sc, f = sizeof(float);
-    // (B, SL, Ne, 20) column partials of ent_fwd2: B * SL <= grid + 2 B for every batch size <= max_batch
-    const size_t cs1p_f = ((size_t)Gf_max + 2 * B + 2) * Ne * HD * f, cs1p_l = B * Se * Ne * HD * f;
-    const bool mixed = fused && !P.mode[1].fused;        // variant 4: fused forward, multi-kernel training
-    const size_t cs1p = !fused ? cs1p_l : (mixed && cs1p_l > cs1p_f ? cs1p_l : cs1p_f);
-    const bool lg = !P.mode[1].fused;     // buffers only the multi-kernel path needs (kept when debugging: dump targets)
-    const bool dbgbuf = lg || h->debug;
-    struct { const char* n; size_t bytes; bool need; } plan[] = {
-        {"RS1", B * Ne * HD * f, h->ent}, {"CS1P", cs1p, h->ent}, {"S1", B * Ne * HD * f, dbgbuf},
-        {"X2", B * Ne * f, dbgbuf}, {"NB", B * Nc * 4 * f, dbgbuf}, {"PH", B * Nc * HD * f, lg}, {"QH", B * Nc * HD * f, lg},
-        {"RS3", B * Nc * HD * f, dbgbuf}, {"CS3P", B * Sc * Nc * HD * f, lg}, {"CS3F", B * Nc * HD * f, dbgbuf},
-        {"PR", B * Nc * HD * f, dbgbuf}, {"PC", B * Nc * HD * f, dbgbuf}, {"CEP", B * Sc * f, true},
-        {"RSM", B * Nc * HD * f, lg}, {"CSMP", B * Sc * Nc * HD * f, lg}, {"LSMP", B * Sc * HD * f, lg},
-        {"HSP", B * Sc * HD * f, lg}, {"DSUMP", B * Sc * f, lg},
-        {"GRH", B * Nc * HD * f, lg}, {"GCH", B * Nc * HD * f, lg},
-        {"RS3D", B * Nc * HD * f, lg}, {"CS3DP", B * Sc * Nc * HD * f, lg}, {"LS3P", B * Sc * HD * f, lg},
-        {"DNB", B * Nc * 4 * f, dbgbuf}, {"GE", B * Ne * HD * f, true}, {"DX2", B * Ne * f, dbgbuf},
-        {"RS1D", B * Ne * HD * f, h->ent && lg}, {"CS1DP", B * Se * Ne * HD * f, h->ent && lg}, {"LS1P", B * Se * HD * f, h->ent && lg},
-        {"GPART", 2 * B * (size_t)h->po.total * f, true},       // second half: spare rows of the cluster form (mid2.cuh)
-        {"GPE", ((size_t)Gb_max + 1) * 4 * HD * f, fused && h->ent}, {"FIN_L2", 256 * f, fused}, {"FIN_CNT", 16, fused},
-        // pack_bits' output for the device entry points taking byte grids
-        {"EBITS0", B * Ne * (size_t)h->WPe * 4, !h->host_bits}, {"YBITS0", B * Nc * (size_t)h->WPc * 4, !h->host_bits},
-        {"EBITS1", B * Ne * (size_t)h->WPe * 4, !h->host_bits}, {"YBITS1", B * Nc * (size_t)h->WPc * 4, !h->host_bits},
-        {"DBG", B * mid2_dbg_floats(h->Ne, h->Nc) * f, fused && h->debug},
-        {"CLK", B * 24 * sizeof(long long), fused && h->debug},
-        {"DLT", B * Nc * (size_t)((h->Nc + 31) / 32 * 32) * f, fused && !P.mode[1].opt.dlt_smem},
-        {"TABS", B * (size_t)mid2_tab_floats(h->Nc) * f, fused && P.gt},
-        {"RSEG", B * Ne * HD * f, P.edge}, {"CSEG", B * Ne * HD * f, P.edge}, {"REG", B * Ne * HD * f, P.edge},
-        {"CEG", B * Ne * HD * f, P.edge}, {"A1F", B * Ne * (Ne - 1) * f, P.edge}, {"PREG", B * Ne * 60 * f, P.edge},
-        {"RSE", B * Ne * HD * f, h->edge}, {"CSEP", B * Se * Ne * HD * f, h->edge}, {"CSEF", B * Ne * HD * f, h->edge},
-        {"PRE", B * Ne * HD * f, h->edge}, {"PCE", B * Ne * HD * f, h->edge},
-        {"SOFT", B * Ne * Ne * 2 * f, h->edge}, {"DSOFT", B * Ne * Ne * 2 * f, h->edge},
-        {"RSME", B * Ne * HD * f, h->edge}, {"CSMEP", B * Se * Ne * HD * f, h->edge}, {"LSMEP", B * Se * HD * f, h->edge},
-        {"HSEP", B * Se * HD * f, h->edge}, {"DSUMEP", B * Se * f, h->edge},
-        {"GRE", B * Ne * HD * f, h->edge}, {"GCE", B * Ne * HD * f, h->edge},
-        {"RSED", B * Ne * HD * f, h->edge}, {"CSEDP", B * Se * Ne * HD * f, h->edge}, {"LSEP", B * Se * HD * f, h->edge},
-        // staging slots of the *_host entry points: the wire block [entity bitmaps][hunk bitmaps][x][hmap][L] (16-byte aligned
-        // sections), and for byte grids the pitched grids pack_bits reads (+ the un-pitched rows, re-pitched on the device)
-        {"H_WIRE0", wire_layout(h, cfg->max_batch).total, true}, {"H_WIRE1", wire_layout(h, cfg->max_batch).total, true},
-        {"H_ADJ0", B * Ne * (size_t)h->pe, !h->host_bits}, {"H_Y0", B * Nc * (size_t)h->pc, !h->host_bits},
-        {"H_ADJ1", B * Ne * (size_t)h->pe, !h->host_bits}, {"H_Y1", B * Nc * (size_t)h->pc, !h->host_bits},
-        {"H_ADJ_RAW0", B * Ne * Ne, !h->host_bits && h->pe != h->Ne}, {"H_Y_RAW0", B * Nc * Nc, !h->host_bits && h->pc != h->Nc},
-        {"H_ADJ_RAW1", B * Ne * Ne, !h->host_bits && h->pe != h->Ne}, {"H_Y_RAW1", B * Nc * Nc, !h->host_bits && h->pc != h->Nc},
-        {"H_FLAG", 16, true}, {"H_PROBS", B * 2 * Nc * (Nc - 1) * f, true}, {"H_LOSS", 4 * f, true}, {"H_GRADS", (size_t)h->po.total * f, true},
-    };
-    for (auto& p : plan) {
-        if (!p.need) continue;
-        int rc = alloc(h, p.n, p.bytes);
+    const std::array<size_t, WS_COUNT> bytes = workspace_bytes(*h);
+    for (int i = 0; i < WS_COUNT; ++i) {
+        if (!bytes[i]) continue;
+        int rc = alloc(h, (WsId)i, bytes[i]);
         if (rc != HDGNN_OK) {
             g_create_error = h->err;
             hdgnn_destroy(h);
@@ -951,7 +996,7 @@ int hdgnn_destroy(hdgnn_handle_t h) {
     cudaSetDevice(h->cfg.device);
     if (h->copy_stream) { cudaStreamSynchronize(h->copy_stream); cudaStreamDestroy(h->copy_stream); }
     for (int i = 0; i < NSLOT; ++i) { if (h->ev_copy[i]) cudaEventDestroy(h->ev_copy[i]); if (h->ev_done[i]) cudaEventDestroy(h->ev_done[i]); }
-    for (auto& kv : h->ws) cudaFree(kv.second.p);
+    for (const Buf& b : h->ws) cudaFree(b.p);
     if (h->tag_table) cudaFreeHost(h->tag_table);
     for (int r = 0; r < PEER_MAX; ++r) if (h->peer_map[r]) cudaIpcCloseMemHandle(h->peer_map[r]);
     if (h->peer_box) cudaFree(h->peer_box);
@@ -994,7 +1039,7 @@ int hdgnn_peer_attach(hdgnn_handle_t h, int rank, int world, const unsigned char
     if (h->peer_ready) return fail(h, HDGNN_E_INVALID, "peers are already attached");
     CK(h, cudaSetDevice(h->cfg.device));
     int rc;
-    if (!h->ws.count("PEER_SEQ") && (rc = alloc(h, "PEER_SEQ", 16))) return rc;      // [0] sequence number, [1] error flag
+    if (!h->ws[WS_PEER_SEQ].p && (rc = alloc(h, WS_PEER_SEQ, 16))) return rc;      // [0] sequence number, [1] error flag
     int stride, ncta; size_t ol, bytes;
     peer_layout(world, h->po.total, &stride, &ncta, &ol, &bytes);
     PeerArgs pa{};
@@ -1010,7 +1055,7 @@ int hdgnn_peer_attach(hdgnn_handle_t h, int rank, int world, const unsigned char
         pa.inbox[r] = (peer_word*)base;
         pa.lossin[r] = (peer_word*)((char*)base + ol);
     }
-    pa.seq = (int*)h->ws["PEER_SEQ"].p;
+    pa.seq = (int*)h->ws[WS_PEER_SEQ].p;
     pa.error = pa.seq + 1;
     {
         const long long ms = env_int("HDGNN_PEER_TIMEOUT_MS", 20000);
@@ -1019,8 +1064,8 @@ int hdgnn_peer_attach(hdgnn_handle_t h, int rank, int world, const unsigned char
     }
     pa.stamps = nullptr;
     if (env_int("HDGNN_PEER_STAMPS", 0)) {
-        if (!h->ws.count("PEER_STAMPS") && (rc = alloc(h, "PEER_STAMPS", 4096 * 2 * sizeof(unsigned long long)))) return rc;
-        pa.stamps = (unsigned long long*)h->ws["PEER_STAMPS"].p;
+        if (!h->ws[WS_PEER_STAMPS].p && (rc = alloc(h, WS_PEER_STAMPS, 4096 * 2 * sizeof(unsigned long long)))) return rc;
+        pa.stamps = (unsigned long long*)h->ws[WS_PEER_STAMPS].p;
     }
     h->peer = pa;
     h->peer_ready = true;
@@ -1065,7 +1110,7 @@ static int run_step(hdgnn_handle_t h, int B, int B_global, const uint8_t* adj, c
         if (!train) {
             if (loss) {
                 PROF_BEGIN(h, st);
-                loss_reduce_kernel<<<1, 256, 0, st>>>(F(h, "CEP"), B, (float)B_global * (float)(h->Nc * (h->Nc - 1)), loss);
+                loss_reduce_kernel<<<1, 256, 0, st>>>(F(h, WS_CEP), B, (float)B_global * (float)(h->Nc * (h->Nc - 1)), loss);
                 LAUNCH_CHECK(h, "loss_reduce_kernel", st);
             }
             return HDGNN_OK;
@@ -1134,15 +1179,13 @@ int hdgnn_train_step(hdgnn_handle_t h, int B, const uint8_t* adj, int adj_pitch,
     if (rc) return rc;
     if (!m || !v || !step_counter || !loss3) return fail(h, HDGNN_E_INVALID, "null pointer");
     const AdamArgs ad{params, m, v, step_counter, lr, beta1, beta2, eps, loss3 + 1};
-    return device_step(h, B, B, adj, x, hmap, L, Y, params, logits, probs, loss3, F(h, "H_GRADS"), &ad, stream);
+    return device_step(h, B, B, adj, x, hmap, L, Y, params, logits, probs, loss3, F(h, WS_H_GRADS), &ad, stream);
 }
 
 // Host buffers -> staging slot `h->cur` (un-pitched rows are re-pitched on the device).  Outside stream capture the
 // copies run on the handle's copy stream: slot s is reused only after the kernels that read it (two calls ago)
 // have finished, and the step waits for the copies (an event, or the tag mid2 polls), so consecutive calls overlap copy
 // and compute.
-static std::string slot_name(const char* base, int slot) { return std::string(base) + (char)('0' + slot); }
-
 static int stage_inputs(hdgnn_handle_t h, int B, const uint8_t* adj_host, const float* x_host, const int32_t* hmap_host,
                         const int32_t* L_host, const uint8_t* Y_host, bool train, cudaStream_t st) {
     const size_t Ne = h->Ne, Nc = h->Nc;
@@ -1159,7 +1202,7 @@ static int stage_inputs(hdgnn_handle_t h, int B, const uint8_t* adj_host, const 
     // (one pinned block, what HostBatch builds) are copied with a single DMA, anything else section by section.  Byte grids
     // go to the slot's pitched buffers instead, and pack_bits fills the block's bitmap sections from them (pack_step).
     const WireOff W = wire_layout(h, B);
-    char* base = (char*)h->ws[slot_name("H_WIRE", slot)].p;
+    char* base = (char*)h->ws[WS_H_WIRE0 + slot].p;
     const char* hb = (const char*)adj_host;
     const bool whole = h->host_bits && (const char*)Y_host == hb + W.yb && (const char*)x_host == hb + W.x &&
                        (const char*)hmap_host == hb + W.hm && (const char*)L_host == hb + W.L;
@@ -1170,17 +1213,16 @@ static int stage_inputs(hdgnn_handle_t h, int B, const uint8_t* adj_host, const 
         CK(h, cudaMemcpyAsync(base + W.yb, Y_host, (size_t)B * Nc * h->WPc * 4, cudaMemcpyHostToDevice, cs));
     } else {
         const uint8_t* srcs[2] = {adj_host, Y_host};
-        const char* raw[2] = {"H_ADJ_RAW", "H_Y_RAW"};
-        const char* dstn[2] = {"H_ADJ", "H_Y"};
+        const WsId raw[2] = {WS_H_ADJ_RAW0, WS_H_Y_RAW0}, dstn[2] = {WS_H_ADJ0, WS_H_Y0};
         const size_t n[2] = {Ne, Nc};
         const int pitch[2] = {h->pe, h->pc};
         for (int t = 0; t < 2; ++t) {
             const size_t rows = (size_t)B * n[t];
-            void* dst = h->ws[slot_name(dstn[t], slot)].p;
+            void* dst = h->ws[dstn[t] + slot].p;
             if (pitch[t] == (int)n[t]) {
                 CK(h, cudaMemcpyAsync(dst, srcs[t], rows * n[t], cudaMemcpyHostToDevice, cs));
             } else {
-                void* rawp = h->ws[slot_name(raw[t], slot)].p;
+                void* rawp = h->ws[raw[t] + slot].p;
                 CK(h, cudaMemcpyAsync(rawp, srcs[t], rows * n[t], cudaMemcpyHostToDevice, cs));
                 const size_t work = rows * (size_t)pitch[t] / 4;
                 int blocks = (int)((work + 255) / 256);
@@ -1201,7 +1243,7 @@ static int stage_inputs(hdgnn_handle_t h, int B, const uint8_t* adj_host, const 
         if (h->tag_table && h->host_bits && h->plan.mode[train].fused && h->plan.mid2_first) {
             // mid2 is the first kernel of the step and reads every staged input: order it by a tag instead of an event
             const int tag = (int)(++h->slot_uses[slot] & 0xffu);
-            CK(h, cudaMemcpyAsync((int*)h->ws["H_FLAG"].p + slot, h->tag_table + tag, sizeof(int), cudaMemcpyHostToDevice, cs));
+            CK(h, cudaMemcpyAsync((int*)h->ws[WS_H_FLAG].p + slot, h->tag_table + tag, sizeof(int), cudaMemcpyHostToDevice, cs));
             h->cur_tag = tag;
         } else {
             CK(h, cudaEventRecord(h->ev_copy[slot], cs));
@@ -1216,12 +1258,12 @@ static int stage_inputs(hdgnn_handle_t h, int B, const uint8_t* adj_host, const 
 static Inputs staged_inputs(hdgnn_handle_t h, const float* params, const uint8_t** adj, const uint8_t** Y) {
     const int s = h->cur;
     const WireOff W = wire_layout(h, h->cur_B);
-    const char* base = (const char*)h->ws[slot_name("H_WIRE", s)].p;
+    const char* base = (const char*)h->ws[WS_H_WIRE0 + s].p;
     Inputs in{(const uint32_t*)(base + W.eb), (const uint32_t*)(base + W.yb), (const float*)(base + W.x),
               (const int32_t*)(base + W.hm), (const int32_t*)(base + W.L), params};
-    if (h->cur_tag >= 0) { in.wait_flag = (const int*)h->ws["H_FLAG"].p + s; in.wait_tag = h->cur_tag; }
-    *adj = h->host_bits ? nullptr : (const uint8_t*)h->ws[slot_name("H_ADJ", s)].p;
-    *Y = h->host_bits ? nullptr : (const uint8_t*)h->ws[slot_name("H_Y", s)].p;
+    if (h->cur_tag >= 0) { in.wait_flag = (const int*)h->ws[WS_H_FLAG].p + s; in.wait_tag = h->cur_tag; }
+    *adj = h->host_bits ? nullptr : (const uint8_t*)h->ws[WS_H_ADJ0 + s].p;
+    *Y = h->host_bits ? nullptr : (const uint8_t*)h->ws[WS_H_Y0 + s].p;
     return in;
 }
 
@@ -1270,9 +1312,9 @@ static int host_step(hdgnn_handle_t h, int B, int B_global, const uint8_t* adj_h
     if (rc) return rc;
     const uint8_t *adj, *Y;
     const Inputs in = staged_inputs(h, params, &adj, &Y);
-    float* probs_d = to_host && probs ? F(h, "H_PROBS") : probs;
+    float* probs_d = to_host && probs ? F(h, WS_H_PROBS) : probs;
     float* alias = to_host && adam && h->plan.mode[1].fused ? host_alias(loss) : nullptr;
-    float* loss_d = to_host ? (alias ? alias : F(h, "H_LOSS")) : loss;
+    float* loss_d = to_host ? (alias ? alias : F(h, WS_H_LOSS)) : loss;
     AdamArgs ad{};
     if (adam) { ad = *adam; ad.reg = loss_d + 1; }
     rc = run_step(h, B, B_global, adj, Y, in, nullptr, probs_d, loss_d, grads, adam ? &ad : nullptr, st);
@@ -1292,7 +1334,7 @@ int hdgnn_train_step_host(hdgnn_handle_t h, int B, const uint8_t* adj_host, cons
     if (rc) return rc;
     if (!m || !v || !step_counter || !loss3_host) return fail(h, HDGNN_E_INVALID, "null pointer");
     const AdamArgs ad{params, m, v, step_counter, lr, beta1, beta2, eps, nullptr};
-    return host_step(h, B, B, adj_host, x_host, hmap_host, L_host, Y_host, params, probs_host, loss3_host, F(h, "H_GRADS"), &ad,
+    return host_step(h, B, B, adj_host, x_host, hmap_host, L_host, Y_host, params, probs_host, loss3_host, F(h, WS_H_GRADS), &ad,
                      true, stream);
 }
 
@@ -1305,7 +1347,7 @@ int hdgnn_train_step_peer(hdgnn_handle_t h, int B, int B_global, const uint8_t* 
     if (!m || !v || !step_counter || !loss3) return fail(h, HDGNN_E_INVALID, "null pointer");
     if ((rc = check_peer(h, B, B_global))) return rc;
     const AdamArgs ad{params, m, v, step_counter, lr, beta1, beta2, eps, loss3 + 1, true};
-    return device_step(h, B, B_global, adj, x, hmap, L, Y, params, logits, probs, loss3, F(h, "H_GRADS"), &ad, stream);
+    return device_step(h, B, B_global, adj, x, hmap, L, Y, params, logits, probs, loss3, F(h, WS_H_GRADS), &ad, stream);
 }
 
 int hdgnn_train_step_peer_host(hdgnn_handle_t h, int B, int B_global, const uint8_t* adj_host, const float* x_host,
@@ -1317,7 +1359,7 @@ int hdgnn_train_step_peer_host(hdgnn_handle_t h, int B, int B_global, const uint
     if (!m || !v || !step_counter || !loss3_host) return fail(h, HDGNN_E_INVALID, "null pointer");
     if ((rc = check_peer(h, B, B_global))) return rc;
     const AdamArgs ad{params, m, v, step_counter, lr, beta1, beta2, eps, nullptr, true};
-    return host_step(h, B, B_global, adj_host, x_host, hmap_host, L_host, Y_host, params, probs_out, loss3_host, F(h, "H_GRADS"),
+    return host_step(h, B, B_global, adj_host, x_host, hmap_host, L_host, Y_host, params, probs_out, loss3_host, F(h, WS_H_GRADS),
                      &ad, true, stream);
 }
 
@@ -1343,19 +1385,19 @@ int hdgnn_infer_host(hdgnn_handle_t h, int B, const uint8_t* adj_host, const flo
 
 int hdgnn_workspace(hdgnn_handle_t h, const char* name, void** ptr, size_t* bytes) {
     if (!h || !name) return HDGNN_E_INVALID;
-    auto it = h->ws.find(name);
-    if (it == h->ws.end()) return fail(h, HDGNN_E_INVALID, std::string("no workspace buffer named ") + name);
-    if (ptr) *ptr = it->second.p;
-    if (bytes) *bytes = it->second.bytes;
+    const Buf* b;
+    if (int rc = find_ws(h, name, &b)) return rc;
+    if (ptr) *ptr = b->p;
+    if (bytes) *bytes = b->bytes;
     return HDGNN_OK;
 }
 
 int hdgnn_workspace_copy(hdgnn_handle_t h, const char* name, void* dst, size_t bytes, void* stream) {
     if (!h || !name || !dst) return HDGNN_E_INVALID;
-    auto it = h->ws.find(name);
-    if (it == h->ws.end()) return fail(h, HDGNN_E_INVALID, std::string("no workspace buffer named ") + name);
-    if (bytes > it->second.bytes) return fail(h, HDGNN_E_INVALID, std::string("workspace buffer too small: ") + name);
-    CK(h, cudaMemcpyAsync(dst, it->second.p, bytes, cudaMemcpyDefault, (cudaStream_t)stream));
+    const Buf* b;
+    if (int rc = find_ws(h, name, &b)) return rc;
+    if (bytes > b->bytes) return fail(h, HDGNN_E_INVALID, std::string("workspace buffer too small: ") + name);
+    CK(h, cudaMemcpyAsync(dst, b->p, bytes, cudaMemcpyDefault, (cudaStream_t)stream));
     return HDGNN_OK;
 }
 

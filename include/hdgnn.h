@@ -288,8 +288,10 @@ int hdgnn_set_hits_accumulator(hdgnn_handle_t h, uint64_t* acc);
  * sorted scores: hdgnn_eval_counts.  Fused path only (HDGNN_E_UNSUPPORTED otherwise). */
 int hdgnn_set_eval_counters(hdgnn_handle_t h, int64_t* counts);
 
-/* Debug / test introspection: device pointer and size in bytes of a named scratch buffer
- * (RS1 CS1 S1 X2 NB PH QH RS3 CS3 PR PC GRH GCH RS3D CS3D DNB GE RS1D CS1D GPART ...). */
+/* Debug / test introspection: device pointer and size in bytes of a named scratch buffer of the handle.  With HDGNN_F_DEBUG
+ * the intermediates of the last step: S1 X2 NB RS3 CS3F PR PC DNB DX2 GE, RS1 beside the dense entity sweeps and on the
+ * multi-kernel path, and on the fused path the per-commit phase clocks CLK; PEER_STAMPS with HDGNN_PEER_STAMPS set.  A name
+ * the library does not know, and a buffer this handle does not have, each return HDGNN_E_INVALID. */
 int hdgnn_workspace(hdgnn_handle_t h, const char* name, void** ptr, size_t* bytes);
 /* copy the first `bytes` bytes of a named scratch buffer to dst (device or host pointer) on `stream` */
 int hdgnn_workspace_copy(hdgnn_handle_t h, const char* name, void* dst, size_t bytes, void* stream);
