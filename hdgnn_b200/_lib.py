@@ -49,6 +49,7 @@ def _load():
         "hdgnn_peer_status": ([vp], i32),
         "hdgnn_set_hits_accumulator": ([vp, vp], i32),
         "hdgnn_set_eval_counters": ([vp, vp], i32),
+        "hdgnn_set_predictions": ([vp, vp], i32),
         "hdgnn_train_step_peer": ([vp, i32, i32, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp, vp, f32, f32, f32, f32, vp, vp, vp, vp], i32),
         "hdgnn_train_step_peer_host": ([vp, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, f32, f32, f32, f32, vp, vp, vp], i32),
         "hdgnn_infer_host": ([vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp], i32),
@@ -60,6 +61,7 @@ def _load():
         "hdgnn_compact_from_raw": ([i32, i32, vp, i32, vp, i32, vp, vp, vp], i32),
         "hdgnn_pack_label_bits": ([i32, i32, vp, i32, vp, vp], i32),
         "hdgnn_eval_counts": ([i32, i32, vp, vp, i32, vp, vp, i32, vp], i32),
+        "hdgnn_hunk_groups": ([i32, i32, vp, vp, vp, vp], i32),
         "hdgnn_workspace": ([vp, C.c_char_p, C.POINTER(vp), C.POINTER(C.c_size_t)], i32),
         "hdgnn_workspace_copy": ([vp, C.c_char_p, vp, C.c_size_t, vp], i32),
         "hdgnn_profile": ([vp, i32], i32),

@@ -181,6 +181,7 @@ struct hdgnn_handle_s {
     // the caller's stream, which would break the programmatic launch chain optimizer -> mid2)
     unsigned long long* hits_acc = nullptr;   // hdgnn_set_hits_accumulator
     unsigned long long* evc = nullptr;        // hdgnn_set_eval_counters
+    uint32_t* pred = nullptr;                 // hdgnn_set_predictions
     uint32_t* tag_table = nullptr;         // pinned, tag_table[i] = i: immutable DMA source
     unsigned int slot_uses[NSLOT] = {};
     int cur_tag = -1;                      // tag of the staging slot filled by the last stage_inputs call, -1 = ordered by event
@@ -271,9 +272,9 @@ template <int CW, bool BWD, bool RANK1>
 cudaError_t pairsum_attr(size_t smem) {
     return cudaFuncSetAttribute(pairsum_kernel<CW, BWD, RANK1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 }
-template <int CW, bool TRAIN>
+template <int CW, bool TRAIN, bool PRED>
 cudaError_t score_attr(size_t smem) {
-    return cudaFuncSetAttribute(score_kernel<CW, TRAIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    return cudaFuncSetAttribute(score_kernel<CW, TRAIN, PRED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 }
 
 // MaxDynamicSharedMemorySize is a per-function hard cap shared by every handle of the process, so it
@@ -285,14 +286,16 @@ cudaError_t set_attrs(hdgnn_handle_t h, int optin) {
     CW_SWITCH(h->CWe, {
         acc(cudaFuncSetAttribute(pairsum_kernel<CW, false, true>, A, optin));
         acc(cudaFuncSetAttribute(pairsum_kernel<CW, true, true>, A, optin));
-        acc(cudaFuncSetAttribute(score_kernel<CW, false>, A, optin));
-        acc(cudaFuncSetAttribute(score_kernel<CW, true>, A, optin));
+        acc(cudaFuncSetAttribute(score_kernel<CW, false, false>, A, optin));
+        acc(cudaFuncSetAttribute(score_kernel<CW, true, false>, A, optin));
     });
     CW_SWITCH(h->CWc, {
         acc(cudaFuncSetAttribute(pairsum_kernel<CW, false, false>, A, optin));
         acc(cudaFuncSetAttribute(pairsum_kernel<CW, true, false>, A, optin));
-        acc(cudaFuncSetAttribute(score_kernel<CW, false>, A, optin));
-        acc(cudaFuncSetAttribute(score_kernel<CW, true>, A, optin));
+        acc(cudaFuncSetAttribute(score_kernel<CW, false, false>, A, optin));
+        acc(cudaFuncSetAttribute(score_kernel<CW, true, false>, A, optin));
+        acc(cudaFuncSetAttribute(score_kernel<CW, false, true>, A, optin));       // the hunk head writing predictions
+        acc(cudaFuncSetAttribute(score_kernel<CW, true, true>, A, optin));
     });
     acc(cudaFuncSetAttribute(pool_fwd_kernel, A, optin));
     acc(cudaFuncSetAttribute(pool_bwd_kernel, A, optin));
@@ -330,8 +333,13 @@ int launch_score(hdgnn_handle_t h, const char* what, const GridCfg& g, int B, bo
     PROF_BEGIN(h, st);
     CW_SWITCH(g.CW, {
         const size_t smem = score_smem_bytes(CW, g.RT, 4 * g.WP, train);
-        if (train) score_kernel<CW, true><<<grid, block, smem, st>>>(a);
-        else score_kernel<CW, false><<<grid, block, smem, st>>>(a);
+        if (a.pred) {
+            if (train) score_kernel<CW, true, true><<<grid, block, smem, st>>>(a);
+            else score_kernel<CW, false, true><<<grid, block, smem, st>>>(a);
+        } else {
+            if (train) score_kernel<CW, true, false><<<grid, block, smem, st>>>(a);
+            else score_kernel<CW, false, false><<<grid, block, smem, st>>>(a);
+        }
     });
     LAUNCH_CHECK(h, what, st);
     return HDGNN_OK;
@@ -421,7 +429,7 @@ int forward_impl(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float*
         ScoreArgs s{};
         s.bits = in.ybits; s.PR = F(h, WS_PR); s.PC = F(h, WS_PC); s.params = in.params;
         s.o_l = po.scr_w1; s.o_w2 = po.scr_w2; s.o_b2 = po.scr_b2;
-        s.logits = logits; s.probs = probs; s.cep = F(h, WS_CEP);
+        s.logits = logits; s.probs = probs; s.cep = F(h, WS_CEP); s.pred = h->pred;
         s.scale = 10.f / ((float)B_global * (float)(h->Nc * (h->Nc - 1)));
         s.RSm = F(h, WS_RSM); s.CSmp = F(h, WS_CSMP); s.LSmp = F(h, WS_LSMP); s.HSp = F(h, WS_HSP); s.dsump = F(h, WS_DSUMP);
         if ((rc = launch_score(h, "score(hunk)", gc, B, train, s, st))) return rc;
@@ -653,6 +661,7 @@ int fused_forward(hdgnn_handle_t h, int B, int B_global, const Inputs& in, float
     m.wait_flag = in.wait_flag; m.wait_tag = in.wait_tag;
     m.hits_acc = h->hits_acc;
     m.evc = h->evc;
+    m.pred = h->pred;
     m.edge = P.edge ? 1 : 0;
     if (m.edge) { m.RSEg = F(h, WS_RSEG); m.CSEg = F(h, WS_CSEG); m.REg = F(h, WS_REG); m.CEg = F(h, WS_CEG); m.A1F = F(h, WS_A1F); m.PREg = F(h, WS_PREG); }
     m.lay = md.lay;
@@ -1087,6 +1096,13 @@ int hdgnn_set_eval_counters(hdgnn_handle_t h, int64_t* counts) {
     return HDGNN_OK;
 }
 
+int hdgnn_set_predictions(hdgnn_handle_t h, uint32_t* pred) {
+    if (!h) return HDGNN_E_INVALID;
+    if ((uintptr_t)pred & 15) return fail(h, HDGNN_E_INVALID, "pred must be 16-byte aligned");
+    h->pred = pred;
+    return HDGNN_OK;
+}
+
 int hdgnn_peer_status(hdgnn_handle_t h) {
     if (!h) return HDGNN_E_INVALID;
     if (!h->peer_ready) return HDGNN_OK;
@@ -1378,7 +1394,6 @@ int hdgnn_infer_host(hdgnn_handle_t h, int B, const uint8_t* adj_host, const flo
                      float* loss_host, void* stream) {
     int rc = check_host_inputs(h, B, adj_host, x_host, hmap_host, L_host, Y_host, params);
     if (rc) return rc;
-    if (!probs_host) return fail(h, HDGNN_E_INVALID, "null pointer");
     return host_step(h, B, B, adj_host, x_host, hmap_host, L_host, Y_host, params, probs_host, loss_host, nullptr, nullptr, true,
                      stream);
 }

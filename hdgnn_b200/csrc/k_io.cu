@@ -6,9 +6,12 @@
 //  * eval_counts_kernel       -- EvaluationFuncs.py:27-37 (top_ACC), :92-117 (prec / recall / f1, with and without the
 //    ceil-on-channel-0 quirk) and :119-153 (AUC) as integer counters per commit, read straight from the probs the
 //    relation head wrote; the (N,2,Ncr) device->host copy and the Python double loops disappear.
+//  * hunk_groups_kernel       -- the commit-level answer of an untangling: the groups of hunks that a label bitmap (the
+//    predicted relations of hdgnn_set_predictions, or the labels) joins, as connected components.
 //
 // Everything here is integer counting => bit-exact and order independent (integer atomics).
 #include "../../include/hdgnn.h"
+#include "bits.cuh"
 #include "common.cuh"
 
 namespace hdgnn {
@@ -145,6 +148,76 @@ __global__ void __launch_bounds__(EV_T) eval_counts_kernel(int Nc, const float* 
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Hunk groups: weakly connected components of per-commit hunk graphs given as label bitmaps (bits.cuh layout).  One warp per
+// commit.  The commit's rows are staged in shared memory and symmetrised in place, S = A | A^T with the diagonal and the padding
+// dropped (32 x 32 ballot transposes, one unordered block pair at a time, so every block is read before it is written).  The
+// sweep then works on bitsets: lane w holds word w of the unvisited set and of the frontier; a component is seeded at the
+// lowest unvisited hunk -- which is therefore its smallest index, the label -- and every hunk of it ORs its row of S in once.
+// Integer work only: the result does not depend on scheduling.
+constexpr int HG_WARPS_MAX = 4;
+constexpr size_t HG_SMEM_MAX = 48 * 1024;   // commits per CTA are chosen to stay within the default dynamic shared memory
+
+__global__ void __launch_bounds__(32 * HG_WARPS_MAX) hunk_groups_kernel(int B, int n, int WP, const uint32_t* __restrict__ bits,
+                                                                       int32_t* __restrict__ groups, int32_t* __restrict__ ngroups) {
+    extern __shared__ __align__(16) uint32_t hg_smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int b = blockIdx.x * (blockDim.x >> 5) + warp;
+    if (b >= B) return;
+    const int CW = (n + 31) >> 5;
+    uint32_t* S = hg_smem + (size_t)warp * n * WP;
+    {
+        const uint4* src = reinterpret_cast<const uint4*>(bits + (size_t)b * n * WP);
+        uint4* dst = reinterpret_cast<uint4*>(S);
+        for (int i = lane; i < n * WP / 4; i += 32) dst[i] = __ldg(src + i);
+    }
+    __syncwarp();
+    auto colmask = [n](int w) { const int c = n - 32 * w; return c >= 32 ? 0xffffffffu : (1u << c) - 1u; };     // w < CW: c >= 1
+    for (int I = 0; I < CW; ++I) {
+        for (int J = I; J < CW; ++J) {
+            // lane l: word J of row 32 I + l (a) and word I of row 32 J + l (c)
+            const int ri = 32 * I + lane, rj = 32 * J + lane;
+            uint32_t a = ri < n ? S[ri * WP + J] & colmask(J) : 0u;
+            uint32_t c = rj < n ? S[rj * WP + I] & colmask(I) : 0u;
+            if (I == J) { a &= ~(1u << lane); c = a; }
+            uint32_t ta = 0u, tc = 0u;          // lane k: bit k of every lane's a (word I of row 32 J + k of A^T), of c likewise
+#pragma unroll
+            for (int k = 0; k < 32; ++k) {
+                const uint32_t x = __ballot_sync(0xffffffffu, (a >> k) & 1u), y = __ballot_sync(0xffffffffu, (c >> k) & 1u);
+                if (lane == k) { ta = x; tc = y; }
+            }
+            if (ri < n) S[ri * WP + J] = a | tc;
+            if (rj < n && I != J) S[rj * WP + I] = c | ta;
+        }
+    }
+    __syncwarp();
+    uint32_t U = lane < CW ? colmask(lane) : 0u;        // unvisited hunks
+    int32_t* g = groups + (size_t)b * n;
+    int ncomp = 0;
+    for (;;) {
+        const uint32_t any = __ballot_sync(0xffffffffu, U != 0u);
+        if (!any) break;
+        const int sl = __ffs(any) - 1;
+        const int seed = 32 * sl + __ffs(__shfl_sync(0xffffffffu, U, sl)) - 1;
+        const uint32_t U0 = U;
+        uint32_t F = lane == sl ? 1u << (seed & 31) : 0u;      // frontier
+        U &= ~F;
+        for (;;) {
+            const uint32_t fa = __ballot_sync(0xffffffffu, F != 0u);
+            if (!fa) break;
+            const int fl = __ffs(fa) - 1;
+            const int v = 32 * fl + __ffs(__shfl_sync(0xffffffffu, F, fl)) - 1;
+            if (lane == fl) F &= F - 1u;
+            const uint32_t nw = lane < CW ? S[v * WP + lane] & U : 0u;
+            U &= ~nw;
+            F |= nw;
+        }
+        for (uint32_t m = U0 & ~U; m; m &= m - 1u) g[32 * lane + __ffs(m) - 1] = seed;
+        ++ncomp;
+    }
+    if (lane == 0 && ngroups) ngroups[b] = ncomp;
+}
+
 }  // namespace hdgnn
 
 using namespace hdgnn;
@@ -183,6 +256,24 @@ extern "C" int hdgnn_eval_counts(int B, int Nc, const float* probs, const uint8_
     dim3 g((Ncr + EV_CHUNK - 1) / EV_CHUNK, B);
     eval_counts_kernel<<<g, EV_T, 0, st>>>(Nc, probs, Y, y_pitch, (unsigned long long*)counts, (unsigned long long*)auc,
                                           auc_first < 0 ? 0 : auc_first);
+    return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+}
+
+extern "C" int hdgnn_hunk_groups(int B, int n, const uint32_t* bits, int32_t* groups, int32_t* ngroups, void* stream) {
+    if (B < 1 || n < 2 || n > HDGNN_MAX_N || !bits || !groups) return HDGNN_E_INVALID;
+    if (((uintptr_t)bits & 15) || ((uintptr_t)groups & 3) || ((uintptr_t)ngroups & 3)) return HDGNN_E_INVALID;
+    int dev = 0, sms = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
+        return HDGNN_E_CUDA;
+    const int WP = bit_words(n);
+    const size_t per = (size_t)n * WP * 4;
+    // one commit per CTA until the batch covers the SMs, then up to HG_WARPS_MAX (as far as the shared memory allows)
+    int cpc = B / sms;
+    const int fit = (int)(HG_SMEM_MAX / per);
+    if (cpc > fit) cpc = fit;
+    if (cpc > HG_WARPS_MAX) cpc = HG_WARPS_MAX;
+    if (cpc < 1) cpc = 1;
+    hunk_groups_kernel<<<(B + cpc - 1) / cpc, 32 * cpc, cpc * per, (cudaStream_t)stream>>>(B, n, WP, bits, groups, ngroups);
     return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
 }
 

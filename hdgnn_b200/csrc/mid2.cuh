@@ -168,6 +168,7 @@ struct Mid2Args {
     unsigned long long* hits_acc;            // running count of arg-max hits (EvaluationFuncs.py:27-37) over all commits, or null
     unsigned long long* evc;                 // (B,8) per-commit evaluation counters in the layout of hdgnn_eval_counts (EvaluationFuncs.py:27-37,
                                              // 92-117), ADDED to by the relation head, or null
+    uint32_t* pred;                          // (B,Nc,WPc) predicted relations [p1 > p0] as a label bitmap, WRITTEN by the relation head, or null
     const int* wait_flag; int wait_tag;      // host-fed step: the staging copies of this step are complete once *wait_flag == wait_tag
                                              // (written by the copy stream's DMA after the data); null = inputs already ordered
     Mid2Smem lay;                            // shared-memory layout (mid2_layout), computed once on the host: the offsets are kernel
@@ -1346,7 +1347,10 @@ __global__ void __launch_bounds__(M2_T, 1) mid2_kernel(const Mid2Args a) {
 
     // ---------------- G1. relation head: logits, softmax, CE (lanes = columns, all 20 channels) ---------
     float ce_acc = 0.f, d_acc = 0.f, hit_acc = 0.f;
-    const bool EVC = a.evc != nullptr;
+    const bool EVC = a.evc != nullptr, PRED = a.pred != nullptr;
+    if (PRED)           // the predicted-relation bitmap's padding words of this CTA's rows
+        for (int idx = tid, ncb = (Nc + 31) >> 5, np = WPc - ncb; idx < (hr1 - hr0) * np; idx += M2_T)
+            a.pred[((size_t)b * Nc + hr0 + idx / np) * WPc + ncb + idx % np] = 0u;
     uint32_t ev_tpc = 0u, ev_fpc = 0u, ev_tpq = 0u, ev_fpq = 0u, ev_pos = 0u;      // warp-uniform partial counts
     const float* PR01s = PR01;          // row tables of the two head sweeps (G1, G2)
     if (GT) { stage_rows(stg, PR01, 2 * T); __syncthreads(); PR01s = stg; }
@@ -1408,14 +1412,18 @@ __global__ void __launch_bounds__(M2_T, 1) mid2_kernel(const Mid2Args a) {
                     ce_acc += fmaxf(z, 0.f) + __logf(1.f + e);     // e in (0, 1]: absolute error ~1e-7
                     hit_acc += ((p1 > p0) == lab) ? 1.f : 0.f;      // np.argmax over the two channels: a tie is class 0
                 }
-                if (EVC) {
+                if (EVC || PRED) {
                     // evaluation counters: two ballots per 32 pairs, then warp-uniform popcounts against the label word (its
-                    // diagonal and padding bits are zero).  am: arg-max is class 1 (a tie is class 0); qp: the reference's
-                    // ceil-on-channel-0 prediction (EvaluationFuncs.py:95-99)
+                    // diagonal and padding bits are zero).  am: arg-max is class 1 (a tie is class 0) -- also word cb of row r
+                    // of the predicted-relation bitmap; qp: the reference's ceil-on-channel-0 prediction (EvaluationFuncs.py:95-99)
                     const uint32_t vm = (r >> 5) == cb ? colmask & ~(1u << (r & 31)) : colmask;
-                    const uint32_t am = __ballot_sync(0xffffffffu, p1 > p0) & vm, qp = __ballot_sync(0xffffffffu, p0 > 0.f) & vm;
-                    ev_tpc += __popc(am & yw); ev_fpc += __popc(am & ~yw); ev_tpq += __popc(qp & ~yw); ev_fpq += __popc(qp & yw);
-                    ev_pos += __popc(yw & vm);
+                    const uint32_t am = __ballot_sync(0xffffffffu, p1 > p0) & vm;
+                    if (PRED && lane == 0) a.pred[((size_t)b * Nc + r) * WPc + cb] = am;
+                    if (EVC) {
+                        const uint32_t qp = __ballot_sync(0xffffffffu, p0 > 0.f) & vm;
+                        ev_tpc += __popc(am & yw); ev_fpc += __popc(am & ~yw); ev_tpq += __popc(qp & ~yw); ev_fpq += __popc(qp & yw);
+                        ev_pos += __popc(yw & vm);
+                    }
                 }
                 if (TRAIN) {
                     const float dv = valid ? a.scale * (p1 - (lab ? 1.f : 0.f)) : 0.f;

@@ -28,6 +28,7 @@ struct ScoreArgs {
     float* logits;        // (B,2,N(N-1)) or nullptr
     float* probs;         // (B,2,N(N-1)) or nullptr
     float* soft;          // (B,N,N,2) soft labels for the entity-edge branch, or nullptr
+    uint32_t* pred;       // (B,N,WP) predicted relations [p1 > p0] as a label bitmap (hdgnn_set_predictions), or nullptr
     float* cep;           // (B,S) sum of CE over the tile
     float scale;          // delta = scale * (p1 - l)            (hunk head, CE loss)
     const float* dsoft;   // (B,N,N,2) upstream d/d(a0,a1): delta = a1*a0*(da1-da0)   (edge head)
@@ -51,7 +52,9 @@ __host__ __device__ inline size_t score_smem_bytes(int CW, int RT, int row_bytes
     return off + 16;
 }
 
-template <int CW, bool TRAIN>
+// PRED: the launch writes the predicted-relation bitmap (a.pred).  The flag is a template parameter so that the instantiations
+// without it keep the plain lane loop and its register allocation.
+template <int CW, bool TRAIN, bool PRED>
 __global__ void __launch_bounds__(32 * HD, 1) score_kernel(const ScoreArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     constexpr int NP = CW * 32;
@@ -129,8 +132,10 @@ __global__ void __launch_bounds__(32 * HD, 1) score_kernel(const ScoreArgs a) {
             for (int kk = 0; kk < HD; ++kk) Rs[kk] = PRt[row * HD + kk];
             const float* lrow = reinterpret_cast<const float*>(labf + (row >> 2) * NP) + (row & 3);
             float* drow = reinterpret_cast<float*>(delt + (row >> 2) * NP) + (row & 3);
-            for (int j = lane; j < N; j += 32) {
-                if (j == i) continue;
+            // PRED: whole 32-column segments, so that the prediction ballot is warp-uniform; columns >= N read the NEG_BIG / zero
+            // padding of PCt and the label tile and store nothing
+            for (int j = lane; j < (PRED ? CW * 32 : N); j += 32) {
+                if (!PRED && j == i) continue;
                 const float l = lrow[4 * j];
                 float l0 = b20, l1 = b21;
 #pragma unroll
@@ -145,6 +150,12 @@ __global__ void __launch_bounds__(32 * HD, 1) score_kernel(const ScoreArgs a) {
                 const float inv = 1.f / (1.f + e);
                 const float pb = inv, ps = e * inv;
                 const float p1 = d >= 0.f ? pb : ps, p0 = d >= 0.f ? ps : pb;
+                if (PRED) {         // predicted relation: np.argmax over the two channels, a tie is class 0
+                    const bool valid = j < N && j != i;
+                    const uint32_t am = __ballot_sync(0xffffffffu, valid && p1 > p0);
+                    if (lane == 0) a.pred[((size_t)b * N + i) * WP + (j >> 5)] = am;
+                    if (!valid) continue;
+                }
                 const size_t q = (size_t)i * (N - 1) + j - (j > i);
                 if (a.logits) {
                     a.logits[((size_t)b * 2 + 0) * npair + q] = l0;
@@ -172,6 +183,7 @@ __global__ void __launch_bounds__(32 * HD, 1) score_kernel(const ScoreArgs a) {
                     d_acc += dl;
                 }
             }
+            if (PRED && lane < WP - CW) a.pred[((size_t)b * N + i) * WP + CW + lane] = 0u;      // padding words of the row
         }
     }
     const float ce_tot = block_sum(ce_acc, scratch);

@@ -122,6 +122,7 @@ class Engine:
         self._h = h
         self.tdev = torch.device("cuda", device)
         self.host_bits = bool(flags & F_LABEL_BITS)      # label grids travel as bitmaps (host and device entry points)
+        self._pred_rows = None                           # rows of the set_predictions buffer, None = predictions off
         # row pitch in bytes of the label arrays the device entry points take
         self.pe, self.pc = (4 * bit_words(Ne), 4 * bit_words(Nc)) if self.host_bits else (label_pitch(Ne), label_pitch(Nc))
 
@@ -139,17 +140,22 @@ class Engine:
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.tdev).cuda_stream)
 
+    def _check_rows(self, B: int):
+        assert self._pred_rows is None or B <= self._pred_rows, "the set_predictions buffer has fewer rows than the batch"
+
     def _check_batch(self, b: DeviceBatch, params: torch.Tensor):
         assert b.Ne == self.Ne and b.Nc == self.Nc, "batch shape does not match the engine"
+        self._check_rows(b.B)
         assert params.dtype == torch.float32 and params.is_cuda and params.numel() == self.n_params
 
     # -- device-resident entry points ---------------------------------------------------------
-    def forward(self, b: DeviceBatch, params: torch.Tensor, want_logits=True):
-        """Inference graph of model_2.py:486-502 -> (probs (B,2,Ncr), logits or None, CE scalar tensor)."""
+    def forward(self, b: DeviceBatch, params: torch.Tensor, want_logits=True, want_probs=True):
+        """Inference graph of model_2.py:486-502 -> (probs (B,2,Ncr) or None, logits or None, CE scalar tensor).
+        want_probs=False: the probabilities are not written (a caller of set_predictions that wants only the bitmap)."""
         self._check_batch(b, params)
         B = b.B
-        probs = torch.empty(B, 2, self.Ncr, dtype=torch.float32, device=self.tdev)
-        logits = torch.empty_like(probs) if want_logits else None
+        probs = torch.empty(B, 2, self.Ncr, dtype=torch.float32, device=self.tdev) if want_probs else None
+        logits = torch.empty(B, 2, self.Ncr, dtype=torch.float32, device=self.tdev) if want_logits else None
         loss = torch.empty(1, dtype=torch.float32, device=self.tdev)
         check(lib.hdgnn_forward(self._h, B, _p(b.adj), self.pe, _p(b.x), _p(b.hmap), _p(b.L), _p(b.Y), self.pc,
                                 _p(params), _p(logits), _p(probs), _p(loss), self._stream()), self._h)
@@ -197,6 +203,7 @@ class Engine:
         tensors (adj / Y as pack_label_bits bitmaps when the engine was created with F_LABEL_BITS);
         loss3 (3,) pinned float32 receives {CE, loss_map, loss_para}.  Asynchronous."""
         B = adj.shape[0]
+        self._check_rows(B)
         check(lib.hdgnn_train_step_host(self._h, B, _p(adj), _p(x), _p(hmap), _p(L), _p(Y), _p(params), _p(m), _p(v),
                                         _p(step_counter), lr, beta1, beta2, eps, _p(probs), _p(loss3),
                                         self._stream()), self._h)
@@ -204,6 +211,7 @@ class Engine:
     def forward_backward_host(self, adj, x, hmap, L, Y, params, grads, B_global, loss=None, probs=None):
         """Commit-sharded training from pinned host tensors: H2D + forward + backward; grads / loss / probs on device."""
         B = adj.shape[0]
+        self._check_rows(B)
         check(lib.hdgnn_forward_backward_host(self._h, B, B_global, _p(adj), _p(x), _p(hmap), _p(L), _p(Y), _p(params),
                                               _p(probs), _p(loss), _p(grads), self._stream()), self._h)
 
@@ -256,6 +264,17 @@ class Engine:
         self._evc_ref = counts          # keep the tensor alive while the handle points at it
         return True
 
+    def set_predictions(self, bits: Optional[torch.Tensor]):
+        """bits: (B, Nc, bit_words(Nc)) int32 CUDA tensor that the relation head of every later forward / training call WRITES the
+        commits' predicted relations to, as a label bitmap (bit (s,t) = [p1 > p0], the arg-max; hdgnn_set_predictions); row b is
+        commit b of a call, so B must cover the batch size of every call made while it is set.  None: off."""
+        if bits is not None:
+            assert bits.dtype == torch.int32 and bits.is_cuda and bits.is_contiguous()
+            assert bits.dim() == 3 and bits.shape[1:] == (self.Nc, bit_words(self.Nc))
+        self._pred_rows = None if bits is None else bits.shape[0]
+        check(lib.hdgnn_set_predictions(self._h, _p(bits)), self._h)
+        self._pred_ref = bits           # keep the tensor alive while the handle points at it
+
     def peer_status(self):
         """Raises HdgnnError(E_PEER) if a gradient exchange timed out since peer_attach (synchronises with the device)."""
         check(lib.hdgnn_peer_status(self._h), self._h)
@@ -271,12 +290,16 @@ class Engine:
     def train_step_peer_host(self, adj, x, hmap, L, Y, params, m, v, step_counter, loss3, probs=None,
                              lr=3e-4, beta1=0.9, beta2=0.999, eps=1e-8):
         B = adj.shape[0]
+        self._check_rows(B)
         check(lib.hdgnn_train_step_peer_host(self._h, B, B * self.peer_world, _p(adj), _p(x), _p(hmap), _p(L), _p(Y), _p(params),
                                              _p(m), _p(v), _p(step_counter), lr, beta1, beta2, eps, _p(probs), _p(loss3),
                                              self._stream()), self._h)
 
-    def infer_host(self, adj, x, hmap, L, Y, params, probs, loss=None):
+    def infer_host(self, adj, x, hmap, L, Y, params, probs=None, loss=None):
+        """Inference from pinned host tensors (layouts of train_step_host).  probs: host or device tensor (B, 2, Ncr), or None
+        when only the predictions (set_predictions), the counters (set_eval_counters) or the loss are wanted."""
         B = adj.shape[0]
+        self._check_rows(B)
         check(lib.hdgnn_infer_host(self._h, B, _p(adj), _p(x), _p(hmap), _p(L), _p(Y), _p(params), _p(probs),
                                    _p(loss), self._stream()), self._h)
 
@@ -451,3 +474,20 @@ def eval_counts(probs: torch.Tensor, Y: torch.Tensor, auc: bool = False, auc_fir
     st = C.c_void_p(torch.cuda.current_stream(probs.device).cuda_stream)
     check(lib.hdgnn_eval_counts(B, Nc, _p(probs), _p(Y), pitch, _p(counts), _p(a), auc_first, st))
     return counts, a
+
+
+def hunk_groups(bits: torch.Tensor):
+    """Hunk groups of label bitmaps (hdgnn_hunk_groups): bits (B, n, bit_words(n)) int32 CUDA tensor, e.g. what set_predictions
+    receives, or the labels.  Hunks s and t share a group when bit (s,t) or bit (t,s) is set.  Returns (groups (B, n) int32: the
+    smallest hunk index of each hunk's group, ngroups (B,) int32)."""
+    if not bits.is_cuda:
+        raise RuntimeError("hunk_groups needs a CUDA tensor; there is no CPU fallback")
+    bits = bits.contiguous()
+    B, n, wp = bits.shape
+    if bits.dtype not in (torch.int32, torch.uint32) or wp != bit_words(n):
+        raise ValueError(f"hunk_groups needs an int32 label bitmap of bit_words({n}) = {bit_words(n)} words per row")
+    groups = torch.empty(B, n, dtype=torch.int32, device=bits.device)
+    ngroups = torch.empty(B, dtype=torch.int32, device=bits.device)
+    st = C.c_void_p(torch.cuda.current_stream(bits.device).cuda_stream)
+    check(lib.hdgnn_hunk_groups(B, n, _p(bits), _p(groups), _p(ngroups), st))
+    return groups, ngroups

@@ -477,6 +477,59 @@ class graph2graph(object):
             log('test time:' + str(end_time - start_time))
         return out, C_edge_t1
 
+    def untangle(self, args=None, data=None, root=".", quirk_q2=True, log=print):
+        """The untangling answer over the test half, with the checkpoint, batches and entity->hunk maps of test(): the predicted
+        relations of every commit as a label bitmap (hdgnn_set_predictions; the probabilities are never written) and the hunk
+        groups they give (hdgnn_hunk_groups), beside the groups of the labels.  Writes C_group_t{Ne}.npy (predicted groups) and
+        C_group_y{Ne}.npy (labelled groups), (n_test, Nc) int32, each hunk labelled with the smallest hunk index of its group, and
+        logs the number of commits whose predicted partition of all Nc hunks equals the labelled one.  Padding hunks are not
+        masked: the library cannot tell them from real hunks that relate to nothing."""
+        from .engine import bit_words, hunk_groups
+        repo = getattr(args, "Repo", self.Repo)
+        train, test = data if data is not None else self._load(root)
+        self.initialize()
+        ckroot = self.checkpoint_dir if os.path.isabs(self.checkpoint_dir) else os.path.join(root, self.checkpoint_dir)
+        if self.load(os.path.join(ckroot, self.Repo)) or self.load(ckroot, note=" [*] (found under the directory save() writes to)"):
+            log(" [*] Load SUCCESS")
+        else:
+            log(" [!] Load failed...")
+        mb = self.mini_batch_num
+        nb = int(test.B / mb)
+        n = nb * mb
+        dev = self.engine.tdev
+        pred = torch.zeros(max(n, 1), self.Nc, bit_words(self.Nc), dtype=torch.int32, device=dev)
+        groups = torch.zeros(max(n, 1), self.Nc, dtype=torch.int32, device=dev)
+        label_groups = torch.zeros_like(groups)
+        start_time = time.time()
+        alive = []       # the library DMAs from these pinned buffers asynchronously: keep them until the final synchronize
+        try:
+            for j in range(nb):
+                saved = (self.world, self.rank)
+                self.world, self.rank = 1, 0                        # inference is not sharded
+                hb = self.host_batch(self._batch(test, train, j, quirk_q2))
+                self.world, self.rank = saved
+                alive.append(hb)
+                rows = slice(j * mb, (j + 1) * mb)
+                self.engine.set_predictions(pred[rows])
+                self.engine.infer_host(*hb.tensors(), self.params, None, None)
+                groups[rows] = hunk_groups(pred[rows])[0]
+                label_groups[rows] = hunk_groups(hb.Yw.to(dev, non_blocking=True))[0]
+        finally:
+            self.engine.set_predictions(None)
+        exact = int((groups[:n] == label_groups[:n]).all(1).sum()) if nb else 0      # synchronises
+        alive.clear()
+        end_time = time.time()
+        out = dict(pred_bits=pred[:n].cpu().numpy(), groups=groups[:n].cpu().numpy(),
+                   label_groups=label_groups[:n].cpu().numpy(), exact_partitions=exact)
+        if self.rank == 0:
+            step_dir = os.path.join(root, 'outputSelf/' + repo + '/model_%d/' % self.variant + str(self.Step) + '/')
+            os.makedirs(step_dir, exist_ok=True)
+            np.save(step_dir + 'C_group_t' + str(self.Ne) + '.npy', out["groups"])
+            np.save(step_dir + 'C_group_y' + str(self.Ne) + '.npy', out["label_groups"])
+            log('exact_partitions: ' + str(exact) + ' / ' + str(n))
+            log('test time:' + str(end_time - start_time))
+        return out
+
     # ------------------------------------------------------------------------------------------
     # checkpoints: same directory layout and naming as tf.train.Saver (model_2.py:427-451), as .npz
     def save(self, checkpoint_dir, step, snapshot=None):

@@ -199,7 +199,9 @@ int hdgnn_train_step_peer_host(hdgnn_handle_t h, int B, int B_global,
                                float lr, float beta1, float beta2, float eps,
                                float* probs_out, float* loss3_host, void* stream);
 
-/* Inference from HOST buffers: H2D, forward, copy-out of probs (B*2*Ncr floats; host or device pointer) and D2H of CE. */
+/* Inference from HOST buffers: H2D, forward, copy-out of probs (B*2*Ncr floats; host or device pointer) and D2H of CE.
+ * probs_host may be NULL: the probabilities are then neither written nor copied (a caller that wants only the predicted
+ * relations of hdgnn_set_predictions, the counters of hdgnn_set_eval_counters or the loss). */
 int hdgnn_infer_host(hdgnn_handle_t h, int B,
                      const uint8_t* adj_host, const float* x_host, const int32_t* hmap_host,
                      const int32_t* L_host, const uint8_t* Y_host,
@@ -265,6 +267,13 @@ int hdgnn_compact_from_raw(int N, int n, const void* raw, int raw_is_f64, uint8_
  * hdgnn_compact_from_raw, bits (N,n,hdgnn_bit_words(n)) uint32; diagonal and padding bits come out zero. */
 int hdgnn_pack_label_bits(int N, int n, const uint8_t* grid, int pitch, uint32_t* bits, void* stream);
 
+/* Weakly connected components of per-commit hunk graphs given as label bitmaps (HDGNN_F_LABEL_BITS layout, e.g. the output of
+ * hdgnn_set_predictions, or the labels Y): hunks s and t are joined when bit (s,t) OR bit (t,s) is set; diagonal and padding
+ * bits are ignored.  bits (B, n, hdgnn_bit_words(n)) uint32, 16-byte aligned; groups (B, n) int32 receives, for every hunk, the
+ * SMALLEST hunk index of its component (a canonical labelling: two partitions are equal iff the arrays are equal); ngroups (B)
+ * int32 or NULL receives the number of components.  2 <= n <= HDGNN_MAX_N.  Integer-exact, deterministic.  Stateless. */
+int hdgnn_hunk_groups(int B, int n, const uint32_t* bits, int32_t* groups, int32_t* ngroups, void* stream);
+
 /* Evaluation counters on the device, replaces the loops of EvaluationFuncs.py:27-37 (top_ACC), :92-117 (prec / recall /
  * f1) and :119-153 (AUC) over the probs the relation head wrote.  probs (B,2,Ncr) f32, Y (B,Nc,y_pitch) u8.
  * counts (B,8) int64: {arg-max hits, quirk tp, fp, fn (ceil of channel 0, as the reference scores), conventional tp, fp,
@@ -287,6 +296,15 @@ int hdgnn_set_hits_accumulator(hdgnn_handle_t h, uint64_t* acc);
  * caller zeroes the rows and re-points `counts` per batch.  NULL switches it off.  AUC (EvaluationFuncs.py:119-153) needs the
  * sorted scores: hdgnn_eval_counts.  Fused path only (HDGNN_E_UNSUPPORTED otherwise). */
 int hdgnn_set_eval_counters(hdgnn_handle_t h, int64_t* counts);
+
+/* The model's answer in the label format: while `pred` (device, (B, Nc, hdgnn_bit_words(Nc)) uint32, 16-byte aligned,
+ * caller-owned; row b = commit b of a call) is set, every forward / training call WRITES (does not add) each commit's
+ * predicted relations in the HDGNN_F_LABEL_BITS layout: bit (s,t) = [p1(s,t) > p0(s,t)] (np.argmax over the two channels, a
+ * tie is class 0: the y_pred of top_ACC and of the conventional prec / recall form, EvaluationFuncs.py:27-37, 92-117);
+ * diagonal bits, padding bits and padding words are written zero.  The relation head stores one word per 32 hunk pairs; the
+ * probabilities may be switched off (probs = NULL).  NULL switches it off.  Available on the fused and on the multi-kernel
+ * path.  hdgnn_hunk_groups turns the bitmap into hunk groups. */
+int hdgnn_set_predictions(hdgnn_handle_t h, uint32_t* pred);
 
 /* Debug / test introspection: device pointer and size in bytes of a named scratch buffer of the handle.  With HDGNN_F_DEBUG
  * the intermediates of the last step: S1 X2 NB RS3 CS3F PR PC DNB DX2 GE, RS1 beside the dense entity sweeps and on the

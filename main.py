@@ -5,7 +5,8 @@ Same flags and defaults, same loop over the three (Step, Ne, Nc, Ner, Ncr) prese
 given on the command line overrides ALL presets, as in the reference.  Extra flags: --variant
 (1-4 = model_1..model_4, default 2 = the model main.py imports), --root (directory holding
 Adjset/ and dataset/), --seed, --no_q2 (feed each batch its own entity->hunk maps instead of the
-reference's first-Mini_batch slice, model_2.py:376-381).
+reference's first-Mini_batch slice, model_2.py:376-381).  Extra value --Type untangle: the hunk groups the trained model
+predicts for every test commit (graph2graph.untangle).
 Multi-GPU: launch with `python -m torch.distributed.run --nproc-per-node N main.py ...`.
 """
 import argparse
@@ -72,6 +73,8 @@ def main(argv=None):
             results.append(model.train(args, root=args.root, quirk_q2=not args.no_q2))
         if args.Type == 'test':
             results.append(model.test(args, root=args.root, quirk_q2=not args.no_q2))
+        if args.Type == 'untangle':
+            results.append(model.untangle(args, root=args.root, quirk_q2=not args.no_q2))
         model.engine.close()
     return results
 

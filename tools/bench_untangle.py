@@ -1,0 +1,163 @@
+"""Cost of the untangling output at Ne = 200, B = 100, Nc in {74, 256, 512} (variant 2, label bitmaps):
+  (a) the device-resident forward writing the probabilities against the same forward writing only the predicted-relation
+      bitmap (hdgnn_set_predictions, probs NULL);
+  (b) host-fed inference end to end: probabilities copied to pinned host memory against predictions + hunk groups copied to
+      pinned host memory (hdgnn_infer_host with probs NULL, then hdgnn_hunk_groups);
+  (c) the hunk_groups kernel alone, on predicted and on label bitmaps.
+Device inputs rotate through copies that together exceed the 126 MB L2; every arm is timed in blocks that alternate with the
+other arm's, and the median block is reported.  The card's name and power limit are read in the same run.
+Usage: python tools/bench_untangle.py [--out result.json]"""
+import argparse, json, os, statistics, subprocess, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+import numpy as np, torch
+from hdgnn_b200.engine import Engine, DeviceBatch, F_LABEL_BITS, bit_words, hunk_groups
+from hdgnn_b200.model import HostBatch
+from hdgnn_b200.synthetic import make_commits
+
+L2_BYTES = 126 << 20
+B, Ne, REPS = 100, 200, 9
+
+
+def card():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                       capture_output=True, text=True).stdout.strip().splitlines()
+    return {"nvidia_smi": q[torch.cuda.current_device()] if q else None, "torch_name": torch.cuda.get_device_name()}
+
+
+def rotate(tensors, nbytes):
+    """Enough device copies of a list of batches that one pass over them reads more than the L2 holds."""
+    copies = max(len(tensors), -(-2 * L2_BYTES // max(nbytes, 1)))
+    return [tensors[i % len(tensors)].clone() if torch.is_tensor(tensors[i % len(tensors)]) else
+            DeviceBatch(*(getattr(tensors[i % len(tensors)], k).clone() for k in ("adj", "x", "hmap", "L", "Y")), Ne=tensors[0].Ne,
+                        Nc=tensors[0].Nc) for i in range(copies)]
+
+
+def timed(arms, calls):
+    """{name: median ms per call} over REPS blocks of `calls` calls, the arms alternating block by block."""
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    got = {k: [] for k in arms}
+    for name, fn in arms.items():          # warm-up of every arm
+        for k in range(3):
+            fn(k)
+    torch.cuda.synchronize()
+    for r in range(REPS):
+        for name, fn in arms.items():
+            e0.record()
+            for k in range(calls):
+                fn(r * calls + k)
+            e1.record()
+            torch.cuda.synchronize()
+            got[name].append(e0.elapsed_time(e1) / calls)
+    return {k: statistics.median(v) for k, v in got.items()}, got
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--out", default=None)
+    args = ap.parse_args()
+    out = {"card": card(), "B": B, "Ne": Ne, "variant": 2, "reps": REPS, "what": __doc__.split("Usage")[0].strip(), "rows": []}
+    for Nc in (74, 256, 512):
+        eng = Engine(Ne, Nc, variant=2, max_batch=B, flags=F_LABEL_BITS)
+        WPc = bit_words(Nc)
+        cbs = [make_commits(B, Ne, Nc, seed=4040 + i) for i in range(4)]
+        dbs = [DeviceBatch.from_numpy(c.adj, c.x, c.hmap, c.L, c.Y, eng.tdev, bits=True) for c in cbs]
+        per_batch = sum(t.numel() * t.element_size() for t in (dbs[0].adj, dbs[0].x, dbs[0].hmap, dbs[0].L, dbs[0].Y))
+        pool = rotate(dbs, per_batch)
+        g = torch.Generator().manual_seed(1)
+        params = (0.1 * torch.randn(eng.n_params, generator=g)).cuda()
+        pred = torch.zeros(B, Nc, WPc, dtype=torch.int32, device="cuda")
+        row = {"Nc": Nc, "device_pool_batches": len(pool)}
+
+        # (a) device-resident forward
+        def fwd_probs(k):
+            eng.forward(pool[k % len(pool)], params, want_logits=False)
+
+        def fwd_pred(k):
+            eng.forward(pool[k % len(pool)], params, want_logits=False, want_probs=False)
+        blocks_a = {"probs": [], "pred": []}
+        for r in range(REPS):
+            eng.set_predictions(None)
+            m1, _ = timed_once(fwd_probs, r, 20)
+            eng.set_predictions(pred)
+            m2, _ = timed_once(fwd_pred, r, 20)
+            blocks_a["probs"].append(m1); blocks_a["pred"].append(m2)
+        eng.set_predictions(None)
+        ms_a = {k: statistics.median(v) for k, v in blocks_a.items()}
+        row["a_device_forward"] = {"ms_per_batch_probs": ms_a["probs"], "ms_per_batch_pred_only": ms_a["pred"],
+                                   "commits_per_s_probs": B / ms_a["probs"] * 1e3, "commits_per_s_pred_only": B / ms_a["pred"] * 1e3,
+                                   "blocks_ms": blocks_a}
+
+        # (b) host-fed inference end to end
+        hbs = [HostBatch(c, bits=True) for c in cbs]
+        probs_h = torch.empty(B, 2, Nc * (Nc - 1), dtype=torch.float32).pin_memory()
+        pred_h = torch.empty(B, Nc, WPc, dtype=torch.int32).pin_memory()
+        groups_h = torch.empty(B, Nc, dtype=torch.int32).pin_memory()
+        loss_h = torch.empty(1, dtype=torch.float32).pin_memory()
+
+        def host_probs(k):
+            eng.infer_host(*hbs[k % len(hbs)].tensors(), params, probs_h, loss_h)
+
+        def host_groups(k):
+            eng.infer_host(*hbs[k % len(hbs)].tensors(), params, None, loss_h)
+            gr, _ = hunk_groups(pred)
+            pred_h.copy_(pred, non_blocking=True)
+            groups_h.copy_(gr, non_blocking=True)
+        calls = 10 if Nc >= 256 else 40
+        blocks_b = {"probs": [], "pred_groups": []}
+        for r in range(REPS):
+            eng.set_predictions(None)
+            blocks_b["probs"].append(timed_once(host_probs, r, calls)[0])
+            eng.set_predictions(pred)
+            blocks_b["pred_groups"].append(timed_once(host_groups, r, calls)[0])
+        eng.set_predictions(None)
+        ms_b = {k: statistics.median(v) for k, v in blocks_b.items()}
+        row["b_host_fed"] = {"ms_per_batch_probs_to_host": ms_b["probs"], "ms_per_batch_pred_groups_to_host": ms_b["pred_groups"],
+                             "commits_per_s_probs_to_host": B / ms_b["probs"] * 1e3,
+                             "commits_per_s_pred_groups_to_host": B / ms_b["pred_groups"] * 1e3,
+                             "probs_bytes_per_batch": probs_h.numel() * 4,
+                             "pred_groups_bytes_per_batch": pred_h.numel() * 4 + groups_h.numel() * 4, "blocks_ms": blocks_b}
+
+        # (c) hunk_groups alone, on predicted and on label bitmaps
+        preds = []
+        eng.set_predictions(pred)
+        for db in dbs:
+            eng.forward(db, params, want_logits=False, want_probs=False)
+            preds.append(pred.clone())
+        eng.set_predictions(None)
+        bitmap_bytes = B * Nc * WPc * 4
+        pred_pool = rotate(preds, bitmap_bytes)
+        lab_pool = rotate([db.Y for db in dbs], bitmap_bytes)
+        ms_c, blocks_c = timed({"pred": lambda k: hunk_groups(pred_pool[k % len(pred_pool)]),
+                                "labels": lambda k: hunk_groups(lab_pool[k % len(lab_pool)])}, 50)
+        ng_pred = float(hunk_groups(pred_pool[0])[1].float().mean())
+        ng_lab = float(hunk_groups(lab_pool[0])[1].float().mean())
+        row["c_hunk_groups"] = {"us_per_batch_pred": ms_c["pred"] * 1e3, "us_per_batch_labels": ms_c["labels"] * 1e3,
+                                "commits_per_s_pred": B / ms_c["pred"] * 1e3, "commits_per_s_labels": B / ms_c["labels"] * 1e3,
+                                "mean_groups_pred": ng_pred, "mean_groups_labels": ng_lab, "bitmap_pool_batches": len(pred_pool),
+                                "blocks_ms": blocks_c}
+        print(json.dumps({k: v for k, v in row.items()}, default=str))
+        out["rows"].append(row)
+        del pool, pred_pool, lab_pool
+        eng.close()
+        torch.cuda.empty_cache()
+    out["card_after"] = card()
+    if args.out:
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        json.dump(out, open(args.out, "w"), indent=1)
+
+
+def timed_once(fn, r, calls):
+    """ms per call of one block of `calls` calls (ends in a device synchronise)."""
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    fn(r * calls)
+    torch.cuda.synchronize()
+    e0.record()
+    for k in range(calls):
+        fn(r * calls + k)
+    e1.record()
+    torch.cuda.synchronize()
+    return e0.elapsed_time(e1) / calls, None
+
+
+if __name__ == "__main__":
+    main()
