@@ -137,3 +137,41 @@ def auc_from_counts(counts, auc, ncr, quirks=True, first=0):
         return float(vals[-1])
     good = vals[first:][~np.isnan(vals[first:])]
     return float(good.mean()) if good.size else float("nan")
+
+
+def partition_metrics_from_counts(counts):
+    """Group-level scores of an untangling from the partition-agreement counters of hdgnn_partition_counts (include/hdgnn.h):
+    counts (N,8) = {real hunks m, pairs joined in both, by pred, by truth, groups of pred, of truth, sum of largest overlaps
+    of the pred groups, of the truth groups}.
+      exact            commits whose two partitions of the real hunks are equal (the three pair counts agree);
+      pair_precision   sum both / sum pred, pair_recall = sum both / sum truth, pair_f1 = 2 sum both / (sum pred + sum truth):
+                       pooled over commits, 0.0 on an empty denominator;
+      rand, ari        mean over the commits with m >= 2 of sklearn's rand_score and adjusted_rand_score (1.0 when no pair
+                       is joined by one partition and split by the other); nan if there is no such commit;
+      purity           sum of largest overlaps of the pred groups / sum m (inverse_purity: of the truth groups), 0.0 if no hunk;
+      groups_pred_mean, groups_truth_mean: groups per commit (nan if there is no commit).
+    Raises ValueError on a row of -1 (a commit the kernel could not score)."""
+    c = np.asarray(counts, dtype=np.int64).reshape(-1, 8)
+    if (c < 0).any():
+        raise ValueError("partition counters hold a row of -1: a commit with nh outside [0, n] or a label outside [0, n)")
+    m, both, jp, jt = (c[:, k] for k in range(4))
+    S = c.sum(0)
+
+    def ratio(a, b):
+        return float(a / b) if b > 0 else 0.0
+
+    M = m * (m - 1) // 2                                     # pairs of real hunks
+    fp, fn = jp - both, jt - both                            # joined by pred only, by truth only
+    tn = M - both - fp - fn
+    sel = m >= 2
+    with np.errstate(divide="ignore", invalid="ignore"):
+        rand = (both + tn) / M
+        den = (both + fn) * (fn + tn) + (both + fp) * (fp + tn)
+        ari = np.where((fp == 0) & (fn == 0), 1.0, 2.0 * (both * tn - fn * fp) / den)
+    return dict(commits=int(c.shape[0]), exact=int(((both == jp) & (both == jt)).sum()),
+                pair_precision=ratio(S[1], S[2]), pair_recall=ratio(S[1], S[3]), pair_f1=ratio(2 * S[1], S[2] + S[3]),
+                rand=float(rand[sel].mean()) if sel.any() else float("nan"),
+                ari=float(ari[sel].mean()) if sel.any() else float("nan"),
+                purity=ratio(S[6], S[0]), inverse_purity=ratio(S[7], S[0]),
+                groups_pred_mean=float(c[:, 4].mean()) if c.shape[0] else float("nan"),
+                groups_truth_mean=float(c[:, 5].mean()) if c.shape[0] else float("nan"))

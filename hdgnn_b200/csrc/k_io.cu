@@ -8,6 +8,9 @@
 //    relation head wrote; the (N,2,Ncr) device->host copy and the Python double loops disappear.
 //  * hunk_groups_kernel       -- the commit-level answer of an untangling: the groups of hunks that a label bitmap (the
 //    predicted relations of hdgnn_set_predictions, or the labels) joins, as connected components.
+//  * partition_counts_kernel  -- how well two such groupings agree, per commit and over its real hunks only: pair counts,
+//    group counts and largest overlaps, from which EvaluationFuncs.partition_metrics_from_counts derives pair precision /
+//    recall / F1, the (adjusted) Rand index and purity.
 //
 // Everything here is integer counting => bit-exact and order independent (integer atomics).
 #include "../../include/hdgnn.h"
@@ -218,6 +221,97 @@ __global__ void __launch_bounds__(32 * HG_WARPS_MAX) hunk_groups_kernel(int B, i
     if (lane == 0 && ngroups) ngroups[b] = ncomp;
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Partition agreement of two hunk labellings per commit, over the real hunks s < m = nh[b].  One warp per commit.  Every label
+// value l owns a bitmap row of its hunks, Gp[l] (pred) and Gt[l] (truth), built by shared-memory atomicOr (integer, order-free);
+// only the words below ceil(m / 32) of a row are used, and only the rows of labels that occur are cleared.  For hunk s with
+// P = Gp[pred[s]], T = Gt[truth[s]]: popc(P & T) is the contingency cell n_ij holding s, so
+//   sum_s (popc(P & T) - 1) = 2 * pairs joined in both, sum_s (popc(P) - 1) = 2 * pairs joined by pred (truth likewise);
+//   s is its pred group's representative when it is the lowest bit of P, so the representatives count the groups;
+//   max_j n_ij of pred group i is the max of popc(P & T) over its hunks (every non-empty cell holds one of them): an atomicMax
+//   per pred label, summed over the representatives, gives counter 6, the same per truth label counter 7.
+// The row stride is odd so that lanes reading word w of different rows mostly hit different banks.
+constexpr int PC_WARPS_MAX = 4;
+constexpr size_t PC_SMEM_MAX = 200 * 1024;   // two commits per CTA at n = 512 (76 KB each)
+
+__host__ __device__ inline int pc_stride(int n) { return ((n + 31) >> 5) | 1; }
+__host__ __device__ inline size_t pc_smem_words(int n) { return (size_t)n * (2 * pc_stride(n) + 4); }
+
+__global__ void __launch_bounds__(32 * PC_WARPS_MAX) partition_counts_kernel(int B, int n, const int32_t* __restrict__ pred,
+                                                                             const int32_t* __restrict__ truth,
+                                                                             const int32_t* __restrict__ nh,
+                                                                             long long* __restrict__ counts) {
+    extern __shared__ __align__(16) uint32_t pc_smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int b = blockIdx.x * (blockDim.x >> 5) + warp;
+    if (b >= B) return;
+    const int ST = pc_stride(n);
+    uint32_t* Gp = pc_smem + (size_t)warp * pc_smem_words(n);
+    uint32_t* Gt = Gp + (size_t)n * ST;
+    int* mp = reinterpret_cast<int*>(Gt + (size_t)n * ST);      // largest cell per pred label
+    int* mt = mp + n;                                           // largest cell per truth label
+    int* ps = mt + n;                                           // the labels of the real hunks
+    int* ts = ps + n;
+    long long* out = counts + (size_t)b * 8;
+    const int m = nh ? __ldg(nh + b) : n;
+    bool bad = m < 0 || m > n;
+    if (!bad) {
+        for (int s = lane; s < m; s += 32) {
+            const int p = __ldg(pred + (size_t)b * n + s), t = __ldg(truth + (size_t)b * n + s);
+            bad |= (unsigned)p >= (unsigned)n || (unsigned)t >= (unsigned)n;
+            ps[s] = p; ts[s] = t;
+        }
+    }
+    if (__any_sync(0xffffffffu, bad)) {
+        if (lane < 8) out[lane] = -1;
+        return;
+    }
+    const int KW = (m + 31) >> 5;                               // bitmap words in use; lane owns hunks lane + 32 k, k < KW
+    for (int s = lane; s < m; s += 32) {
+        const int p = ps[s], t = ts[s];
+        for (int w = 0; w < KW; ++w) { Gp[p * ST + w] = 0u; Gt[t * ST + w] = 0u; }
+        mp[p] = 0; mt[t] = 0;
+    }
+    __syncwarp();
+    for (int k = 0; k < KW && lane + 32 * k < m; ++k) {
+        const int s = lane + 32 * k;
+        atomicOr(&Gp[ps[s] * ST + k], 1u << lane);
+        atomicOr(&Gt[ts[s] * ST + k], 1u << lane);
+    }
+    __syncwarp();
+    unsigned both = 0u, jp = 0u, jt = 0u, gp = 0u, gt = 0u, repP = 0u, repT = 0u;
+    const uint32_t below = (1u << lane) - 1u;
+    for (int k = 0; k < KW && lane + 32 * k < m; ++k) {
+        const int s = lane + 32 * k;
+        const int p = ps[s], t = ts[s];
+        const uint32_t* P = Gp + p * ST;
+        const uint32_t* T = Gt + t * ST;
+        int a = 0, c = 0, d = 0;
+        bool lowP = true, lowT = true;                           // s is the lowest hunk of its pred / truth group
+        for (int w = 0; w < KW; ++w) {
+            const uint32_t x = P[w], y = T[w];
+            a += __popc(x); d += __popc(y); c += __popc(x & y);
+            const uint32_t lim = w < k ? 0xffffffffu : w == k ? below : 0u;
+            lowP &= !(x & lim); lowT &= !(y & lim);
+        }
+        both += c - 1; jp += a - 1; jt += d - 1;
+        gp += lowP; gt += lowT;
+        repP |= (uint32_t)lowP << k; repT |= (uint32_t)lowT << k;
+        atomicMax(&mp[p], c);
+        atomicMax(&mt[t], c);
+    }
+    __syncwarp();
+    unsigned op = 0u, ot = 0u;
+    for (uint32_t r = repP; r; r &= r - 1u) op += mp[ps[lane + 32 * (__ffs(r) - 1)]];
+    for (uint32_t r = repT; r; r &= r - 1u) ot += mt[ts[lane + 32 * (__ffs(r) - 1)]];
+    both = __reduce_add_sync(0xffffffffu, both); jp = __reduce_add_sync(0xffffffffu, jp); jt = __reduce_add_sync(0xffffffffu, jt);
+    gp = __reduce_add_sync(0xffffffffu, gp); gt = __reduce_add_sync(0xffffffffu, gt);
+    op = __reduce_add_sync(0xffffffffu, op); ot = __reduce_add_sync(0xffffffffu, ot);
+    const unsigned v = lane == 0 ? (unsigned)m : lane == 1 ? both / 2 : lane == 2 ? jp / 2 : lane == 3 ? jt / 2
+                     : lane == 4 ? gp : lane == 5 ? gt : lane == 6 ? op : ot;
+    if (lane < 8) out[lane] = (long long)v;
+}
+
 }  // namespace hdgnn
 
 using namespace hdgnn;
@@ -274,6 +368,32 @@ extern "C" int hdgnn_hunk_groups(int B, int n, const uint32_t* bits, int32_t* gr
     if (cpc > HG_WARPS_MAX) cpc = HG_WARPS_MAX;
     if (cpc < 1) cpc = 1;
     hunk_groups_kernel<<<(B + cpc - 1) / cpc, 32 * cpc, cpc * per, (cudaStream_t)stream>>>(B, n, WP, bits, groups, ngroups);
+    return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+}
+
+extern "C" int hdgnn_partition_counts(int B, int n, const int32_t* pred, const int32_t* truth, const int32_t* nh, int64_t* counts,
+                                      void* stream) {
+    if (B < 1 || n < 2 || n > HDGNN_MAX_N || !pred || !truth || !counts) return HDGNN_E_INVALID;
+    if (((uintptr_t)pred & 3) || ((uintptr_t)truth & 3) || ((uintptr_t)nh & 3) || ((uintptr_t)counts & 7)) return HDGNN_E_INVALID;
+    int dev = 0, sms = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
+        return HDGNN_E_CUDA;
+    const size_t per = pc_smem_words(n) * 4;
+    // one commit per CTA until the batch covers the SMs, then up to PC_WARPS_MAX (as far as PC_SMEM_MAX allows)
+    int cpc = B / sms;
+    const int fit = (int)(PC_SMEM_MAX / per);
+    if (cpc > fit) cpc = fit;
+    if (cpc > PC_WARPS_MAX) cpc = PC_WARPS_MAX;
+    if (cpc < 1) cpc = 1;
+    const size_t smem = cpc * per;
+    // above the 48 KB default (one commit from n = 410 on, or several smaller ones) the launch needs the opt-in.  It is set to
+    // the largest launch there can be, so concurrent callers never lower it under each other; it is not a stream operation,
+    // so it is allowed while a graph is captured.
+    if (smem > 48 * 1024 &&
+        cudaFuncSetAttribute(partition_counts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PC_SMEM_MAX) != cudaSuccess)
+        return HDGNN_E_CUDA;
+    partition_counts_kernel<<<(B + cpc - 1) / cpc, 32 * cpc, smem, (cudaStream_t)stream>>>(B, n, pred, truth, nh,
+                                                                                           (long long*)counts);
     return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
 }
 

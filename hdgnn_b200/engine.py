@@ -491,3 +491,30 @@ def hunk_groups(bits: torch.Tensor):
     st = C.c_void_p(torch.cuda.current_stream(bits.device).cuda_stream)
     check(lib.hdgnn_hunk_groups(B, n, _p(bits), _p(groups), _p(ngroups), st))
     return groups, ngroups
+
+
+def partition_counts(pred: torch.Tensor, truth: torch.Tensor, nh: Optional[torch.Tensor] = None):
+    """Partition-agreement counters of two hunk groupings per commit (hdgnn_partition_counts), e.g. hunk_groups of the predicted
+    relations and of the labels: pred, truth (B, n) int32 CUDA tensors, any labels in [0, n) on the real hunks; nh (B,) int32
+    CUDA tensor, the number of real hunks of each commit (hunks >= nh[b] are ignored), or None: all n.  Returns counts (B, 8)
+    int64 = {real hunks, pairs joined in both, by pred, by truth, groups of pred, of truth, sum of largest overlaps of the pred
+    groups, of the truth groups}; a row of -1 marks a commit with nh outside [0, n] or a real hunk labelled outside [0, n).
+    Feed them to EvaluationFuncs.partition_metrics_from_counts."""
+    tensors = (pred, truth) if nh is None else (pred, truth, nh)
+    if not all(t.is_cuda for t in tensors):
+        raise RuntimeError("partition_counts needs CUDA tensors; there is no CPU fallback")
+    if any(t.device != pred.device for t in tensors):
+        raise ValueError("partition_counts needs all tensors on one device")
+    if any(t.dtype != torch.int32 for t in tensors):
+        raise ValueError("partition_counts needs int32 tensors")
+    if pred.dim() != 2 or truth.shape != pred.shape:
+        raise ValueError(f"partition_counts needs pred and truth of one shape (B, n), got {tuple(pred.shape)} / {tuple(truth.shape)}")
+    B, n = pred.shape
+    if nh is not None and nh.shape != (B,):
+        raise ValueError(f"partition_counts needs nh of shape ({B},), got {tuple(nh.shape)}")
+    pred, truth = pred.contiguous(), truth.contiguous()
+    nh = None if nh is None else nh.contiguous()
+    counts = torch.empty(B, 8, dtype=torch.int64, device=pred.device)
+    st = C.c_void_p(torch.cuda.current_stream(pred.device).cuda_stream)
+    check(lib.hdgnn_partition_counts(B, n, _p(pred), _p(truth), _p(nh), _p(counts), st))
+    return counts

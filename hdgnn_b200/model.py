@@ -481,10 +481,15 @@ class graph2graph(object):
         """The untangling answer over the test half, with the checkpoint, batches and entity->hunk maps of test(): the predicted
         relations of every commit as a label bitmap (hdgnn_set_predictions; the probabilities are never written) and the hunk
         groups they give (hdgnn_hunk_groups), beside the groups of the labels.  Writes C_group_t{Ne}.npy (predicted groups) and
-        C_group_y{Ne}.npy (labelled groups), (n_test, Nc) int32, each hunk labelled with the smallest hunk index of its group, and
-        logs the number of commits whose predicted partition of all Nc hunks equals the labelled one.  Padding hunks are not
-        masked: the library cannot tell them from real hunks that relate to nothing."""
-        from .engine import bit_words, hunk_groups
+        C_group_y{Ne}.npy (labelled groups), (n_test, Nc) int32, each hunk labelled with the smallest hunk index of its group, over
+        all Nc hunks, and logs the number of commits whose predicted partition of all Nc hunks equals the labelled one
+        (exact_partitions).  The group-level scores (hdgnn_partition_counts -> EvaluationFuncs.partition_metrics_from_counts:
+        pair precision / recall / F1, Rand and adjusted Rand index, purity, groups per commit; out["partition_counts"] and
+        out["partition"], one log line each before exact_partitions) count only each commit's real hunks 0 .. nh-1, the hunk
+        count the loader read from the commit's hunk map (test.nh); padding hunks, singletons on both sides, would inflate every
+        agreement measure.  A loader without hunk counts (test.nh None) scores all Nc hunks."""
+        from .EvaluationFuncs import partition_metrics_from_counts
+        from .engine import bit_words, hunk_groups, partition_counts
         repo = getattr(args, "Repo", self.Repo)
         train, test = data if data is not None else self._load(root)
         self.initialize()
@@ -500,6 +505,9 @@ class graph2graph(object):
         pred = torch.zeros(max(n, 1), self.Nc, bit_words(self.Nc), dtype=torch.int32, device=dev)
         groups = torch.zeros(max(n, 1), self.Nc, dtype=torch.int32, device=dev)
         label_groups = torch.zeros_like(groups)
+        pcounts = torch.zeros(max(n, 1), 8, dtype=torch.int64, device=dev)
+        # the hunk counts of the commits whose labels Y are scored (never those of the Q2-substituted maps)
+        nh = None if test.nh is None or not nb else torch.as_tensor(np.ascontiguousarray(test.nh[:n], dtype=np.int32)).to(dev)
         start_time = time.time()
         alive = []       # the library DMAs from these pinned buffers asynchronously: keep them until the final synchronize
         try:
@@ -514,18 +522,23 @@ class graph2graph(object):
                 self.engine.infer_host(*hb.tensors(), self.params, None, None)
                 groups[rows] = hunk_groups(pred[rows])[0]
                 label_groups[rows] = hunk_groups(hb.Yw.to(dev, non_blocking=True))[0]
+                pcounts[rows] = partition_counts(groups[rows], label_groups[rows], None if nh is None else nh[rows])
         finally:
             self.engine.set_predictions(None)
         exact = int((groups[:n] == label_groups[:n]).all(1).sum()) if nb else 0      # synchronises
         alive.clear()
         end_time = time.time()
         out = dict(pred_bits=pred[:n].cpu().numpy(), groups=groups[:n].cpu().numpy(),
-                   label_groups=label_groups[:n].cpu().numpy(), exact_partitions=exact)
+                   label_groups=label_groups[:n].cpu().numpy(), exact_partitions=exact,
+                   partition_counts=pcounts[:n].cpu().numpy())
+        out["partition"] = partition_metrics_from_counts(out["partition_counts"])
         if self.rank == 0:
             step_dir = os.path.join(root, 'outputSelf/' + repo + '/model_%d/' % self.variant + str(self.Step) + '/')
             os.makedirs(step_dir, exist_ok=True)
             np.save(step_dir + 'C_group_t' + str(self.Ne) + '.npy', out["groups"])
             np.save(step_dir + 'C_group_y' + str(self.Ne) + '.npy', out["label_groups"])
+            for k, v in out["partition"].items():
+                log('partition_' + k + ': ' + str(v))
             log('exact_partitions: ' + str(exact) + ' / ' + str(n))
             log('test time:' + str(end_time - start_time))
         return out

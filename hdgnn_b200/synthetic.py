@@ -10,6 +10,7 @@ and a planted, learnable hunk adjacency.
 from __future__ import annotations
 
 from dataclasses import dataclass
+from typing import Optional
 
 import numpy as np
 
@@ -23,12 +24,14 @@ class CommitBatch:
     hmap (B,Ne)    int32  hunk id of entity line i; -1 = 'null' or id >= Nc (utils2.py:129-136)
     L    (B,)      int32  number of index lines read, <= Ne              (utils2.py:121)
     Y    (B,Nc,Nc) uint8  off-diagonal hunk adjacency = label            (utils2.py:47)
+    nh   (B,)      int32  number of real hunks, rows 0 .. nh-1 of Y; None = not known (every Nc hunk counts)
     """
     adj: np.ndarray
     x: np.ndarray
     hmap: np.ndarray
     L: np.ndarray
     Y: np.ndarray
+    nh: Optional[np.ndarray] = None
 
     @property
     def B(self):
@@ -43,7 +46,8 @@ class CommitBatch:
         return self.Y.shape[1]
 
     def slice(self, lo, hi):
-        return CommitBatch(self.adj[lo:hi], self.x[lo:hi], self.hmap[lo:hi], self.L[lo:hi], self.Y[lo:hi])
+        return CommitBatch(self.adj[lo:hi], self.x[lo:hi], self.hmap[lo:hi], self.L[lo:hi], self.Y[lo:hi],
+                           None if self.nh is None else self.nh[lo:hi])
 
 
 def make_commits(B, Ne, Nc, seed=20260, p_edge=0.05, p_null=0.15, p_short=0.2, p_noise=0.02,

@@ -85,7 +85,10 @@ def _index_maps(index_lines, hunk_maps, N, Ne, Nc):
 def compact_from_raw(x_raw, y_raw, index_lines, hunk_maps, Ne, Nc, device=None) -> CommitBatch:
     """x_raw (N,Ne,Ne), y_raw (N,Nc,Nc): arrays as stored; index_lines: per commit the list of lines of
     its IndexPath file; hunk_maps: per commit dict key -> number.  device: CUDA device -> the array half runs on
-    the GPU (what graph2graph uses); None -> NumPy (CPU tests, the checker)."""
+    the GPU (what graph2graph uses); None -> NumPy (CPU tests, the checker).
+    The number of real hunks of commit b is taken as nh[b] = min(Nc, len(hunk_maps[b])).  This assumes that the hunk numbers
+    0 .. len-1 of a commit's map occupy rows 0 .. len-1 of its CHunkAdjs grid and that the rest is padding, which is what
+    write_dataset writes; it has not been verified against the reference's data blob, which is missing."""
     x_raw = np.asarray(x_raw)
     y_raw = np.asarray(y_raw)
     N = x_raw.shape[0]
@@ -93,14 +96,17 @@ def compact_from_raw(x_raw, y_raw, index_lines, hunk_maps, Ne, Nc, device=None) 
         raise ValueError(f"adjacency shapes {x_raw.shape} / {y_raw.shape} do not match Ne={Ne}, Nc={Nc}")
     adj, x, Y = _grids_host(x_raw, y_raw, Ne, Nc) if device is None else _grids_device(x_raw, y_raw, Ne, Nc, device)
     hmap, L = _index_maps(index_lines, hunk_maps, N, Ne, Nc)
-    return CommitBatch(adj, x, hmap, L, Y)
+    nh = np.array([min(Nc, len(m)) for m in hunk_maps], dtype=np.int32)
+    return CommitBatch(adj, x, hmap, L, Y, nh)
 
 
 def read_compact(repo: str, step: int, Ne: int, Nc: int, root: str = ".", cache: bool = True, device=None) -> CommitBatch:
+    """compact_from_raw of the files of utils2.py:22-25, through the cache Intermediate_products/{repo}/compact_*.npz.  A cache
+    written before the hunk counts were stored loads with nh = None (every Nc hunk counts as real)."""
     cp = _cache_path(root, repo, step, Ne, Nc)
     if cache and os.path.exists(cp):
         z = np.load(cp)
-        return CommitBatch(z["adj"], z["x"], z["hmap"], z["L"], z["Y"])
+        return CommitBatch(z["adj"], z["x"], z["hmap"], z["L"], z["Y"], z["nh"] if "nh" in z.files else None)
     import joblib
     pa, py, pi, ph = _paths(root, repo, step)
     for p in (pa, py, pi, ph):
@@ -122,7 +128,7 @@ def read_compact(repo: str, step: int, Ne: int, Nc: int, root: str = ".", cache:
         # one writer (rank 0), temporary file + atomic rename: a rank arriving later never sees a half-written zip
         os.makedirs(os.path.dirname(cp), exist_ok=True)          # the reference needs this dir to pre-exist (Q14)
         tmp = f"{cp}.{os.getpid()}.tmp.npz"
-        np.savez_compressed(tmp, adj=cb.adj, x=cb.x, hmap=cb.hmap, L=cb.L, Y=cb.Y)
+        np.savez_compressed(tmp, adj=cb.adj, x=cb.x, hmap=cb.hmap, L=cb.L, Y=cb.Y, nh=cb.nh)
         os.replace(tmp, cp)
     return cb
 

@@ -274,6 +274,18 @@ int hdgnn_pack_label_bits(int N, int n, const uint8_t* grid, int pitch, uint32_t
  * int32 or NULL receives the number of components.  2 <= n <= HDGNN_MAX_N.  Integer-exact, deterministic.  Stateless. */
 int hdgnn_hunk_groups(int B, int n, const uint32_t* bits, int32_t* groups, int32_t* ngroups, void* stream);
 
+/* Partition agreement of two hunk groupings per commit (e.g. hdgnn_hunk_groups of the predicted relations and of the labels),
+ * over the REAL hunks 0 .. m-1 of each commit, m = nh[b] (nh (B) int32, or NULL: m = n).  pred, truth (B, n) int32: any
+ * labelling with values in [0, n) on the real hunks (hunks >= m are ignored, whatever they hold).  counts (B, 8) int64 is
+ * WRITTEN (not added), row b =
+ *   {m, pairs joined in both, pairs joined by pred, pairs joined by truth, groups of pred, groups of truth,
+ *    sum over pred groups of the largest overlap with a truth group, sum over truth groups of the largest overlap with a pred group}
+ * (pairs = unordered pairs {s,t}, s < t < m).  A commit with nh[b] outside [0, n] or a real hunk labelled outside [0, n) gets
+ * the row all -1.  pred, truth, nh 4-byte and counts 8-byte aligned.  2 <= n <= HDGNN_MAX_N.  Integer-exact, deterministic,
+ * stateless, asynchronous on `stream`. */
+int hdgnn_partition_counts(int B, int n, const int32_t* pred, const int32_t* truth, const int32_t* nh,
+                           int64_t* counts, void* stream);
+
 /* Evaluation counters on the device, replaces the loops of EvaluationFuncs.py:27-37 (top_ACC), :92-117 (prec / recall /
  * f1) and :119-153 (AUC) over the probs the relation head wrote.  probs (B,2,Ncr) f32, Y (B,Nc,y_pitch) u8.
  * counts (B,8) int64: {arg-max hits, quirk tp, fp, fn (ceil of channel 0, as the reference scores), conventional tp, fp,

@@ -6,7 +6,8 @@ given on the command line overrides ALL presets, as in the reference.  Extra fla
 (1-4 = model_1..model_4, default 2 = the model main.py imports), --root (directory holding
 Adjset/ and dataset/), --seed, --no_q2 (feed each batch its own entity->hunk maps instead of the
 reference's first-Mini_batch slice, model_2.py:376-381).  Extra value --Type untangle: the hunk groups the trained model
-predicts for every test commit (graph2graph.untangle).
+predicts for every test commit (graph2graph.untangle), scored against the labelled groups over each commit's real hunks
+(pair precision / recall / F1, Rand and adjusted Rand index, purity).
 Multi-GPU: launch with `python -m torch.distributed.run --nproc-per-node N main.py ...`.
 """
 import argparse

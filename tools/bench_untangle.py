@@ -3,14 +3,18 @@
       bitmap (hdgnn_set_predictions, probs NULL);
   (b) host-fed inference end to end: probabilities copied to pinned host memory against predictions + hunk groups copied to
       pinned host memory (hdgnn_infer_host with probs NULL, then hdgnn_hunk_groups);
-  (c) the hunk_groups kernel alone, on predicted and on label bitmaps.
+  (c) the hunk_groups kernel alone, on predicted and on label bitmaps;
+  (d) the partition_counts kernel alone (the untangling scores) on the hunk groups of two label sets, every hunk real (the
+      costliest case), at B = 100 and Nc in {74, 256, 512} and at B = 4096, Nc = 74, alternating with hunk_groups on the
+      same commits; the per-call times of these eager blocks include the Python wrapper and the launch, so the kernel
+      times are read from torch.profiler as well, in a pass of their own.
 Device inputs rotate through copies that together exceed the 126 MB L2; every arm is timed in blocks that alternate with the
 other arm's, and the median block is reported.  The card's name and power limit are read in the same run.
-Usage: python tools/bench_untangle.py [--out result.json]"""
+Usage: python tools/bench_untangle.py [--sections abcd] [--out result.json]"""
 import argparse, json, os, statistics, subprocess, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
-from hdgnn_b200.engine import Engine, DeviceBatch, F_LABEL_BITS, bit_words, hunk_groups
+from hdgnn_b200.engine import Engine, DeviceBatch, F_LABEL_BITS, bit_words, hunk_groups, pack_label_bits, partition_counts
 from hdgnn_b200.model import HostBatch
 from hdgnn_b200.synthetic import make_commits
 
@@ -54,9 +58,10 @@ def timed(arms, calls):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=None)
+    ap.add_argument("--sections", default="abcd", help="which of the sections (a)-(d) to run")
     args = ap.parse_args()
     out = {"card": card(), "B": B, "Ne": Ne, "variant": 2, "reps": REPS, "what": __doc__.split("Usage")[0].strip(), "rows": []}
-    for Nc in (74, 256, 512):
+    for Nc in ((74, 256, 512) if set("abc") & set(args.sections) else ()):
         eng = Engine(Ne, Nc, variant=2, max_batch=B, flags=F_LABEL_BITS)
         WPc = bit_words(Nc)
         cbs = [make_commits(B, Ne, Nc, seed=4040 + i) for i in range(4)]
@@ -140,10 +145,50 @@ def main():
         del pool, pred_pool, lab_pool
         eng.close()
         torch.cuda.empty_cache()
+    if "d" in args.sections:
+        out["d_partition_counts"] = [scores(Bd, Nc) for Bd, Nc in ((B, 74), (B, 256), (B, 512), (4096, 74))]
     out["card_after"] = card()
     if args.out:
         os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
         json.dump(out, open(args.out, "w"), indent=1)
+
+
+def scores(Bd, Nc):
+    """(d): partition_counts of two groupings of Bd commits (the hunk groups of two synthetic label sets, nh = Nc), in blocks
+    alternating with hunk_groups of the first label set."""
+    lab = [torch.as_tensor(pack_label_bits(make_commits(Bd, 8, Nc, seed=5050 + i, p_noise=1.0 / Nc).Y).view(np.int32)).cuda()
+           for i in range(2)]
+    groups = [hunk_groups(x)[0] for x in lab]
+    nh = torch.full((Bd,), Nc, dtype=torch.int32, device="cuda")
+    pairs = rotate([torch.stack(groups)], 2 * Bd * Nc * 4)
+    bits = rotate([lab[0]], lab[0].numel() * 4)
+    ms, blocks = timed({"partition_counts": lambda k: partition_counts(pairs[k % len(pairs)][0], pairs[k % len(pairs)][1], nh),
+                        "hunk_groups": lambda k: hunk_groups(bits[k % len(bits)])}, 50)
+    kern = kernel_us({"partition_counts": lambda k: partition_counts(pairs[k % len(pairs)][0], pairs[k % len(pairs)][1], nh),
+                      "hunk_groups": lambda k: hunk_groups(bits[k % len(bits)])}, 200)
+    c = partition_counts(groups[0], groups[1], nh).cpu().numpy()
+    row = {"B": Bd, "Nc": Nc, "us_per_batch_partition_counts": ms["partition_counts"] * 1e3,
+           "us_per_batch_hunk_groups": ms["hunk_groups"] * 1e3, "commits_per_s_partition_counts": Bd / ms["partition_counts"] * 1e3,
+           "kernel_us_partition_counts": kern.get("partition_counts"), "kernel_us_hunk_groups": kern.get("hunk_groups"),
+           "mean_groups": [float(c[:, 4].mean()), float(c[:, 5].mean())], "pool_batches": len(pairs), "blocks_ms": blocks}
+    print(json.dumps(row, default=str))
+    return row
+
+
+def kernel_us(arms, calls):
+    """{name: mean device time in µs of the kernel `{name}_kernel`} over `calls` calls of each arm, from torch.profiler."""
+    from torch.profiler import profile, ProfilerActivity
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for fn in arms.values():
+            for k in range(calls):
+                fn(k)
+        torch.cuda.synchronize()
+    got = {}
+    for e in prof.key_averages():
+        for name in arms:
+            if f"{name}_kernel" in e.key and e.count:
+                got[name] = e.device_time_total / e.count
+    return got
 
 
 def timed_once(fn, r, calls):
