@@ -11,8 +11,11 @@
 //  * partition_counts_kernel  -- how well two such groupings agree, per commit and over its real hunks only: pair counts,
 //    group counts and largest overlaps, from which EvaluationFuncs.partition_metrics_from_counts derives pair precision /
 //    recall / F1, the (adjusted) Rand index and purity.
+//  * hunk_clusters_kernel     -- hunk groups formed from the relation probabilities instead of the arg-max bitmap: average
+//    linkage over each commit's real hunks, merging two groups only while their mean relation probability clears a threshold.
 //
-// Everything here is integer counting => bit-exact and order independent (integer atomics).
+// Everything here except hunk_clusters_kernel is integer counting => bit-exact and order independent (integer atomics).  The
+// clustering is fp32, but its merge sequence fixes every rounding, so it is deterministic and reproducible on the host.
 #include "../../include/hdgnn.h"
 #include "bits.cuh"
 #include "common.cuh"
@@ -312,6 +315,205 @@ __global__ void __launch_bounds__(32 * PC_WARPS_MAX) partition_counts_kernel(int
     if (lane < 8) out[lane] = (long long)v;
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Hunk clusters: average linkage (UPGMA) of the relation probabilities per commit, over the real hunks s < m = nh[b].  One CTA
+// per commit (the workspace form: persistent CTAs, one slice of `work` each, walking the commits).
+//   w(s,t) = fmaxf(p1(s,t), p1(t,s)); S(A,C) = sum of w over A x C, kept for every pair of live clusters (the full symmetric
+//   m x m table, row r = the cluster whose representative -- smallest hunk -- is r) and updated by Lance-Williams,
+//   S(A u B, C) = S(A,C) + S(B,C): one fp32 add per entry per merge, so the merge sequence fixes every rounding;
+//   mean(A,C) = __fdiv_rn(S(A,C), (float)(|A| |C|)) (|A| |C| <= 256^2: exact in fp32).
+//   Beside S, the table O holds the ordered bits of every live pair's mean (0: NaN, dead or diagonal), so a rescan of a row is
+//   an integer max over it: no division, no sizes.
+// A pair is ranked by the 64-bit key  [ordered bits of its mean | ~(lo << 16 | hi)]  (lo < hi its representatives): the larger
+// key has the larger mean, and among equal means the smaller (lo, hi).  -0 is keyed as +0, NaN gets key 0 ("no pair"; every
+// real pair's key is > 0), so a NaN mean never merges.  Row r keeps key[r] = the largest key over the live partners of r.
+// Argmax over the row bests = argmax over all pairs: every pair (r, t) is a candidate of row r, so max_r key[r] >= its key,
+// and every key[r] is the key of a live pair; the keys are distinct (they encode the pair), so the maximum is one pair.
+// One merge of the best pair (a, c), a < c, keeping a:
+//   A. block arg-max over key[]; stop when it is 0 (one cluster left, or only NaN) or its mean is not > threshold;
+//   B. thread per row x: S(a,x) = S(x,a) = S(a,x) + S(c,x), O(a,x) = O(x,a) = the new mean's bits, O(x,c) = 0, and the new
+//      key of (x, a); a row whose best partner was a or c goes on the rescan list, every other row takes max(key[x], key(x, a))
+//      -- exact, since the pairs that left (x,a), (x,c) were not its best and the one that came is compared; row a's best is
+//      the block max of the new keys (x, a);
+//   C. warp per listed row: full rescan of its row of O.
+// Barriers: A, B and C (C only when the list is not empty).  The sizes of a and c change only at the start of the next A (each
+// row's owner thread writes its own row), so every thread reads the old sizes in B.
+// The tables live in shared memory when they fit beside the row arrays (n <= 169), else in a slice of `work`; the same code
+// reaches both through generic pointers.
+constexpr int HC_T_MAX = 512;
+constexpr int HC_WARPS = HC_T_MAX / 32;
+constexpr int HC_WORK_SLICES = 296;                        // CTAs of the workspace form: two per SM of a B200
+constexpr size_t HC_SMEM_MAX = 227 * 1024;
+
+__host__ __device__ inline int hc_stride(int n) { return n | 1; }                      // odd: column writes spread over banks
+__host__ __device__ inline size_t hc_table_words(int n) { return (size_t)n * hc_stride(n); }
+// key u64[n], two u64 slot arrays, size / lab / list int32[n], two list counters and two spare words; then S and O
+__host__ __device__ inline size_t hc_rows_bytes(int n) { return (size_t)n * 8 + 2 * HC_WARPS * 8 + (size_t)n * 12 + 16; }
+inline bool hc_table_in_smem(int n) { return hc_rows_bytes(n) + 2 * hc_table_words(n) * 4 <= HC_SMEM_MAX; }
+inline int hc_threads(int n) { return n <= 128 ? 128 : n <= 256 ? 256 : HC_T_MAX; }
+
+// ordered bits of a mean: larger mean <=> larger bits, -0 as +0, NaN -> 0 (every other value gives >= 0x007fffff)
+__device__ __forceinline__ uint32_t hc_ord(float v) {
+    uint32_t u = __float_as_uint(v);
+    if ((u & 0x7fffffffu) > 0x7f800000u) return 0u;       // NaN
+    if ((u << 1) == 0u) u = 0u;                             // -0 -> +0
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ unsigned long long hc_key(uint32_t o, int s, int t) {
+    if (!o) return 0ull;
+    const uint32_t lo = (uint32_t)min(s, t), hi = (uint32_t)max(s, t);
+    return ((unsigned long long)o << 32) | (uint32_t)~((lo << 16) | hi);
+}
+__device__ __forceinline__ float hc_key_mean(unsigned long long k) {
+    const uint32_t o = (uint32_t)(k >> 32);
+    return __uint_as_float((o & 0x80000000u) ? (o ^ 0x80000000u) : ~o);
+}
+__device__ __forceinline__ int hc_key_lo(unsigned long long k) { return (int)((~(uint32_t)k) >> 16); }
+__device__ __forceinline__ int hc_key_hi(unsigned long long k) { return (int)((~(uint32_t)k) & 0xffffu); }
+__device__ __forceinline__ unsigned long long hc_max(unsigned long long x, unsigned long long y) { return x > y ? x : y; }
+__device__ __forceinline__ unsigned long long hc_warp_max(unsigned long long k) {
+    const uint32_t h = __reduce_max_sync(0xffffffffu, (uint32_t)(k >> 32));
+    const uint32_t l = __reduce_max_sync(0xffffffffu, (uint32_t)(k >> 32) == h ? (uint32_t)k : 0u);
+    return ((unsigned long long)h << 32) | l;
+}
+
+// The best key of row x over its live partners (one warp): the largest bits of its row of O, the smallest column among equals.
+__device__ __forceinline__ unsigned long long hc_rescan(const uint32_t* O, int ST, int m, int x, int lane) {
+    const uint32_t* Ox = O + (size_t)x * ST;
+    uint32_t bo = 0u;
+    int bt = 0xffff;
+    for (int t = lane; t < m; t += 32) {
+        const uint32_t o = Ox[t];
+        if (o > bo) { bo = o; bt = t; }                     // t ascends: the first of equal bits is the smallest column
+    }
+    const uint32_t h = __reduce_max_sync(0xffffffffu, bo);
+    const int t = (int)__reduce_min_sync(0xffffffffu, bo == h ? (uint32_t)bt : 0xffffu);
+    return hc_key(h, x, t);
+}
+
+__global__ void __launch_bounds__(HC_T_MAX) hunk_clusters_kernel(int B, int n, const float* __restrict__ probs,
+                                                                 const int32_t* __restrict__ nh, float threshold,
+                                                                 int32_t* __restrict__ groups, int32_t* __restrict__ ngroups,
+                                                                 float* work) {
+    extern __shared__ __align__(16) unsigned char hc_smem[];
+    const int T = blockDim.x, NW = T >> 5, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    unsigned long long* key = reinterpret_cast<unsigned long long*>(hc_smem);
+    unsigned long long* slot = key + n;                    // per-warp maxima of phase A
+    unsigned long long* slotA = slot + HC_WARPS;           // per-warp maxima of the new keys (x, a) of phase B
+    int* size = reinterpret_cast<int*>(slotA + HC_WARPS);  // cluster size of a representative, 0 = not a live cluster
+    int* lab = size + n;                                   // representative of every hunk's cluster
+    int* list = lab + n;                                   // rows to rescan
+    int* cnt = list + n;                                   // list lengths of even / odd merges
+    const int ST = hc_stride(n);
+    const size_t TW = hc_table_words(n);
+    float* S = work ? work + (size_t)blockIdx.x * 2 * TW : reinterpret_cast<float*>(cnt + 4);
+    uint32_t* O = reinterpret_cast<uint32_t*>(S + TW);
+    const size_t Ncr = (size_t)n * (n - 1);
+    for (int b = blockIdx.x; b < B; b += gridDim.x) {
+        const int m = nh ? __ldg(nh + b) : n;
+        int32_t* g = groups + (size_t)b * n;
+        if (m < 0 || m > n) {
+            for (int s = tid; s < n; s += T) g[s] = -1;
+            if (tid == 0 && ngroups) ngroups[b] = -1;
+            continue;
+        }
+        // channel 1 of the real block, row s of p1 (pairs s(n-1) .. s(n-1)+n-2) read along t; the padding pairs are never read
+        const float* p1 = probs + (size_t)b * 2 * Ncr + Ncr;
+        for (int s = warp; s < m; s += NW) {
+            const float* row = p1 + (size_t)s * (n - 1);
+            for (int t = lane; t < m; t += 32)
+                if (t != s) S[(size_t)s * ST + t] = __ldg(row + t - (t > s));
+        }
+        for (int s = tid; s < n; s += T) {
+            size[s] = s < m ? 1 : 0;
+            lab[s] = s;
+            if (s < m) O[(size_t)s * ST + s] = 0u;
+        }
+        if (tid < 2) cnt[tid] = 0;
+        __syncthreads();
+        for (int s = warp; s < m; s += NW)                  // w = fmaxf of both directions, each unordered pair by one lane
+            for (int t = s + 1 + lane; t < m; t += 32) {
+                const float v = fmaxf(S[(size_t)s * ST + t], S[(size_t)t * ST + s]);
+                const uint32_t o = hc_ord(v);                   // mean of two singletons = w
+                S[(size_t)s * ST + t] = v;
+                S[(size_t)t * ST + s] = v;
+                O[(size_t)s * ST + t] = o;
+                O[(size_t)t * ST + s] = o;
+            }
+        __syncthreads();
+        for (int x = warp; x < m; x += NW) {
+            const unsigned long long k = hc_rescan(O, ST, m, x, lane);
+            if (lane == 0) key[x] = k;
+        }
+        __syncthreads();
+        int merges = 0, pa = -1, pc = -1, psz = 0;         // the last merge, whose sizes the owner threads write in A
+        for (;;) {
+            // A: block arg-max over the row bests (thread tid owns rows tid + k T throughout)
+            if (pa >= 0) {
+                if (pa % T == tid) size[pa] = psz;
+                if (pc % T == tid) size[pc] = 0;
+            }
+            unsigned long long kb = 0ull;
+            for (int x = tid; x < m; x += T) kb = hc_max(kb, key[x]);
+            kb = hc_warp_max(kb);
+            if (lane == 0) slot[warp] = kb;
+            __syncthreads();
+            kb = 0ull;
+            for (int w = 0; w < NW; ++w) kb = hc_max(kb, slot[w]);
+            if (kb == 0ull || !(hc_key_mean(kb) > threshold)) break;
+            // B: Lance-Williams update of row / column a, compare-and-update or rescan listing of every other row
+            const int a = hc_key_lo(kb), c = hc_key_hi(kb);
+            const int sn = size[a] + size[c];
+            int* L = cnt + (merges & 1);
+            if (tid == 0) cnt[(merges & 1) ^ 1] = 0;       // the other counter was last read before this merge's A barrier
+            unsigned long long kA = 0ull;
+            for (int x = tid; x < m; x += T) {
+                if (lab[x] == c) lab[x] = a;
+                if (x == c) key[x] = 0ull;
+                if (x == a) O[(size_t)a * ST + c] = 0u;
+                const int sx = size[x];
+                if (x == a || x == c || sx == 0) continue;
+                const float v = S[(size_t)a * ST + x] + S[(size_t)c * ST + x];
+                const uint32_t o = hc_ord(__fdiv_rn(v, (float)(sx * sn)));
+                S[(size_t)a * ST + x] = v;
+                S[(size_t)x * ST + a] = v;
+                O[(size_t)a * ST + x] = o;
+                O[(size_t)x * ST + a] = o;
+                O[(size_t)x * ST + c] = 0u;
+                const unsigned long long k = hc_key(o, x, a);
+                kA = hc_max(kA, k);
+                const unsigned long long kx = key[x];
+                const int px = kx ? (hc_key_lo(kx) == x ? hc_key_hi(kx) : hc_key_lo(kx)) : -1;
+                if (px == a || px == c) list[atomicAdd(L, 1)] = x;
+                else if (k > kx) key[x] = k;
+            }
+            kA = hc_warp_max(kA);
+            if (lane == 0) slotA[warp] = kA;
+            __syncthreads();
+            // C: row a from the new keys, full rescans of the listed rows
+            if (a % T == tid) {
+                kA = 0ull;
+                for (int w = 0; w < NW; ++w) kA = hc_max(kA, slotA[w]);
+                key[a] = kA;
+            }
+            const int nl = *L;
+            if (nl) {
+                for (int i = warp; i < nl; i += NW) {
+                    const int x = list[i];
+                    const unsigned long long k = hc_rescan(O, ST, m, x, lane);
+                    if (lane == 0) key[x] = k;
+                }
+                __syncthreads();
+            }
+            pa = a; pc = c; psz = sn;
+            ++merges;
+        }
+        for (int s = tid; s < n; s += T) g[s] = s < m ? lab[s] : s;
+        if (tid == 0 && ngroups) ngroups[b] = n - merges;
+        __syncthreads();                                    // before the next commit reuses the arrays and the table
+    }
+}
+
 }  // namespace hdgnn
 
 using namespace hdgnn;
@@ -394,6 +596,31 @@ extern "C" int hdgnn_partition_counts(int B, int n, const int32_t* pred, const i
         return HDGNN_E_CUDA;
     partition_counts_kernel<<<(B + cpc - 1) / cpc, 32 * cpc, smem, (cudaStream_t)stream>>>(B, n, pred, truth, nh,
                                                                                            (long long*)counts);
+    return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+}
+
+extern "C" size_t hdgnn_hunk_clusters_work(int B, int n) {
+    if (B < 1 || n < 2 || n > HDGNN_MAX_N || hc_table_in_smem(n)) return 0;
+    return (size_t)(B < HC_WORK_SLICES ? B : HC_WORK_SLICES) * 2 * hc_table_words(n) * sizeof(float);
+}
+
+extern "C" int hdgnn_hunk_clusters(int B, int n, const float* probs, const int32_t* nh, float threshold, int32_t* groups,
+                                   int32_t* ngroups, void* work, void* stream) {
+    if (B < 1 || n < 2 || n > HDGNN_MAX_N || !probs || !groups || threshold != threshold) return HDGNN_E_INVALID;
+    if (((uintptr_t)probs & 3) || ((uintptr_t)nh & 3) || ((uintptr_t)groups & 3) || ((uintptr_t)ngroups & 3) || ((uintptr_t)work & 3))
+        return HDGNN_E_INVALID;
+    const bool in_smem = hc_table_in_smem(n);
+    if (!in_smem && !work) return HDGNN_E_INVALID;
+    const size_t smem = hc_rows_bytes(n) + (in_smem ? 2 * hc_table_words(n) * 4 : 0);
+    // the opt-in is set to the largest launch there can be, so concurrent callers never lower it under each other; it is not a
+    // stream operation, so it is allowed while a graph is captured
+    if (smem > 48 * 1024 &&
+        cudaFuncSetAttribute(hunk_clusters_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)HC_SMEM_MAX) != cudaSuccess)
+        return HDGNN_E_CUDA;
+    // one CTA per commit; the workspace form walks the commits with one slice (S and O) per CTA
+    const int grid = in_smem ? B : (B < HC_WORK_SLICES ? B : HC_WORK_SLICES);
+    hunk_clusters_kernel<<<grid, hc_threads(n), smem, (cudaStream_t)stream>>>(B, n, probs, nh, threshold, groups, ngroups,
+                                                                             in_smem ? nullptr : (float*)work);
     return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
 }
 

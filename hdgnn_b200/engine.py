@@ -518,3 +518,35 @@ def partition_counts(pred: torch.Tensor, truth: torch.Tensor, nh: Optional[torch
     st = C.c_void_p(torch.cuda.current_stream(pred.device).cuda_stream)
     check(lib.hdgnn_partition_counts(B, n, _p(pred), _p(truth), _p(nh), _p(counts), st))
     return counts
+
+
+def hunk_clusters(probs: torch.Tensor, nh: Optional[torch.Tensor] = None, threshold: float = 0.5):
+    """Hunk groups by average-linkage clustering of the relation probabilities (hdgnn_hunk_clusters): probs (B, 2, n(n-1))
+    float32 CUDA tensor as the relation head writes it (only channel 1 is read); nh (B,) int32 CUDA tensor, the number of real
+    hunks of each commit, or None: all n.  Two groups merge while the mean of max(p1(s,t), p1(t,s)) over their hunk pairs is
+    > threshold, the closest first.  Returns (groups (B, n) int32: the smallest hunk index of each real hunk's group, s for a
+    hunk s >= nh[b]; ngroups (B,) int32), the labelling of hunk_groups; a commit with nh outside [0, n] gets -1 throughout."""
+    tensors = (probs,) if nh is None else (probs, nh)
+    if not all(t.is_cuda for t in tensors):
+        raise RuntimeError("hunk_clusters needs CUDA tensors; there is no CPU fallback")
+    if any(t.device != probs.device for t in tensors):
+        raise ValueError("hunk_clusters needs all tensors on one device")
+    if probs.dtype != torch.float32 or (nh is not None and nh.dtype != torch.int32):
+        raise ValueError("hunk_clusters needs float32 probs and int32 nh")
+    if probs.dim() != 3 or probs.shape[1] != 2:
+        raise ValueError(f"hunk_clusters needs probs of shape (B, 2, n(n-1)), got {tuple(probs.shape)}")
+    B, _, ncr = probs.shape
+    n = (1 + int(round((1 + 4 * ncr) ** 0.5))) // 2
+    if n < 2 or n * (n - 1) != ncr:
+        raise ValueError(f"hunk_clusters needs n(n-1) pairs per channel, got {ncr}")
+    if nh is not None and nh.shape != (B,):
+        raise ValueError(f"hunk_clusters needs nh of shape ({B},), got {tuple(nh.shape)}")
+    probs = probs.contiguous()
+    nh = None if nh is None else nh.contiguous()
+    groups = torch.empty(B, n, dtype=torch.int32, device=probs.device)
+    ngroups = torch.empty(B, dtype=torch.int32, device=probs.device)
+    nwork = lib.hdgnn_hunk_clusters_work(B, n)
+    work = torch.empty(nwork, dtype=torch.uint8, device=probs.device) if nwork else None
+    st = C.c_void_p(torch.cuda.current_stream(probs.device).cuda_stream)
+    check(lib.hdgnn_hunk_clusters(B, n, _p(probs), _p(nh), float(threshold), _p(groups), _p(ngroups), _p(work), st))
+    return groups, ngroups

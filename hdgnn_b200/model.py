@@ -477,19 +477,26 @@ class graph2graph(object):
             log('test time:' + str(end_time - start_time))
         return out, C_edge_t1
 
-    def untangle(self, args=None, data=None, root=".", quirk_q2=True, log=print):
+    def untangle(self, args=None, data=None, root=".", quirk_q2=True, log=print, grouping="components", threshold=0.5):
         """The untangling answer over the test half, with the checkpoint, batches and entity->hunk maps of test(): the predicted
-        relations of every commit as a label bitmap (hdgnn_set_predictions; the probabilities are never written) and the hunk
-        groups they give (hdgnn_hunk_groups), beside the groups of the labels.  Writes C_group_t{Ne}.npy (predicted groups) and
+        relations of every commit as a label bitmap (hdgnn_set_predictions; by default no probabilities are written) and the
+        hunk groups they give (hdgnn_hunk_groups), beside the groups of the labels.  Writes C_group_t{Ne}.npy (predicted groups) and
         C_group_y{Ne}.npy (labelled groups), (n_test, Nc) int32, each hunk labelled with the smallest hunk index of its group, over
         all Nc hunks, and logs the number of commits whose predicted partition of all Nc hunks equals the labelled one
         (exact_partitions).  The group-level scores (hdgnn_partition_counts -> EvaluationFuncs.partition_metrics_from_counts:
         pair precision / recall / F1, Rand and adjusted Rand index, purity, groups per commit; out["partition_counts"] and
         out["partition"], one log line each before exact_partitions) count only each commit's real hunks 0 .. nh-1, the hunk
         count the loader read from the commit's hunk map (test.nh); padding hunks, singletons on both sides, would inflate every
-        agreement measure.  A loader without hunk counts (test.nh None) scores all Nc hunks."""
+        agreement measure.  A loader without hunk counts (test.nh None) scores all Nc hunks.
+        grouping="components" forms the predicted groups as above.  grouping="average" forms them by average-linkage clustering
+        of the relation probabilities (hdgnn_hunk_clusters) over the same real hunks: two groups merge only while the mean of
+        max(p1(s,t), p1(t,s)) over their hunk pairs is > threshold, so one confident cross pair cannot join two groups and a few
+        missing pairs cannot split one.  Each batch's probabilities go to a device buffer (never to the host); pred_bits keep
+        their meaning, and one log line names the grouping before the partition_* lines."""
         from .EvaluationFuncs import partition_metrics_from_counts
-        from .engine import bit_words, hunk_groups, partition_counts
+        from .engine import bit_words, hunk_clusters, hunk_groups, partition_counts
+        if grouping not in ("components", "average"):
+            raise ValueError(f"grouping must be 'components' or 'average', got {grouping!r}")
         repo = getattr(args, "Repo", self.Repo)
         train, test = data if data is not None else self._load(root)
         self.initialize()
@@ -508,6 +515,8 @@ class graph2graph(object):
         pcounts = torch.zeros(max(n, 1), 8, dtype=torch.int64, device=dev)
         # the hunk counts of the commits whose labels Y are scored (never those of the Q2-substituted maps)
         nh = None if test.nh is None or not nb else torch.as_tensor(np.ascontiguousarray(test.nh[:n], dtype=np.int32)).to(dev)
+        average = grouping == "average"
+        probs = torch.empty(mb, 2, self.Ncr, dtype=torch.float32, device=dev) if average and nb else None
         start_time = time.time()
         alive = []       # the library DMAs from these pinned buffers asynchronously: keep them until the final synchronize
         try:
@@ -519,8 +528,11 @@ class graph2graph(object):
                 alive.append(hb)
                 rows = slice(j * mb, (j + 1) * mb)
                 self.engine.set_predictions(pred[rows])
-                self.engine.infer_host(*hb.tensors(), self.params, None, None)
-                groups[rows] = hunk_groups(pred[rows])[0]
+                self.engine.infer_host(*hb.tensors(), self.params, probs, None)
+                if average:
+                    groups[rows] = hunk_clusters(probs, None if nh is None else nh[rows], threshold)[0]
+                else:
+                    groups[rows] = hunk_groups(pred[rows])[0]
                 label_groups[rows] = hunk_groups(hb.Yw.to(dev, non_blocking=True))[0]
                 pcounts[rows] = partition_counts(groups[rows], label_groups[rows], None if nh is None else nh[rows])
         finally:
@@ -537,6 +549,8 @@ class graph2graph(object):
             os.makedirs(step_dir, exist_ok=True)
             np.save(step_dir + 'C_group_t' + str(self.Ne) + '.npy', out["groups"])
             np.save(step_dir + 'C_group_y' + str(self.Ne) + '.npy', out["label_groups"])
+            if average:
+                log('grouping: average linkage, threshold ' + str(threshold))
             for k, v in out["partition"].items():
                 log('partition_' + k + ': ' + str(v))
             log('exact_partitions: ' + str(exact) + ' / ' + str(n))

@@ -286,6 +286,24 @@ int hdgnn_hunk_groups(int B, int n, const uint32_t* bits, int32_t* groups, int32
 int hdgnn_partition_counts(int B, int n, const int32_t* pred, const int32_t* truth, const int32_t* nh,
                            int64_t* counts, void* stream);
 
+/* Hunk groups by average-linkage (UPGMA) clustering of the relation probabilities, over the REAL hunks 0 .. m-1 of each commit,
+ * m = nh[b] (nh (B) int32, or NULL: m = n).  probs (B, 2, n(n-1)) f32 as the relation head writes it (pair order
+ * p(s,t) = s(n-1)+t-[t>s]); only channel 1 of the real pairs is read.  The similarity of hunks s != t is
+ * w(s,t) = fmaxf(p1(s,t), p1(t,s)) (either direction joins, as in hdgnn_hunk_groups).  From the m singletons, the two clusters
+ * with the largest mean similarity mean(A,C) = S(A,C) / (float)(|A| |C|) (S the fp32 sum of w over A x C, updated by
+ * S(A u B, C) = S(A,C) + S(B,C); IEEE division) are merged while that mean is > threshold; ties go to the smaller
+ * (min representative, max representative), a cluster's representative being its smallest hunk; a NaN mean never merges.
+ * A confident pair between two groups therefore does not join them unless the groups' mean clears the threshold.
+ * groups (B, n) int32 receives the representative of every real hunk's cluster and s for every hunk s >= m (the canonical
+ * labelling of hdgnn_hunk_groups, which hdgnn_partition_counts takes); ngroups (B) int32 or NULL the number of distinct values.
+ * A commit with nh[b] outside [0, n] gets groups all -1 and ngroups -1.  `work`: device scratch of
+ * hdgnn_hunk_clusters_work(B, n) bytes (0 for n <= 169: the commit's tables live in shared memory; else min(B, 296)
+ * pairs of tables of n (n|1) 4-byte words), may be NULL when that is 0.  probs, nh, groups, ngroups, work 4-byte aligned; 2 <= n <= HDGNN_MAX_N;
+ * threshold not NaN.  Deterministic (the merge sequence fixes every rounding), stateless, asynchronous on `stream`. */
+size_t hdgnn_hunk_clusters_work(int B, int n);
+int hdgnn_hunk_clusters(int B, int n, const float* probs, const int32_t* nh, float threshold,
+                        int32_t* groups, int32_t* ngroups, void* work, void* stream);
+
 /* Evaluation counters on the device, replaces the loops of EvaluationFuncs.py:27-37 (top_ACC), :92-117 (prec / recall /
  * f1) and :119-153 (AUC) over the probs the relation head wrote.  probs (B,2,Ncr) f32, Y (B,Nc,y_pitch) u8.
  * counts (B,8) int64: {arg-max hits, quirk tp, fp, fn (ceil of channel 0, as the reference scores), conventional tp, fp,

@@ -7,7 +7,9 @@ given on the command line overrides ALL presets, as in the reference.  Extra fla
 Adjset/ and dataset/), --seed, --no_q2 (feed each batch its own entity->hunk maps instead of the
 reference's first-Mini_batch slice, model_2.py:376-381).  Extra value --Type untangle: the hunk groups the trained model
 predicts for every test commit (graph2graph.untangle), scored against the labelled groups over each commit's real hunks
-(pair precision / recall / F1, Rand and adjusted Rand index, purity).
+(pair precision / recall / F1, Rand and adjusted Rand index, purity).  With --Type untangle, --grouping average forms the
+groups by average-linkage clustering of the relation probabilities instead of connected components of the arg-max relations:
+two groups merge only while their mean relation probability is > --threshold (default 0.5).
 Multi-GPU: launch with `python -m torch.distributed.run --nproc-per-node N main.py ...`.
 """
 import argparse
@@ -52,6 +54,11 @@ def main(argv=None):
         parser.add_argument('--root', type=str, default='.', help='directory holding Adjset/ and dataset/')
         parser.add_argument('--seed', type=int, default=None, help='weight-init seed (the reference is unseeded)')
         parser.add_argument('--no_q2', action='store_true', help='per-batch entity->hunk maps (fixes model_2.py:376-381)')
+        parser.add_argument('--grouping', choices=['components', 'average'], default='components',
+                            help='untangle: hunk groups as connected components of the arg-max relations, or by average '
+                                 'linkage of the relation probabilities')
+        parser.add_argument('--threshold', type=float, default=0.5,
+                            help='untangle --grouping average: merge two groups while their mean relation probability is above it')
         args = parser.parse_args(argv)
 
         ck = args.checkpoint_dir if os.path.isabs(args.checkpoint_dir) else os.path.join(args.root, args.checkpoint_dir)
@@ -75,7 +82,8 @@ def main(argv=None):
         if args.Type == 'test':
             results.append(model.test(args, root=args.root, quirk_q2=not args.no_q2))
         if args.Type == 'untangle':
-            results.append(model.untangle(args, root=args.root, quirk_q2=not args.no_q2))
+            results.append(model.untangle(args, root=args.root, quirk_q2=not args.no_q2, grouping=args.grouping,
+                                          threshold=args.threshold))
         model.engine.close()
     return results
 

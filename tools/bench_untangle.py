@@ -7,14 +7,24 @@
   (d) the partition_counts kernel alone (the untangling scores) on the hunk groups of two label sets, every hunk real (the
       costliest case), at B = 100 and Nc in {74, 256, 512} and at B = 4096, Nc = 74, alternating with hunk_groups on the
       same commits; the per-call times of these eager blocks include the Python wrapper and the launch, so the kernel
-      times are read from torch.profiler as well, in a pass of their own.
+      times are read from torch.profiler as well, in a pass of their own;
+  (e) the hunk_clusters kernel alone (average linkage of the relation probabilities) at B = 100 and Nc in {74, 256, 512} and
+      at B = 4096, Nc = 74, every hunk real, on planted groups of 8 hunks plus noise (nearly every merge happens: the costly
+      case), alternating with hunk_groups on the arg-max bitmap of the same probabilities, kernel times from torch.profiler in
+      a pass of their own; host-fed inference end to end as graph2graph.untangle runs it (Ne = 200, B = 100, random weights),
+      grouping "average" (probabilities written to a device buffer, then hunk_clusters) against "components" (hunk_groups of
+      the predicted relations); and the partition scores of both groupings against the planted groups when a few confident
+      cross-group false positives are added.
 Device inputs rotate through copies that together exceed the 126 MB L2; every arm is timed in blocks that alternate with the
 other arm's, and the median block is reported.  The card's name and power limit are read in the same run.
-Usage: python tools/bench_untangle.py [--sections abcd] [--out result.json]"""
+Usage: python tools/bench_untangle.py [--sections abcde] [--out result.json]"""
 import argparse, json, os, statistics, subprocess, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
-from hdgnn_b200.engine import Engine, DeviceBatch, F_LABEL_BITS, bit_words, hunk_groups, pack_label_bits, partition_counts
+from hdgnn_b200.EvaluationFuncs import partition_metrics_from_counts
+from hdgnn_b200._lib import lib
+from hdgnn_b200.engine import (Engine, DeviceBatch, F_LABEL_BITS, bit_words, hunk_clusters, hunk_groups, pack_label_bits,
+                               partition_counts)
 from hdgnn_b200.model import HostBatch
 from hdgnn_b200.synthetic import make_commits
 
@@ -58,7 +68,7 @@ def timed(arms, calls):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=None)
-    ap.add_argument("--sections", default="abcd", help="which of the sections (a)-(d) to run")
+    ap.add_argument("--sections", default="abcde", help="which of the sections (a)-(e) to run")
     args = ap.parse_args()
     out = {"card": card(), "B": B, "Ne": Ne, "variant": 2, "reps": REPS, "what": __doc__.split("Usage")[0].strip(), "rows": []}
     for Nc in ((74, 256, 512) if set("abc") & set(args.sections) else ()):
@@ -147,6 +157,10 @@ def main():
         torch.cuda.empty_cache()
     if "d" in args.sections:
         out["d_partition_counts"] = [scores(Bd, Nc) for Bd, Nc in ((B, 74), (B, 256), (B, 512), (4096, 74))]
+    if "e" in args.sections:
+        out["e_hunk_clusters"] = [clusters(Bd, Nc) for Bd, Nc in ((B, 74), (B, 256), (B, 512), (4096, 74))]
+        out["e_untangle_end_to_end"] = [untangle_e2e(Nc) for Nc in (74, 256, 512)]
+        out["e_quality"] = [quality(Nc) for Nc in (74, 256)]
     out["card_after"] = card()
     if args.out:
         os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
@@ -171,6 +185,104 @@ def scores(Bd, Nc):
            "us_per_batch_hunk_groups": ms["hunk_groups"] * 1e3, "commits_per_s_partition_counts": Bd / ms["partition_counts"] * 1e3,
            "kernel_us_partition_counts": kern.get("partition_counts"), "kernel_us_hunk_groups": kern.get("hunk_groups"),
            "mean_groups": [float(c[:, 4].mean()), float(c[:, 5].mean())], "pool_batches": len(pairs), "blocks_ms": blocks}
+    print(json.dumps(row, default=str))
+    return row
+
+
+def planted(Bd, Nc, seed, group=8, p_false=0.0):
+    """(probs (Bd, 2, Nc(Nc-1)) f32, truth (Bd, Nc) int32) on the device: each commit's hunks in random groups of `group`;
+    p1 ~ U(0.55, 0.95) inside a group (15 % of the inner pairs missing at U(0, 0.3)), U(0, 0.35) across, plus a fraction
+    p_false of the cross pairs at U(0.8, 1); both directions drawn on their own; p0 = 1 - p1.  truth = the smallest hunk of
+    each hunk's planted group."""
+    g = torch.Generator(device="cuda").manual_seed(seed)
+    u = lambda lo, hi: lo + (hi - lo) * torch.rand(Bd, Nc, Nc, generator=g, device="cuda")
+    lab = torch.argsort(torch.rand(Bd, Nc, generator=g, device="cuda"), dim=1) // group
+    same = lab[:, :, None] == lab[:, None, :]
+    P = torch.where(same, u(0.55, 0.95), u(0.0, 0.35))
+    P = torch.where(same & (torch.rand(Bd, Nc, Nc, generator=g, device="cuda") < 0.15), u(0.0, 0.3), P)
+    P = torch.where(~same & (torch.rand(Bd, Nc, Nc, generator=g, device="cuda") < p_false), u(0.8, 1.0), P)
+    off = ~torch.eye(Nc, dtype=torch.bool, device="cuda")
+    p1 = P[:, off]                                   # row-major without the diagonal: the pair order s(Nc-1)+t-[t>s]
+    probs = torch.stack([1 - p1, p1], dim=1).contiguous()
+    idx = torch.arange(Nc, device="cuda").expand(Bd, Nc)
+    first = torch.full((Bd, Nc), Nc, dtype=torch.int64, device="cuda").scatter_reduce(1, lab, idx, "amin")
+    return probs, torch.gather(first, 1, lab).to(torch.int32)
+
+
+def argmax_bits(probs, Nc):
+    p = probs.cpu().numpy()
+    grid = np.zeros((p.shape[0], Nc, Nc), dtype=np.uint8)
+    grid[:, ~np.eye(Nc, dtype=bool)] = p[:, 1] > p[:, 0]
+    return torch.as_tensor(pack_label_bits(grid).view(np.int32)).cuda()
+
+
+def clusters(Bd, Nc):
+    """(e): hunk_clusters of Bd commits (every hunk real, planted groups of 8), in blocks alternating with hunk_groups of the
+    arg-max bitmap of the same probabilities."""
+    probs, _ = planted(Bd, Nc, 6060)
+    bits = argmax_bits(probs, Nc)
+    nh = torch.full((Bd,), Nc, dtype=torch.int32, device="cuda")
+    ppool = rotate([probs], probs.numel() * 4)
+    bpool = rotate([bits], bits.numel() * 4)
+    arms = {"hunk_clusters": lambda k: hunk_clusters(ppool[k % len(ppool)], nh, 0.5),
+            "hunk_groups": lambda k: hunk_groups(bpool[k % len(bpool)])}
+    calls = 5 if Nc >= 256 else 20
+    ms, blocks = timed(arms, calls)
+    kern = kernel_us(arms, 4 * calls)
+    ng_avg = hunk_clusters(probs, nh, 0.5)[1].float().mean().item()
+    ng_cc = hunk_groups(bits)[1].float().mean().item()
+    row = {"B": Bd, "Nc": Nc, "us_per_batch_hunk_clusters": ms["hunk_clusters"] * 1e3, "us_per_batch_hunk_groups": ms["hunk_groups"] * 1e3,
+           "commits_per_s_hunk_clusters": Bd / ms["hunk_clusters"] * 1e3,
+           "kernel_us_hunk_clusters": kern.get("hunk_clusters"), "kernel_us_hunk_groups": kern.get("hunk_groups"),
+           "merges_per_commit": Nc - ng_avg, "mean_groups_average": ng_avg, "mean_groups_components": ng_cc,
+           "work_bytes": int(lib.hdgnn_hunk_clusters_work(Bd, Nc)),
+           "pool_batches": len(ppool), "blocks_ms": blocks}
+    print(json.dumps(row, default=str))
+    del ppool, bpool
+    torch.cuda.empty_cache()
+    return row
+
+
+def untangle_e2e(Nc):
+    """(e): host-fed inference + groups per batch as graph2graph.untangle runs it, "average" against "components"."""
+    eng = Engine(Ne, Nc, variant=2, max_batch=B, flags=F_LABEL_BITS)
+    cbs = [make_commits(B, Ne, Nc, seed=7070 + i) for i in range(4)]
+    hbs = [HostBatch(c, bits=True) for c in cbs]
+    params = (0.1 * torch.randn(eng.n_params, generator=torch.Generator().manual_seed(1))).cuda()
+    pred = torch.zeros(B, Nc, bit_words(Nc), dtype=torch.int32, device="cuda")
+    probs = torch.empty(B, 2, Nc * (Nc - 1), dtype=torch.float32, device="cuda")
+    nh = torch.full((B,), Nc, dtype=torch.int32, device="cuda")
+    groups = torch.empty(B, Nc, dtype=torch.int32, device="cuda")
+    eng.set_predictions(pred)
+
+    def average(k):
+        eng.infer_host(*hbs[k % len(hbs)].tensors(), params, probs, None)
+        groups.copy_(hunk_clusters(probs, nh, 0.5)[0])
+
+    def components(k):
+        eng.infer_host(*hbs[k % len(hbs)].tensors(), params, None, None)
+        groups.copy_(hunk_groups(pred)[0])
+    ms, blocks = timed({"average": average, "components": components}, 5 if Nc >= 256 else 20)
+    ng = hunk_clusters(probs, nh, 0.5)[1].float().mean().item()
+    eng.set_predictions(None)
+    eng.close()
+    row = {"Nc": Nc, "B": B, "Ne": Ne, "ms_per_batch_average": ms["average"], "ms_per_batch_components": ms["components"],
+           "commits_per_s_average": B / ms["average"] * 1e3, "commits_per_s_components": B / ms["components"] * 1e3,
+           "mean_groups_average_random_weights": ng, "blocks_ms": blocks}
+    print(json.dumps(row, default=str))
+    return row
+
+
+def quality(Nc, Bq=200):
+    """(e): partition scores against the planted groups of both groupings, on planted probabilities with 1 % of the cross pairs
+    confident false positives."""
+    probs, truth = planted(Bq, Nc, 8080, p_false=0.01)
+    nh = torch.full((Bq,), Nc, dtype=torch.int32, device="cuda")
+    avg = hunk_clusters(probs, nh, 0.5)[0]
+    cc = hunk_groups(argmax_bits(probs, Nc))[0]
+    row = {"Nc": Nc, "B": Bq, "p_false": 0.01, "group": 8,
+           "average": partition_metrics_from_counts(partition_counts(avg, truth, nh).cpu().numpy()),
+           "components": partition_metrics_from_counts(partition_counts(cc, truth, nh).cpu().numpy())}
     print(json.dumps(row, default=str))
     return row
 
