@@ -43,12 +43,13 @@
 #include "pack.cuh"
 #include "fused.h"
 #include "final.cuh"
+#include "host.cuh"
 
 using namespace hdgnn;
 
-namespace {
+thread_local std::string hdgnn::g_error;
 
-thread_local std::string g_create_error;
+namespace {
 
 struct Block { const char* name; int rows, cols; };
 const Block kEnt[] = {{"ent_w1", 4, 20}, {"ent_b1", 1, 20}, {"ent_w5", 20, 20}, {"ent_b5", 1, 20},
@@ -225,7 +226,7 @@ namespace {
     } while (0)
 
 int fail(hdgnn_handle_t h, int code, const std::string& msg) {
-    if (h) h->err = msg; else g_create_error = msg;
+    if (h) h->err = msg; else g_error = msg;
     return code;
 }
 
@@ -908,22 +909,24 @@ int hdgnn_param_offset(int variant, const char* name) {
 }
 
 int hdgnn_pack_label_bits(int N, int n, const uint8_t* grid, int pitch, uint32_t* bits, void* stream) {
-    if (N < 1 || n < 2 || n > HDGNN_MAX_N || !grid || !bits) return HDGNN_E_INVALID;
-    if (pitch < n || (pitch & 15) || pitch > 528 || ((uintptr_t)grid & 15) || ((uintptr_t)bits & 15)) return HDGNN_E_INVALID;
+    const Call c{"hdgnn_pack_label_bits"};
+    if (int rc = c.sizes("N", N, "n", n)) return rc;
+    if (pitch < n || (pitch & 15) || pitch > 528) return c.invalid("pitch must be a multiple of 16 in [n, 528]");
+    if (int rc = c.pointers({{"grid", grid, 16}, {"bits", bits, 16}})) return rc;
     PackArgs p{};
     p.adj = grid; p.Ne = n; p.pe = pitch; p.WPe = bit_words(n); p.ebits = bits; p.B = N;
     p.Y = nullptr; p.Nc = 0; p.pc = 0; p.WPc = 0; p.ybits = nullptr;
     const long long rows = (long long)N * n;
     if (pitch <= 256) pack_bits_kernel<16><<<(int)((rows + 15) / 16), 256, 0, (cudaStream_t)stream>>>(p);
     else pack_bits_kernel<32><<<(int)((rows + 7) / 8), 256, 0, (cudaStream_t)stream>>>(p);
-    return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+    return c.launched();
 }
 
 int hdgnn_bit_words(int n) { return n > 0 && n <= HDGNN_MAX_N ? bit_words(n) : -1; }
 
 int hdgnn_label_pitch(int n) { return n < 1 ? HDGNN_E_INVALID : round_up(n, 16); }
 
-const char* hdgnn_last_error(hdgnn_handle_t h) { return h ? h->err.c_str() : g_create_error.c_str(); }
+const char* hdgnn_last_error(hdgnn_handle_t h) { return h ? h->err.c_str() : g_error.c_str(); }
 
 int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
     if (!cfg || !out) return fail(nullptr, HDGNN_E_INVALID, "null cfg/out");
@@ -979,7 +982,7 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
         if (!bytes[i]) continue;
         int rc = alloc(h, (WsId)i, bytes[i]);
         if (rc != HDGNN_OK) {
-            g_create_error = h->err;
+            g_error = h->err;
             hdgnn_destroy(h);
             return rc;
         }
@@ -992,7 +995,7 @@ int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out) {
         ok = cudaEventCreateWithFlags(&h->ev_copy[i], cudaEventDisableTiming) == cudaSuccess &&
              cudaEventCreateWithFlags(&h->ev_done[i], cudaEventDisableTiming) == cudaSuccess;
     if (!ok) {
-        g_create_error = "cudaStreamCreate / cudaEventCreate failed";
+        g_error = "cudaStreamCreate / cudaEventCreate failed";
         hdgnn_destroy(h);
         return HDGNN_E_CUDA;
     }

@@ -24,6 +24,7 @@
 
 #include "../../include/hdgnn.h"
 #include "bits.cuh"
+#include "host.cuh"
 
 namespace hdgnn {
 
@@ -789,21 +790,15 @@ __global__ void mean_kernel(const float* v, int n, float* out) {
 
 using namespace hdgnn;
 
-static int conv_check(int B, int N, int pitch, const void* adj, int flags) {
-    if (B < 1 || N < 2 || N > HDGNN_MAX_N || !adj || !legacy_adj_ok(N, pitch, adj, flags)) return HDGNN_E_INVALID;
-    return HDGNN_OK;
-}
-
 extern "C" int hdgnn_normalize_propagate(int B, int N, const uint8_t* adj, int pitch, const float* H, int d_in, const float* W,
                                          const float* bias, int d_out, float eps, int flags, float* out, float* dinv_out,
                                          void* stream) {
-    int rc = conv_check(B, N, pitch, adj, flags);
-    if (rc) return rc;
-    if (!H || !out || d_in < 1 || d_in > CONV_MAXD || d_out < 1 || d_out > CONV_MAXD) return HDGNN_E_INVALID;
-    if (!W && d_in != d_out) return HDGNN_E_INVALID;
-    int dev = 0, optin = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
-        return HDGNN_E_CUDA;
+    const Call c{"hdgnn_normalize_propagate"};
+    if (int rc = legacy_check(c, B, N, pitch, adj, flags)) return rc;
+    if (d_in < 1 || d_in > CONV_MAXD || d_out < 1 || d_out > CONV_MAXD || (!W && d_in != d_out))
+        return c.invalid("d_in or d_out outside [1, 32], or W null with d_in != d_out");
+    if (int rc = c.pointers({{"H", H, 4}, {"W", W, 4, false}, {"bias", bias, 4, false}, {"out", out, 4}, {"dinv_out", dinv_out, 4, false}})) return rc;
+    Device d; if (int rc = c.device(&d)) return rc;
     const bool bits = flags & HDGNN_P_LABEL_BITS;
     ConvArgs a{};
     a.B = B; a.N = N; a.pitch = pitch; a.d_in = d_in; a.d_out = d_out; a.flags = flags; a.eps = eps;
@@ -813,64 +808,54 @@ extern "C" int hdgnn_normalize_propagate(int B, int N, const uint8_t* adj, int p
     // that of the tile as staged (N * pitch bytes): a bitmap tile is 1/8 of a byte tile, so the persistent kernel takes
     // bitmaps up to N = 240 at d_in = 20 where byte grids fall back to the one-CTA-per-commit kernel above N = 208.
     const size_t smem_tc2 = tc2_smem_bytes(N, pitch, d_in);
-    if (!(flags & (HDGNN_P_NO_TENSOR | HDGNN_P_TENSOR_V1)) && N <= 256 && smem_tc2 <= (size_t)optin) {
-        int sms = 148;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (!(flags & (HDGNN_P_NO_TENSOR | HDGNN_P_TENSOR_V1)) && N <= 256 && smem_tc2 <= (size_t)d.optin) {
         const auto k = bits ? propagate_tc2_kernel<true> : propagate_tc2_kernel<false>;
-        if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) != cudaSuccess) return HDGNN_E_CUDA;
-        k<<<B < sms ? B : sms, TC2_T, smem_tc2, (cudaStream_t)stream>>>(a);
-        return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+        if (int rc = c.raise_smem(k, d)) return rc;
+        k<<<B < d.sms ? B : d.sms, TC2_T, smem_tc2, (cudaStream_t)stream>>>(a);
+        return c.launched();
     }
     const size_t smem_tc = tc_smem_bytes(N, pitch, d_in, d_out);
-    if (!(flags & HDGNN_P_NO_TENSOR) && N <= 256 && smem_tc <= (size_t)optin) {
+    if (!(flags & HDGNN_P_NO_TENSOR) && N <= 256 && smem_tc <= (size_t)d.optin) {
         const auto k = bits ? propagate_tc_kernel<true> : propagate_tc_kernel<false>;
-        if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) != cudaSuccess) return HDGNN_E_CUDA;
+        if (int rc = c.raise_smem(k, d)) return rc;
         k<<<B, TC_T, smem_tc, (cudaStream_t)stream>>>(a);
-        return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+        return c.launched();
     }
     const size_t smem = conv_smem_bytes(N, pitch, d_out);
-    if (smem > (size_t)optin) return HDGNN_E_UNSUPPORTED;       // the per-commit tile must fit one SM
+    if (smem > (size_t)d.optin) return c.fail(HDGNN_E_UNSUPPORTED, "the per-commit tile does not fit one SM's shared memory");
     const auto k = bits ? propagate_kernel<true> : propagate_kernel<false>;
-    if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) != cudaSuccess) return HDGNN_E_CUDA;
+    if (int rc = c.raise_smem(k, d)) return rc;
     k<<<B, CONV_T, smem, (cudaStream_t)stream>>>(a);
-    return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+    return c.launched();
 }
 
 extern "C" int hdgnn_map_conv(int B, int N, const uint8_t* adj, int pitch, const float* x, const float* theta, float lam_max,
                               float eps, int flags, float* per_commit, float* loss, void* stream) {
-    int rc = conv_check(B, N, pitch, adj, flags);
-    if (rc) return rc;
-    if (!x || !theta || !per_commit || lam_max <= 0.f) return HDGNN_E_INVALID;
+    const Call c{"hdgnn_map_conv"};
+    if (int rc = legacy_check(c, B, N, pitch, adj, flags)) return rc;
+    if (!(lam_max > 0.f)) return c.invalid("lam_max must be > 0");
+    if (int rc = c.pointers({{"x", x, 4}, {"theta", theta, 4}, {"per_commit", per_commit, 4}, {"loss", loss, 4, false}})) return rc;
+    Device d; if (int rc = c.device(&d)) return rc;
     const bool bits = flags & HDGNN_P_LABEL_BITS;
-    const size_t smem = conv_smem_bytes(N, pitch, 1);
-    int dev = 0, optin = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
-        return HDGNN_E_CUDA;
-    // the reference's (transposed) form: persistent kernel on the staged tile, several tiles in flight per SM
-    const size_t smem2 = mc2_smem_bytes(N, pitch, bits ? round_up(N, 16) / 4 : pitch / 4);
-    if (!(flags & (HDGNN_P_NO_TRANSPOSE | HDGNN_P_TENSOR_V1)) && smem2 <= (size_t)optin) {
-        int sms = 148;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        const auto k2 = bits ? map_conv2_kernel<true> : map_conv2_kernel<false>;
-        if (cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2) != cudaSuccess) return HDGNN_E_CUDA;
-        ConvArgs a2{};
-        a2.B = B; a2.N = N; a2.pitch = pitch; a2.flags = flags; a2.eps = eps; a2.lam_max = lam_max;
-        a2.adj = adj; a2.x = x; a2.theta = theta; a2.per_commit = per_commit;
-        int per_sm = (int)((size_t)(228 * 1024) / (smem2 + 1024));       // resident CTAs an SM's shared memory allows
-        per_sm = per_sm < 1 ? 1 : (per_sm > 8 ? 8 : per_sm);
-        const int grid = B < sms * per_sm ? B : sms * per_sm;
-        if (!x || !theta || !per_commit || lam_max <= 0.f) return HDGNN_E_INVALID;
-        k2<<<grid, MC2_T, smem2, (cudaStream_t)stream>>>(a2);
-        if (loss) mean_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(per_commit, B, loss);
-        return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
-    }
-    if (smem > (size_t)optin) return HDGNN_E_UNSUPPORTED;
-    const auto k = bits ? map_conv_kernel<true> : map_conv_kernel<false>;
-    if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) != cudaSuccess) return HDGNN_E_CUDA;
     ConvArgs a{};
     a.B = B; a.N = N; a.pitch = pitch; a.flags = flags; a.eps = eps; a.lam_max = lam_max;
     a.adj = adj; a.x = x; a.theta = theta; a.per_commit = per_commit;
-    k<<<B, CONV_T, smem, (cudaStream_t)stream>>>(a);
+    // the reference's (transposed) form: persistent kernel on the staged tile, several tiles in flight per SM
+    const size_t smem2 = mc2_smem_bytes(N, pitch, bits ? round_up(N, 16) / 4 : pitch / 4);
+    if (!(flags & (HDGNN_P_NO_TRANSPOSE | HDGNN_P_TENSOR_V1)) && smem2 <= (size_t)d.optin) {
+        const auto k2 = bits ? map_conv2_kernel<true> : map_conv2_kernel<false>;
+        if (int rc = c.raise_smem(k2, d)) return rc;
+        int per_sm = (int)((size_t)d.per_sm / (smem2 + 1024));       // resident CTAs an SM's shared memory allows
+        per_sm = per_sm < 1 ? 1 : (per_sm > 8 ? 8 : per_sm);
+        const int grid = B < d.sms * per_sm ? B : d.sms * per_sm;
+        k2<<<grid, MC2_T, smem2, (cudaStream_t)stream>>>(a);
+    } else {
+        const size_t smem = conv_smem_bytes(N, pitch, 1);
+        if (smem > (size_t)d.optin) return c.fail(HDGNN_E_UNSUPPORTED, "the per-commit tile does not fit one SM's shared memory");
+        const auto k = bits ? map_conv_kernel<true> : map_conv_kernel<false>;
+        if (int rc = c.raise_smem(k, d)) return rc;
+        k<<<B, CONV_T, smem, (cudaStream_t)stream>>>(a);
+    }
     if (loss) mean_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(per_commit, B, loss);
-    return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+    return c.launched();
 }

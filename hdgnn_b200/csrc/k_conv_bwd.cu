@@ -17,6 +17,7 @@
 // All sums run in a fixed order (no float atomics).
 #include "../../include/hdgnn.h"
 #include "bits.cuh"
+#include "host.cuh"
 
 namespace hdgnn {
 
@@ -226,10 +227,18 @@ extern "C" size_t hdgnn_propagate_backward_work(int B, int N, int d_in, int d_ou
 extern "C" int hdgnn_normalize_propagate_backward(int B, int N, const uint8_t* adj, int adj_pitch, const float* H, int d_in,
                                                   const float* W, int d_out, float eps, int flags, const float* out, const float* dOut,
                                                   float* dH, float* dW, float* dbias, float* work, void* stream) {
-    if (B < 1 || N < 2 || N > HDGNN_MAX_N || !adj || !H || !dOut || !work) return HDGNN_E_INVALID;
-    if (!legacy_adj_ok(N, adj_pitch, adj, flags)) return HDGNN_E_INVALID;
-    if (d_in < 1 || d_in > CB_MAXD || d_out < 1 || d_out > CB_MAXD || (!W && d_in != d_out)) return HDGNN_E_INVALID;
-    if ((flags & HDGNN_P_RELU) && !out) return HDGNN_E_INVALID;
+    const Call c{"hdgnn_normalize_propagate_backward"};
+    if (int rc = legacy_check(c, B, N, adj_pitch, adj, flags)) return rc;
+    if (d_in < 1 || d_in > CB_MAXD || d_out < 1 || d_out > CB_MAXD || (!W && d_in != d_out))
+        return c.invalid("d_in or d_out outside [1, 32], or W null with d_in != d_out");
+    if (int rc = c.pointers({{"H", H, 4}, {"W", W, 4, false}, {"out", out, 4, (flags & HDGNN_P_RELU) != 0}, {"dOut", dOut, 4},
+                             {"dH", dH, 4, false}, {"dW", dW, 4, false}, {"dbias", dbias, 4, false}, {"work", work, 4}}))
+        return rc;
+    size_t smem = ((size_t)N * (d_in + d_out) + (size_t)d_in * d_out) * sizeof(float);
+    if (smem < CB_T * sizeof(float)) smem = CB_T * sizeof(float);      // the bias slots reuse the head of the tile
+    Device d; if (int rc = c.device(&d)) return rc;
+    if (smem > (size_t)d.optin) return c.fail(HDGNN_E_UNSUPPORTED, "the per-commit tile does not fit one SM's shared memory");
+    if (int rc = c.raise_smem(prop_bwd_commit_kernel, d)) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const size_t nel = (size_t)B * N * d_out;
     float* dPre = work; float* dZ = work + nel; float* partial = work + 2 * nel;
@@ -243,39 +252,33 @@ extern "C" int hdgnn_normalize_propagate_backward(int B, int N, const uint8_t* a
     const int flipped = keep | ((flags & HDGNN_P_NO_TRANSPOSE) ? 0 : HDGNN_P_NO_TRANSPOSE);
     int rc = hdgnn_normalize_propagate(B, N, adj, adj_pitch, dpre_src, d_out, nullptr, nullptr, d_out, eps, flipped, dZ, nullptr, stream);
     if (rc) return rc;
-    size_t smem = ((size_t)N * (d_in + d_out) + (size_t)d_in * d_out) * sizeof(float);
-    if (smem < CB_T * sizeof(float)) smem = CB_T * sizeof(float);      // the bias slots reuse the head of the tile
-    int dev = 0, optin = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
-        return HDGNN_E_CUDA;
-    if (smem > (size_t)optin) return HDGNN_E_UNSUPPORTED;
-    if (cudaFuncSetAttribute(prop_bwd_commit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return HDGNN_E_CUDA;
     prop_bwd_commit_kernel<<<B, CB_T, smem, st>>>(N, d_in, d_out, H, W, dZ, dpre_src, dH, partial);
     const int stride = d_in * d_out + d_out;
     float* part2 = partial + (size_t)B * stride;
     if ((dW && W) || dbias) batch_sum1_kernel<<<dim3((stride + 127) / 128, BS_CH), 128, 0, st>>>(partial, B, stride, part2);
     if (dW && W) batch_sum2_kernel<<<(d_in * d_out + 127) / 128, 128, 0, st>>>(part2, stride, 0, d_in * d_out, dW);
     if (dbias) batch_sum2_kernel<<<1, 128, 0, st>>>(part2, stride, d_in * d_out, d_out, dbias);
-    return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+    return c.launched();
 }
 
 extern "C" int hdgnn_map_conv_backward(int B, int N, const uint8_t* adj, int adj_pitch, const float* x, const float* theta, float lam_max,
                                        float eps, int flags, float gscale, float* dx, float* dtheta, float* work, void* stream) {
-    if (B < 1 || N < 2 || N > HDGNN_MAX_N || !adj || !x || !theta || lam_max <= 0.f) return HDGNN_E_INVALID;
-    if (!legacy_adj_ok(N, adj_pitch, adj, flags)) return HDGNN_E_INVALID;
-    if (dtheta && !work) return HDGNN_E_INVALID;
-    cudaStream_t st = (cudaStream_t)stream;
+    const Call c{"hdgnn_map_conv_backward"};
+    if (int rc = legacy_check(c, B, N, adj_pitch, adj, flags)) return rc;
+    if (!(lam_max > 0.f)) return c.invalid("lam_max must be > 0");
+    if (int rc = c.pointers({{"x", x, 4}, {"theta", theta, 4}, {"dx", dx, 4, false}, {"dtheta", dtheta, 4, false},
+                             {"work", work, 4, dtheta != nullptr}}))
+        return rc;
     const size_t smem = 16 + (size_t)round_up(N * adj_pitch, 16) + (size_t)(5 * N + 32) * sizeof(float);
-    int dev = 0, optin = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
-        return HDGNN_E_CUDA;
-    if (smem > (size_t)optin) return HDGNN_E_UNSUPPORTED;
+    Device d; if (int rc = c.device(&d)) return rc;
+    if (smem > (size_t)d.optin) return c.fail(HDGNN_E_UNSUPPORTED, "the per-commit tile does not fit one SM's shared memory");
     const auto k = (flags & HDGNN_P_LABEL_BITS) ? map_conv_bwd_kernel<true> : map_conv_bwd_kernel<false>;
-    if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return HDGNN_E_CUDA;
+    if (int rc = c.raise_smem(k, d)) return rc;
     McbArgs a{};
     a.B = B; a.N = N; a.pitch = adj_pitch; a.flags = flags; a.eps = eps; a.lam_max = lam_max; a.gscale = gscale;
     a.adj = adj; a.x = x; a.theta = theta; a.dx = dx; a.part = dtheta ? work : nullptr;
+    cudaStream_t st = (cudaStream_t)stream;
     k<<<B, CB_T, smem, st>>>(a);
     if (dtheta) theta_grad_kernel<<<1, 256, 0, st>>>(work, B, theta, dtheta);
-    return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+    return c.launched();
 }

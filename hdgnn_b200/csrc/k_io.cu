@@ -19,6 +19,7 @@
 #include "../../include/hdgnn.h"
 #include "bits.cuh"
 #include "common.cuh"
+#include "host.cuh"
 
 namespace hdgnn {
 
@@ -520,16 +521,16 @@ using namespace hdgnn;
 
 extern "C" int hdgnn_compact_from_raw(int N, int n, const void* raw, int raw_is_f64, uint8_t* grid, int pitch, float* diag,
                                       int32_t* err, void* stream) {
-    if (N < 1 || n < 2 || n > HDGNN_MAX_N || !raw || !grid) return HDGNN_E_INVALID;
-    if (pitch < n || (pitch & 15) || pitch > 512 + 16) return HDGNN_E_INVALID;
+    const Call c{"hdgnn_compact_from_raw"};
+    if (int rc = c.sizes("N", N, "n", n)) return rc;
+    if (pitch < n || (pitch & 15) || pitch > 512 + 16) return c.invalid("pitch must be a multiple of 16 in [n, 528]");
     const long long rows = (long long)N * n;
-    if (rows > 0x7fffffffLL) return HDGNN_E_INVALID;
-    int dev = 0, sms = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
-        return HDGNN_E_CUDA;
+    if (rows > 0x7fffffffLL) return c.invalid("N * n above 2^31 - 1");
+    if (int rc = c.pointers({{"raw", raw, raw_is_f64 ? 8u : 4u}, {"grid", grid, 1}, {"diag", diag, 4, false}, {"err", err, 4, false}})) return rc;
+    Device d; if (int rc = c.device(&d)) return rc;
     const int wpb = 8;
     long long want = (rows + wpb - 1) / wpb;
-    const int grid_x = (int)(want < (long long)sms * 8 ? want : (long long)sms * 8);      // 8 CTAs of 8 warps per SM, grid-stride
+    const int grid_x = (int)(want < (long long)d.sms * 8 ? want : (long long)d.sms * 8);      // 8 CTAs of 8 warps per SM, grid-stride
     cudaStream_t st = (cudaStream_t)stream;
     const int kmax = (pitch + 31) / 32;
 #define LAUNCH(T, K) compact_from_raw_kernel<T, K><<<grid_x, 256, 0, st>>>((const T*)raw, (int)rows, n, grid, pitch, diag, err)
@@ -539,64 +540,50 @@ extern "C" int hdgnn_compact_from_raw(int N, int n, const void* raw, int raw_is_
         if (kmax <= 4) LAUNCH(float, 4); else if (kmax <= 8) LAUNCH(float, 8); else if (kmax <= 12) LAUNCH(float, 12); else LAUNCH(float, 17);
     }
 #undef LAUNCH
-    return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+    return c.launched();
 }
 
 extern "C" int hdgnn_eval_counts(int B, int Nc, const float* probs, const uint8_t* Y, int y_pitch, int64_t* counts, int64_t* auc,
                                  int auc_first, void* stream) {
-    if (B < 1 || Nc < 2 || Nc > HDGNN_MAX_N || !probs || !Y || !counts || y_pitch < Nc) return HDGNN_E_INVALID;
+    const Call c{"hdgnn_eval_counts"};
+    if (int rc = c.sizes("B", B, "Nc", Nc)) return rc;
+    if (y_pitch < Nc) return c.invalid("y_pitch < Nc");
+    if (int rc = c.pointers({{"probs", probs, 4}, {"Y", Y, 1}, {"counts", counts, 8}, {"auc", auc, 8, false}})) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    if (cudaMemsetAsync(counts, 0, (size_t)B * 8 * sizeof(int64_t), st) != cudaSuccess) return HDGNN_E_CUDA;
-    if (auc && cudaMemsetAsync(auc, 0, (size_t)B * 2 * sizeof(int64_t), st) != cudaSuccess) return HDGNN_E_CUDA;
+    if (int rc = c.cuda(cudaMemsetAsync(counts, 0, (size_t)B * 8 * sizeof(int64_t), st))) return rc;
+    if (int rc = c.cuda(auc ? cudaMemsetAsync(auc, 0, (size_t)B * 2 * sizeof(int64_t), st) : cudaSuccess)) return rc;
     const int Ncr = Nc * (Nc - 1);
     dim3 g((Ncr + EV_CHUNK - 1) / EV_CHUNK, B);
     eval_counts_kernel<<<g, EV_T, 0, st>>>(Nc, probs, Y, y_pitch, (unsigned long long*)counts, (unsigned long long*)auc,
                                           auc_first < 0 ? 0 : auc_first);
-    return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+    return c.launched();
 }
 
 extern "C" int hdgnn_hunk_groups(int B, int n, const uint32_t* bits, int32_t* groups, int32_t* ngroups, void* stream) {
-    if (B < 1 || n < 2 || n > HDGNN_MAX_N || !bits || !groups) return HDGNN_E_INVALID;
-    if (((uintptr_t)bits & 15) || ((uintptr_t)groups & 3) || ((uintptr_t)ngroups & 3)) return HDGNN_E_INVALID;
-    int dev = 0, sms = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
-        return HDGNN_E_CUDA;
+    const Call c{"hdgnn_hunk_groups"};
+    if (int rc = c.sizes("B", B, "n", n)) return rc;
+    if (int rc = c.pointers({{"bits", bits, 16}, {"groups", groups, 4}, {"ngroups", ngroups, 4, false}})) return rc;
+    Device d; if (int rc = c.device(&d)) return rc;
     const int WP = bit_words(n);
     const size_t per = (size_t)n * WP * 4;
-    // one commit per CTA until the batch covers the SMs, then up to HG_WARPS_MAX (as far as the shared memory allows)
-    int cpc = B / sms;
-    const int fit = (int)(HG_SMEM_MAX / per);
-    if (cpc > fit) cpc = fit;
-    if (cpc > HG_WARPS_MAX) cpc = HG_WARPS_MAX;
-    if (cpc < 1) cpc = 1;
+    const int cpc = commits_per_cta(B, d.sms, per, HG_SMEM_MAX, HG_WARPS_MAX);
     hunk_groups_kernel<<<(B + cpc - 1) / cpc, 32 * cpc, cpc * per, (cudaStream_t)stream>>>(B, n, WP, bits, groups, ngroups);
-    return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+    return c.launched();
 }
 
 extern "C" int hdgnn_partition_counts(int B, int n, const int32_t* pred, const int32_t* truth, const int32_t* nh, int64_t* counts,
                                       void* stream) {
-    if (B < 1 || n < 2 || n > HDGNN_MAX_N || !pred || !truth || !counts) return HDGNN_E_INVALID;
-    if (((uintptr_t)pred & 3) || ((uintptr_t)truth & 3) || ((uintptr_t)nh & 3) || ((uintptr_t)counts & 7)) return HDGNN_E_INVALID;
-    int dev = 0, sms = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
-        return HDGNN_E_CUDA;
+    const Call c{"hdgnn_partition_counts"};
+    if (int rc = c.sizes("B", B, "n", n)) return rc;
+    if (int rc = c.pointers({{"pred", pred, 4}, {"truth", truth, 4}, {"nh", nh, 4, false}, {"counts", counts, 8}})) return rc;
+    Device d; if (int rc = c.device(&d)) return rc;
     const size_t per = pc_smem_words(n) * 4;
-    // one commit per CTA until the batch covers the SMs, then up to PC_WARPS_MAX (as far as PC_SMEM_MAX allows)
-    int cpc = B / sms;
-    const int fit = (int)(PC_SMEM_MAX / per);
-    if (cpc > fit) cpc = fit;
-    if (cpc > PC_WARPS_MAX) cpc = PC_WARPS_MAX;
-    if (cpc < 1) cpc = 1;
-    const size_t smem = cpc * per;
-    // above the 48 KB default (one commit from n = 410 on, or several smaller ones) the launch needs the opt-in.  It is set to
-    // the largest launch there can be, so concurrent callers never lower it under each other; it is not a stream operation,
-    // so it is allowed while a graph is captured.
-    if (smem > 48 * 1024 &&
-        cudaFuncSetAttribute(partition_counts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PC_SMEM_MAX) != cudaSuccess)
-        return HDGNN_E_CUDA;
+    const int cpc = commits_per_cta(B, d.sms, per, PC_SMEM_MAX, PC_WARPS_MAX);
+    const size_t smem = cpc * per;     // above the 48 KB default: one commit from n = 410 on, or several smaller ones
+    if (int rc = smem > 48 * 1024 ? c.raise_smem(partition_counts_kernel, d) : HDGNN_OK) return rc;
     partition_counts_kernel<<<(B + cpc - 1) / cpc, 32 * cpc, smem, (cudaStream_t)stream>>>(B, n, pred, truth, nh,
                                                                                            (long long*)counts);
-    return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+    return c.launched();
 }
 
 extern "C" size_t hdgnn_hunk_clusters_work(int B, int n) {
@@ -606,22 +593,21 @@ extern "C" size_t hdgnn_hunk_clusters_work(int B, int n) {
 
 extern "C" int hdgnn_hunk_clusters(int B, int n, const float* probs, const int32_t* nh, float threshold, int32_t* groups,
                                    int32_t* ngroups, void* work, void* stream) {
-    if (B < 1 || n < 2 || n > HDGNN_MAX_N || !probs || !groups || threshold != threshold) return HDGNN_E_INVALID;
-    if (((uintptr_t)probs & 3) || ((uintptr_t)nh & 3) || ((uintptr_t)groups & 3) || ((uintptr_t)ngroups & 3) || ((uintptr_t)work & 3))
-        return HDGNN_E_INVALID;
+    const Call c{"hdgnn_hunk_clusters"};
+    if (int rc = c.sizes("B", B, "n", n)) return rc;
+    if (threshold != threshold) return c.invalid("threshold is NaN");
     const bool in_smem = hc_table_in_smem(n);
-    if (!in_smem && !work) return HDGNN_E_INVALID;
+    if (int rc = c.pointers({{"probs", probs, 4}, {"nh", nh, 4, false}, {"groups", groups, 4}, {"ngroups", ngroups, 4, false},
+                             {"work", work, 4, !in_smem}}))
+        return rc;
+    Device d; if (int rc = c.device(&d)) return rc;
     const size_t smem = hc_rows_bytes(n) + (in_smem ? 2 * hc_table_words(n) * 4 : 0);
-    // the opt-in is set to the largest launch there can be, so concurrent callers never lower it under each other; it is not a
-    // stream operation, so it is allowed while a graph is captured
-    if (smem > 48 * 1024 &&
-        cudaFuncSetAttribute(hunk_clusters_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)HC_SMEM_MAX) != cudaSuccess)
-        return HDGNN_E_CUDA;
+    if (int rc = smem > 48 * 1024 ? c.raise_smem(hunk_clusters_kernel, d) : HDGNN_OK) return rc;
     // one CTA per commit; the workspace form walks the commits with one slice (S and O) per CTA
     const int grid = in_smem ? B : (B < HC_WORK_SLICES ? B : HC_WORK_SLICES);
     hunk_clusters_kernel<<<grid, hc_threads(n), smem, (cudaStream_t)stream>>>(B, n, probs, nh, threshold, groups, ngroups,
                                                                              in_smem ? nullptr : (float*)work);
-    return cudaGetLastError() == cudaSuccess ? HDGNN_OK : HDGNN_E_CUDA;
+    return c.launched();
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -661,14 +647,14 @@ __global__ void __launch_bounds__(256) fma_peak_kernel(int iters, float seed, fl
 }  // namespace hdgnn
 
 extern "C" int hdgnn_measure_fp32_peak(int packed, float* tflops_out) {
-    if (!tflops_out) return HDGNN_E_INVALID;
-    int dev = 0, nsm = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return HDGNN_E_CUDA;
+    const Call c{"hdgnn_measure_fp32_peak"};
+    if (int rc = c.pointers({{"tflops_out", tflops_out, 4}})) return rc;
+    Device d; if (int rc = c.device(&d)) return rc;
     float* sink = nullptr;
     if (cudaMalloc(&sink, 16) != cudaSuccess) return HDGNN_E_NOMEM;
     cudaEvent_t e0, e1;
     cudaEventCreate(&e0); cudaEventCreate(&e1);
-    const int iters = 20000, grid = nsm * 8, block = 256;
+    const int iters = 20000, grid = d.sms * 8, block = 256;
     float best = 0.f;
     for (int rep = 0; rep < 5; ++rep) {
         cudaEventRecord(e0);

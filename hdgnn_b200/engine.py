@@ -95,17 +95,51 @@ class DeviceBatch:
 
 def pack_label_bits_device(grid: torch.Tensor) -> torch.Tensor:
     """(N,n,pitch) u8 CUDA byte grid (pitch = label_pitch(n)) -> (N,n,bit_words(n)) int32 bitmap (hdgnn_pack_label_bits)."""
-    if not grid.is_cuda:
-        raise RuntimeError("pack_label_bits_device needs a CUDA tensor; pack_label_bits is the host form")
+    if grid.dim() != 3:
+        raise ValueError(f"pack_label_bits_device needs a (N, n, pitch) byte grid, got {tuple(grid.shape)}")
     N, n, pitch = grid.shape
     bits = torch.empty(N, n, bit_words(n), dtype=torch.int32, device=grid.device)
-    st = C.c_void_p(torch.cuda.current_stream(grid.device).cuda_stream)
-    check(lib.hdgnn_pack_label_bits(N, n, C.c_void_p(grid.data_ptr()), pitch, C.c_void_p(bits.data_ptr()), st))
+    _launch("pack_label_bits_device", lib.hdgnn_pack_label_bits, N, n, (grid.contiguous(), U8), pitch, bits)
     return bits
 
 
 def _p(t: Optional[torch.Tensor]):
     return None if t is None else C.c_void_p(t.data_ptr())
+
+
+F32, I32, U8, BITMAP = (torch.float32,), (torch.int32,), (torch.uint8,), (torch.int32, torch.uint32)
+
+
+def _launch(name: str, fn, *args):
+    """Call the stateless libhdgnn entry point `fn` on `args` and the stream.  Tensors are passed by pointer; an input is given
+    as (tensor or None, allowed dtypes).  Every tensor must be a CUDA tensor (RuntimeError), all of them on one device and of
+    their dtypes (ValueError).  The call runs with that device current, on its current stream; a refusal raises HdgnnError
+    with the library's message."""
+    want = [a for a in args if isinstance(a, tuple)]
+    args = [a[0] if isinstance(a, tuple) else a for a in args]
+    tensors = [t for t in args if isinstance(t, torch.Tensor)]
+    if not all(t.is_cuda for t in tensors):
+        raise RuntimeError(f"{name} needs CUDA tensors; there is no CPU fallback")
+    devices = {t.device for t in tensors}
+    if len(devices) > 1:
+        raise ValueError(f"{name} needs all tensors on one device, got {sorted(map(str, devices))}")
+    for t, dtypes in want:
+        if t is not None and t.dtype not in dtypes:
+            raise ValueError(f"{name} needs {' or '.join(map(str, dtypes))}, got {t.dtype}")
+    dev = tensors[0].device
+    with torch.cuda.device(dev):
+        check(fn(*[_p(a) if isinstance(a, torch.Tensor) else a for a in args], C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
+
+
+def _shape(name: str, arg: str, t: Optional[torch.Tensor], *shape):
+    """ValueError unless t (None passes) has `shape`; an extent None matches any."""
+    if t is not None and (t.dim() != len(shape) or any(s is not None and s != e for s, e in zip(shape, t.shape))):
+        want = ", ".join("*" if s is None else str(s) for s in shape)
+        raise ValueError(f"{name} needs {arg} of shape ({want}), got {tuple(t.shape)}")
+
+
+def _f32(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
+    return None if t is None else t.contiguous().float()
 
 
 class Engine:
@@ -364,19 +398,17 @@ def normalize_propagate(adj: torch.Tensor, H: torch.Tensor, W: Optional[torch.Te
     """act(A_hat (H W) + b) with the reference's normalize_adj (model.py:360-367).  adj (B,N,N|pitch) uint8 cuda, or a
     (B,N,bit_words(N)) int32 / uint32 label bitmap (the same operator, P_LABEL_BITS is set here), H (B,N,d_in) float32
     cuda.  Returns (out (B,N,d_out), dinv (B,N))."""
+    name = "normalize_propagate"
     a, pitch, flags = _adjacency(adj, flags)
-    if not (adj.is_cuda and H.is_cuda):
-        raise RuntimeError("normalize_propagate needs CUDA tensors; there is no CPU fallback")
     B, N = a.shape[:2]
-    H = H.contiguous().float()
+    _shape(name, "H", H, B, N, None)
     d_in = H.shape[2]
+    _shape(name, "W", W, d_in, None)
     d_out = d_in if W is None else W.shape[1]
+    _shape(name, "bias", bias, d_out)
     out = torch.empty(B, N, d_out, dtype=torch.float32, device=a.device)
     dinv = torch.empty(B, N, dtype=torch.float32, device=a.device)
-    st = C.c_void_p(torch.cuda.current_stream(a.device).cuda_stream)
-    check(lib.hdgnn_normalize_propagate(B, N, _p(a), pitch, _p(H), d_in, _p(None if W is None else W.contiguous().float()),
-                                        _p(None if bias is None else bias.contiguous().float()), d_out, eps, flags,
-                                        _p(out), _p(dinv), st))
+    _launch(name, lib.hdgnn_normalize_propagate, B, N, a, pitch, _f32(H), d_in, _f32(W), _f32(bias), d_out, eps, flags, out, dinv)
     return out, dinv
 
 
@@ -385,14 +417,12 @@ def map_conv(adj: torch.Tensor, x: torch.Tensor, theta: torch.Tensor, lam_max: f
     """map_conv of model.py:394-403 (k = 2, Ds = 1); adj as for normalize_propagate.  Returns (loss scalar tensor,
     per-commit (B,))."""
     a, pitch, flags = _adjacency(adj, flags)
-    if not (adj.is_cuda and x.is_cuda):
-        raise RuntimeError("map_conv needs CUDA tensors; there is no CPU fallback")
     B, N = a.shape[:2]
+    _shape("map_conv", "x", x, B, N)
+    _shape("map_conv", "theta", theta.reshape(-1), 2)
     per = torch.empty(B, dtype=torch.float32, device=a.device)
     loss = torch.empty(1, dtype=torch.float32, device=a.device)
-    st = C.c_void_p(torch.cuda.current_stream(a.device).cuda_stream)
-    check(lib.hdgnn_map_conv(B, N, _p(a), pitch, _p(x.contiguous().float()), _p(theta.reshape(-1).contiguous().float()),
-                             lam_max, eps, flags, _p(per), _p(loss), st))
+    _launch("map_conv", lib.hdgnn_map_conv, B, N, a, pitch, _f32(x), _f32(theta.reshape(-1)), lam_max, eps, flags, per, loss)
     return loss, per
 
 
@@ -401,20 +431,20 @@ def normalize_propagate_backward(adj: torch.Tensor, H: torch.Tensor, dOut: torch
     """Backward of normalize_propagate w.r.t. H, W and the bias (the adjacency carries no gradient: model.py:337 takes its
     argmax); adj as for normalize_propagate.  `out` = the forward's output, needed with P_RELU.  Returns (dH (B,N,d_in),
     dW (d_in,d_out) or None, dbias (d_out))."""
+    name = "normalize_propagate_backward"
     a, pitch, flags = _adjacency(adj, flags)
-    if not (adj.is_cuda and H.is_cuda and dOut.is_cuda):
-        raise RuntimeError("normalize_propagate_backward needs CUDA tensors; there is no CPU fallback")
     B, N = a.shape[:2]
-    H = H.contiguous().float(); dOut = dOut.contiguous().float()
+    _shape(name, "H", H, B, N, None)
+    _shape(name, "dOut", dOut, B, N, None)
     d_in, d_out = H.shape[2], dOut.shape[2]
+    _shape(name, "W", W, d_in, d_out)
+    _shape(name, "out", out, B, N, d_out)
     dH = torch.empty(B, N, d_in, dtype=torch.float32, device=a.device)
     dW = torch.empty(d_in, d_out, dtype=torch.float32, device=a.device) if W is not None else None
     db = torch.empty(d_out, dtype=torch.float32, device=a.device)
     work = torch.empty(lib.hdgnn_propagate_backward_work(B, N, d_in, d_out), dtype=torch.float32, device=a.device)
-    st = C.c_void_p(torch.cuda.current_stream(a.device).cuda_stream)
-    check(lib.hdgnn_normalize_propagate_backward(B, N, _p(a), pitch, _p(H), d_in, _p(None if W is None else W.contiguous().float()), d_out,
-                                                 eps, flags, _p(None if out is None else out.contiguous().float()), _p(dOut),
-                                                 _p(dH), _p(dW), _p(db), _p(work), st))
+    _launch(name, lib.hdgnn_normalize_propagate_backward, B, N, a, pitch, _f32(H), d_in, _f32(W), d_out, eps, flags, _f32(out),
+            _f32(dOut), dH, dW, db, work)
     return dH, dW, db
 
 
@@ -423,15 +453,14 @@ def map_conv_backward(adj: torch.Tensor, x: torch.Tensor, theta: torch.Tensor, l
     """Gradient of map_conv's loss w.r.t. x (B,N) and theta (2) (model.py:394-403; no gradient to the adjacency); adj as
     for normalize_propagate."""
     a, pitch, flags = _adjacency(adj, flags)
-    if not (adj.is_cuda and x.is_cuda):
-        raise RuntimeError("map_conv_backward needs CUDA tensors; there is no CPU fallback")
     B, N = a.shape[:2]
+    _shape("map_conv_backward", "x", x, B, N)
+    _shape("map_conv_backward", "theta", theta.reshape(-1), 2)
     dx = torch.empty(B, N, dtype=torch.float32, device=a.device)
     dth = torch.empty(2, dtype=torch.float32, device=a.device)
     work = torch.empty(2 * B, dtype=torch.float32, device=a.device)
-    st = C.c_void_p(torch.cuda.current_stream(a.device).cuda_stream)
-    check(lib.hdgnn_map_conv_backward(B, N, _p(a), pitch, _p(x.contiguous().float()), _p(theta.reshape(-1).contiguous().float()),
-                                      lam_max, eps, flags, gscale, _p(dx), _p(dth), _p(work), st))
+    _launch("map_conv_backward", lib.hdgnn_map_conv_backward, B, N, a, pitch, _f32(x), _f32(theta.reshape(-1)), lam_max, eps, flags,
+            gscale, dx, dth, work)
     return dx, dth
 
 
@@ -440,20 +469,17 @@ def compact_from_raw_device(raw: torch.Tensor, want_diag: bool = True):
     """utils2.py:29-47 + the int() label indexing of :82,:105 on the device.  raw: (N,n,n) float64 / float32 CUDA tensor
     as stored in CAdjs / CHunkAdjs.  Returns (grid u8 (N,n,pitch), diag f32 (N,n) or None); raises IndexError where
     the reference would (an off-diagonal entry that does not truncate to -2, -1, 0 or 1)."""
-    if not raw.is_cuda:
-        raise RuntimeError("compact_from_raw_device needs a CUDA tensor; there is no CPU fallback")
+    if raw.dim() != 3 or raw.shape[1] != raw.shape[2]:
+        raise ValueError(f"compact_from_raw_device needs raw of shape (N, n, n), got {tuple(raw.shape)}")
+    N, n, _ = raw.shape
     if raw.dtype not in (torch.float64, torch.float32):
         raw = raw.to(torch.float64)
-    raw = raw.contiguous()
-    N, n, n2 = raw.shape
-    assert n == n2
     pitch = label_pitch(n)
     grid = torch.empty(N, n, pitch, dtype=torch.uint8, device=raw.device)
     diag = torch.empty(N, n, dtype=torch.float32, device=raw.device) if want_diag else None
     err = torch.zeros(1, dtype=torch.int32, device=raw.device)
-    st = C.c_void_p(torch.cuda.current_stream(raw.device).cuda_stream)
-    check(lib.hdgnn_compact_from_raw(N, n, _p(raw), 1 if raw.dtype == torch.float64 else 0, _p(grid), pitch, _p(diag),
-                                     _p(err), st))
+    _launch("compact_from_raw_device", lib.hdgnn_compact_from_raw, N, n, raw.contiguous(), 1 if raw.dtype == torch.float64 else 0,
+            grid, pitch, diag, err)
     if int(err.item()):
         raise IndexError("off-diagonal entries must truncate to 0 or 1 (utils2.py:82,105)")
     return grid, diag
@@ -463,16 +489,12 @@ def eval_counts(probs: torch.Tensor, Y: torch.Tensor, auc: bool = False, auc_fir
     """Evaluation counters of EvaluationFuncs.py on the device.  probs (B,2,Ncr) f32 CUDA, Y (B,Nc,Nc|pitch) u8 CUDA.
     Returns (counts (B,8) int64, auc (B,2) int64 or None), see include/hdgnn.h; feed them to
     EvaluationFuncs.metrics_from_counts."""
-    if not (probs.is_cuda and Y.is_cuda):
-        raise RuntimeError("eval_counts needs CUDA tensors; there is no CPU fallback")
-    probs = probs.contiguous()
-    Y = Y.contiguous()
+    _shape("eval_counts", "Y", Y, None, None, None)
     B, Nc, pitch = Y.shape
-    assert probs.dtype == torch.float32 and probs.shape == (B, 2, Nc * (Nc - 1)) and Y.dtype == torch.uint8
+    _shape("eval_counts", "probs", probs, B, 2, Nc * (Nc - 1))
     counts = torch.empty(B, 8, dtype=torch.int64, device=probs.device)
     a = torch.empty(B, 2, dtype=torch.int64, device=probs.device) if auc else None
-    st = C.c_void_p(torch.cuda.current_stream(probs.device).cuda_stream)
-    check(lib.hdgnn_eval_counts(B, Nc, _p(probs), _p(Y), pitch, _p(counts), _p(a), auc_first, st))
+    _launch("eval_counts", lib.hdgnn_eval_counts, B, Nc, (probs.contiguous(), F32), (Y.contiguous(), U8), pitch, counts, a, auc_first)
     return counts, a
 
 
@@ -480,16 +502,12 @@ def hunk_groups(bits: torch.Tensor):
     """Hunk groups of label bitmaps (hdgnn_hunk_groups): bits (B, n, bit_words(n)) int32 CUDA tensor, e.g. what set_predictions
     receives, or the labels.  Hunks s and t share a group when bit (s,t) or bit (t,s) is set.  Returns (groups (B, n) int32: the
     smallest hunk index of each hunk's group, ngroups (B,) int32)."""
-    if not bits.is_cuda:
-        raise RuntimeError("hunk_groups needs a CUDA tensor; there is no CPU fallback")
-    bits = bits.contiguous()
-    B, n, wp = bits.shape
-    if bits.dtype not in (torch.int32, torch.uint32) or wp != bit_words(n):
-        raise ValueError(f"hunk_groups needs an int32 label bitmap of bit_words({n}) = {bit_words(n)} words per row")
+    if bits.dim() != 3 or bits.shape[2] != bit_words(bits.shape[1]):
+        raise ValueError(f"hunk_groups needs a (B, n, bit_words(n)) label bitmap, got {tuple(bits.shape)}")
+    B, n, _ = bits.shape
     groups = torch.empty(B, n, dtype=torch.int32, device=bits.device)
     ngroups = torch.empty(B, dtype=torch.int32, device=bits.device)
-    st = C.c_void_p(torch.cuda.current_stream(bits.device).cuda_stream)
-    check(lib.hdgnn_hunk_groups(B, n, _p(bits), _p(groups), _p(ngroups), st))
+    _launch("hunk_groups", lib.hdgnn_hunk_groups, B, n, (bits.contiguous(), BITMAP), groups, ngroups)
     return groups, ngroups
 
 
@@ -500,23 +518,13 @@ def partition_counts(pred: torch.Tensor, truth: torch.Tensor, nh: Optional[torch
     int64 = {real hunks, pairs joined in both, by pred, by truth, groups of pred, of truth, sum of largest overlaps of the pred
     groups, of the truth groups}; a row of -1 marks a commit with nh outside [0, n] or a real hunk labelled outside [0, n).
     Feed them to EvaluationFuncs.partition_metrics_from_counts."""
-    tensors = (pred, truth) if nh is None else (pred, truth, nh)
-    if not all(t.is_cuda for t in tensors):
-        raise RuntimeError("partition_counts needs CUDA tensors; there is no CPU fallback")
-    if any(t.device != pred.device for t in tensors):
-        raise ValueError("partition_counts needs all tensors on one device")
-    if any(t.dtype != torch.int32 for t in tensors):
-        raise ValueError("partition_counts needs int32 tensors")
-    if pred.dim() != 2 or truth.shape != pred.shape:
-        raise ValueError(f"partition_counts needs pred and truth of one shape (B, n), got {tuple(pred.shape)} / {tuple(truth.shape)}")
+    _shape("partition_counts", "pred", pred, None, None)
     B, n = pred.shape
-    if nh is not None and nh.shape != (B,):
-        raise ValueError(f"partition_counts needs nh of shape ({B},), got {tuple(nh.shape)}")
-    pred, truth = pred.contiguous(), truth.contiguous()
-    nh = None if nh is None else nh.contiguous()
+    _shape("partition_counts", "truth", truth, B, n)
+    _shape("partition_counts", "nh", nh, B)
     counts = torch.empty(B, 8, dtype=torch.int64, device=pred.device)
-    st = C.c_void_p(torch.cuda.current_stream(pred.device).cuda_stream)
-    check(lib.hdgnn_partition_counts(B, n, _p(pred), _p(truth), _p(nh), _p(counts), st))
+    _launch("partition_counts", lib.hdgnn_partition_counts, B, n, (pred.contiguous(), I32), (truth.contiguous(), I32),
+            (None if nh is None else nh.contiguous(), I32), counts)
     return counts
 
 
@@ -526,27 +534,16 @@ def hunk_clusters(probs: torch.Tensor, nh: Optional[torch.Tensor] = None, thresh
     hunks of each commit, or None: all n.  Two groups merge while the mean of max(p1(s,t), p1(t,s)) over their hunk pairs is
     > threshold, the closest first.  Returns (groups (B, n) int32: the smallest hunk index of each real hunk's group, s for a
     hunk s >= nh[b]; ngroups (B,) int32), the labelling of hunk_groups; a commit with nh outside [0, n] gets -1 throughout."""
-    tensors = (probs,) if nh is None else (probs, nh)
-    if not all(t.is_cuda for t in tensors):
-        raise RuntimeError("hunk_clusters needs CUDA tensors; there is no CPU fallback")
-    if any(t.device != probs.device for t in tensors):
-        raise ValueError("hunk_clusters needs all tensors on one device")
-    if probs.dtype != torch.float32 or (nh is not None and nh.dtype != torch.int32):
-        raise ValueError("hunk_clusters needs float32 probs and int32 nh")
-    if probs.dim() != 3 or probs.shape[1] != 2:
-        raise ValueError(f"hunk_clusters needs probs of shape (B, 2, n(n-1)), got {tuple(probs.shape)}")
+    _shape("hunk_clusters", "probs", probs, None, 2, None)
     B, _, ncr = probs.shape
     n = (1 + int(round((1 + 4 * ncr) ** 0.5))) // 2
     if n < 2 or n * (n - 1) != ncr:
         raise ValueError(f"hunk_clusters needs n(n-1) pairs per channel, got {ncr}")
-    if nh is not None and nh.shape != (B,):
-        raise ValueError(f"hunk_clusters needs nh of shape ({B},), got {tuple(nh.shape)}")
-    probs = probs.contiguous()
-    nh = None if nh is None else nh.contiguous()
+    _shape("hunk_clusters", "nh", nh, B)
     groups = torch.empty(B, n, dtype=torch.int32, device=probs.device)
     ngroups = torch.empty(B, dtype=torch.int32, device=probs.device)
     nwork = lib.hdgnn_hunk_clusters_work(B, n)
     work = torch.empty(nwork, dtype=torch.uint8, device=probs.device) if nwork else None
-    st = C.c_void_p(torch.cuda.current_stream(probs.device).cuda_stream)
-    check(lib.hdgnn_hunk_clusters(B, n, _p(probs), _p(nh), float(threshold), _p(groups), _p(ngroups), _p(work), st))
+    _launch("hunk_clusters", lib.hdgnn_hunk_clusters, B, n, (probs.contiguous(), F32), (None if nh is None else nh.contiguous(), I32),
+            float(threshold), groups, ngroups, work)
     return groups, ngroups

@@ -14,7 +14,10 @@
  *  - every call is asynchronous on the caller's `stream` (a cudaStream_t passed as void*),
  *    no hidden synchronisation, CUDA-graph capturable; the *_host entry points enqueue
  *    their own copies on that stream and are asynchronous as well;
- *  - return value: 0 = ok, <0 = error (HDGNN_E_*); text via hdgnn_last_error();
+ *  - every pointer is aligned to its element type (8 bytes for int64 / double, 4 for float / int32); label bitmaps, and the
+ *    adj / Y byte grids of the handle's entry points and of the legacy operator, to 16 bytes; an optional pointer may be NULL;
+ *  - return value: 0 = ok, <0 = error (HDGNN_E_*); text via hdgnn_last_error(), which names the entry point and the
+ *    argument of a refused stateless call;
  *  - a handle belongs to one device and one host thread at a time;
  *  - the caller owns params / grads / Adam moments (one flat fp32 blob each, laid out in
  *    the TF variable-creation order of the variant's build_model, see hdgnn_param_layout);
@@ -94,7 +97,8 @@ int hdgnn_param_offset(int variant, const char* name);
 
 int hdgnn_create(const hdgnn_config_t* cfg, hdgnn_handle_t* out);
 int hdgnn_destroy(hdgnn_handle_t h);
-const char* hdgnn_last_error(hdgnn_handle_t h);       /* h may be NULL: last create() error */
+/* h may be NULL: the message of the calling thread's last failed call without a handle (hdgnn_create or a stateless entry point) */
+const char* hdgnn_last_error(hdgnn_handle_t h);
 int hdgnn_label_pitch(int n);                         /* required row pitch for an n x n byte grid */
 int hdgnn_bit_words(int n);                           /* uint32 words per row of an n x n label bitmap (16-byte rows) */
 
@@ -216,7 +220,7 @@ int hdgnn_infer_host(hdgnn_handle_t h, int B,
  *   - a byte grid: uint8 (B, N, adj_pitch), A_ij != 0 is an edge, adj_pitch >= N and a multiple of 16; or
  *   - with HDGNN_P_LABEL_BITS, a label bitmap in the layout of HDGNN_F_LABEL_BITS: (B, N, hdgnn_bit_words(N)) uint32,
  *     bit k of word w of row i = A_i,32w+k, adj_pitch = 4 * hdgnn_bit_words(N) exactly (what hdgnn_pack_label_bits writes).
- * Either way adj is 16-byte aligned, and the diagonal (and for bitmaps the padding bits, columns >= N) is ignored.
+ * Either way the diagonal (and for bitmaps the padding bits, columns >= N) is ignored.
  * The per-commit state (N * adj_pitch bytes of adjacency + two bitmaps + N * d_out floats) must fit one SM's shared
  * memory, else HDGNN_E_UNSUPPORTED: byte grids up to N ~ 380 at d_out = 20, label bitmaps up to N = HDGNN_MAX_N = 512
  * (a 32 KB tile).  With bitmaps the persistent tcgen05 kernel is the default up to N = 240 at d_in = 20 (byte grids: N = 208). */
@@ -263,13 +267,13 @@ int hdgnn_map_conv_backward(int B, int N, const uint8_t* adj, int adj_pitch, con
 int hdgnn_compact_from_raw(int N, int n, const void* raw, int raw_is_f64, uint8_t* grid, int pitch, float* diag,
                            int32_t* err, void* stream);
 
-/* Byte grids -> label bitmaps (the format of HDGNN_F_LABEL_BITS) on the device: grid (N,n,pitch) u8 as written by
- * hdgnn_compact_from_raw, bits (N,n,hdgnn_bit_words(n)) uint32; diagonal and padding bits come out zero. */
+/* Byte grids -> label bitmaps (the format of HDGNN_F_LABEL_BITS) on the device: grid (N,n,pitch) u8, 16-byte aligned, as
+ * written by hdgnn_compact_from_raw, bits (N,n,hdgnn_bit_words(n)) uint32; diagonal and padding bits come out zero. */
 int hdgnn_pack_label_bits(int N, int n, const uint8_t* grid, int pitch, uint32_t* bits, void* stream);
 
 /* Weakly connected components of per-commit hunk graphs given as label bitmaps (HDGNN_F_LABEL_BITS layout, e.g. the output of
  * hdgnn_set_predictions, or the labels Y): hunks s and t are joined when bit (s,t) OR bit (t,s) is set; diagonal and padding
- * bits are ignored.  bits (B, n, hdgnn_bit_words(n)) uint32, 16-byte aligned; groups (B, n) int32 receives, for every hunk, the
+ * bits are ignored.  bits (B, n, hdgnn_bit_words(n)) uint32; groups (B, n) int32 receives, for every hunk, the
  * SMALLEST hunk index of its component (a canonical labelling: two partitions are equal iff the arrays are equal); ngroups (B)
  * int32 or NULL receives the number of components.  2 <= n <= HDGNN_MAX_N.  Integer-exact, deterministic.  Stateless. */
 int hdgnn_hunk_groups(int B, int n, const uint32_t* bits, int32_t* groups, int32_t* ngroups, void* stream);
@@ -281,7 +285,7 @@ int hdgnn_hunk_groups(int B, int n, const uint32_t* bits, int32_t* groups, int32
  *   {m, pairs joined in both, pairs joined by pred, pairs joined by truth, groups of pred, groups of truth,
  *    sum over pred groups of the largest overlap with a truth group, sum over truth groups of the largest overlap with a pred group}
  * (pairs = unordered pairs {s,t}, s < t < m).  A commit with nh[b] outside [0, n] or a real hunk labelled outside [0, n) gets
- * the row all -1.  pred, truth, nh 4-byte and counts 8-byte aligned.  2 <= n <= HDGNN_MAX_N.  Integer-exact, deterministic,
+ * the row all -1.  2 <= n <= HDGNN_MAX_N.  Integer-exact, deterministic,
  * stateless, asynchronous on `stream`. */
 int hdgnn_partition_counts(int B, int n, const int32_t* pred, const int32_t* truth, const int32_t* nh,
                            int64_t* counts, void* stream);
@@ -298,7 +302,7 @@ int hdgnn_partition_counts(int B, int n, const int32_t* pred, const int32_t* tru
  * labelling of hdgnn_hunk_groups, which hdgnn_partition_counts takes); ngroups (B) int32 or NULL the number of distinct values.
  * A commit with nh[b] outside [0, n] gets groups all -1 and ngroups -1.  `work`: device scratch of
  * hdgnn_hunk_clusters_work(B, n) bytes (0 for n <= 169: the commit's tables live in shared memory; else min(B, 296)
- * pairs of tables of n (n|1) 4-byte words), may be NULL when that is 0.  probs, nh, groups, ngroups, work 4-byte aligned; 2 <= n <= HDGNN_MAX_N;
+ * pairs of tables of n (n|1) 4-byte words), may be NULL when that is 0.  2 <= n <= HDGNN_MAX_N;
  * threshold not NaN.  Deterministic (the merge sequence fixes every rounding), stateless, asynchronous on `stream`. */
 size_t hdgnn_hunk_clusters_work(int B, int n);
 int hdgnn_hunk_clusters(int B, int n, const float* probs, const int32_t* nh, float threshold,

@@ -1,7 +1,6 @@
 """The legacy operator (model.py:335-403) fed label bitmaps (HDGNN_P_LABEL_BITS) instead of byte grids: normalize_propagate,
 map_conv and both backwards.  Where both formats run the same kernel the results are bitwise equal to the byte-grid call;
 where the kernel selection may differ, and beyond the byte grid's size limit, they match the fp64 oracle."""
-import ctypes as C
 import os
 
 import numpy as np
@@ -296,33 +295,6 @@ def test_bits_match_reference_model_py_golden():
 
 
 # ---- argument checks -------------------------------------------------------------------------------------------------------
-def _c_calls(N, adj_ptr, pitch, flags):
-    """The four legacy entry points with fake device pointers: each must refuse the adjacency before any CUDA call."""
-    from hdgnn_b200._lib import lib
-    f = C.c_void_p(1 << 20)
-    return {
-        "normalize_propagate": lib.hdgnn_normalize_propagate(2, N, adj_ptr, pitch, f, 20, None, None, 20, 1e-3, flags, f, None, None),
-        "map_conv": lib.hdgnn_map_conv(2, N, adj_ptr, pitch, f, f, 1.5, 1e-3, flags, f, None, None),
-        "normalize_propagate_backward": lib.hdgnn_normalize_propagate_backward(2, N, adj_ptr, pitch, f, 20, None, 20, 1e-3, flags,
-                                                                              None, f, f, None, None, f, None),
-        "map_conv_backward": lib.hdgnn_map_conv_backward(2, N, adj_ptr, pitch, f, f, 1.5, 1e-3, flags, 1.0, f, None, None, None),
-    }
-
-
-@pytest.mark.parametrize("N", [9, 200, 512])
-def test_bitmap_pitch_and_alignment_are_checked_before_launch(N):
-    from hdgnn_b200 import _lib
-    from hdgnn_b200.engine import P_LABEL_BITS, bit_words, label_pitch
-    aligned, pitch = C.c_void_p(1 << 24), 4 * bit_words(N)
-    wrong = {label_pitch(N), pitch + 16, pitch - 16, 4 * ((N + 31) // 32)} - {pitch, 0}     # byte pitch, unpadded rows, ...
-    bad = [(aligned, p) for p in sorted(wrong)] + [(C.c_void_p((1 << 24) + 4), pitch)]      # ... and a misaligned base
-    for adj, p in bad:
-        for name, rc in _c_calls(N, adj, p, P_LABEL_BITS).items():
-            assert rc == _lib.E_INVALID, (name, p, adj.value)
-    for name, rc in _c_calls(_lib.MAX_N + 1, aligned, 4 * 16, P_LABEL_BITS).items():
-        assert rc == _lib.E_INVALID, name
-
-
 def test_bitmap_arguments_are_checked_in_python():
     from hdgnn_b200.engine import (P_LABEL_BITS, bit_words, map_conv, map_conv_backward, normalize_propagate,
                                    normalize_propagate_backward)

@@ -1,45 +1,13 @@
-"""CPU checks of the average-linkage hunk clusters: hdgnn_hunk_clusters rejects bad arguments before any CUDA call, and the NumPy
-restatement of its specification (oracle/hunk_clusters.py) equals scipy's average linkage cut at 1 - threshold and keeps apart
-two groups that one confident false-positive pair chains together under connected components."""
-import ctypes as C
-
+"""CPU checks of the average-linkage hunk clusters: the NumPy restatement of their specification (oracle/hunk_clusters.py)
+equals scipy's average linkage cut at 1 - threshold and keeps apart two groups that one confident false-positive pair chains
+together under connected components."""
 import numpy as np
-import torch
 from scipy.cluster.hierarchy import fcluster, linkage
 from scipy.sparse import csr_matrix
 from scipy.sparse.csgraph import connected_components
 from scipy.spatial.distance import squareform
 
 from oracle.hunk_clusters import hunk_clusters, hunk_clusters_one, pair_index
-
-
-def test_hunk_clusters_validates_arguments_without_a_gpu():
-    from hdgnn_b200 import _lib
-    f, work_of = _lib.lib.hdgnn_hunk_clusters, _lib.lib.hdgnn_hunk_clusters_work
-    probs, nh, groups, ngroups, work = (C.c_void_p(a) for a in (0x10000, 0x20000, 0x30000, 0x40000, 0x50000))  # never read
-    nan = float("nan")
-    bad = [
-        (1, 1, probs, nh, 0.5, groups, ngroups, work),                   # n below 2
-        (1, 513, probs, nh, 0.5, groups, ngroups, work),                 # n above HDGNN_MAX_N
-        (0, 74, probs, nh, 0.5, groups, ngroups, work),                  # B below 1
-        (1, 74, None, nh, 0.5, groups, ngroups, work),                   # null probs
-        (1, 74, probs, nh, 0.5, None, ngroups, work),                    # null groups
-        (1, 74, probs, nh, nan, groups, ngroups, work),                  # NaN threshold
-        (1, 74, C.c_void_p(0x10002), nh, 0.5, groups, ngroups, work),    # probs not 4-byte aligned
-        (1, 74, probs, C.c_void_p(0x20001), 0.5, groups, ngroups, work), # nh not 4-byte aligned
-        (1, 74, probs, nh, 0.5, C.c_void_p(0x30002), ngroups, work),     # groups not 4-byte aligned
-        (1, 74, probs, nh, 0.5, groups, C.c_void_p(0x40003), work),      # ngroups not 4-byte aligned
-        (1, 300, probs, nh, 0.5, groups, ngroups, C.c_void_p(0x50002)),  # work not 4-byte aligned
-        (1, 300, probs, nh, 0.5, groups, ngroups, None),                 # the table needs the workspace, and there is none
-    ]
-    for args in bad:
-        assert f(*args, None) == _lib.E_INVALID, args
-    # the two tables of a commit live in shared memory up to n = 169, above that in one slice of the workspace per CTA
-    assert work_of(100, 74) == 0 and work_of(100, 169) == 0
-    assert work_of(100, 170) == 100 * 2 * 170 * 171 * 4 and work_of(4096, 512) == 296 * 2 * 512 * 513 * 4
-    assert work_of(0, 300) == 0 and work_of(1, 513) == 0 and work_of(1, 1) == 0
-    if not torch.cuda.is_available():                                    # valid arguments reach the device and fail loudly there
-        assert f(1, 74, probs, None, 0.5, groups, None, None, None) == _lib.E_CUDA
 
 
 def _probs_of(P1: np.ndarray) -> np.ndarray:
