@@ -65,6 +65,8 @@ def _load():
         "hdgnn_partition_counts": ([i32, i32, vp, vp, vp, vp, vp], i32),
         "hdgnn_hunk_clusters_work": ([i32, i32], C.c_size_t),
         "hdgnn_hunk_clusters": ([i32, i32, vp, vp, f32, vp, vp, vp, vp], i32),
+        "hdgnn_hunk_linkage": ([i32, i32, vp, vp, vp, vp, vp, vp, vp], i32),
+        "hdgnn_linkage_cut": ([i32, i32, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp], i32),
         "hdgnn_workspace": ([vp, C.c_char_p, C.POINTER(vp), C.POINTER(C.c_size_t)], i32),
         "hdgnn_workspace_copy": ([vp, C.c_char_p, vp, C.c_size_t, vp], i32),
         "hdgnn_profile": ([vp, i32], i32),

@@ -12,7 +12,9 @@
 //    group counts and largest overlaps, from which EvaluationFuncs.partition_metrics_from_counts derives pair precision /
 //    recall / F1, the (adjusted) Rand index and purity.
 //  * hunk_clusters_kernel     -- hunk groups formed from the relation probabilities instead of the arg-max bitmap: average
-//    linkage over each commit's real hunks, merging two groups only while their mean relation probability clears a threshold.
+//    linkage over each commit's real hunks, merging two groups only while their mean relation probability clears a threshold;
+//    its LINK instantiation records the whole merge sequence instead (hdgnn_hunk_linkage).
+//  * linkage_cut_kernel       -- hunk groups from such a record at many thresholds, or at a group count, in one pass.
 //
 // Everything here except hunk_clusters_kernel is integer counting => bit-exact and order independent (integer atomics).  The
 // clustering is fp32, but its merge sequence fixes every rounding, so it is deterministic and reproducible on the host.
@@ -341,6 +343,9 @@ __global__ void __launch_bounds__(32 * PC_WARPS_MAX) partition_counts_kernel(int
 // row's owner thread writes its own row), so every thread reads the old sizes in B.
 // The tables live in shared memory when they fit beside the row arrays (n <= 169), else in a slice of `work`; the same code
 // reaches both through generic pointers.
+// LINK (hdgnn_hunk_linkage): the same merges without a threshold -- A stops only when the arg-max key is 0 -- and thread 0
+// records each one, (a, c) and the winning key's mean, after the A barrier; the trailing parameters are used only then, so the
+// threshold form keeps its code.  Rows past the last merge are filled with (-1, -1) and NaN.
 constexpr int HC_T_MAX = 512;
 constexpr int HC_WARPS = HC_T_MAX / 32;
 constexpr int HC_WORK_SLICES = 296;                        // CTAs of the workspace form: two per SM of a B200
@@ -392,10 +397,12 @@ __device__ __forceinline__ unsigned long long hc_rescan(const uint32_t* O, int S
     return hc_key(h, x, t);
 }
 
+template <bool LINK>
 __global__ void __launch_bounds__(HC_T_MAX) hunk_clusters_kernel(int B, int n, const float* __restrict__ probs,
                                                                  const int32_t* __restrict__ nh, float threshold,
                                                                  int32_t* __restrict__ groups, int32_t* __restrict__ ngroups,
-                                                                 float* work) {
+                                                                 float* work, int32_t* __restrict__ rec_pairs,
+                                                                 float* __restrict__ rec_heights, int32_t* __restrict__ rec_count) {
     extern __shared__ __align__(16) unsigned char hc_smem[];
     const int T = blockDim.x, NW = T >> 5, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     unsigned long long* key = reinterpret_cast<unsigned long long*>(hc_smem);
@@ -413,9 +420,16 @@ __global__ void __launch_bounds__(HC_T_MAX) hunk_clusters_kernel(int B, int n, c
     for (int b = blockIdx.x; b < B; b += gridDim.x) {
         const int m = nh ? __ldg(nh + b) : n;
         int32_t* g = groups + (size_t)b * n;
+        int32_t* rp = rec_pairs + (size_t)b * (n - 1) * 2;
+        float* rh = rec_heights + (size_t)b * (n - 1);
         if (m < 0 || m > n) {
-            for (int s = tid; s < n; s += T) g[s] = -1;
-            if (tid == 0 && ngroups) ngroups[b] = -1;
+            if constexpr (LINK) {
+                for (int i = tid; i < n - 1; i += T) { rp[2 * i] = -1; rp[2 * i + 1] = -1; rh[i] = __int_as_float(0x7fffffff); }
+                if (tid == 0) rec_count[b] = -1;
+            } else {
+                for (int s = tid; s < n; s += T) g[s] = -1;
+                if (tid == 0 && ngroups) ngroups[b] = -1;
+            }
             continue;
         }
         // channel 1 of the real block, row s of p1 (pairs s(n-1) .. s(n-1)+n-2) read along t; the padding pairs are never read
@@ -461,9 +475,16 @@ __global__ void __launch_bounds__(HC_T_MAX) hunk_clusters_kernel(int B, int n, c
             __syncthreads();
             kb = 0ull;
             for (int w = 0; w < NW; ++w) kb = hc_max(kb, slot[w]);
-            if (kb == 0ull || !(hc_key_mean(kb) > threshold)) break;
+            if constexpr (LINK) {
+                if (kb == 0ull) break;
+            } else {
+                if (kb == 0ull || !(hc_key_mean(kb) > threshold)) break;
+            }
             // B: Lance-Williams update of row / column a, compare-and-update or rescan listing of every other row
             const int a = hc_key_lo(kb), c = hc_key_hi(kb);
+            if constexpr (LINK) {
+                if (tid == 0) { rp[2 * merges] = a; rp[2 * merges + 1] = c; rh[merges] = hc_key_mean(kb); }
+            }
             const int sn = size[a] + size[c];
             int* L = cnt + (merges & 1);
             if (tid == 0) cnt[(merges & 1) ^ 1] = 0;       // the other counter was last read before this merge's A barrier
@@ -509,9 +530,83 @@ __global__ void __launch_bounds__(HC_T_MAX) hunk_clusters_kernel(int B, int n, c
             pa = a; pc = c; psz = sn;
             ++merges;
         }
-        for (int s = tid; s < n; s += T) g[s] = s < m ? lab[s] : s;
-        if (tid == 0 && ngroups) ngroups[b] = n - merges;
+        if constexpr (LINK) {
+            for (int i = merges + tid; i < n - 1; i += T) { rp[2 * i] = -1; rp[2 * i + 1] = -1; rh[i] = __int_as_float(0x7fffffff); }
+            if (tid == 0) rec_count[b] = merges;
+        } else {
+            for (int s = tid; s < n; s += T) g[s] = s < m ? lab[s] : s;
+            if (tid == 0 && ngroups) ngroups[b] = n - merges;
+        }
         __syncthreads();                                    // before the next commit reuses the arrays and the table
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Cuts of recorded merge sequences (hdgnn_hunk_linkage) at K thresholds, or at one group count per commit.  One CTA per commit.
+// The record is checked once and turned into parent[c] = a and step[c] = i (the row that absorbed c; LC_LIVE: none).  The
+// checks -- every row 0 <= a < c < m, no c twice, no a absorbed at an earlier row -- make each hunk's chain of absorptions run
+// to ever smaller hunks at ever later rows, so the first hunk of the chain not absorbed before the cut's merge count is the
+// representative (smallest hunk) of the hunk's cluster after those merges, and the walk ends within m steps.  The record may
+// come from a file: a commit that fails a check gets -1 throughout, and nothing is read past its nmerges rows.
+// Then one warp per cut: the threshold cut's merge count is the longest prefix of heights > t (ballot scan), and every real
+// hunk follows its chain while step < count.  Integer work: exact and deterministic.
+constexpr int LC_K_MAX = 64;
+constexpr int LC_WARPS = 8;
+constexpr int LC_LIVE = 0x7fffffff;
+struct LcThresholds { float t[LC_K_MAX]; };                // by value, so a captured graph keeps the caller's thresholds
+
+__global__ void __launch_bounds__(32 * LC_WARPS) linkage_cut_kernel(int B, int n, const int32_t* __restrict__ pairs,
+                                                                    const float* __restrict__ heights,
+                                                                    const int32_t* __restrict__ count,
+                                                                    const int32_t* __restrict__ nh, int K, LcThresholds thr,
+                                                                    const int32_t* __restrict__ target,
+                                                                    int32_t* __restrict__ groups, int32_t* __restrict__ ngroups) {
+    __shared__ int parent[HDGNN_MAX_N], step[HDGNN_MAX_N];
+    const int b = blockIdx.x, T = blockDim.x, tid = threadIdx.x, lane = tid & 31;
+    const int m = nh ? __ldg(nh + b) : n;
+    const int nm = __ldg(count + b);
+    const int32_t* rp = pairs + (size_t)b * (n - 1) * 2;
+    const float* rh = heights + (size_t)b * (n - 1);
+    int bad = m < 0 || m > n || nm < 0 || nm > max(m - 1, 0);
+    if (!bad)
+        for (int s = tid; s < m; s += T) step[s] = LC_LIVE;
+    __syncthreads();
+    if (!bad)
+        for (int i = tid; i < nm; i += T) {
+            const int a = __ldg(rp + 2 * i), c = __ldg(rp + 2 * i + 1);
+            if (!(0 <= a && a < c && c < m)) bad = 1;
+            else if (atomicCAS(&step[c], LC_LIVE, i) != LC_LIVE) bad = 1;      // c absorbed twice
+            else parent[c] = a;
+        }
+    bad = __syncthreads_or(bad);
+    if (!bad)
+        for (int i = tid; i < nm; i += T)
+            if (step[__ldg(rp + 2 * i)] < i) bad = 1;                          // a absorbed before row i
+    bad = __syncthreads_or(bad);
+    for (int k = tid >> 5; k < K; k += T >> 5) {
+        int32_t* g = groups + ((size_t)k * B + b) * n;
+        int c = -1;
+        if (!bad) {
+            if (target) {
+                c = min(nm, max(0, m - max(__ldg(target + b), 1)));
+            } else {
+                const float t = thr.t[k];
+                c = nm;
+                for (int base = 0; base < nm; base += 32) {
+                    const int i = base + lane;
+                    const uint32_t stop = __ballot_sync(0xffffffffu, i < nm && !(__ldg(rh + i) > t));
+                    if (stop) { c = base + __ffs(stop) - 1; break; }
+                }
+            }
+        }
+        for (int s = lane; s < n; s += 32) {
+            int x = s;
+            if (bad) x = -1;
+            else if (s < m)
+                while (step[x] < c) x = parent[x];
+            g[s] = x;
+        }
+        if (lane == 0 && ngroups) ngroups[(size_t)k * B + b] = bad ? -1 : n - c;
     }
 }
 
@@ -586,6 +681,22 @@ extern "C" int hdgnn_partition_counts(int B, int n, const int32_t* pred, const i
     return c.launched();
 }
 
+// One CTA per commit; the workspace form walks the commits with one slice (S and O) per CTA.  Called once the entry point has
+// checked its arguments.
+template <bool LINK>
+static int hc_launch(const Call& c, int B, int n, const float* probs, const int32_t* nh, float threshold, int32_t* groups,
+                     int32_t* ngroups, void* work, int32_t* merges, float* heights, int32_t* nmerges, void* stream) {
+    Device d; if (int rc = c.device(&d)) return rc;
+    const bool in_smem = hc_table_in_smem(n);
+    const size_t smem = hc_rows_bytes(n) + (in_smem ? 2 * hc_table_words(n) * 4 : 0);
+    if (int rc = smem > 48 * 1024 ? c.raise_smem(hunk_clusters_kernel<LINK>, d) : HDGNN_OK) return rc;
+    const int grid = in_smem ? B : (B < HC_WORK_SLICES ? B : HC_WORK_SLICES);
+    hunk_clusters_kernel<LINK><<<grid, hc_threads(n), smem, (cudaStream_t)stream>>>(B, n, probs, nh, threshold, groups, ngroups,
+                                                                                   in_smem ? nullptr : (float*)work, merges,
+                                                                                   heights, nmerges);
+    return c.launched();
+}
+
 extern "C" size_t hdgnn_hunk_clusters_work(int B, int n) {
     if (B < 1 || n < 2 || n > HDGNN_MAX_N || hc_table_in_smem(n)) return 0;
     return (size_t)(B < HC_WORK_SLICES ? B : HC_WORK_SLICES) * 2 * hc_table_words(n) * sizeof(float);
@@ -600,13 +711,38 @@ extern "C" int hdgnn_hunk_clusters(int B, int n, const float* probs, const int32
     if (int rc = c.pointers({{"probs", probs, 4}, {"nh", nh, 4, false}, {"groups", groups, 4}, {"ngroups", ngroups, 4, false},
                              {"work", work, 4, !in_smem}}))
         return rc;
-    Device d; if (int rc = c.device(&d)) return rc;
-    const size_t smem = hc_rows_bytes(n) + (in_smem ? 2 * hc_table_words(n) * 4 : 0);
-    if (int rc = smem > 48 * 1024 ? c.raise_smem(hunk_clusters_kernel, d) : HDGNN_OK) return rc;
-    // one CTA per commit; the workspace form walks the commits with one slice (S and O) per CTA
-    const int grid = in_smem ? B : (B < HC_WORK_SLICES ? B : HC_WORK_SLICES);
-    hunk_clusters_kernel<<<grid, hc_threads(n), smem, (cudaStream_t)stream>>>(B, n, probs, nh, threshold, groups, ngroups,
-                                                                             in_smem ? nullptr : (float*)work);
+    return hc_launch<false>(c, B, n, probs, nh, threshold, groups, ngroups, work, nullptr, nullptr, nullptr, stream);
+}
+
+extern "C" int hdgnn_hunk_linkage(int B, int n, const float* probs, const int32_t* nh, int32_t* merges, float* heights,
+                                  int32_t* nmerges, void* work, void* stream) {
+    const Call c{"hdgnn_hunk_linkage"};
+    if (int rc = c.sizes("B", B, "n", n)) return rc;
+    if (int rc = c.pointers({{"probs", probs, 4}, {"nh", nh, 4, false}, {"merges", merges, 4}, {"heights", heights, 4},
+                             {"nmerges", nmerges, 4}, {"work", work, 4, !hc_table_in_smem(n)}}))
+        return rc;
+    return hc_launch<true>(c, B, n, probs, nh, 0.f, nullptr, nullptr, work, merges, heights, nmerges, stream);
+}
+
+extern "C" int hdgnn_linkage_cut(int B, int n, const int32_t* merges, const float* heights, const int32_t* nmerges,
+                                 const int32_t* nh, int K, const float* thresholds_host, const int32_t* target, int32_t* groups,
+                                 int32_t* ngroups, void* stream) {
+    const Call c{"hdgnn_linkage_cut"};
+    if (int rc = c.sizes("B", B, "n", n)) return rc;
+    if (K < 1 || K > LC_K_MAX) return c.invalid("K outside [1, 64]");
+    if (int rc = c.pointers({{"merges", merges, 4}, {"heights", heights, 4}, {"nmerges", nmerges, 4}, {"nh", nh, 4, false},
+                             {"thresholds_host", thresholds_host, 4, false}, {"target", target, 4, false},
+                             {"groups", groups, 4}, {"ngroups", ngroups, 4, false}}))
+        return rc;
+    if (!thresholds_host == !target) return c.invalid("thresholds_host and target: exactly one must be given");
+    if (target && K != 1) return c.invalid("K must be 1 with target");
+    LcThresholds thr{};
+    for (int k = 0; thresholds_host && k < K; ++k) {
+        if (thresholds_host[k] != thresholds_host[k]) return c.invalid("thresholds_host[" + std::to_string(k) + "] is NaN");
+        thr.t[k] = thresholds_host[k];
+    }
+    linkage_cut_kernel<<<B, 32 * std::min(K, LC_WARPS), 0, (cudaStream_t)stream>>>(B, n, merges, heights, nmerges, nh, K, thr,
+                                                                                    target, groups, ngroups);
     return c.launched();
 }
 

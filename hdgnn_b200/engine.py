@@ -534,12 +534,7 @@ def hunk_clusters(probs: torch.Tensor, nh: Optional[torch.Tensor] = None, thresh
     hunks of each commit, or None: all n.  Two groups merge while the mean of max(p1(s,t), p1(t,s)) over their hunk pairs is
     > threshold, the closest first.  Returns (groups (B, n) int32: the smallest hunk index of each real hunk's group, s for a
     hunk s >= nh[b]; ngroups (B,) int32), the labelling of hunk_groups; a commit with nh outside [0, n] gets -1 throughout."""
-    _shape("hunk_clusters", "probs", probs, None, 2, None)
-    B, _, ncr = probs.shape
-    n = (1 + int(round((1 + 4 * ncr) ** 0.5))) // 2
-    if n < 2 or n * (n - 1) != ncr:
-        raise ValueError(f"hunk_clusters needs n(n-1) pairs per channel, got {ncr}")
-    _shape("hunk_clusters", "nh", nh, B)
+    B, n = _probs_shape("hunk_clusters", probs, nh)
     groups = torch.empty(B, n, dtype=torch.int32, device=probs.device)
     ngroups = torch.empty(B, dtype=torch.int32, device=probs.device)
     nwork = lib.hdgnn_hunk_clusters_work(B, n)
@@ -547,3 +542,84 @@ def hunk_clusters(probs: torch.Tensor, nh: Optional[torch.Tensor] = None, thresh
     _launch("hunk_clusters", lib.hdgnn_hunk_clusters, B, n, (probs.contiguous(), F32), (None if nh is None else nh.contiguous(), I32),
             float(threshold), groups, ngroups, work)
     return groups, ngroups
+
+
+def _probs_shape(name: str, probs: torch.Tensor, nh: Optional[torch.Tensor]):
+    """(B, n) of relation-head probabilities (B, 2, n(n-1)) with nh (B,) or None; ValueError otherwise."""
+    _shape(name, "probs", probs, None, 2, None)
+    B, _, ncr = probs.shape
+    n = (1 + int(round((1 + 4 * ncr) ** 0.5))) // 2
+    if n < 2 or n * (n - 1) != ncr:
+        raise ValueError(f"{name} needs n(n-1) pairs per channel, got {ncr}")
+    _shape(name, "nh", nh, B)
+    return B, n
+
+
+def hunk_linkage(probs: torch.Tensor, nh: Optional[torch.Tensor] = None):
+    """The dendrogram of hunk_clusters (hdgnn_hunk_linkage): the same average-linkage merges on the same inputs, without a
+    threshold.  Returns (merges (B, n-1, 2) int32: row i = (a, c), a < c, cluster c joined cluster a; heights (B, n-1) float32:
+    the mean of w over the two clusters at that merge; nmerges (B,) int32: the rows recorded, m - 1 unless NaN means were left,
+    -1 for a commit with nh outside [0, n]).  Rows past nmerges hold (-1, -1) and NaN.  linkage_cut turns it into groups;
+    scipy_linkage into scipy's linkage matrix."""
+    B, n = _probs_shape("hunk_linkage", probs, nh)
+    merges = torch.empty(B, n - 1, 2, dtype=torch.int32, device=probs.device)
+    heights = torch.empty(B, n - 1, dtype=torch.float32, device=probs.device)
+    nmerges = torch.empty(B, dtype=torch.int32, device=probs.device)
+    nwork = lib.hdgnn_hunk_clusters_work(B, n)
+    work = torch.empty(nwork, dtype=torch.uint8, device=probs.device) if nwork else None
+    _launch("hunk_linkage", lib.hdgnn_hunk_linkage, B, n, (probs.contiguous(), F32), (None if nh is None else nh.contiguous(), I32),
+            merges, heights, nmerges, work)
+    return merges, heights, nmerges
+
+
+def linkage_cut(merges: torch.Tensor, heights: torch.Tensor, nmerges: torch.Tensor, nh: Optional[torch.Tensor] = None,
+                thresholds=None, target: Optional[torch.Tensor] = None):
+    """Hunk groups from hunk_linkage's record (hdgnn_linkage_cut), at each of `thresholds` (a sequence of 1 to 64 floats: the
+    longest prefix of merges whose heights are all > t, which is exactly hunk_clusters(probs, nh, t)) or at `target` ((B,) int32
+    CUDA tensor: the merges that leave max(target, 1) groups of the real hunks, or all of them); exactly one of the two.
+    Returns (groups (K, B, n) int32, ngroups (K, B) int32) in hunk_clusters' labelling (K = 1 with target); a commit whose
+    record is inconsistent gets -1 throughout."""
+    if (thresholds is None) == (target is None):
+        raise ValueError("linkage_cut needs exactly one of thresholds and target")
+    _shape("linkage_cut", "merges", merges, None, None, 2)
+    B, n = merges.shape[0], merges.shape[1] + 1
+    _shape("linkage_cut", "heights", heights, B, n - 1)
+    _shape("linkage_cut", "nmerges", nmerges, B)
+    _shape("linkage_cut", "nh", nh, B)
+    _shape("linkage_cut", "target", target, B)
+    host = None
+    if thresholds is not None:
+        thresholds = [float(t) for t in thresholds]
+        host = (C.c_float * max(len(thresholds), 1))(*thresholds)
+    K = 1 if thresholds is None else len(thresholds)
+    groups = torch.empty(K, B, n, dtype=torch.int32, device=merges.device)
+    ngroups = torch.empty(K, B, dtype=torch.int32, device=merges.device)
+    _launch("linkage_cut", lib.hdgnn_linkage_cut, B, n, (merges.contiguous(), I32), (heights.contiguous(), F32),
+            (nmerges.contiguous(), I32), (None if nh is None else nh.contiguous(), I32), K, host,
+            (None if target is None else target.contiguous(), I32), groups, ngroups)
+    return groups, ngroups
+
+
+def scipy_linkage(merges, heights, nmerges, nh=None) -> list:
+    """hunk_linkage's record (tensors or arrays) as scipy's linkage matrices, one per commit: Z (m-1, 4) float64, row i =
+    [id of a's cluster, id of c's cluster, 1 - height, size of the new cluster], where a singleton s has id s and the cluster
+    formed at row i has id m + i, as scipy.cluster.hierarchy.linkage numbers them; dendrogram and fcluster(Z, 1 - t,
+    "distance") then work on the device's result.  ValueError for a commit whose sequence did not join all m real hunks
+    (NaN means left over, or nmerges -1)."""
+    merges, heights, nmerges = (np.asarray(x.cpu() if torch.is_tensor(x) else x) for x in (merges, heights, nmerges))
+    n = merges.shape[1] + 1
+    out = []
+    for b in range(merges.shape[0]):
+        m = n if nh is None else int(np.asarray(nh.cpu() if torch.is_tensor(nh) else nh)[b])
+        if int(nmerges[b]) != max(m - 1, 0):
+            raise ValueError(f"commit {b}: {int(nmerges[b])} merges of {m} hunks do not form one tree")
+        ident = np.arange(max(m, 0))                         # scipy id of the cluster each representative stands for
+        size = np.ones(max(m, 0), np.int64)
+        Z = np.empty((max(m - 1, 0), 4), np.float64)
+        for i in range(max(m - 1, 0)):
+            a, c = int(merges[b, i, 0]), int(merges[b, i, 1])
+            size[a] += size[c]
+            Z[i] = (ident[a], ident[c], 1.0 - float(heights[b, i]), size[a])
+            ident[a] = m + i
+        out.append(Z)
+    return out

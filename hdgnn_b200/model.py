@@ -477,7 +477,8 @@ class graph2graph(object):
             log('test time:' + str(end_time - start_time))
         return out, C_edge_t1
 
-    def untangle(self, args=None, data=None, root=".", quirk_q2=True, log=print, grouping="components", threshold=0.5):
+    def untangle(self, args=None, data=None, root=".", quirk_q2=True, log=print, grouping="components", threshold=0.5,
+                 sweep=None):
         """The untangling answer over the test half, with the checkpoint, batches and entity->hunk maps of test(): the predicted
         relations of every commit as a label bitmap (hdgnn_set_predictions; by default no probabilities are written) and the
         hunk groups they give (hdgnn_hunk_groups), beside the groups of the labels.  Writes C_group_t{Ne}.npy (predicted groups) and
@@ -492,11 +493,21 @@ class graph2graph(object):
         of the relation probabilities (hdgnn_hunk_clusters) over the same real hunks: two groups merge only while the mean of
         max(p1(s,t), p1(t,s)) over their hunk pairs is > threshold, so one confident cross pair cannot join two groups and a few
         missing pairs cannot split one.  Each batch's probabilities go to a device buffer (never to the host); pred_bits keep
-        their meaning, and one log line names the grouping before the partition_* lines."""
+        their meaning, and one log line names the grouping before the partition_* lines.
+        sweep (grouping="average" only): a sequence of further thresholds to score.  Each batch then runs hunk_linkage once and
+        linkage_cut at [threshold, *sweep]; the groups at `threshold` are those of hunk_clusters, so everything above is
+        unchanged.  Every sweep threshold is scored like the groups (out["sweep"]: threshold -> partition metrics, in the order
+        given), and so is the cut at the labelled number of groups of each commit's real hunks (out["sweep_labelled_k"]: the
+        score with the number of concerns known).  out["linkage"] = (merges, heights, nmerges) of every commit, also written as
+        C_linkage{Ne}.npz; one log line per sweep threshold and one for the labelled-k cut come before the grouping line."""
         from .EvaluationFuncs import partition_metrics_from_counts
-        from .engine import bit_words, hunk_clusters, hunk_groups, partition_counts
+        from .engine import bit_words, hunk_clusters, hunk_groups, hunk_linkage, linkage_cut, partition_counts
         if grouping not in ("components", "average"):
             raise ValueError(f"grouping must be 'components' or 'average', got {grouping!r}")
+        if sweep is not None:
+            if grouping != "average":
+                raise ValueError("sweep needs grouping='average'")
+            sweep = [float(t) for t in sweep]
         repo = getattr(args, "Repo", self.Repo)
         train, test = data if data is not None else self._load(root)
         self.initialize()
@@ -517,6 +528,11 @@ class graph2graph(object):
         nh = None if test.nh is None or not nb else torch.as_tensor(np.ascontiguousarray(test.nh[:n], dtype=np.int32)).to(dev)
         average = grouping == "average"
         probs = torch.empty(mb, 2, self.Ncr, dtype=torch.float32, device=dev) if average and nb else None
+        if sweep is not None:
+            link = (torch.full((max(n, 1), self.Nc - 1, 2), -1, dtype=torch.int32, device=dev),
+                    torch.full((max(n, 1), self.Nc - 1), float("nan"), dtype=torch.float32, device=dev),
+                    torch.zeros(max(n, 1), dtype=torch.int32, device=dev))
+            scounts = torch.zeros(len(sweep) + 1, max(n, 1), 8, dtype=torch.int64, device=dev)   # the sweep, then labelled k
         start_time = time.time()
         alive = []       # the library DMAs from these pinned buffers asynchronously: keep them until the final synchronize
         try:
@@ -529,12 +545,25 @@ class graph2graph(object):
                 rows = slice(j * mb, (j + 1) * mb)
                 self.engine.set_predictions(pred[rows])
                 self.engine.infer_host(*hb.tensors(), self.params, probs, None)
-                if average:
-                    groups[rows] = hunk_clusters(probs, None if nh is None else nh[rows], threshold)[0]
+                nh_j = None if nh is None else nh[rows]
+                if sweep is not None:
+                    rec = hunk_linkage(probs, nh_j)
+                    for dst, src in zip(link, rec):
+                        dst[rows] = src
+                    cuts = linkage_cut(*rec, nh_j, thresholds=[threshold, *sweep])[0]
+                    groups[rows] = cuts[0]
+                elif average:
+                    groups[rows] = hunk_clusters(probs, nh_j, threshold)[0]
                 else:
                     groups[rows] = hunk_groups(pred[rows])[0]
                 label_groups[rows] = hunk_groups(hb.Yw.to(dev, non_blocking=True))[0]
-                pcounts[rows] = partition_counts(groups[rows], label_groups[rows], None if nh is None else nh[rows])
+                pcounts[rows] = partition_counts(groups[rows], label_groups[rows], nh_j)
+                if sweep is not None:
+                    for k in range(len(sweep)):
+                        scounts[k, rows] = partition_counts(cuts[k + 1], label_groups[rows], nh_j)
+                    # the labelled groups of the real hunks: column 5 of the counts just computed
+                    at_k = linkage_cut(*rec, nh_j, target=pcounts[rows, 5].to(torch.int32))[0][0]
+                    scounts[-1, rows] = partition_counts(at_k, label_groups[rows], nh_j)
         finally:
             self.engine.set_predictions(None)
         exact = int((groups[:n] == label_groups[:n]).all(1).sum()) if nb else 0      # synchronises
@@ -544,11 +573,21 @@ class graph2graph(object):
                    label_groups=label_groups[:n].cpu().numpy(), exact_partitions=exact,
                    partition_counts=pcounts[:n].cpu().numpy())
         out["partition"] = partition_metrics_from_counts(out["partition_counts"])
+        if sweep is not None:
+            sc = scounts[:, :n].cpu().numpy()
+            out["sweep"] = {t: partition_metrics_from_counts(sc[k]) for k, t in enumerate(sweep)}
+            out["sweep_labelled_k"] = partition_metrics_from_counts(sc[-1])
+            out["linkage"] = tuple(x[:n].cpu().numpy() for x in link)
         if self.rank == 0:
             step_dir = os.path.join(root, 'outputSelf/' + repo + '/model_%d/' % self.variant + str(self.Step) + '/')
             os.makedirs(step_dir, exist_ok=True)
             np.save(step_dir + 'C_group_t' + str(self.Ne) + '.npy', out["groups"])
             np.save(step_dir + 'C_group_y' + str(self.Ne) + '.npy', out["label_groups"])
+            if sweep is not None:
+                np.savez(step_dir + 'C_linkage' + str(self.Ne) + '.npz', **dict(zip(("merges", "heights", "nmerges"), out["linkage"])))
+                for t, v in out["sweep"].items():
+                    log('sweep threshold ' + str(t) + ': ' + str(v))
+                log('sweep labelled groups: ' + str(out["sweep_labelled_k"]))
             if average:
                 log('grouping: average linkage, threshold ' + str(threshold))
             for k, v in out["partition"].items():

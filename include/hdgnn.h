@@ -308,6 +308,35 @@ size_t hdgnn_hunk_clusters_work(int B, int n);
 int hdgnn_hunk_clusters(int B, int n, const float* probs, const int32_t* nh, float threshold,
                         int32_t* groups, int32_t* ngroups, void* work, void* stream);
 
+/* The dendrogram of hdgnn_hunk_clusters: the same clustering (inputs, w, fp32 sums, tie rule, `work` of
+ * hdgnn_hunk_clusters_work) without a threshold, recording every merge.  It stops only when no pair with a non-NaN mean is
+ * left; a mean of +-inf merges like any other.  merges (B, n-1, 2) int32: row i = (a, c), a < c, cluster c joined cluster a,
+ * which stays the representative; heights (B, n-1) f32: that pair's mean (-0 stored as +0); nmerges (B) int32: the rows
+ * recorded, m - 1 unless NaN means were left over.  Rows from nmerges on hold (-1, -1) and NaN.  A commit with nh[b] outside
+ * [0, n] gets nmerges -1 and every row -1 / NaN.  2 <= n <= HDGNN_MAX_N.  Deterministic, stateless, asynchronous on `stream`.
+ *
+ * Merge heights need not be monotone: UPGMA is in exact arithmetic, but the fp32 sums and the division can put a later height
+ * one ulp above an earlier one.  So a threshold cut is defined as a PREFIX: hdgnn_hunk_clusters(t) performs the same merges
+ * and stops at the first whose mean is not > t, hence hdgnn_linkage_cut(hdgnn_hunk_linkage(p), t) equals
+ * hdgnn_hunk_clusters(p, t) bit for bit, groups and ngroups, for every non-NaN t. */
+int hdgnn_hunk_linkage(int B, int n, const float* probs, const int32_t* nh, int32_t* merges, float* heights, int32_t* nmerges,
+                       void* work, void* stream);
+
+/* Hunk groups at K cuts of recorded merge sequences (the outputs of hdgnn_hunk_linkage, or the same arrays read back from a
+ * file).  Cut k of commit b applies the commit's first c merges, m = nh[b] (nh NULL: m = n):
+ *   threshold mode (thresholds_host: K host floats, 1 <= K <= 64, none NaN, taken by value; target NULL): c = the length of
+ *     the longest prefix of the commit's merges whose heights are all > thresholds_host[k];
+ *   group-count mode (target: device (B) int32; K = 1; thresholds_host NULL): c = min(nmerges[b], max(0, m - max(target[b], 1))),
+ *     scipy's maxclust, except that a sequence stopped early by NaN means leaves more groups than asked for.
+ * groups (K, B, n) int32: the representative (smallest hunk) of s's cluster after those merges for s < m, s for s >= m;
+ * ngroups (K, B) int32 or NULL: n - c.  This is the labelling of hdgnn_hunk_clusters, which hdgnn_partition_counts takes.
+ * A commit whose record is inconsistent -- nh[b] outside [0, n], nmerges[b] outside [0, max(m - 1, 0)], a row without
+ * 0 <= a < c < m, a c that appears twice, or an a absorbed at an earlier row -- gets groups and ngroups -1 for every cut; no
+ * row past nmerges[b] is read.  2 <= n <= HDGNN_MAX_N.  Integer-exact, deterministic, stateless, asynchronous on `stream`. */
+int hdgnn_linkage_cut(int B, int n, const int32_t* merges, const float* heights, const int32_t* nmerges, const int32_t* nh,
+                      int K, const float* thresholds_host, const int32_t* target, int32_t* groups, int32_t* ngroups,
+                      void* stream);
+
 /* Evaluation counters on the device, replaces the loops of EvaluationFuncs.py:27-37 (top_ACC), :92-117 (prec / recall /
  * f1) and :119-153 (AUC) over the probs the relation head wrote.  probs (B,2,Ncr) f32, Y (B,Nc,y_pitch) u8.
  * counts (B,8) int64: {arg-max hits, quirk tp, fp, fn (ceil of channel 0, as the reference scores), conventional tp, fp,

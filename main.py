@@ -9,13 +9,26 @@ reference's first-Mini_batch slice, model_2.py:376-381).  Extra value --Type unt
 predicts for every test commit (graph2graph.untangle), scored against the labelled groups over each commit's real hunks
 (pair precision / recall / F1, Rand and adjusted Rand index, purity).  With --Type untangle, --grouping average forms the
 groups by average-linkage clustering of the relation probabilities instead of connected components of the arg-max relations:
-two groups merge only while their mean relation probability is > --threshold (default 0.5).
+two groups merge only while their mean relation probability is > --threshold (default 0.5).  --sweep 0.3,0.4,... (with
+--grouping average only) scores those thresholds as well, and the cut at each commit's labelled number of groups, from one
+dendrogram per batch, so a threshold can be chosen from the scores; the groups written stay those at --threshold.
 Multi-GPU: launch with `python -m torch.distributed.run --nproc-per-node N main.py ...`.
 """
 import argparse
 import os
 
 import torch
+
+
+def _thresholds(text):
+    """'0.3,0.4' -> [0.3, 0.4]: 1 to 63 thresholds, none NaN (one hdgnn_linkage_cut call takes --threshold and 63 more)."""
+    try:
+        ts = [float(t) for t in text.split(',')]
+    except ValueError:
+        raise argparse.ArgumentTypeError(f'not a comma-separated list of numbers: {text!r}')
+    if not 1 <= len(ts) <= 63 or any(t != t for t in ts):
+        raise argparse.ArgumentTypeError(f'1 to 63 thresholds, none NaN: {text!r}')
+    return ts
 
 
 def main(argv=None):
@@ -59,7 +72,11 @@ def main(argv=None):
                                  'linkage of the relation probabilities')
         parser.add_argument('--threshold', type=float, default=0.5,
                             help='untangle --grouping average: merge two groups while their mean relation probability is above it')
+        parser.add_argument('--sweep', type=_thresholds, default=None,
+                            help='untangle --grouping average: comma-separated thresholds to score beside --threshold')
         args = parser.parse_args(argv)
+        if args.sweep is not None and (args.Type != 'untangle' or args.grouping != 'average'):
+            parser.error('--sweep needs --Type untangle --grouping average')
 
         ck = args.checkpoint_dir if os.path.isabs(args.checkpoint_dir) else os.path.join(args.root, args.checkpoint_dir)
         if not os.path.exists(ck):
@@ -83,7 +100,7 @@ def main(argv=None):
             results.append(model.test(args, root=args.root, quirk_q2=not args.no_q2))
         if args.Type == 'untangle':
             results.append(model.untangle(args, root=args.root, quirk_q2=not args.no_q2, grouping=args.grouping,
-                                          threshold=args.threshold))
+                                          threshold=args.threshold, sweep=args.sweep))
         model.engine.close()
     return results
 

@@ -14,17 +14,23 @@
       a pass of their own; host-fed inference end to end as graph2graph.untangle runs it (Ne = 200, B = 100, random weights),
       grouping "average" (probabilities written to a device buffer, then hunk_clusters) against "components" (hunk_groups of
       the predicted relations); and the partition scores of both groupings against the planted groups when a few confident
-      cross-group false positives are added.
+      cross-group false positives are added;
+  (f) the dendrogram: hunk_linkage (the whole merge sequence) against hunk_clusters at 0.5 on the same commits, at B = 100 and
+      Nc in {74, 256, 512} and at B = 4096, Nc = 74, every hunk real, on planted groups of 8 and on random-weight
+      probabilities (p1 ~ U(0, 1): the merges a threshold of 0.5 skips are many), and linkage_cut of the record at K = 1, 16
+      and 64 thresholds, kernel times from torch.profiler in a pass per arm; and a sweep of 9 thresholds as
+      graph2graph.untangle(sweep=...) runs it (one hunk_linkage, one linkage_cut, 9 partition_counts) against 9 hunk_clusters
+      calls each followed by partition_counts, with the two arms' counters compared.
 Device inputs rotate through copies that together exceed the 126 MB L2; every arm is timed in blocks that alternate with the
 other arm's, and the median block is reported.  The card's name and power limit are read in the same run.
-Usage: python tools/bench_untangle.py [--sections abcde] [--out result.json]"""
+Usage: python tools/bench_untangle.py [--sections abcdef] [--out result.json]"""
 import argparse, json, os, statistics, subprocess, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from hdgnn_b200.EvaluationFuncs import partition_metrics_from_counts
 from hdgnn_b200._lib import lib
-from hdgnn_b200.engine import (Engine, DeviceBatch, F_LABEL_BITS, bit_words, hunk_clusters, hunk_groups, pack_label_bits,
-                               partition_counts)
+from hdgnn_b200.engine import (Engine, DeviceBatch, F_LABEL_BITS, bit_words, hunk_clusters, hunk_groups, hunk_linkage,
+                               linkage_cut, pack_label_bits, partition_counts)
 from hdgnn_b200.model import HostBatch
 from hdgnn_b200.synthetic import make_commits
 
@@ -68,7 +74,7 @@ def timed(arms, calls):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=None)
-    ap.add_argument("--sections", default="abcde", help="which of the sections (a)-(e) to run")
+    ap.add_argument("--sections", default="abcdef", help="which of the sections (a)-(f) to run")
     args = ap.parse_args()
     out = {"card": card(), "B": B, "Ne": Ne, "variant": 2, "reps": REPS, "what": __doc__.split("Usage")[0].strip(), "rows": []}
     for Nc in ((74, 256, 512) if set("abc") & set(args.sections) else ()):
@@ -161,6 +167,10 @@ def main():
         out["e_hunk_clusters"] = [clusters(Bd, Nc) for Bd, Nc in ((B, 74), (B, 256), (B, 512), (4096, 74))]
         out["e_untangle_end_to_end"] = [untangle_e2e(Nc) for Nc in (74, 256, 512)]
         out["e_quality"] = [quality(Nc) for Nc in (74, 256)]
+    if "f" in args.sections:
+        out["f_linkage"] = [linkage_row(Bd, Nc, kind) for Bd, Nc in ((B, 74), (B, 256), (B, 512), (4096, 74))
+                            for kind in ("planted", "random")]
+        out["f_sweep"] = [sweep_row(Nc) for Nc in (74, 256, 512)]
     out["card_after"] = card()
     if args.out:
         os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
@@ -284,6 +294,95 @@ def quality(Nc, Bq=200):
            "average": partition_metrics_from_counts(partition_counts(avg, truth, nh).cpu().numpy()),
            "components": partition_metrics_from_counts(partition_counts(cc, truth, nh).cpu().numpy())}
     print(json.dumps(row, default=str))
+    return row
+
+
+def random_probs(Bd, Nc, seed):
+    """(Bd, 2, Nc(Nc-1)) f32 on the device: p1 ~ U(0, 1) for every pair, p0 = 1 - p1 (a forward with random weights is
+    about as unstructured)."""
+    p1 = torch.rand(Bd, Nc * (Nc - 1), generator=torch.Generator(device="cuda").manual_seed(seed), device="cuda")
+    return torch.stack([1 - p1, p1], dim=1).contiguous()
+
+
+# kernel of each arm of section (f): the threshold and the recording instantiation of hunk_clusters_kernel share a name
+F_KERNELS = {"hunk_clusters": ("hunk_clusters_kernel", ("<false>", "ILb0E")), "hunk_linkage": ("hunk_clusters_kernel", ("<true>", "ILb1E")),
+             "cut_K1": ("linkage_cut_kernel", ("",)), "cut_K16": ("linkage_cut_kernel", ("",)), "cut_K64": ("linkage_cut_kernel", ("",))}
+
+
+def kernel_us_each(arms, calls):
+    """{arm: mean device time in µs of its kernel (F_KERNELS)}, one torch.profiler pass per arm."""
+    from torch.profiler import profile, ProfilerActivity
+    got = {}
+    for name, fn in arms.items():
+        kern, tags = F_KERNELS[name]
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            for k in range(calls):
+                fn(k)
+            torch.cuda.synchronize()
+        for e in prof.key_averages():
+            if kern in e.key and any(t in e.key for t in tags) and e.count:
+                got[name] = e.device_time_total / e.count
+    return got
+
+
+def linkage_row(Bd, Nc, kind):
+    """(f): hunk_linkage against hunk_clusters(0.5), and linkage_cut at K = 1, 16, 64, on the same Bd commits."""
+    probs = planted(Bd, Nc, 6161)[0] if kind == "planted" else random_probs(Bd, Nc, 6161)
+    nh = torch.full((Bd,), Nc, dtype=torch.int32, device="cuda")
+    rec = hunk_linkage(probs, nh)
+    ppool = rotate([probs], probs.numel() * 4)
+    rbytes = sum(x.numel() * 4 for x in rec)
+    rpool = [tuple(x.clone() for x in rec) for _ in range(max(1, -(-2 * L2_BYTES // rbytes)))]
+    ts = [float(t) for t in np.linspace(0.05, 0.95, 64)]
+    arms = {"hunk_clusters": lambda k: hunk_clusters(ppool[k % len(ppool)], nh, 0.5),
+            "hunk_linkage": lambda k: hunk_linkage(ppool[k % len(ppool)], nh)}
+    for K in (1, 16, 64):
+        arms[f"cut_K{K}"] = (lambda K: lambda k: linkage_cut(*rpool[k % len(rpool)], nh, thresholds=ts[:K]))(K)
+    calls = 5 if Nc >= 256 else 20
+    ms, blocks = timed(arms, calls)
+    kern = kernel_us_each(arms, 4 * calls)
+    g, ng = linkage_cut(*rec, nh, thresholds=[0.5])
+    gc, ngc = hunk_clusters(probs, nh, 0.5)
+    row = {"B": Bd, "Nc": Nc, "probs": kind, **{f"us_per_call_{k}": v * 1e3 for k, v in ms.items()},
+           **{f"kernel_us_{k}": kern.get(k) for k in arms},
+           "merges_per_commit_linkage": float(rec[2].float().mean()), "merges_per_commit_clusters_0.5": Nc - float(ngc.float().mean()),
+           "cut_0.5_equals_hunk_clusters": bool(torch.equal(g[0], gc) and torch.equal(ng[0], ngc)),
+           "pool_batches": len(ppool), "record_pool_batches": len(rpool), "blocks_ms": blocks}
+    print(json.dumps(row, default=str))
+    del ppool, rpool
+    torch.cuda.empty_cache()
+    return row
+
+
+def sweep_row(Nc, Bd=B):
+    """(f): 9 thresholds scored as graph2graph.untangle(sweep=...) does it, against 9 hunk_clusters + partition_counts."""
+    probs, truth = planted(Bd, Nc, 6262, p_false=0.01)
+    nh = torch.full((Bd,), Nc, dtype=torch.int32, device="cuda")
+    ppool = rotate([probs], probs.numel() * 4)
+    ts = [0.1, 0.2, 0.3, 0.4, 0.5, 0.6, 0.7, 0.8, 0.9]
+    counts = torch.empty(2, len(ts), Bd, 8, dtype=torch.int64, device="cuda")
+
+    def linkage_sweep(k):
+        p = ppool[k % len(ppool)]
+        g = linkage_cut(*hunk_linkage(p, nh), nh, thresholds=ts)[0]
+        for i in range(len(ts)):
+            counts[0, i] = partition_counts(g[i], truth, nh)
+
+    def clusters_x9(k):
+        p = ppool[k % len(ppool)]
+        for i, t in enumerate(ts):
+            counts[1, i] = partition_counts(hunk_clusters(p, nh, t)[0], truth, nh)
+    ms, blocks = timed({"linkage_sweep": linkage_sweep, "clusters_x9": clusters_x9}, 2 if Nc >= 256 else 5)
+    linkage_sweep(0)
+    clusters_x9(0)
+    row = {"B": Bd, "Nc": Nc, "thresholds": ts, "ms_per_batch_linkage_sweep": ms["linkage_sweep"],
+           "ms_per_batch_9_hunk_clusters": ms["clusters_x9"], "counts_equal": bool(torch.equal(counts[0], counts[1])),
+           "pair_f1": [partition_metrics_from_counts(counts[0, i].cpu().numpy())["pair_f1"] for i in range(len(ts))],
+           "ari": [partition_metrics_from_counts(counts[0, i].cpu().numpy())["ari"] for i in range(len(ts))],
+           "pool_batches": len(ppool), "blocks_ms": blocks}
+    print(json.dumps(row, default=str))
+    del ppool
+    torch.cuda.empty_cache()
     return row
 
 
